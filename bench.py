@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ray segments/s and ms/frame of the render hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Workload (config.workload): the cornell_box mesh at 3840x2160, fov 1.5, camera origin, depth cap 3
 -- the configuration BASELINE.json's metric and north_star target are quoted on (configs[2]; the
@@ -326,7 +326,8 @@ def verify_frames(tr, backend, cameras, world, rank, dev):
 
 def timed_frames(tr, flush, steps, warmup, world, dev):
     """`warmup` untimed frames, then `steps` frames each bracketed by CUDA events on the launching stream, the L2 flushed
-    before each (outside its events), barrier + synchronize on both sides; returns ms per step, max over ranks."""
+    before each (outside its events), barrier + synchronize on both sides; returns (ms per step, max over ranks; the RGB8
+    frame of the last step on rank 0, None elsewhere -- valid until the next frame is issued)."""
     import torch
     import torch.distributed as dist
 
@@ -340,10 +341,11 @@ def timed_frames(tr, flush, steps, warmup, world, dev):
     barrier()
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
     barrier()
+    frame = None
     for a, b in ev:
         flush.fill_(0)
         a.record()
-        tr.render()
+        frame = tr.render()
         b.record()
     barrier()
     if tr.peer is not None:
@@ -351,7 +353,28 @@ def timed_frames(tr, flush, steps, warmup, world, dev):
     total = torch.tensor([sum(a.elapsed_time(b) for a, b in ev)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(total, op=dist.ReduceOp.MAX)
-    return float(total[0]) / steps
+    return float(total[0]) / steps, frame
+
+
+DUMP_PIXELS = 1 << 20        # pixels kept of a larger frame: 3 x 12 MB of float32 + 8 MB of float64 indices
+
+
+def dump_outputs(out_dir, tr, frame8):
+    """Writes what the last timed step computed, so that two builds can be compared output for output: the RGB8 frame a
+    caller receives (frame_rgb8), the float frame it was quantised from (frame_rgb) and the frame's maximum (frame_max).
+    A frame of more than DUMP_PIXELS pixels is cut to a fixed sample of pixels drawn with a fixed seed; sample_pixel_index
+    holds their flat indices (row * width + column).  Rank 0's buffers only."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    n = tr.height * tr.width
+    idx = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    sel = torch.from_numpy(idx).to(tr.rgb.device)
+    arrays = {"frame_rgb8": frame8.reshape(n, 3)[sel].float(), "frame_rgb": tr.rgb.reshape(n, 3)[sel], "frame_max": tr.dmax}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "sample_pixel_index.npy"), idx.astype(np.float64))
 
 
 def heavy_leg(name, world, rank, dev, flush, steps=3, warmup=3):
@@ -371,7 +394,7 @@ def heavy_leg(name, world, rank, dev, flush, steps=3, warmup=3):
     tr = tiled.TiledRenderer(backend, w, h, dev)
     try:
         L = backend.L
-        ms = timed_frames(tr, flush, steps, warmup, world, dev)
+        ms = timed_frames(tr, flush, steps, warmup, world, dev)[0]
         ok, sha, detail = verify_frames(tr, backend, VERIFY_CAMERAS["stress"][:2], world, rank, dev)
         segs = None
         if rank == 0:                                       # segments of the frame: pixels + the queries the kernel counted behind them
@@ -511,7 +534,9 @@ def run_ours(args):
     # ---- the timed region: K frames, each bracketed by CUDA events on the launching stream (a frame is the K0 -> K1 pair and
     # nothing else), L2 flushed before each, barrier + synchronize on both sides, max over ranks
     graphs_before = int(L.rm_graph_launch_count())
-    ms_per_step = timed_frames(tr, flush, args.steps, max(args.warmup, 3), world, dev)
+    ms_per_step, last_frame = timed_frames(tr, flush, args.steps, max(args.warmup, 3), world, dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr, last_frame)
     value = segs / (ms_per_step * 1e-3)
     graphs_headline = int(L.rm_graph_launch_count()) - graphs_before      # frames (warm-up included) issued as one graph launch
 
@@ -519,7 +544,7 @@ def run_ours(args):
     # the split of a frame between the kernels.  Not the headline pass: the extra event records between the two launches
     # cost ~5 us per frame (0.0697 against 0.0645 ms on the 4K cornell frame, profiles/r5l_*).
     _abi.check(L.rm_set_profiling(1))
-    profiled_ms_per_step = timed_frames(tr, flush, args.steps, 3, world, dev)
+    profiled_ms_per_step = timed_frames(tr, flush, args.steps, 3, world, dev)[0]
     k0_ms, k1_ms, k4_ms = [], [], []
     if tr.exchange == "peer":
         t0, t1, t4 = C.c_double(0), C.c_double(0), C.c_double(0)
@@ -552,7 +577,7 @@ def run_ours(args):
         for _block in range(3):
             for arm in ("1", "0"):
                 os.environ["RM_B200_GRAPH"] = arm
-                arms[arm].append(timed_frames(tr, flush, n_g, 3, world, dev))
+                arms[arm].append(timed_frames(tr, flush, n_g, 3, world, dev)[0])
         del os.environ["RM_B200_GRAPH"]
         graph_ab = {"one_graph_launch_ms_per_frame": sum(arms["1"]) / 3, "two_launches_ms_per_frame": sum(arms["0"]) / 3,
                     "blocks": {"graph": arms["1"], "two_launches": arms["0"]}, "frames_per_block": n_g,
@@ -819,7 +844,11 @@ def main():
     ap.add_argument("--no-cull", action="store_true", help="trace every primitive like the reference's brute force")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--heavy", default="stress_8k_bvh", help="second, short leg on a workload that can scale ('' = none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float arrays; a seeded pixel sample of a large frame)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

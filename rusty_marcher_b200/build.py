@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "librm_b200.so")
 SOURCES = ["rm_api.cu", "rm_kernels.cu", "rm_scene.cpp", "rm_bvh.cpp", "rm_host.cpp"]
-HEADERS = ["rm_math.cuh", "rm_trace.cuh", "rm_fast.cuh", "rm_bvh.cuh", "rm_scene.h", "rm_kernels.h",
+HEADERS = ["rm_math.cuh", "rm_trace.cuh", "rm_fast.cuh", "rm_bvh.cuh", "rm_scene.h", "rm_kernels.h", "rm_pool.h",
            os.path.join("..", "..", "include", "rm_b200.h"), os.path.join("..", "..", "include", "rm_b200_host.h")]
 
 NVCC_FLAGS = [

@@ -7,7 +7,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE = "/root/reference"
+# a checkout of the original Rust project (rusty-marcher), for the tests that need its sources; they skip without one
+REFERENCE = os.environ.get("RM_REFERENCE_DIR", "")
 
 
 def pytest_configure(config):
@@ -36,7 +37,7 @@ def has_gpu():
 @pytest.fixture(scope="session")
 def reference_dir():
     if not os.path.isdir(REFERENCE):
-        pytest.skip("reference tree not present (GPU box)")
+        pytest.skip("RM_REFERENCE_DIR does not name a checkout of the original rusty-marcher project")
     return REFERENCE
 
 

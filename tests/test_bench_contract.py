@@ -44,6 +44,32 @@ def test_gpu_arm_refuses_to_run_without_a_device():
     assert not [l for l in r.stdout.splitlines() if l.startswith("{")]
 
 
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_frame_as_float_arrays(tmp_path):
+    """--dump-outputs DIR: the RGB8 frame of the last timed step, its float frame and maximum, as a seeded pixel sample
+    of a frame larger than bench.DUMP_PIXELS, float32 / float64 only, 64 MB at most."""
+    import numpy as np
+    r = run("--workload", "cornell_1080p", "--steps", "2", "--warmup", "0", "--heavy", "", "--no-cpu-baseline",
+            "--dump-outputs", str(tmp_path))
+    assert r.returncode == 0, r.stderr
+    names = sorted(os.listdir(tmp_path))
+    assert names == ["frame_max.npy", "frame_rgb.npy", "frame_rgb8.npy", "sample_pixel_index.npy"]
+    assert sum(os.path.getsize(tmp_path / n) for n in names) <= 64 << 20
+    a = {n[:-4]: np.load(tmp_path / n) for n in names}
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    idx = a["sample_pixel_index"]
+    assert idx.shape == (1 << 20,) and np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < 1920 * 1080
+    rgb8 = a["frame_rgb8"]
+    assert rgb8.shape == a["frame_rgb"].shape == (1 << 20, 3)
+    assert np.array_equal(rgb8, np.round(rgb8)) and rgb8.min() >= 0 and 0 < rgb8.max() <= 255
+    assert a["frame_max"].shape == (1,) and a["frame_max"][0] > 0
+
+
+def test_dump_outputs_is_refused_by_the_reference_arm():
+    r = run("--impl", "reference", "--dump-outputs", "unused")
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+
+
 def test_workload_table_holds_the_baseline_configurations():
     sys.path.insert(0, ROOT)
     import bench

@@ -11,6 +11,8 @@ import rusty_marcher_b200 as rm
 from oracle import oracle as O
 from rusty_marcher_b200 import _abi, obj, workloads
 
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")     # stored geometry of test_data/*.obj
+
 
 def flat_of_builder(b):
     return _abi.load().rm_builder_flatten(b).contents
@@ -141,8 +143,8 @@ def test_obj_load_missing_file_returns_none():
     assert obj.load("/nonexistent/thing.obj") is None          # obj.rs:53-56
 
 
-def test_cornell_box_from_reference_file(reference_dir):
-    models = obj.load(os.path.join(reference_dir, "test_data", "cornell_box.obj"))
+def test_cornell_box_from_reference_file():
+    models = obj.load(os.path.join(GOLDEN, "cornell_box.obj"))
     assert [(m.name, m.triangles.shape[0]) for m in models] == [
         ("floor", 6), ("light", 2), ("ceiling", 2), ("back_wall", 2), ("green_wall", 2), ("red_wall", 2),
         ("short_block", 10), ("tall_block", 10)]
@@ -151,8 +153,8 @@ def test_cornell_box_from_reference_file(reference_dir):
         assert m.name == name and np.array_equal(m.triangles[:, 0:9].reshape(-1, 3, 3), v)
 
 
-def test_scene_from_obj_equals_workload_scene(reference_dir):
-    a = rm.Scene.from_obj(os.path.join(reference_dir, "test_data", "dodecahedron.obj")).flatten()
+def test_scene_from_obj_equals_workload_scene():
+    a = rm.Scene.from_obj(os.path.join(GOLDEN, "dodecahedron.obj")).flatten()
     b = workloads.scene("dodecahedron").flatten()
     assert a.c.n_triangles == b.c.n_triangles == 36
     assert np.array_equal(a._tris, b._tris) and np.array_equal(a._refl, b._refl)

@@ -1,5 +1,6 @@
 """Pins the oracle: golden image of the reference (engine/out.ppm), the reference's own unit tests
 restated (SURVEY.md 4), and the independently derived known answers of SURVEY.md 8c."""
+import gzip
 import hashlib
 import json
 import os
@@ -35,8 +36,11 @@ def test_demo_matches_reference_golden_ppm(demo_800):
     assert hashlib.sha256(ppm).hexdigest() == OUT_PPM_SHA
 
 
-def test_demo_matches_reference_file_if_present(demo_800, reference_dir):
-    ref = open(os.path.join(reference_dir, "engine", "out.ppm"), "rb").read()
+def test_demo_matches_reference_file_if_present(demo_800):
+    """Byte-for-byte against a stored copy of the reference's engine/out.ppm (make_reference_inputs.py)."""
+    with gzip.open(os.path.join(GOLDEN, "out.ppm.gz"), "rb") as f:
+        ref = f.read()
+    assert hashlib.sha256(ref).hexdigest() == OUT_PPM_SHA
     assert demo_ppm(demo_800) == ref
 
 
@@ -160,10 +164,10 @@ def test_triangle_intersect_cyclic_orders():
 
 # ---- OBJ ingest (tobj restatement; parity unpinned, see oracle/rm_oracle.h) ---------------------
 
-def test_cornell_box_loads_like_the_reference_expects(reference_dir):
-    """obj.rs:229-233 (is_some) + SURVEY.md 8c known answers."""
+def test_cornell_box_loads_like_the_reference_expects():
+    """obj.rs:229-233 (is_some) + SURVEY.md 8c known answers, on the stored geometry of test_data/cornell_box.obj."""
     s = O.Scene()
-    assert s.add_obj_file(os.path.join(reference_dir, "test_data", "cornell_box.obj")) == 8
+    assert s.add_obj_file(os.path.join(GOLDEN, "cornell_box.obj")) == 8
     assert [s.obj_triangles(i).shape[0] for i in range(8)] == [6, 2, 2, 2, 2, 2, 10, 10]
     s.add_default_lights()
     r = O.render(s, 320, 256)
@@ -174,9 +178,9 @@ def test_cornell_box_loads_like_the_reference_expects(reference_dir):
     assert r["degenerate_hits"] == 0
 
 
-def test_dodecahedron_known_answers(reference_dir):
+def test_dodecahedron_known_answers():
     s = O.Scene()
-    assert s.add_obj_file(os.path.join(reference_dir, "test_data", "dodecahedron.obj")) == 1
+    assert s.add_obj_file(os.path.join(GOLDEN, "dodecahedron.obj")) == 1
     tris = s.obj_triangles(0)
     assert tris.shape[0] == 36
     s.add_default_lights()
@@ -185,12 +189,12 @@ def test_dodecahedron_known_answers(reference_dir):
     assert r["rgb"].max() == 1.2948687004360002
 
 
-def test_fixture_meshes_equal_the_reference_files(reference_dir):
-    """The committed scenes/*.npz are exactly what the OBJ reader produces from the reference files."""
+def test_fixture_meshes_equal_the_reference_files():
+    """The committed scenes/*.npz are exactly what the OBJ reader produces from the stored geometry of the reference files."""
     from rusty_marcher_b200 import workloads
     for name in ("cornell_box", "dodecahedron"):
         s = O.Scene()
-        s.add_obj_file(os.path.join(reference_dir, "test_data", name + ".obj"), offset=(0., 0., 0.))
+        s.add_obj_file(os.path.join(GOLDEN, name + ".obj"), offset=(0., 0., 0.))
         models = workloads.load_models(name)
         assert s.num_shapes == len(models)
         for i, (_n, v) in enumerate(models):
