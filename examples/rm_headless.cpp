@@ -7,6 +7,8 @@
 //   render           main.rs:329-351  Renderer::render + the status label   (every run; --frames N re-renders N times,
 //                                      the scene resident, like the re-render loop)
 //   "Save to file"   main.rs:353-362  FrameBuffer::normalize + write_ppm("out.ppm")   --out FILE
+//                                      --samples S (2..8): the saved frame anti-aliased, S x S primary rays per pixel
+//                                      (rm_render_supersampled; an extension, the reference has no such mode)
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -25,7 +27,7 @@ static void die(const char* what, int rc) {
 }
 
 int main(int argc, char** argv) {
-    int width = 1600, height = 1280, depth = 3, frames = 1, accel = 0;     // main.rs:240: the frame buffer is 1600 x 1280
+    int width = 1600, height = 1280, depth = 3, frames = 1, accel = 0, samples = 1;     // main.rs:240: the frame buffer is 1600 x 1280
     bool f64 = false, rows64 = false;
     const char* obj = nullptr;
     const char* out = "out.ppm";
@@ -43,7 +45,12 @@ int main(int argc, char** argv) {
         else if (a == "--f64") f64 = true;              // the validation kernels: the reference's own f64 arithmetic
         else if (a == "--rows-f64") rows64 = true;      // FP32 kernels into the reference's frame type (one allocation per row, f64)
         else if (a == "--accel") accel = 1;
+        else if (a == "--samples") { need(1); samples = std::atoi(argv[++i]); }
         else { std::fprintf(stderr, "rm_headless: unknown option %s\n", a.c_str()); return 2; }
+    }
+    if (samples < 1 || samples > 8 || (samples > 1 && f64)) {
+        std::fprintf(stderr, "rm_headless: --samples takes 1 to 8, with the FP32 kernels\n");
+        return 2;
     }
     int rc = rm_init(0);
     if (rc != RM_OK) die("rm_init", rc);
@@ -97,7 +104,10 @@ int main(int argc, char** argv) {
         std::printf("Scene rendered in %lld ms (%u fps, %.2f MP/s)\n", ms, ms > 0 ? (unsigned)fps : 4294967295u, fps * (double)n_px / 1e6);
     }
     // "Save to file": normalize + to_vec on the device (framebuffer.rs:40-82), then the P6 stream (framebuffer.rs:26-38)
-    if (!f64) {
+    if (samples > 1) {
+        std::memset(&st, 0, sizeof st);
+        if ((rc = rm_render_supersampled(scene, &p, samples, nullptr, rgb8.data(), &st)) != RM_OK) die("render (supersampled 8-bit frame)", rc);
+    } else if (!f64) {
         std::memset(&st, 0, sizeof st);
         if ((rc = rm_render(scene, &p, nullptr, nullptr, rgb8.data(), &st)) != RM_OK) die("render (8-bit frame)", rc);
     }

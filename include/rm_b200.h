@@ -229,6 +229,31 @@ int rm_render_rows_f32(RmScene scene, const RmParams* params, float* const* rows
 int rm_render_dispersive(const RmScene scenes[3], const RmParams* params, float* out_rgb, int32_t* out_prim_id,
                          RmStats* stats);
 
+/* ---- extension mode: supersampled anti-aliasing, s x s samples per pixel -------------------------------------------------- *
+ * The reference traces one primary ray per pixel (renderer.rs:63-89); there is no reference behaviour for anti-aliasing.
+ * Defined here -- and identically in the tests' f64 restatement over the oracle -- in terms of the FP32 production render:
+ * for samples = s in [1, 8], pixel (x, y) of the frame is the mean of the FP32 render of the same scene and camera at width
+ * s*W and height s*H over the s x s block of sub-pixels (s*x + j, s*y + i), i, j in [0, s).  backproject (renderer.rs:128-135)
+ * divides by the width, so the sub-pixel rays are the reference's rays at x + j/s; the aspect ratio (s*W)/(s*H) rounds to the
+ * same double as W/H.  The mean is FP32 in this order (normative; no fused multiply-add):
+ *     acc = 0.f;  for i in [0, s): for j in [0, s): acc += v[i][j];  out = acc / (float)(s*s)      (IEEE division)
+ * Rows: the output patch rows [b, e) of the call (patch_row_end = -1: floor(H/32)), like rm_render; the s x frame renders
+ * exactly its patch rows [s*b, s*e) -- not floor(s*H/32) bands.  Other rows of the caller's buffers are left untouched.
+ *   out_rgb   H*W*3 floats, or NULL: the resolved frame.
+ *   out_rgb8  H*W*3 bytes, or NULL: normalize() + to_vec() of the resolved rows by their own maximum (framebuffer.rs:40-82).
+ *             At least one of the two must be given.
+ *   stats     optional: max_value (FrameBuffer::normalize's max over the resolved rows), ms_render (device time of the s x
+ *             frame's render kernels), ms_total, kernel_launches (the resolve included), resident_prims, d2h_bytes.  Event
+ *             counters are not collected.
+ * s = 1 gives rm_render's frame bit for bit.  accel and cull_backfacing apply to the s x render.  Device memory: a scratch of
+ * 12 * s^2 * W * rows bytes for the s x frame (rows = rendered pixel rows; 1.6 GB for a 3840 x 2160 frame at s = 4), kept for
+ * the next call.  The call writes the caller's float frame, so the library forgets its previous deliveries into that memory
+ * (RM_ROWS_RETAINED, above): the next retained delivery there clears every black tile.
+ * RM_ERR_INVALID_ARGUMENT: samples outside [1, 8], precision other than RM_FP32, patch_row_stride > 1, unknown scene, both
+ * outputs NULL.  RM_ERR_DIMENSIONS: the s x frame is not a valid frame (s*W or s*H above 65535, 2^22 patches or more). */
+int rm_render_supersampled(RmScene scene, const RmParams* params, int samples, float* out_rgb, uint8_t* out_rgb8,
+                           RmStats* stats);
+
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device
  * scalar of the same type as d_rgb that receives max(previous value, tile max) -- zero it first.

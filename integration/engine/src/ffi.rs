@@ -195,6 +195,9 @@ extern "C" {
                               stats: *mut RmStats) -> c_int;
     pub fn rm_render_dispersive(scenes: *const RmScene, params: *const RmParams, out_rgb: *mut f32,
                                 out_prim_id: *mut i32, stats: *mut RmStats) -> c_int;
+    /// s x s samples per pixel (samples in [1, 8]): the s x frame box-filtered down to W x H
+    pub fn rm_render_supersampled(scene: RmScene, params: *const RmParams, samples: c_int, out_rgb: *mut f32,
+                                  out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
     // ---- the hot path, device buffers
     pub fn rm_render_device(scene: RmScene, params: *const RmParams, d_rgb: *mut c_void, d_prim_id: *mut i32,
                             d_max: *mut c_void, stream: *mut c_void) -> c_int;

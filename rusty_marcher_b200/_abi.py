@@ -113,6 +113,7 @@ SYMBOLS = {
     "rm_last_kernel_times": (C.c_int, [_P(C.c_double), _P(C.c_double)]),
     "rm_kernel_times": (C.c_int, [C.c_int, _P(C.c_double), _P(C.c_double), _P(C.c_double)]),
     "rm_render_dispersive": (C.c_int, [_P(C.c_int64), _P(RmParams), C.c_void_p, C.c_void_p, _P(RmStats)]),
+    "rm_render_supersampled": (C.c_int, [C.c_int64, _P(RmParams), C.c_int, C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_scene_query_count": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),
     "rm_scene_accel_status": (C.c_int, [C.c_int64, _P(C.c_int32)]),
     "rm_scene_walk_stats": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),

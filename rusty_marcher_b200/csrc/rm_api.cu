@@ -151,6 +151,7 @@ struct Context {
     RmScene next_handle = 1;
     Scratch rgb, prim, rgb8, small;   // small: [0,8) max scalar, [64, 64+17*8) counters
     Scratch mix;                      // rm_render_dispersive: the frame assembled from the three passes
+    Scratch sub;                      // rm_render_supersampled: the s x frame before the resolve
     Scratch pack;                     // host delivery: the busy tiles of a frame, packed in schedule order
     std::vector<Arena> arena_cache;   // device allocations of freed scenes, for the next upload
     // Host packs of the last few scenes by content (SURVEY.md 8f row 2, ingest): a caller that hands over the same scene
@@ -986,7 +987,7 @@ void rm_shutdown(void) {
     for (auto& a : g.arena_cache) cudaFree(a.p);
     g.arena_cache.clear();
     g.pack_cache.clear();
-    g.rgb.release(); g.prim.release(); g.rgb8.release(); g.small.release(); g.mix.release(); g.pack.release();
+    g.rgb.release(); g.prim.release(); g.rgb8.release(); g.small.release(); g.mix.release(); g.pack.release(); g.sub.release();
     g.h_stage.release(); g.h_order.release(); g.h_upload.release(); g.h_early.release();
     if (g.side_stream) cudaStreamDestroy(g.side_stream);
     g.side_stream = nullptr;
@@ -1166,6 +1167,83 @@ int rm_render_dispersive(const RmScene scenes[3], const RmParams* params, float*
         stats->ms_total = ms;
         stats->kernel_launches = launches;
         stats->resident_prims = resident;
+    }
+    return RM_OK;
+}
+
+// Extension mode (include/rm_b200.h): the unchanged render kernels on the s x frame into a scratch of its own, then
+// resolve_box_kernel (the W-wide rows and their maximum) and, for the 8-bit frame, the tone-map kernel.
+int rm_render_supersampled(RmScene scene, const RmParams* params, int samples, float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
+    std::lock_guard<std::mutex> lock(g.mu);
+    if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+    int rc = check_params(params);
+    if (rc != RM_OK) return rc;
+    if (samples < 1 || samples > 8) return fail(RM_ERR_INVALID_ARGUMENT, "samples must be in [1, 8]");
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_supersampled computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_supersampled renders contiguous patch rows (patch_row_stride <= 1)");
+    if (g.scenes.find(scene) == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
+    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
+    // the s x frame renders exactly the sub-rows of the call's patch rows [b, e): its patch rows [s b, s e)
+    RmParams sp = *params;
+    sp.width = samples * params->width;
+    sp.height = samples * params->height;
+    sp.patch_row_begin = samples * (fp.row_begin / 32);
+    sp.patch_row_end = samples * (fp.row_end / 32);
+    sp.patch_row_stride = 1;
+    if ((rc = check_params(&sp)) != RM_OK) return rc;
+    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    if ((rc = g.sub.ensure(std::max<size_t>(n_px * samples * samples * 12, 16))) != RM_OK) return rc;
+    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
+    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
+    float* d_max = static_cast<float*>(g.small.p);              // of the resolved rows
+    float* d_sub_max = d_max + 2;                               // of the s x frame (not reported)
+    cudaStream_t s = g.stream;
+    CK(cudaEventRecord(g.ev[0], s));
+    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
+    CK(cudaEventRecord(g.ev[1], s));
+    int resident = 0, launches = 0;
+    rc = render_device_impl<float>(scene, &sp, static_cast<float*>(g.sub.p), nullptr, d_sub_max, s, 1, nullptr, nullptr, &resident, &launches);
+    if (rc != RM_OK) return rc;
+    CK(cudaEventRecord(g.ev[2], s));
+    if (rows) {
+        CK(rm::launch_resolve_box(static_cast<const float*>(g.sub.p), samples, static_cast<float*>(g.rgb.p), fp.width, (int)rows, d_max, s));
+        launches++;
+        if (out_rgb8) {
+            CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
+            launches++;
+        }
+    }
+    // this call writes the caller's float frame: what the library last delivered there (RM_ROWS_RETAINED) no longer holds.
+    // A record goes when the frame it describes -- at most `height` rows from its key on -- overlaps the rows written here.
+    const size_t host_px = (size_t)fp.row_begin * fp.width;
+    if (out_rgb && n_px) {
+        const char* lo = reinterpret_cast<const char*>(out_rgb + host_px * 3);
+        const char* hi = lo + n_px * 12;
+        g.delivered.erase(std::remove_if(g.delivered.begin(), g.delivered.end(), [&](const Delivered& d) {
+                              const char* k = static_cast<const char*>(d.key);
+                              return k < hi && k + (size_t)d.height * d.width * 3 * d.elem > lo;
+                          }), g.delivered.end());
+        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
+    }
+    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
+    float h_max = 0.f;
+    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
+    CK(cudaEventRecord(g.ev[3], s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) {
+        std::memset(stats, 0, sizeof(*stats));
+        stats->max_value = (double)h_max;
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
+        stats->ms_render = ms;
+        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
+        stats->ms_total = ms;
+        stats->kernel_launches = launches;
+        stats->resident_prims = resident;
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
     }
     return RM_OK;
 }

@@ -900,6 +900,58 @@ deliver_busy_kernel(const float* __restrict__ rgb, const FrameParams<float> fp, 
     }
 }
 
+// Supersampled anti-aliasing (rm_render_supersampled): the S x frame box-filtered down to `rows` W-wide output rows
+// (rm::resolve_box), and their channel maximum (FrameBuffer::normalize) into *dmax.  A pure streaming pass: 12 S^2 bytes in,
+// 12 out per output pixel.  A warp covers 32 consecutive output pixels of one row, so each sub-row it reads is one contiguous
+// run of 32 * 12 S bytes; a lane's share of a sub-row (12 S bytes, at a multiple of 12 S from a 16-byte aligned row start:
+// W is a multiple of 32) is read as float4 when S is a multiple of 4, as float2 when S is even.
+template <int S>
+__global__ void __launch_bounds__(256)
+resolve_box_kernel(const float* __restrict__ sub, float* __restrict__ out, const int width, const int rows,
+                   float* __restrict__ dmax) {
+    __shared__ int cta_max;
+    const int lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) cta_max = 0;
+    __syncthreads();
+    const int warps_x = width >> 5;
+    const long long g = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+    const int y = (int)(g / warps_x);
+    const int x = (int)(g - (long long)y * warps_x) * 32 + lane;
+    float m = 0.f;
+    if (y < rows) {
+        const size_t sub_row = (size_t)S * width * 3;          // floats per row of the S x frame
+        const float* p = sub + (size_t)S * y * sub_row + (size_t)S * 3 * x;
+        float o[3];
+        resolve_box<S>([&](int i, float (&r)[3 * S]) {
+            const float* q = p + i * sub_row;
+            if constexpr (S % 4 == 0) {
+#pragma unroll
+                for (int k = 0; k < 3 * S / 4; k++) {
+                    const float4 f = reinterpret_cast<const float4*>(q)[k];
+                    r[4 * k] = f.x; r[4 * k + 1] = f.y; r[4 * k + 2] = f.z; r[4 * k + 3] = f.w;
+                }
+            } else if constexpr (S % 2 == 0) {
+#pragma unroll
+                for (int k = 0; k < 3 * S / 2; k++) {
+                    const float2 f = reinterpret_cast<const float2*>(q)[k];
+                    r[2 * k] = f.x; r[2 * k + 1] = f.y;
+                }
+            } else {
+#pragma unroll
+                for (int k = 0; k < 3 * S; k++) r[k] = q[k];
+            }
+        }, o);
+        float* d = out + ((size_t)y * width + x) * 3;
+        d[0] = o[0]; d[1] = o[1]; d[2] = o[2];
+        m = fmaxf(fmaxf(o[0], o[1]), o[2]);
+    }
+    // values are >= 0, so the integer order of the bit patterns is the float order
+    const int wm = __reduce_max_sync(0xffffffffu, __float_as_int(m));
+    if (lane == 0 && wm > 0) atomicMax(&cta_max, wm);
+    __syncthreads();
+    if (threadIdx.x == 0 && cta_max > 0) atomicMax(reinterpret_cast<int*>(dmax), cta_max);
+}
+
 __global__ void publish_zero_kernel(const PeerLink link, float* __restrict__ dmax) {
     *dmax = 0.f;
     publish_max(link, 0.f);
@@ -1094,6 +1146,24 @@ cudaError_t launch_deliver_busy(const DeviceScene<float>& ds, const FrameParams<
     if (n_busy <= 0) return cudaSuccess;
     deliver_busy_kernel<<<std::min(n_busy, 148 * 8), 256, 0, stream>>>(rgb, fp, tiles_x, ds.tile_order, ds.tile_order + ds.tile_order_cap / 2,
                                                                        n_full, n_busy, host_frame, host_row_floats);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_resolve_box(const float* sub, int samples, float* out, int width, int rows, float* dmax, cudaStream_t stream) {
+    const long long warps = (long long)(width / 32) * rows;
+    if (warps <= 0) return cudaSuccess;
+    const unsigned blocks = (unsigned)((warps + 7) / 8);
+    switch (samples) {
+        case 1: resolve_box_kernel<1><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        case 2: resolve_box_kernel<2><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        case 3: resolve_box_kernel<3><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        case 4: resolve_box_kernel<4><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        case 5: resolve_box_kernel<5><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        case 6: resolve_box_kernel<6><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        case 7: resolve_box_kernel<7><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        case 8: resolve_box_kernel<8><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        default: return cudaErrorInvalidValue;
+    }
     return cudaGetLastError();
 }
 

@@ -107,6 +107,10 @@ cudaError_t launch_deliver_busy(const DeviceScene<float>& ds, const FrameParams<
 cudaError_t launch_tonemap_peer(const DeviceScene<float>& ds, const FrameParams<float>& fp, const float* rgb, const float* dmax,
                                 bool normalise, unsigned char* rgb8, cudaStream_t stream, const PeerLink& link);
 
+// resolve_box_kernel: `rows` output rows of `width` pixels (out: rows * width * 3 floats) from the samples x frame `sub`
+// (samples * rows rows of samples * width pixels), samples in [1, 8]; *dmax receives max(old, channel maximum of out).
+cudaError_t launch_resolve_box(const float* sub, int samples, float* out, int width, int rows, float* dmax, cudaStream_t stream);
+
 // A rank without rows: zero maximum to every mailbox (the others wait for a word of every rank).
 cudaError_t launch_publish_zero(const PeerLink& link, float* dmax, cudaStream_t stream);
 

@@ -196,4 +196,27 @@ template <typename R> RM_HD void pin(Vec3<R>& v) { pin(v.x); pin(v.y); pin(v.z);
 
 template <typename R> RM_HD Vec3<R> xyz(const R4<R>& v) { return {v.x, v.y, v.z}; }
 
+// Supersampled anti-aliasing (rm_render_supersampled): one output pixel as the mean of its S x S sub-pixels.
+// sub_row(i, r) fills r[3 j + c] with channel c of sub-pixel j of sub-row i.  The order is normative (include/rm_b200.h):
+// sub-rows outer, sub-pixels inner, FP32 adds without contraction (-fmad=false), then one IEEE division by S*S.  Sub-rows
+// are handed over one at a time: a kernel need not hold all 3 S^2 values at once (S = 8: 192 floats).
+template <int S, typename SubRow> RM_HD void resolve_box(const SubRow& sub_row, float out[3]) {
+    float a0 = 0.f, a1 = 0.f, a2 = 0.f;
+#pragma unroll
+    for (int i = 0; i < S; i++) {
+        float r[3 * S];
+        sub_row(i, r);
+#pragma unroll
+        for (int j = 0; j < S; j++) {
+            a0 += r[3 * j];
+            a1 += r[3 * j + 1];
+            a2 += r[3 * j + 2];
+        }
+    }
+    const float n = (float)(S * S);
+    out[0] = a0 / n;
+    out[1] = a1 / n;
+    out[2] = a2 / n;
+}
+
 }  // namespace rm

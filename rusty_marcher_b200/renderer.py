@@ -150,6 +150,37 @@ class Renderer:
         print(message)
         return message
 
+    def render_supersampled(self, frame, scene, samples=2, rgb8=None, patch_rows=(0, -1)):
+        """EXTENSION MODE (no reference counterpart): anti-aliasing with samples x samples primary rays per pixel.  Pixel
+        (x, y) is the mean of the FP32 frame rendered at samples times the width and height over its samples x samples
+        block of sub-pixels (rm_render_supersampled; samples = 1 is render()'s frame).  Fills frame.buffer (float32) over
+        the rendered rows and, if given, rgb8 (H, W, 3) uint8 with normalize + to_vec of the resolved frame; returns the
+        same kind of status message as render()."""
+        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
+            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
+        if self.precision != _abi.RM_FP32:
+            raise ValueError("render_supersampled computes in RM_FP32")
+        if int(self.width) != frame.width or int(self.height) != frame.height:
+            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
+        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
+                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
+            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
+        L = _abi.load()
+        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
+        now = time.perf_counter()
+        p = self.params(frame, scene, patch_rows)
+        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
+            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
+        stats = _abi.RmStats()
+        _abi.check(L.rm_render_supersampled(scene.device_handle(), C.byref(p), int(samples), frame.buffer.ctypes.data,
+                                            rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
+        self.last_stats = stats
+        ms = int((time.perf_counter() - now) * 1000)
+        fps = 1000. / ms if ms > 0 else float("inf")
+        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
+        print(message)
+        return message
+
 
 def create_renderer(fov, height, width):
     return Renderer(fov, height, width)
