@@ -9,6 +9,9 @@
 //   "Save to file"   main.rs:353-362  FrameBuffer::normalize + write_ppm("out.ppm")   --out FILE
 //                                      --samples S (2..8): the saved frame anti-aliased, S x S primary rays per pixel
 //                                      (rm_render_supersampled; an extension, the reference has no such mode)
+//                                      --contrast C: S x S rays only where a pixel's 3x3 neighbourhood changes primitive
+//                                      or exceeds the contrast C, one ray elsewhere (rm_render_adaptive; S = 1 without
+//                                      --samples); prints the number of refined pixels
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -31,6 +34,8 @@ int main(int argc, char** argv) {
     bool f64 = false, rows64 = false;
     const char* obj = nullptr;
     const char* out = "out.ppm";
+    bool adaptive = false;
+    double contrast = 0.;
     double cam[3] = {0., 0., 0.};
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
@@ -46,10 +51,15 @@ int main(int argc, char** argv) {
         else if (a == "--rows-f64") rows64 = true;      // FP32 kernels into the reference's frame type (one allocation per row, f64)
         else if (a == "--accel") accel = 1;
         else if (a == "--samples") { need(1); samples = std::atoi(argv[++i]); }
+        else if (a == "--contrast") { need(1); contrast = std::strtod(argv[++i], nullptr); adaptive = true; }
         else { std::fprintf(stderr, "rm_headless: unknown option %s\n", a.c_str()); return 2; }
     }
-    if (samples < 1 || samples > 8 || (samples > 1 && f64)) {
+    if (samples < 1 || samples > 8 || ((samples > 1 || adaptive) && f64)) {
         std::fprintf(stderr, "rm_headless: --samples takes 1 to 8, with the FP32 kernels\n");
+        return 2;
+    }
+    if (contrast != contrast) {
+        std::fprintf(stderr, "rm_headless: --contrast takes a number (not NaN)\n");
         return 2;
     }
     int rc = rm_init(0);
@@ -104,7 +114,14 @@ int main(int argc, char** argv) {
         std::printf("Scene rendered in %lld ms (%u fps, %.2f MP/s)\n", ms, ms > 0 ? (unsigned)fps : 4294967295u, fps * (double)n_px / 1e6);
     }
     // "Save to file": normalize + to_vec on the device (framebuffer.rs:40-82), then the P6 stream (framebuffer.rs:26-38)
-    if (samples > 1) {
+    if (adaptive) {
+        std::vector<unsigned char> mask(n_px, 0);
+        std::memset(&st, 0, sizeof st);
+        if ((rc = rm_render_adaptive(scene, &p, samples, contrast, nullptr, rgb8.data(), mask.data(), &st)) != RM_OK) die("render (adaptive 8-bit frame)", rc);
+        size_t refined = 0;
+        for (unsigned char m : mask) refined += m;
+        std::printf("adaptive anti-aliasing: %zu of %zu pixels refined (%d x %d samples, contrast %g)\n", refined, n_px, samples, samples, contrast);
+    } else if (samples > 1) {
         std::memset(&st, 0, sizeof st);
         if ((rc = rm_render_supersampled(scene, &p, samples, nullptr, rgb8.data(), &st)) != RM_OK) die("render (supersampled 8-bit frame)", rc);
     } else if (!f64) {

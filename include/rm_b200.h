@@ -254,6 +254,34 @@ int rm_render_dispersive(const RmScene scenes[3], const RmParams* params, float*
 int rm_render_supersampled(RmScene scene, const RmParams* params, int samples, float* out_rgb, uint8_t* out_rgb8,
                            RmStats* stats);
 
+/* ---- extension mode: adaptive anti-aliasing, s x s samples only where the frame changes abruptly ---------------------------- *
+ * Whitted's (1980) adaptive supersampling with Mitchell's (1987) contrast test; no reference behaviour.  Defined by two calls:
+ * P = rm_render's FP32 frame of the scene and camera with its primary ids, S = rm_render_supersampled(..., samples)'s frame.
+ * With R = 32 * floor(H/32) (the rendered rows), pixel p = (x, y) is REFINED if contrast < 0 (every pixel), or else if one of
+ * its 8 neighbours q inside [0, W) x [0, R) has id(q) != id(p), or, for some channel c with a = P[p][c], b = P[q][c],
+ *     fabsf(a - b) > k * (a + b),     k = (float)contrast, every operation rounded to FP32, no fused multiply-add.
+ * contrast = +inf refines geometric edges only (inf * 0 is NaN, the comparison false).  The output pixel is S[p] if p is
+ * refined, P[p] otherwise: samples = 1 gives rm_render's frame, contrast < 0 rm_render_supersampled's, and every other frame
+ * follows bit for bit from those two and the mask.  Sub-pixel detail wholly inside one pixel (a thin object that no pixel
+ * centre hits, a highlight between two samples) changes no 1x pixel and is missed by design.
+ * Rows: the output patch rows [b, e) of the call (patch_row_end = -1: floor(H/32)), like rm_render; rows outside are left
+ * untouched in all three outputs.  The mask looks at neighbours outside the call's rows as well (the 1x frame is rendered
+ * over one more patch row on either side), so a call over some patch rows gives the same rows as a full-frame call.
+ *   out_rgb   H*W*3 floats, or NULL: the frame.
+ *   out_rgb8  H*W*3 bytes, or NULL: normalize() + to_vec() of the output rows by their own maximum.  At least one of the two.
+ *   out_mask  H*W bytes, or NULL: 1 = refined, 0 = not.
+ *   stats     optional: max_value (over the output rows), ms_render (device time from the start of the 1x render to the
+ *             resolved float rows: no tone map, no copies), ms_total, kernel_launches, resident_prims, d2h_bytes.
+ * Device memory, kept for the next call: the 1x frame's rows (16 W bytes per row, halo included), W * rows * 5 bytes for the
+ * mask and the list of refined pixels, and the refined pixels' sub-pixel values, sized for the worst case (every pixel
+ * refined): 12 * s^2 * W * rows bytes, as rm_render_supersampled's scratch (1.6 GB for a 3840 x 2160 frame at s = 4).
+ * The call writes the caller's float frame, so the library forgets its previous deliveries into that memory (RM_ROWS_RETAINED).
+ * RM_ERR_INVALID_ARGUMENT: samples outside [1, 8], NaN contrast, precision other than RM_FP32, patch_row_stride > 1,
+ * max_depth < 1, unknown scene, out_rgb and out_rgb8 both NULL.  RM_ERR_DIMENSIONS: the s x frame is not a valid frame (as for
+ * rm_render_supersampled). */
+int rm_render_adaptive(RmScene scene, const RmParams* params, int samples, double contrast, float* out_rgb, uint8_t* out_rgb8,
+                       uint8_t* out_mask, RmStats* stats);
+
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device
  * scalar of the same type as d_rgb that receives max(previous value, tile max) -- zero it first.

@@ -151,7 +151,9 @@ struct Context {
     RmScene next_handle = 1;
     Scratch rgb, prim, rgb8, small;   // small: [0,8) max scalar, [64, 64+17*8) counters
     Scratch mix;                      // rm_render_dispersive: the frame assembled from the three passes
-    Scratch sub;                      // rm_render_supersampled: the s x frame before the resolve
+    Scratch sub;                      // rm_render_supersampled: the s x frame before the resolve; rm_render_adaptive: the
+                                      // sub-pixel values of the refined pixels
+    Scratch adapt;                    // rm_render_adaptive: the mask bytes and the list of refined pixels
     Scratch pack;                     // host delivery: the busy tiles of a frame, packed in schedule order
     std::vector<Arena> arena_cache;   // device allocations of freed scenes, for the next upload
     // Host packs of the last few scenes by content (SURVEY.md 8f row 2, ingest): a caller that hands over the same scene
@@ -177,6 +179,18 @@ struct Context {
     std::mutex mu;
 };
 Context g;
+
+// A call that writes the caller's float frame [lo, lo + bytes) itself (rm_render_supersampled, rm_render_adaptive): what the
+// library last delivered there (RM_ROWS_RETAINED) no longer holds.  A record goes when the frame it describes -- at most
+// `height` rows from its key on -- overlaps the bytes written.
+void forget_deliveries(const void* lo, size_t bytes) {
+    const char* a = static_cast<const char*>(lo);
+    const char* b = a + bytes;
+    g.delivered.erase(std::remove_if(g.delivered.begin(), g.delivered.end(), [&](const Delivered& d) {
+                          const char* k = static_cast<const char*>(d.key);
+                          return k < b && k + (size_t)d.height * d.width * 3 * d.elem > a;
+                      }), g.delivered.end());
+}
 
 size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
@@ -987,7 +1001,7 @@ void rm_shutdown(void) {
     for (auto& a : g.arena_cache) cudaFree(a.p);
     g.arena_cache.clear();
     g.pack_cache.clear();
-    g.rgb.release(); g.prim.release(); g.rgb8.release(); g.small.release(); g.mix.release(); g.pack.release(); g.sub.release();
+    g.rgb.release(); g.prim.release(); g.rgb8.release(); g.small.release(); g.mix.release(); g.pack.release(); g.sub.release(); g.adapt.release();
     g.h_stage.release(); g.h_order.release(); g.h_upload.release(); g.h_early.release();
     if (g.side_stream) cudaStreamDestroy(g.side_stream);
     g.side_stream = nullptr;
@@ -1216,16 +1230,9 @@ int rm_render_supersampled(RmScene scene, const RmParams* params, int samples, f
             launches++;
         }
     }
-    // this call writes the caller's float frame: what the library last delivered there (RM_ROWS_RETAINED) no longer holds.
-    // A record goes when the frame it describes -- at most `height` rows from its key on -- overlaps the rows written here.
     const size_t host_px = (size_t)fp.row_begin * fp.width;
     if (out_rgb && n_px) {
-        const char* lo = reinterpret_cast<const char*>(out_rgb + host_px * 3);
-        const char* hi = lo + n_px * 12;
-        g.delivered.erase(std::remove_if(g.delivered.begin(), g.delivered.end(), [&](const Delivered& d) {
-                              const char* k = static_cast<const char*>(d.key);
-                              return k < hi && k + (size_t)d.height * d.width * 3 * d.elem > lo;
-                          }), g.delivered.end());
+        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
         CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
     }
     if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
@@ -1244,6 +1251,108 @@ int rm_render_supersampled(RmScene scene, const RmParams* params, int samples, f
         stats->kernel_launches = launches;
         stats->resident_prims = resident;
         stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
+    }
+    return RM_OK;
+}
+
+// Extension mode (include/rm_b200.h): the unchanged render kernels on the 1x frame of the call's rows plus one patch row
+// of halo on either side, adaptive_mark_kernel (mask, list of refined pixels, maximum of the others), adaptive_subpixel_kernel
+// (the s x frame's sub-pixels of the listed pixels only), adaptive_resolve_kernel over the list and, for the 8-bit frame,
+// the tone-map kernel.  The list length stays on the device: no host round trip between the launches.
+int rm_render_adaptive(RmScene scene, const RmParams* params, int samples, double contrast, float* out_rgb, uint8_t* out_rgb8,
+                       uint8_t* out_mask, RmStats* stats) {
+    std::lock_guard<std::mutex> lock(g.mu);
+    if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+    int rc = check_params(params);
+    if (rc != RM_OK) return rc;
+    if (samples < 1 || samples > 8) return fail(RM_ERR_INVALID_ARGUMENT, "samples must be in [1, 8]");
+    if (contrast != contrast) return fail(RM_ERR_INVALID_ARGUMENT, "contrast is NaN");
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_adaptive computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_adaptive renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_adaptive needs max_depth >= 1");
+    auto it = g.scenes.find(scene);
+    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    const rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);      // the output rows [row_begin, row_end)
+    // the s x frame, whose sub-pixels the refined pixels get: only its FrameParams are used, but it must be a valid frame
+    RmParams sp = *params;
+    sp.width = samples * params->width;
+    sp.height = samples * params->height;
+    sp.patch_row_begin = 0;
+    sp.patch_row_end = -1;
+    sp.patch_row_stride = 1;
+    if ((rc = check_params(&sp)) != RM_OK) return rc;
+    const rm::FrameParams<float> fs = rm::make_frame_params<float>(sp);
+    // the 1x frame: the call's patch rows and one more above and below where the frame has one (the mask's neighbours)
+    const int b = fp.row_begin / 32, e = fp.row_end / 32;
+    RmParams hp = *params;
+    hp.patch_row_begin = e > b ? std::max(b - 1, 0) : b;
+    hp.patch_row_end = e > b ? std::min(e + 1, params->height / 32) : b;
+    hp.patch_row_stride = 1;
+    const int lo = 32 * hp.patch_row_begin, hi = 32 * hp.patch_row_end;
+    const size_t halo_px = (size_t)(hi - lo) * fp.width, rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    const size_t ss = (size_t)samples * samples;
+    if ((rc = g.rgb.ensure(std::max<size_t>(halo_px * 12, 16))) != RM_OK) return rc;
+    if ((rc = g.prim.ensure(std::max<size_t>(halo_px * 4, 16))) != RM_OK) return rc;
+    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(halo_px * 3, 16))) != RM_OK) return rc;
+    if ((rc = g.sub.ensure(std::max<size_t>(n_px * ss * 12, 16))) != RM_OK) return rc;
+    const size_t list_off = align256(n_px);
+    if ((rc = g.adapt.ensure(std::max<size_t>(list_off + n_px * 4, 16))) != RM_OK) return rc;
+    if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
+    float* d_max = static_cast<float*>(g.small.p);              // of the output rows
+    float* d_max1 = d_max + 2;                                  // of the 1x frame with its halo (not reported)
+    unsigned* d_count = reinterpret_cast<unsigned*>(static_cast<char*>(g.small.p) + 16);
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
+    unsigned char* d_mask = static_cast<unsigned char*>(g.adapt.p);
+    unsigned* d_list = reinterpret_cast<unsigned*>(static_cast<char*>(g.adapt.p) + list_off);
+    float* d_rgb = static_cast<float*>(g.rgb.p);
+    const size_t dev_px = (size_t)(fp.row_begin - lo) * fp.width;     // first output pixel in the 1x scratch
+    cudaStream_t s = g.stream;
+    CK(cudaEventRecord(g.ev[0], s));
+    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
+    CK(cudaEventRecord(g.ev[1], s));
+    int resident = 0, launches = 0;
+    rc = render_device_impl<float>(scene, &hp, d_rgb, static_cast<int*>(g.prim.p), d_max1, s, 1, nullptr, nullptr, &resident, &launches);
+    if (rc != RM_OK) return rc;
+    if (rows) {
+        CK(rm::launch_adaptive_mark(d_rgb, static_cast<const int*>(g.prim.p), fp.width, lo, hi, fp.row_begin, (int)rows, (float)contrast,
+                                    contrast < 0., d_mask, d_list, d_count, d_max, s));
+        CK(rm::launch_adaptive_subpixel(it->second.f32.ds, fs, params->cull_backfacing != 0, samples, d_list, d_count, d_next,
+                                        static_cast<float*>(g.sub.p), params->camera, s));
+        CK(rm::launch_adaptive_resolve(static_cast<const float*>(g.sub.p), samples, d_list, d_count, d_rgb, fp.width, lo, (long long)n_px,
+                                       d_max, s));
+        launches += 3;
+    }
+    CK(cudaEventRecord(g.ev[2], s));
+    if (out_rgb8 && rows) {
+        rm::FrameParams<float> fo = fp;
+        fo.buf_row0 = lo;                                       // both scratch frames are indexed from the halo's first row
+        CK(rm::launch_tonemap<float>(fo, d_rgb, d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
+        launches++;
+    }
+    const size_t host_px = (size_t)fp.row_begin * fp.width;
+    if (out_rgb && n_px) {
+        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
+        CK(cudaMemcpyAsync(out_rgb + host_px * 3, d_rgb + dev_px * 3, n_px * 12, cudaMemcpyDeviceToHost, s));
+    }
+    if (out_rgb8 && n_px)
+        CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, static_cast<unsigned char*>(g.rgb8.p) + dev_px * 3, n_px * 3, cudaMemcpyDeviceToHost, s));
+    if (out_mask && n_px) CK(cudaMemcpyAsync(out_mask + host_px, d_mask, n_px, cudaMemcpyDeviceToHost, s));
+    float h_max = 0.f;
+    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
+    CK(cudaEventRecord(g.ev[3], s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) {
+        std::memset(stats, 0, sizeof(*stats));
+        stats->max_value = (double)h_max;
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
+        stats->ms_render = ms;
+        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
+        stats->ms_total = ms;
+        stats->kernel_launches = launches;
+        stats->resident_prims = resident;
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0) + (out_mask ? 1 : 0));
     }
     return RM_OK;
 }

@@ -952,6 +952,231 @@ resolve_box_kernel(const float* __restrict__ sub, float* __restrict__ out, const
     if (threadIdx.x == 0 && cta_max > 0) atomicMax(reinterpret_cast<int*>(dmax), cta_max);
 }
 
+// ---- Adaptive anti-aliasing (rm_render_adaptive): mark -> sub-pixel rays of the marked pixels -> resolve ----------------
+// Mark: one thread per pixel of the call's n_px = rows * W pixels from frame row row_begin (a warp: 32 pixels of one row,
+// W being a multiple of 32).  The 1x frame (rgb, id) holds rows [lo, hi).  Pixels that are not refined keep their 1x value,
+// which is already in place in rgb, and fold it into *dmax; refined ones go to `list` as x | y << 16 (one atomic per warp:
+// the order of the list varies from run to run, what is computed for each entry does not).  mask[i]: 1 = refined.
+__global__ void __launch_bounds__(256)
+adaptive_mark_kernel(const float* __restrict__ rgb, const int* __restrict__ id, const int width, const int lo, const int hi,
+                     const int row_begin, const long long n_px, const float k, const int all, unsigned char* __restrict__ mask,
+                     unsigned* __restrict__ list, unsigned* __restrict__ count, float* __restrict__ dmax) {
+    __shared__ int cta_max;
+    const int lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) cta_max = 0;
+    __syncthreads();
+    const long long t = (long long)blockIdx.x * 256 + threadIdx.x;
+    bool refine = false;
+    float m = 0.f;
+    int x = 0, y = 0;
+    if (t < n_px) {
+        const long long r = t / width;
+        y = row_begin + (int)r;
+        x = (int)(t - r * width);
+        refine = adaptive_mark(rgb, id, width, lo, hi, x, y, k, all != 0);
+        mask[t] = refine ? 1 : 0;
+        if (!refine) {
+            const float* v = rgb + 3 * ((size_t)(y - lo) * width + x);
+            m = fmaxf(fmaxf(v[0], v[1]), v[2]);
+        }
+    }
+    const unsigned b = __ballot_sync(0xffffffffu, refine);
+    if (b) {
+        unsigned base = 0;
+        if (lane == 0) base = atomicAdd(count, (unsigned)__popc(b));
+        base = __shfl_sync(0xffffffffu, base, 0);
+        if (refine) list[base + __popc(b & ((1u << lane) - 1u))] = (unsigned)x | ((unsigned)y << 16);
+    }
+    // values are >= 0, so the integer order of the bit patterns is the float order
+    const int wm = __reduce_max_sync(0xffffffffu, __float_as_int(m));
+    if (lane == 0 && wm > 0) atomicMax(&cta_max, wm);
+    __syncthreads();
+    if (threadIdx.x == 0 && cta_max > 0) atomicMax(reinterpret_cast<int*>(dmax), cta_max);
+}
+
+// Sub-pixel rays of the listed pixels: entry e of the list, sub-pixel r = i * s + j (i, j in [0, s)), is the s x frame's
+// pixel (s x + j, s y + i), and its value goes to sub[3 (e s^2 + r) ...] -- every listed pixel's s^2 values contiguous,
+// sub-rows outer, in resolve_box's order.  fp is the s x frame's FrameParams.  Every value is the one render_fast_kernel
+// (K1) writes for that pixel of the s x frame, bit for bit: the same device functions with the same operands per pixel --
+// primary_begin, primary_tri over the raster records K0 wrote for this camera (they depend on the camera only, not on the
+// frame size) or primary_bvh, primary_rest, fast_shade -- and misses are 0.
+// Persistent grid: a warp draws 32 consecutive sub-rays at a time from a 64-bit counter (*next, zero at launch) up to
+// *count * s^2 -- the list length stays on the device.  Stage A runs one sub-ray per lane; the warp's triangles are first
+// bounded against the rectangle of its 32 sub-pixels (tri_may_touch: exact, see rect_max).  Hits go to the warp's queue,
+// compacted with ballot / popc, and are shaded 32 at a time (stage B on full warps, like K1); the last partial round runs
+// when the work has run out.
+constexpr int kAdaptiveQueue = 64;
+template <bool kSmem, bool kBvh, int kGlass>
+__global__ void __launch_bounds__(kFastBlock, RM_K1_MIN_BLOCKS)
+adaptive_subpixel_kernel(const DeviceScene<float> ds, const FrameParams<float> fp, const int cull, const int samples,
+                         const unsigned* __restrict__ list, const unsigned* __restrict__ count,
+                         unsigned long long* __restrict__ next, float* __restrict__ sub, const int stage_mat) {
+    extern __shared__ __align__(32) unsigned char smem_raw[];
+    __shared__ float4 queue[kFastBlock / 32][kAdaptiveQueue];       // {t, slot, id, sub-ray index}
+    const BlobLayout& L = ds.lay;
+    const int n_tri = tri_count(L, cull != 0);
+    const unsigned char* base = ds.blob;
+    const R4<float>* tri_r = ds.tri_r;
+    if (kSmem) {                                                // as K1: blob | raster records | materials (if they fit)
+        const uint4* src = reinterpret_cast<const uint4*>(ds.blob);
+        uint4* dst = reinterpret_cast<uint4*>(smem_raw);
+        const int n16 = L.bytes / 16;
+        for (int i = threadIdx.x; i < n16; i += kFastBlock) dst[i] = __ldg(src + i);
+        const uint4* rsrc = reinterpret_cast<const uint4*>(ds.tri_r);
+        for (int i = threadIdx.x; i < n_tri * 4; i += kFastBlock) dst[n16 + i] = rsrc[i];
+        if (stage_mat) {
+            uint4* m = dst + n16 + L.n_tri * 4;
+            const uint4* a = reinterpret_cast<const uint4*>(ds.mat_a);
+            const uint4* b = reinterpret_cast<const uint4*>(ds.mat_b);
+            for (int i = threadIdx.x; i < ds.n_mat; i += kFastBlock) {
+                m[i] = __ldg(a + i);
+                m[ds.n_mat + i] = __ldg(b + i);
+                reinterpret_cast<int*>(m + 2 * ds.n_mat)[i] = __ldg(ds.mat_f + i);
+            }
+        }
+        base = smem_raw;
+        tri_r = reinterpret_cast<const R4<float>*>(smem_raw + L.bytes);
+    }
+    __syncthreads();
+    FastViewT<kBvh, false> fv;
+    fv.bvh = ds.bvh;
+    fv.sph = reinterpret_cast<const R4<float>*>(base + L.off_sph);
+    fv.sph_id = reinterpret_cast<const int*>(base + L.off_sph_id);
+    fv.n_sph = L.n_sph;
+    fv.tri_g = reinterpret_cast<const R4<float>*>(base + L.off_tri_g);
+    fv.tri_r = tri_r;
+    fv.n_tri = n_tri;
+    fv.poly_slot = reinterpret_cast<const int*>(base + L.off_poly_slot);
+    fv.n_poly = poly_count(L, cull != 0);
+    fv.pln_n = reinterpret_cast<const R4<float>*>(base + L.off_pln_n);
+    fv.pln_c = reinterpret_cast<const R4<float>*>(base + L.off_pln_c);
+    fv.pln_v = reinterpret_cast<const I2*>(base + L.off_pln_v);
+    fv.pln_id = reinterpret_cast<const int*>(base + L.off_pln_id);
+    fv.vert = reinterpret_cast<const R4<float>*>(base + L.off_vert);
+    fv.mat_a = ds.mat_a;
+    fv.mat_b = ds.mat_b;
+    fv.mat_f = ds.mat_f;
+    if (kSmem && stage_mat) {
+        fv.mat_a = reinterpret_cast<const R4<float>*>(smem_raw + L.bytes + (size_t)L.n_tri * 64);
+        fv.mat_b = fv.mat_a + ds.n_mat;
+        fv.mat_f = reinterpret_cast<const int*>(fv.mat_b + ds.n_mat);
+    }
+    fv.lgt_p = reinterpret_cast<const R4<float>*>(base + L.off_lgt_p);
+    fv.lgt_c = reinterpret_cast<const R4<float>*>(base + L.off_lgt_c);
+    fv.n_lgt = L.n_lgt;
+    fv.sph64 = ds.sph64;
+    fv.tri64 = ds.tri_src;
+    fv.pln64 = ds.pln64;
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const unsigned lane_lt = (1u << lane) - 1u;
+    const bool rest = fv.n_sph + fv.n_poly > 0;
+    const unsigned ss = (unsigned)(samples * samples);
+    const unsigned long long total = (unsigned long long)*count * ss;
+    float4* const wq = queue[warp];
+    int qn = 0;                                                 // entries in this warp's queue (warp-uniform)
+    // sub-ray g -> its pixel of the s x frame
+    auto sub_pixel = [&](const unsigned long long g, int& sx, int& sy) {
+        const unsigned long long e = g / ss;
+        const int r = (int)(g - e * ss), i = r / samples, j = r - i * samples;
+        const unsigned xy = __ldg(list + e);
+        sx = samples * (int)(xy & 0xffffu) + j;
+        sy = samples * (int)(xy >> 16) + i;
+    };
+    auto shade_entry = [&](const float4 e) {
+        const unsigned long long g = (unsigned long long)__float_as_uint(e.w);
+        int sx, sy;
+        sub_pixel(g, sx, sy);
+        RM_CHECK(g < total && sx >= 0 && sx < fp.width && sy >= 0 && sy < fp.height);
+        const Vec3<float> c = fast_shade<kGlass>(fv, fp, sx, sy, e.x, __float_as_int(e.y), __float_as_int(e.z));
+        float* dst = sub + 3 * g;
+        dst[0] = c.x;
+        dst[1] = c.y;
+        dst[2] = c.z;
+    };
+    for (;;) {
+        unsigned long long g0 = 0;
+        if (lane == 0) g0 = atomicAdd(next, 32ull);
+        g0 = __shfl_sync(0xffffffffu, g0, 0);
+        if (g0 >= total) break;
+        const unsigned long long g = g0 + lane;
+        const bool live = g < total;
+        int sx = 0, sy = 0;
+        if (live) sub_pixel(g, sx, sy);
+        PrimaryState<1> ps;
+        primary_begin<1>(ps, fp, sx, sy);
+        if constexpr (kBvh) {
+            primary_bvh<1, false>(ps, fv, fp);
+        } else {
+            // the rectangle of the warp's live sub-pixels (lane 0 is always live)
+            const int xa = __reduce_min_sync(0xffffffffu, live ? sx : 0x7fffffff), xb = __reduce_max_sync(0xffffffffu, live ? sx : -1);
+            const int ya = __reduce_min_sync(0xffffffffu, live ? sy : 0x7fffffff), yb = __reduce_max_sync(0xffffffffu, live ? sy : -1);
+            const float Xa = pixel_X(fp, xa), Xb = pixel_X(fp, xb), Ya = pixel_Y(fp, ya), Yb = pixel_Y(fp, yb);
+            for (int jb = 0; jb < n_tri; jb += 32) {
+                const int j = jb + lane;
+                bool cand = false;
+                if (j < n_tri) cand = tri_may_touch(tri_r[4 * j], tri_r[4 * j + 1], tri_r[4 * j + 2], tri_r[4 * j + 3], Xa, Xb, Ya, Yb);
+                unsigned cm = __ballot_sync(0xffffffffu, cand);
+                while (cm) {                                    // uniform across the warp
+                    const int jj = jb + __ffs(cm) - 1;
+                    cm &= cm - 1;
+                    primary_tri<1>(ps, tri_r[4 * jj], tri_r[4 * jj + 1], tri_r[4 * jj + 2], tri_r[4 * jj + 3], fv.n_sph + jj);
+                }
+            }
+            if (rest) primary_rest<1>(ps, fv, fp);
+        }
+        const bool hit = live && ps.slot[0] >= 0;
+        if (live && !hit) {                                     // renderer.rs:300-306: a primary miss is black
+            float* dst = sub + 3 * g;
+            dst[0] = 0.f;
+            dst[1] = 0.f;
+            dst[2] = 0.f;
+        }
+        const unsigned mh = __ballot_sync(0xffffffffu, hit);
+        RM_CHECK(qn + __popc(mh) <= kAdaptiveQueue);
+        if (hit) wq[qn + __popc(mh & lane_lt)] = make_float4(ps.t[0], __int_as_float(ps.slot[0]), __int_as_float(ps.id[0]), __uint_as_float((unsigned)g));
+        qn += __popc(mh);
+        __syncwarp();
+        if (qn >= 32) {
+            qn -= 32;
+            shade_entry(wq[qn + lane]);
+            __syncwarp();                                       // reads done before the next round appends
+        }
+    }
+    if (lane < qn) shade_entry(wq[lane]);
+}
+
+// Resolve of the refined pixels: list entry e's s^2 sub-pixel values (sub, laid out as above) -> rm::resolve_box<S> -> its
+// pixel of rgb (rows from frame row lo), and their maximum into *dmax.  Grid-stride over the *count entries.
+template <int S>
+__global__ void __launch_bounds__(256)
+adaptive_resolve_kernel(const float* __restrict__ sub, const unsigned* __restrict__ list, const unsigned* __restrict__ count,
+                        float* __restrict__ rgb, const int width, const int lo, float* __restrict__ dmax) {
+    __shared__ int cta_max;
+    const int lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) cta_max = 0;
+    __syncthreads();
+    const unsigned n = *count;
+    float m = 0.f;
+    for (unsigned e = blockIdx.x * 256u + threadIdx.x; e < n; e += gridDim.x * 256u) {
+        const unsigned xy = list[e];
+        const int x = (int)(xy & 0xffffu), y = (int)(xy >> 16);
+        const float* p = sub + (size_t)e * (3 * S * S);
+        float o[3];
+        resolve_box<S>([&](int i, float (&r)[3 * S]) {
+#pragma unroll
+            for (int k = 0; k < 3 * S; k++) r[k] = p[i * 3 * S + k];
+        }, o);
+        float* d = rgb + 3 * ((size_t)(y - lo) * width + x);
+        d[0] = o[0]; d[1] = o[1]; d[2] = o[2];
+        m = fmaxf(m, fmaxf(fmaxf(o[0], o[1]), o[2]));
+    }
+    const int wm = __reduce_max_sync(0xffffffffu, __float_as_int(m));
+    if (lane == 0 && wm > 0) atomicMax(&cta_max, wm);
+    __syncthreads();
+    if (threadIdx.x == 0 && cta_max > 0) atomicMax(reinterpret_cast<int*>(dmax), cta_max);
+}
+
 __global__ void publish_zero_kernel(const PeerLink link, float* __restrict__ dmax) {
     *dmax = 0.f;
     publish_max(link, 0.f);
@@ -1162,6 +1387,70 @@ cudaError_t launch_resolve_box(const float* sub, int samples, float* out, int wi
         case 6: resolve_box_kernel<6><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
         case 7: resolve_box_kernel<7><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
         case 8: resolve_box_kernel<8><<<blocks, 256, 0, stream>>>(sub, out, width, rows, dmax); break;
+        default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_adaptive_mark(const float* rgb, const int* id, int width, int lo, int hi, int row_begin, int rows, float k,
+                                 bool all, unsigned char* mask, unsigned* list, unsigned* count, float* dmax, cudaStream_t stream) {
+    const long long n_px = (long long)width * rows;
+    if (n_px <= 0) return cudaSuccess;
+    adaptive_mark_kernel<<<(unsigned)((n_px + 255) / 256), 256, 0, stream>>>(rgb, id, width, lo, hi, row_begin, n_px, k, all ? 1 : 0,
+                                                                             mask, list, count, dmax);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_adaptive_subpixel(const DeviceScene<float>& ds, const FrameParams<float>& fp, bool cull, int samples,
+                                     const unsigned* list, const unsigned* count, unsigned long long* next, float* sub,
+                                     const double camera[3], cudaStream_t stream) {
+    // the instantiation launch_fast would pick for this scene and camera: hierarchy or not, glass mode, staged scene
+    using K = decltype(&adaptive_subpixel_kernel<true, false, GLASS_NONE>);
+    static const K table[3][3] = {
+        {adaptive_subpixel_kernel<true, false, GLASS_NONE>, adaptive_subpixel_kernel<true, false, GLASS_F32>, adaptive_subpixel_kernel<true, false, GLASS_F64>},
+        {adaptive_subpixel_kernel<false, false, GLASS_NONE>, adaptive_subpixel_kernel<false, false, GLASS_F32>, adaptive_subpixel_kernel<false, false, GLASS_F64>},
+        {adaptive_subpixel_kernel<false, true, GLASS_NONE>, adaptive_subpixel_kernel<false, true, GLASS_F32>, adaptive_subpixel_kernel<false, true, GLASS_F64>}};
+    static int sm_count = 0, dyn_limit = 0;
+    cudaError_t e;
+    if (!sm_count) {
+        int dev = 0, optin = 0;
+        cudaFuncAttributes fa;
+        if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+        if ((e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
+        if ((e = cudaFuncGetAttributes(&fa, table[0][GLASS_F64])) != cudaSuccess) return e;
+        dyn_limit = std::min(kSmemLimit, optin - (int)fa.sharedSizeBytes - 1024);
+        for (int gm = 0; gm < 3; gm++)
+            if ((e = cudaFuncSetAttribute(table[0][gm], cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
+        if ((e = cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
+    }
+    const bool bvh = fp.accel != 0 && ds.bvh.n_nodes > 0 && ds.lay.n_lgt <= kBvhMaxLights;
+    const size_t smem_geo = (size_t)ds.lay.bytes + (size_t)ds.lay.n_tri * 64;
+    const size_t smem_mat = (((size_t)ds.n_mat * 36) + 15) / 16 * 16;
+    const int stage_mat = smem_geo + smem_mat <= (size_t)dyn_limit ? 1 : 0;
+    const size_t smem = smem_geo + (stage_mat ? smem_mat : 0);
+    const bool use_smem = !bvh && smem <= (size_t)dyn_limit;
+    const int glass = glass_mode(ds.lay.any_glass != 0, ds.lay.n_sph, ds.lay.coord_max, ds.lay.r_min, camera);
+    const K k = table[bvh ? 2 : use_smem ? 0 : 1][glass];
+    const size_t dyn = use_smem ? smem : 0;
+    int occ = 1;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, kFastBlock, dyn)) != cudaSuccess) return e;
+    k<<<sm_count * std::max(occ, 1), kFastBlock, dyn, stream>>>(ds, fp, cull ? 1 : 0, samples, list, count, next, sub, stage_mat);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_adaptive_resolve(const float* sub, int samples, const unsigned* list, const unsigned* count, float* rgb, int width,
+                                    int lo, long long max_entries, float* dmax, cudaStream_t stream) {
+    if (max_entries <= 0) return cudaSuccess;
+    const unsigned blocks = (unsigned)std::min<long long>((max_entries + 255) / 256, 148 * 8);
+    switch (samples) {
+        case 1: adaptive_resolve_kernel<1><<<blocks, 256, 0, stream>>>(sub, list, count, rgb, width, lo, dmax); break;
+        case 2: adaptive_resolve_kernel<2><<<blocks, 256, 0, stream>>>(sub, list, count, rgb, width, lo, dmax); break;
+        case 3: adaptive_resolve_kernel<3><<<blocks, 256, 0, stream>>>(sub, list, count, rgb, width, lo, dmax); break;
+        case 4: adaptive_resolve_kernel<4><<<blocks, 256, 0, stream>>>(sub, list, count, rgb, width, lo, dmax); break;
+        case 5: adaptive_resolve_kernel<5><<<blocks, 256, 0, stream>>>(sub, list, count, rgb, width, lo, dmax); break;
+        case 6: adaptive_resolve_kernel<6><<<blocks, 256, 0, stream>>>(sub, list, count, rgb, width, lo, dmax); break;
+        case 7: adaptive_resolve_kernel<7><<<blocks, 256, 0, stream>>>(sub, list, count, rgb, width, lo, dmax); break;
+        case 8: adaptive_resolve_kernel<8><<<blocks, 256, 0, stream>>>(sub, list, count, rgb, width, lo, dmax); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();

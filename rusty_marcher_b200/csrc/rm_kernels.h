@@ -111,6 +111,21 @@ cudaError_t launch_tonemap_peer(const DeviceScene<float>& ds, const FrameParams<
 // (samples * rows rows of samples * width pixels), samples in [1, 8]; *dmax receives max(old, channel maximum of out).
 cudaError_t launch_resolve_box(const float* sub, int samples, float* out, int width, int rows, float* dmax, cudaStream_t stream);
 
+// Adaptive anti-aliasing (rm_render_adaptive), three launches after K0 + K1 rendered the 1x frame's rows [lo, hi) into rgb / id:
+// adaptive_mark_kernel: rows [row_begin, row_begin + rows) -> mask (1 byte per pixel, from row_begin), the refined pixels
+//   appended to list (x | y << 16; *count, zero at launch, receives their number), the unrefined values' maximum into *dmax.
+cudaError_t launch_adaptive_mark(const float* rgb, const int* id, int width, int lo, int hi, int row_begin, int rows, float k,
+                                 bool all, unsigned char* mask, unsigned* list, unsigned* count, float* dmax, cudaStream_t stream);
+// adaptive_subpixel_kernel: the samples^2 sub-pixel values of every listed pixel in the samples x frame fp (sub: 3 samples^2
+//   floats per entry), K0's raster records of the same camera reused; *next: a zeroed 64-bit work counter.
+cudaError_t launch_adaptive_subpixel(const DeviceScene<float>& ds, const FrameParams<float>& fp, bool cull, int samples,
+                                     const unsigned* list, const unsigned* count, unsigned long long* next, float* sub,
+                                     const double camera[3], cudaStream_t stream);
+// adaptive_resolve_kernel: every listed pixel's resolve_box of its sub-pixel values into rgb (rows from lo), their maximum into
+//   *dmax; max_entries bounds *count (sizes the grid).
+cudaError_t launch_adaptive_resolve(const float* sub, int samples, const unsigned* list, const unsigned* count, float* rgb, int width,
+                                    int lo, long long max_entries, float* dmax, cudaStream_t stream);
+
 // A rank without rows: zero maximum to every mailbox (the others wait for a word of every rank).
 cudaError_t launch_publish_zero(const PeerLink& link, float* dmax, cudaStream_t stream);
 

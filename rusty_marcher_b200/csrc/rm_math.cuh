@@ -219,4 +219,31 @@ template <int S, typename SubRow> RM_HD void resolve_box(const SubRow& sub_row, 
     out[2] = a2 / n;
 }
 
+// Adaptive anti-aliasing (rm_render_adaptive): whether pixel (x, y) of the 1x frame is refined (supersampled).  rgb (3
+// floats per pixel) and id hold the frame's rows [lo, hi), row lo first, rows of `width` pixels; the caller makes [lo, hi)
+// cover every row of [0, R) (R: the rendered rows) that the 3x3 neighbourhood of (x, y) reaches, and nothing beyond R.
+// Normative (include/rm_b200.h): refined when `all`, or when one of the 8 neighbours inside [0, width) x [lo, hi) has
+// another primitive id, or differs in some channel by more than k times the two values' sum -- Mitchell's contrast test,
+// fabsf(a - b) > k * (a + b), FP32 without contraction.  k = +inf refines geometric edges only (inf * 0 is NaN).
+RM_HD bool adaptive_mark(const float* rgb, const int* id, const int width, const int lo, const int hi, const int x, const int y,
+                         const float k, const bool all) {
+    if (all) return true;
+    const size_t p = (size_t)(y - lo) * width + x;
+    const int ip = id[p];
+    const float a0 = rgb[3 * p], a1 = rgb[3 * p + 1], a2 = rgb[3 * p + 2];
+    for (int dy = -1; dy <= 1; dy++) {
+        const int qy = y + dy;
+        if (qy < lo || qy >= hi) continue;
+        for (int dx = -1; dx <= 1; dx++) {
+            const int qx = x + dx;
+            if ((dx == 0 && dy == 0) || qx < 0 || qx >= width) continue;
+            const size_t q = (size_t)(qy - lo) * width + qx;
+            if (id[q] != ip) return true;
+            const float b0 = rgb[3 * q], b1 = rgb[3 * q + 1], b2 = rgb[3 * q + 2];
+            if (fabsf(a0 - b0) > k * (a0 + b0) || fabsf(a1 - b1) > k * (a1 + b1) || fabsf(a2 - b2) > k * (a2 + b2)) return true;
+        }
+    }
+    return false;
+}
+
 }  // namespace rm

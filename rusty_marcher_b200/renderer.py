@@ -181,6 +181,42 @@ class Renderer:
         print(message)
         return message
 
+    def render_adaptive(self, frame, scene, samples=4, contrast=0.1, rgb8=None, mask=None, patch_rows=(0, -1)):
+        """EXTENSION MODE (no reference counterpart): adaptive anti-aliasing.  A pixel gets render_supersampled()'s value
+        when one of its 8 neighbours in render()'s frame has another primitive id or differs in some channel by more than
+        contrast * (a + b) (contrast < 0: every pixel; +inf: geometric edges only), and render()'s value otherwise
+        (rm_render_adaptive).  Fills frame.buffer (float32) over the rendered rows, rgb8 (H, W, 3) uint8 with normalize +
+        to_vec of that frame if given, and mask (H, W) uint8 with 1 where a pixel was refined; returns the same kind of
+        status message as render()."""
+        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
+            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
+        if not isinstance(contrast, (int, float, np.integer, np.floating)) or isinstance(contrast, bool) or np.isnan(contrast):
+            raise ValueError("contrast must be a real number (not NaN), got %r" % (contrast,))
+        if self.precision != _abi.RM_FP32:
+            raise ValueError("render_adaptive computes in RM_FP32")
+        if int(self.width) != frame.width or int(self.height) != frame.height:
+            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
+        for name, a, shape in (("rgb8", rgb8, (frame.height, frame.width, 3)), ("mask", mask, (frame.height, frame.width))):
+            if a is not None and (not isinstance(a, np.ndarray) or a.dtype != np.uint8 or a.shape != shape or not a.flags.c_contiguous
+                                  or not a.flags.writeable):
+                raise ValueError("%s must be a writeable C-contiguous uint8 array of shape %s" % (name, shape))
+        L = _abi.load()
+        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
+        now = time.perf_counter()
+        p = self.params(frame, scene, patch_rows)
+        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
+            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
+        stats = _abi.RmStats()
+        _abi.check(L.rm_render_adaptive(scene.device_handle(), C.byref(p), int(samples), float(contrast), frame.buffer.ctypes.data,
+                                        rgb8.ctypes.data if rgb8 is not None else None,
+                                        mask.ctypes.data if mask is not None else None, C.byref(stats)))
+        self.last_stats = stats
+        ms = int((time.perf_counter() - now) * 1000)
+        fps = 1000. / ms if ms > 0 else float("inf")
+        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
+        print(message)
+        return message
+
 
 def create_renderer(fov, height, width):
     return Renderer(fov, height, width)
