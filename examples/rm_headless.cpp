@@ -12,6 +12,9 @@
 //                                      --contrast C: S x S rays only where a pixel's 3x3 neighbourhood changes primitive
 //                                      or exceeds the contrast C, one ray elsewhere (rm_render_adaptive; S = 1 without
 //                                      --samples); prints the number of refined pixels
+//   --look-at X,Y,Z                    the camera turned to look at that point (rm_render_view; an extension: the reference
+//                                      always looks down -z), --up X,Y,Z its up direction (default 0,1,0).  Combines with
+//                                      --camera, --accel, --f64 and --out; not with --samples, --contrast or --rows-f64
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -37,6 +40,10 @@ int main(int argc, char** argv) {
     bool adaptive = false;
     double contrast = 0.;
     double cam[3] = {0., 0., 0.};
+    bool look = false;
+    double target[3] = {0., 0., 0.};
+    RmView view = {{0., 0., -1.}, {0., 1., 0.}};
+    auto triple = [](const char* s, double v[3]) { char end = 0; return std::sscanf(s, "%lf,%lf,%lf%c", &v[0], &v[1], &v[2], &end) == 3; };
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
         auto need = [&](int n) { if (i + n >= argc) { std::fprintf(stderr, "rm_headless: %s needs %d value(s)\n", a.c_str(), n); std::exit(2); } };
@@ -52,10 +59,19 @@ int main(int argc, char** argv) {
         else if (a == "--accel") accel = 1;
         else if (a == "--samples") { need(1); samples = std::atoi(argv[++i]); }
         else if (a == "--contrast") { need(1); contrast = std::strtod(argv[++i], nullptr); adaptive = true; }
+        else if (a == "--look-at" || a == "--up") {
+            need(1);
+            if (!triple(argv[++i], a == "--up" ? view.up : target)) { std::fprintf(stderr, "rm_headless: %s takes X,Y,Z\n", a.c_str()); return 2; }
+            look = look || a == "--look-at";
+        }
         else { std::fprintf(stderr, "rm_headless: unknown option %s\n", a.c_str()); return 2; }
     }
     if (samples < 1 || samples > 8 || ((samples > 1 || adaptive) && f64)) {
         std::fprintf(stderr, "rm_headless: --samples takes 1 to 8, with the FP32 kernels\n");
+        return 2;
+    }
+    if (look && (samples > 1 || adaptive || rows64)) {
+        std::fprintf(stderr, "rm_headless: --look-at does not combine with --samples, --contrast or --rows-f64\n");
         return 2;
     }
     if (contrast != contrast) {
@@ -87,6 +103,14 @@ int main(int argc, char** argv) {
     p.max_depth = depth;
     p.accel = accel;
     p.precision = f64 ? RM_FP64 : RM_FP32;
+    if (look) {
+        for (int k = 0; k < 3; k++) view.forward[k] = target[k] - p.camera[k];
+        double basis[9];
+        if ((rc = rm_view_basis(&view, basis)) != RM_OK) {
+            std::fprintf(stderr, "rm_headless: %s\n", rm_last_error());
+            return 2;
+        }
+    }
     const size_t n_px = (size_t)width * height;
     std::vector<unsigned char> rgb8(n_px * 3, 0);
     std::vector<float> rgb32;
@@ -105,7 +129,9 @@ int main(int argc, char** argv) {
     for (int f = 0; f < frames; f++) {
         const auto t0 = std::chrono::steady_clock::now();
         std::memset(&st, 0, sizeof st);
-        if (f64) rc = rm_render_f64(scene, &p, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
+        if (look && f64) rc = rm_render_view_f64(scene, &p, &view, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
+        else if (look) rc = rm_render_view(scene, &p, &view, rgb32.data(), nullptr, nullptr, &st);
+        else if (f64) rc = rm_render_f64(scene, &p, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (rows64) rc = rm_render_rows_f64(scene, &p, row_ptrs.data(), RM_ROWS_RETAINED, &st);
         else rc = rm_render(scene, &p, rgb32.data(), nullptr, nullptr, &st);
         if (rc != RM_OK) die("render", rc);
@@ -124,6 +150,9 @@ int main(int argc, char** argv) {
     } else if (samples > 1) {
         std::memset(&st, 0, sizeof st);
         if ((rc = rm_render_supersampled(scene, &p, samples, nullptr, rgb8.data(), &st)) != RM_OK) die("render (supersampled 8-bit frame)", rc);
+    } else if (look && !f64) {
+        std::memset(&st, 0, sizeof st);
+        if ((rc = rm_render_view(scene, &p, &view, nullptr, nullptr, rgb8.data(), &st)) != RM_OK) die("render (8-bit frame)", rc);
     } else if (!f64) {
         std::memset(&st, 0, sizeof st);
         if ((rc = rm_render(scene, &p, nullptr, nullptr, rgb8.data(), &st)) != RM_OK) die("render (8-bit frame)", rc);

@@ -282,6 +282,48 @@ int rm_render_supersampled(RmScene scene, const RmParams* params, int samples, f
 int rm_render_adaptive(RmScene scene, const RmParams* params, int samples, double contrast, float* out_rgb, uint8_t* out_rgb8,
                        uint8_t* out_mask, RmStats* stats);
 
+/* ---- extension mode: camera orientation -- render from any view direction, not only down -z ------------------------------- *
+ * The reference's camera looks down -z (backproject, renderer.rs:128-135); it has a position and a field of view only.
+ * Definition (normative; the tests' f64 restatement over the oracle is the same):
+ *   Basis, in f64 without fused multiply-add; normalized(a) = a.scale(1 / norm), norm = sqrt(x*x + y*y + z*z)
+ *   (geometry.rs:104-109); cross(a, b) = (a.y*b.z - a.z*b.y, a.z*b.x - a.x*b.z, a.x*b.y - a.y*b.x):
+ *       w = normalized(-forward);   u = normalized(cross(up, w));   v = cross(w, u)
+ *   A view is invalid (RM_ERR_INVALID_ARGUMENT) if a component is not finite, if forward.forward == 0, or if
+ *   |cross(up, w)|^2 <= 1e-20 * (up.up) -- up = 0 or parallel to forward.
+ *   Primary rays: with (dx, dy, dz) the reference's normalised backproject direction of pixel (j, i), the primary ray leaves
+ *   the camera position along
+ *       d = ((u.x*dx + v.x*dy) + w.x*dz,  (u.y*dx + v.y*dy) + w.y*dz,  (u.z*dx + v.z*dy) + w.z*dz)
+ *   without renormalisation.  Everything after the primary ray is the reference's: recursion, shading, lights.
+ *   Identity: a view whose basis is exactly u = (1,0,0), v = (0,1,0), w = (0,0,1) (forward = (0,0,-1), up = (0,1,0) is one)
+ *   is rendered by rm_render's own path: the frame, ids and 8-bit frame equal rm_render's bit for bit.
+ *   Kept on purpose: the reference's triangle and polygon inside test looks at world z only (triangle.rs:13-15), so a turned
+ *   camera still sees only planar primitives whose world normal has z > 0, and cull_backfacing (a world-space criterion) stays
+ *   valid.  The scene is not rotated into camera space: that would change which primitives can be hit.
+ * FP32 production path: K0 writes the raster records rotated by the transposed basis (in f64), stage A runs on them unchanged,
+ * and the world direction of a primary ray (spheres, n-gons, the hierarchy walk, shading) is the FP32 basis applied to the
+ * unit camera-space direction; frames meet the same FP32 parity criteria against the f64 definition as rm_render's.  With
+ * accel = 2 a view call renders as accel = 1 (the hierarchy without its work counters).
+ * Out of scope: views for rm_render_supersampled, rm_render_adaptive, rm_render_dispersive, rm_render_rows_* and
+ * rm_render_frame; projections other than the reference's pinhole; an up vector that turns with the camera. */
+typedef struct RmView {
+    double forward[3];   /* direction the camera looks in (need not be unit length) */
+    double up[3];        /* approximate up; only its component orthogonal to forward matters */
+} RmView;
+/* u, v, w of `view` into out_basis[0..2], [3..5], [6..8], or RM_ERR_INVALID_ARGUMENT.  Needs no GPU. */
+int rm_view_basis(const RmView* view, double out_basis[9]);
+/* rm_render from the camera turned to `view`: the same outputs, rows (patch_row_begin / end / stride), stats semantics and
+ * counter collection (stats->pixels = 1).  RM_FP32.  The call writes the caller's float frame itself, so the library forgets
+ * its previous deliveries into that memory (RM_ROWS_RETAINED).  RM_ERR_INVALID_ARGUMENT: a NULL or invalid view, a precision
+ * other than RM_FP32, and whatever rm_render rejects. */
+int rm_render_view(RmScene scene, const RmParams* params, const RmView* view, float* out_rgb, int32_t* out_prim_id,
+                   uint8_t* out_rgb8, RmStats* stats);
+/* The same with RM_FP64 arithmetic and a double frame (validation mode, like rm_render_f64); params->precision RM_FP64. */
+int rm_render_view_f64(RmScene scene, const RmParams* params, const RmView* view, double* out_rgb, int32_t* out_prim_id,
+                       uint8_t* out_rgb8, RmStats* stats);
+/* rm_render_device from the camera turned to `view` (RM_FP32 or RM_FP64 by params->precision). */
+int rm_render_view_device(RmScene scene, const RmParams* params, const RmView* view, void* d_rgb, int32_t* d_prim_id,
+                          void* d_max, void* stream);
+
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device
  * scalar of the same type as d_rgb that receives max(previous value, tile max) -- zero it first.

@@ -160,6 +160,14 @@ pub struct RmStats {
 
 pub type RmScene = i64;
 
+/// camera orientation of rm_render_view: the basis is w = -forward, u = up x w, v = w x u (all normalised, f64)
+#[repr(C)]
+#[derive(Copy, Clone, Debug)]
+pub struct RmView {
+    pub forward: [f64; 3],
+    pub up: [f64; 3],
+}
+
 /// one frame on the GPUs of one box (one process per GPU)
 #[repr(C)]
 pub struct RmExchange {
@@ -201,6 +209,15 @@ extern "C" {
     /// s x s samples only at the pixels the 3x3 id and contrast test refines, one sample elsewhere
     pub fn rm_render_adaptive(scene: RmScene, params: *const RmParams, samples: c_int, contrast: f64, out_rgb: *mut f32,
                               out_rgb8: *mut u8, out_mask: *mut u8, stats: *mut RmStats) -> c_int;
+    /// u, v, w of a view (no GPU needed)
+    pub fn rm_view_basis(view: *const RmView, out_basis: *mut f64) -> c_int;
+    /// rm_render / rm_render_f64 / rm_render_device from the camera turned to `view`
+    pub fn rm_render_view(scene: RmScene, params: *const RmParams, view: *const RmView, out_rgb: *mut f32,
+                          out_prim_id: *mut i32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
+    pub fn rm_render_view_f64(scene: RmScene, params: *const RmParams, view: *const RmView, out_rgb: *mut f64,
+                              out_prim_id: *mut i32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
+    pub fn rm_render_view_device(scene: RmScene, params: *const RmParams, view: *const RmView, d_rgb: *mut c_void,
+                                 d_prim_id: *mut i32, d_max: *mut c_void, stream: *mut c_void) -> c_int;
     // ---- the hot path, device buffers
     pub fn rm_render_device(scene: RmScene, params: *const RmParams, d_rgb: *mut c_void, d_prim_id: *mut i32,
                             d_max: *mut c_void, stream: *mut c_void) -> c_int;

@@ -74,6 +74,10 @@ class RmStats(C.Structure):
         return {n: int(getattr(self, n)) for n in COUNTER_FIELDS}
 
 
+class RmView(C.Structure):
+    _fields_ = [("forward", d3), ("up", d3)]
+
+
 RM_MAX_RANKS, RM_IPC_HANDLE_BYTES, RM_MAILBOX_BYTES = 16, 64, 512
 
 
@@ -115,6 +119,10 @@ SYMBOLS = {
     "rm_render_dispersive": (C.c_int, [_P(C.c_int64), _P(RmParams), C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_render_supersampled": (C.c_int, [C.c_int64, _P(RmParams), C.c_int, C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_render_adaptive": (C.c_int, [C.c_int64, _P(RmParams), C.c_int, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, _P(RmStats)]),
+    "rm_view_basis": (C.c_int, [_P(RmView), _P(C.c_double)]),
+    "rm_render_view": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), C.c_void_p, C.c_void_p, C.c_void_p, _P(RmStats)]),
+    "rm_render_view_f64": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), C.c_void_p, C.c_void_p, C.c_void_p, _P(RmStats)]),
+    "rm_render_view_device": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rm_scene_query_count": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),
     "rm_scene_accel_status": (C.c_int, [C.c_int64, _P(C.c_int32)]),
     "rm_scene_walk_stats": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),

@@ -455,7 +455,8 @@ int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_p
                        int buf_row0_is_tile, unsigned long long* d_counters, rm::FrameParams<R>* out_fp, int* resident,
                        int* launches = nullptr, unsigned char* d_rgb8_zero = nullptr, bool* scheduled = nullptr,
                        const rm::PeerLink* link = nullptr, unsigned char* d_rgb8_out = nullptr, bool normalise = true,
-                       unsigned char* d_rgb8_next = nullptr, bool as_graph = false, cudaEvent_t ev_after_k0 = nullptr) {
+                       unsigned char* d_rgb8_next = nullptr, bool as_graph = false, cudaEvent_t ev_after_k0 = nullptr,
+                       const rm::ViewBasis* view = nullptr) {
     if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
     int rc = check_params(params);
     if (rc != RM_OK) return rc;
@@ -511,7 +512,7 @@ int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_p
         if (!g.cap_stream) e = cudaStreamCreateWithFlags(&g.cap_stream, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaStreamBeginCapture(g.cap_stream, cudaStreamCaptureModeRelaxed);
         if (e == cudaSuccess) {
-            const cudaError_t el = rm::launch_render<R>(dp.ds, fp, cull, d_rgb, d_prim, d_max, d_counters, g.cap_stream, params->camera, launches, &ex);
+            const cudaError_t el = rm::launch_render<R>(dp.ds, fp, cull, d_rgb, d_prim, d_max, d_counters, g.cap_stream, params->camera, launches, &ex, view);
             e = cudaStreamEndCapture(g.cap_stream, &graph);
             if (el != cudaSuccess) e = el;
         }
@@ -542,7 +543,7 @@ int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_p
             ex.ev_rendered = ev_rendered;
         }
     }
-    if (!launched) CK(rm::launch_render<R>(dp.ds, fp, cull, d_rgb, d_prim, d_max, d_counters, stream, params->camera, launches, &ex));
+    if (!launched) CK(rm::launch_render<R>(dp.ds, fp, cull, d_rgb, d_prim, d_max, d_counters, stream, params->camera, launches, &ex, view));
     se.frames++;
     LastFrame& lf = it->second.last;
     lf.classified = sizeof(R) == 4 && ex.scheduled;
@@ -554,7 +555,8 @@ int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_p
 }
 
 template <typename R>
-int render_host_impl(RmScene scene, const RmParams* params, R* out_rgb, int32_t* out_prim, uint8_t* out_rgb8, RmStats* stats) {
+int render_host_impl(RmScene scene, const RmParams* params, R* out_rgb, int32_t* out_prim, uint8_t* out_rgb8, RmStats* stats,
+                     const rm::ViewBasis* view = nullptr) {
     std::lock_guard<std::mutex> lock(g.mu);
     if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
     int rc = check_params(params);
@@ -580,8 +582,11 @@ int render_host_impl(RmScene scene, const RmParams* params, R* out_rgb, int32_t*
     bool scheduled = false;
     rc = render_device_impl<R>(scene, params, static_cast<R*>(g.rgb.p), out_prim ? static_cast<int*>(g.prim.p) : nullptr,
                                d_max, s, 1, want_counters ? d_cnt : nullptr, &fp, &resident, &launches,
-                               out_rgb8 ? static_cast<unsigned char*>(g.rgb8.p) : nullptr, &scheduled);
+                               out_rgb8 ? static_cast<unsigned char*>(g.rgb8.p) : nullptr, &scheduled, nullptr, nullptr, true, nullptr,
+                               false, nullptr, view);
     if (rc != RM_OK) return rc;
+    // a view call writes the caller's float frame itself: what the library delivered there before no longer holds
+    if (view && out_rgb && rows) forget_deliveries(out_rgb + (size_t)fp.row_begin * fp.width * 3, rows * fp.width * 3 * sizeof(R));
     CK(cudaEventRecord(g.ev[2], s));
     if (out_rgb8 && rows) {
         if (scheduled) {
@@ -1135,6 +1140,51 @@ int rm_render_f64(RmScene scene, const RmParams* params, double* out_rgb, int32_
     return render_host_impl<double>(scene, params, out_rgb, out_prim_id, out_rgb8, stats);
 }
 
+int rm_view_basis(const RmView* view, double out_basis[9]) {
+    if (!view || !out_basis) return fail(RM_ERR_INVALID_ARGUMENT, "view and out_basis must not be null");
+    const char* err = "";
+    const int rc = rm::view_basis(*view, out_basis, &err);
+    return rc == RM_OK ? RM_OK : fail(rc, err);
+}
+
+namespace {
+// The kernels' form of a view (f64 basis and its FP32 rounding).  *identity: the basis is exactly x, y, z -- such a call is
+// rm_render's own (include/rm_b200.h).
+int kernel_view(const RmView* view, rm::ViewBasis& vb, bool* identity) {
+    if (!view) return fail(RM_ERR_INVALID_ARGUMENT, "view is null");
+    const char* err = "";
+    if (rm::view_basis(*view, vb.m, &err) != RM_OK) return fail(RM_ERR_INVALID_ARGUMENT, err);
+    *identity = true;
+    for (int k = 0; k < 9; k++) {
+        vb.f[k] = (float)vb.m[k];
+        *identity = *identity && vb.m[k] == (k % 4 == 0 ? 1. : 0.);
+    }
+    return RM_OK;
+}
+}  // namespace
+
+int rm_render_view(RmScene scene, const RmParams* params, const RmView* view, float* out_rgb, int32_t* out_prim_id, uint8_t* out_rgb8,
+                   RmStats* stats) {
+    if (params && params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_view computes in RM_FP32; use rm_render_view_f64 for RM_FP64");
+    rm::ViewBasis vb;
+    bool identity = false;
+    int rc = kernel_view(view, vb, &identity);
+    if (rc != RM_OK) return rc;
+    if (identity) return rm_render(scene, params, out_rgb, out_prim_id, out_rgb8, stats);
+    return render_host_impl<float>(scene, params, out_rgb, out_prim_id, out_rgb8, stats, &vb);
+}
+
+int rm_render_view_f64(RmScene scene, const RmParams* params, const RmView* view, double* out_rgb, int32_t* out_prim_id,
+                       uint8_t* out_rgb8, RmStats* stats) {
+    if (params && params->precision != RM_FP64) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_view_f64 computes in RM_FP64; use rm_render_view for RM_FP32");
+    rm::ViewBasis vb;
+    bool identity = false;
+    int rc = kernel_view(view, vb, &identity);
+    if (rc != RM_OK) return rc;
+    if (identity) return rm_render_f64(scene, params, out_rgb, out_prim_id, out_rgb8, stats);
+    return render_host_impl<double>(scene, params, out_rgb, out_prim_id, out_rgb8, stats, &vb);
+}
+
 // Extension mode (include/rm_b200.h): three passes of the unchanged render kernels, channel c of pass c kept.  The merge
 // is three pitched device-to-device copies (one float of every pixel: width 4 bytes, pitch 12) -- no kernel of its own.
 int rm_render_dispersive(const RmScene scenes[3], const RmParams* params, float* out_rgb, int32_t* out_prim_id, RmStats* stats) {
@@ -1365,6 +1415,24 @@ int rm_render_device(RmScene scene, const RmParams* params, void* d_rgb, int32_t
                                           static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr);
     return render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max),
                                      static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr);
+}
+
+int rm_render_view_device(RmScene scene, const RmParams* params, const RmView* view, void* d_rgb, int32_t* d_prim_id, void* d_max,
+                          void* stream) {
+    rm::ViewBasis vb;
+    bool identity = false;
+    int rc = kernel_view(view, vb, &identity);
+    if (rc != RM_OK) return rc;
+    if (identity) return rm_render_device(scene, params, d_rgb, d_prim_id, d_max, stream);
+    std::lock_guard<std::mutex> lock(g.mu);
+    if (!d_rgb || !d_max) return fail(RM_ERR_INVALID_ARGUMENT, "d_rgb and d_max must be device pointers");
+    if (params && params->precision == RM_FP64)
+        return render_device_impl<double>(scene, params, static_cast<double*>(d_rgb), d_prim_id, static_cast<double*>(d_max),
+                                          static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                          nullptr, nullptr, true, nullptr, false, nullptr, &vb);
+    return render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max),
+                                     static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                     nullptr, nullptr, true, nullptr, false, nullptr, &vb);
 }
 
 int rm_render_device_rgb8(RmScene scene, const RmParams* params, void* d_rgb, int32_t* d_prim_id, void* d_max, uint8_t* d_rgb8,

@@ -37,13 +37,17 @@ constexpr int kTriSrcDoubles = 16;   // n[3], dn, v0x, v0y, A0, B0, A1, B1, C1, 
 // Camera-specialised record of one triangle (4 x R4<float>), from its FP64 source record.
 //   r0 = {n'x, n'y, -n'z, |K|}   r1 = {G0x, G0y, -G0z, thr^2}   r2 = {G1x, G1y, -G1z, id}   r3 = {G2x, G2y, -G2z, 0}
 // with everything multiplied by sign(K) so that a hit needs dpD > 0 and s_i > 0.
-RM_HD void prepare_raster(const double* __restrict__ src, const double cam[3], R4<float>* __restrict__ out) {
+// Under a view (ViewBasis M) the world direction is M D, and n.(M D) = (M^T n).D, G_i.(M D) = (M^T G_i).D: the records
+// carry M^T n and M^T G_i, the world-space K, thr and edge terms unchanged, and stage A runs on them as it is.
+template <class VW = NoView>
+RM_HD void prepare_raster(const double* __restrict__ src, const double cam[3], R4<float>* __restrict__ out, const VW& vw = VW()) {
     const double nx = src[0], ny = src[1], nz = src[2], dn = src[3];
     const double wx = cam[0] - src[4], wy = cam[1] - src[5];
     const double K = dn - (cam[0] * nx + cam[1] * ny + cam[2] * nz);
     const double A[3] = {src[6], src[8], src[11]}, B[3] = {src[7], src[9], src[12]}, Cc[3] = {0., src[10], 0.};
     const double s = (K < 0.) ? -1. : 1.;
-    out[0] = {(float)(s * nx), (float)(s * ny), (float)(-s * nz), (float)fabs(K)};
+    const Vec3<double> n = vw.to_camera(Vec3<double>{nx, ny, nz});
+    out[0] = {(float)(s * n.x), (float)(s * n.y), (float)(-s * n.z), (float)fabs(K)};
     float last[3] = {(float)(src[13] * src[13]), 0.f, 0.f};    // thr^2: the test runs on squared quantities
     int id = (int)src[14];
 #if defined(__CUDA_ARCH__)
@@ -53,7 +57,12 @@ RM_HD void prepare_raster(const double* __restrict__ src, const double cam[3], R
 #endif
     for (int i = 0; i < 3; i++) {
         const double E = A[i] * wx + B[i] * wy + Cc[i];
-        out[1 + i] = {(float)(s * (E * nx + K * A[i])), (float)(s * (E * ny + K * B[i])), (float)(-s * (E * nz)), last[i]};
+        if constexpr (std::is_same<VW, NoView>::value) {       // (the statement as it was before views: the same code)
+            out[1 + i] = {(float)(s * (E * nx + K * A[i])), (float)(s * (E * ny + K * B[i])), (float)(-s * (E * nz)), last[i]};
+        } else {
+            const Vec3<double> G = vw.to_camera(Vec3<double>{E * nx + K * A[i], E * ny + K * B[i], E * nz});
+            out[1 + i] = {(float)(s * G.x), (float)(s * G.y), (float)(-s * G.z), last[i]};
+        }
     }
 }
 
@@ -502,11 +511,13 @@ RM_HD void primary_tri(PrimaryState<kPx>& ps, const R4<float> r0, const R4<float
 // UNROLLED: as a rolled loop (`#pragma unroll 1`) it had the shape that went wrong in primary_bvh on the B200 -- a trip
 // counter ptxas keeps in a uniform register around per-lane divergent inner loops (here: the per-edge early exits of
 // plane_intersect), see the note at primary_bvh.  Unrolled there is no counter to share.
-template <int kPx, class FV> RM_HD void primary_rest(PrimaryState<kPx>& ps, const FV& fv, const FrameParams<float>& fp) {
+// vw: the camera's orientation (ViewBasis under a view); the rays leave along the world direction vw.apply(D / |D|).
+template <int kPx, class FV, class VW = NoView>
+RM_HD void primary_rest(PrimaryState<kPx>& ps, const FV& fv, const FrameParams<float>& fp, const VW& vw = VW()) {
 #pragma unroll
     for (int r = 0; r < kPx; r++) {
         const float inv = fast_rsqrt(ps.len2[0]);
-        const Vec3<float> d = {ps.X[0] * inv, ps.Y * inv, -inv};
+        const Vec3<float> d = vw.apply(Vec3<float>{ps.X[0] * inv, ps.Y * inv, -inv});
         bool hit = ps.slot[0] >= 0;
         HitRec<float> best;
         best.dist = ps.t[0] * (ps.len2[0] * inv);              // to the unit direction
@@ -546,7 +557,10 @@ template <int kPx, class FV> RM_HD void primary_rest(PrimaryState<kPx>& ps, cons
 // triangle leaf runs primary_tri on the triangle's raster record, a sphere / n-gon leaf the general routine from the
 // camera, and the two partial winners are merged the way primary_rest merges them -- the same arithmetic per (pixel,
 // primitive) and the same (distance, id) order as the brute-force stage A, hence the same t / slot / id, bit for bit.
-template <int kPx, bool kCount> RM_HD void primary_bvh(PrimaryState<kPx>& ps, const FastViewT<true, kCount>& fv, const FrameParams<float>& fp) {
+// (Under a view the walk follows the world direction, and the triangle leaves test the rotated raster records: |M D| = |D|,
+// so their distances in units of |D| stay what they are.)
+template <int kPx, bool kCount, class VW = NoView>
+RM_HD void primary_bvh(PrimaryState<kPx>& ps, const FastViewT<true, kCount>& fv, const FrameParams<float>& fp, const VW& vw = VW()) {
     using FastViewBvh = FastViewT<true, kCount>;
     const bool rest = fv.n_sph + fv.n_poly > 0;
     // One walk per pixel, the loop over the thread's pixels fully unrolled.  As a rolled loop (`#pragma unroll 1`, like
@@ -566,7 +580,7 @@ template <int kPx, bool kCount> RM_HD void primary_bvh(PrimaryState<kPx>& ps, co
         p1.id[0] = -1;
         const float inv = fast_rsqrt(p1.len2[0]);
         const float len = p1.len2[0] * inv;                    // |D|: stage A's triangle distances are in units of it
-        const Vec3<float> d = {p1.X[0] * inv, p1.Y * inv, -inv};
+        const Vec3<float> d = vw.apply(Vec3<float>{p1.X[0] * inv, p1.Y * inv, -inv});
         HitRec<float> other;                                   // closest sphere / n-gon, unit-direction distance
         other.dist = INFINITY;
         other.slot = -1;
@@ -676,9 +690,11 @@ RM_HD Vec3<float> to_f32(const Vec3<double> v) { return {(float)v.x, (float)v.y,
 RM_HD Vec3<float> to_f32(const Vec3<float> v) { return v; }
 
 // renderer.rs:254-309 from the primary hit of pixel (x, y); t1 = FP32 ray parameter of that hit (unit direction).
-template <typename G, class FV>
+// Under a view the primary direction is the camera-space one taken to the world by vw: in f64 from the f64 basis (the
+// normative definition of include/rm_b200.h), in FP32 from its FP32 rounding.
+template <typename G, class FV, class VW = NoView>
 RM_HD Vec3<float> cast_glass_impl(const FV& fv, const FrameParams<float>& fp, const int x, const int y, const float t1,
-                                  const int slot1, const int id1) {
+                                  const int slot1, const int id1, const VW& vw = VW()) {
     struct Frame {
         Vec3<float> c;
         Vec3<G> ro, rd;
@@ -691,13 +707,13 @@ RM_HD Vec3<float> cast_glass_impl(const FV& fv, const FrameParams<float>& fp, co
     Vec3<G> o, d;
     if constexpr (sizeof(G) == 8) {                             // renderer.rs:128-135 in the reference's own arithmetic
         o = {fp.cam64[0], fp.cam64[1], fp.cam64[2]};
-        d = Fast64::normalized(Vec3<double>{2. * ((double)x * fp.inv_w64 - 0.5) * fp.hf64 * fp.ratio64,
-                                            -2. * ((double)y * fp.inv_h64 - 0.5) * fp.hf64, -1.});
+        d = vw.apply(Fast64::normalized(Vec3<double>{2. * ((double)x * fp.inv_w64 - 0.5) * fp.hf64 * fp.ratio64,
+                                                     -2. * ((double)y * fp.inv_h64 - 0.5) * fp.hf64, -1.}));
     } else {
         const float X = pixel_X(fp, x), Y = pixel_Y(fp, y);
         const float inv = fast_rsqrt(fmaf(X, X, fmaf(Y, Y, 1.f)));     // geometry.rs:104-109: scale(1/norm)
         o = fp.camera;
-        d = {X * inv, Y * inv, -inv};
+        d = vw.apply(Vec3<float>{X * inv, Y * inv, -inv});
     }
     Counters<false> st;
     Vec3<float> v;
@@ -785,18 +801,18 @@ RM_HD Vec3<float> cast_glass_impl(const FV& fv, const FrameParams<float>& fp, co
         }
     }
 }
-template <class FV>
+template <class FV, class VW = NoView>
 RM_GLASS_FN Vec3<float> cast_glass64(const FV& fv, const FrameParams<float>& fp, const int x, const int y, const float t1,
-                                     const int slot1, const int id1) {
-    return cast_glass_impl<double, FV>(fv, fp, x, y, t1, slot1, id1);
+                                     const int slot1, const int id1, const VW& vw = VW()) {
+    return cast_glass_impl<double, FV, VW>(fv, fp, x, y, t1, slot1, id1, vw);
 }
 
 // One pixel whose primary ray hit (t in units of |D|, slot, id): renderer.rs:254-309 from level 1.
 // kGlass = GLASS_NONE: the scene has neither glass-like materials nor spheres (every OBJ scene of the reference: obj.rs:125-138
 // loads meshes opaque) -- the kernel instantiated for it carries no recursion, no f64 code and fewer registers.
-template <int kGlass = GLASS_F64, class FV>
+template <int kGlass = GLASS_F64, class FV, class VW = NoView>
 RM_HD Vec3<float> fast_shade(FV& fv, const FrameParams<float>& fp, const int x, const int y, const float t, const int slot,
-                             const int id) {
+                             const int id, const VW& vw = VW()) {
     const float X = pixel_X(fp, x), Y = pixel_Y(fp, y);
     const float len2 = fmaf(X, X, fmaf(Y, Y, 1.f));
     const float inv = fast_rsqrt(len2);                            // geometry.rs:104-109: scale(1/norm)
@@ -805,9 +821,9 @@ RM_HD Vec3<float> fast_shade(FV& fv, const FrameParams<float>& fp, const int x, 
     // warp's 32 queue entries mix glass-like and opaque hits, and two routines would run the expensive part of both --
     // the shadow rays of direct() -- one after the other for the two groups of lanes (measured on the demo frame: 170
     // instead of 156 us).
-    if constexpr (kGlass == GLASS_F64) return cast_glass64(fv, fp, x, y, dist, slot, id);
-    if constexpr (kGlass == GLASS_F32) return cast_glass_impl<float, FV>(fv, fp, x, y, dist, slot, id);
-    const Vec3<float> d = {X * inv, Y * inv, -inv};
+    if constexpr (kGlass == GLASS_F64) return cast_glass64(fv, fp, x, y, dist, slot, id, vw);
+    if constexpr (kGlass == GLASS_F32) return cast_glass_impl<float, FV, VW>(fv, fp, x, y, dist, slot, id, vw);
+    const Vec3<float> d = vw.apply(Vec3<float>{X * inv, Y * inv, -inv});
     HitRec<float> h;
     h.dist = dist;
     h.slot = slot;

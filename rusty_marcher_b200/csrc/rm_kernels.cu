@@ -162,11 +162,13 @@ template <> struct Tone<double> {
     }
 };
 
-template <typename R, bool S>
+// kView (rm_render_view): the primary ray leaves along view.apply(backproject(x, y)) -- the basis in f64 for R = double,
+// its FP32 rounding for R = float.  `view` is the last argument so that the instantiations without it keep their code.
+template <typename R, bool S, bool kView = false>
 __global__ void __launch_bounds__(kBlock)
 render_kernel(const DeviceScene<R> ds, const FrameParams<R> fp, const int cull, const int use_smem,
               R* __restrict__ rgb, int* __restrict__ prim_id, R* __restrict__ dmax,
-              unsigned long long* __restrict__ counters) {
+              unsigned long long* __restrict__ counters, const ViewBasis view) {
     extern __shared__ __align__(32) unsigned char smem_raw[];
     __shared__ R warp_max[kBlock / 32];
 
@@ -192,7 +194,7 @@ render_kernel(const DeviceScene<R> ds, const FrameParams<R> fp, const int cull, 
     if (x < fp.width && yl < fp.n_bands * 32) {
         st.add(C_PIXELS);
         int pid;
-        const Vec3<R> dir = backproject<R>(fp, x, y);
+        const Vec3<R> dir = typename ViewOf<kView>::type(view).apply(backproject<R>(fp, x, y));
         const Vec3<R> c = cast_ray<R, S, SceneView<R>>(sc, fp.camera, dir, fp.background, fp.max_depth, pid, st);
         const size_t px = (size_t)(y - fp.buf_row0) * fp.width + x;
         rgb[3 * px] = c.x;
@@ -221,17 +223,19 @@ render_kernel(const DeviceScene<R> ds, const FrameParams<R> fp, const int cull, 
     }
 }
 
-// K0: camera-specialised raster records of every fast-path triangle, in FP64, once per frame.
+// K0: camera-specialised raster records of every fast-path triangle, in FP64, once per frame.  kView: rotated into the
+// camera's basis (prepare_raster).
+template <bool kView = false>
 __global__ void __launch_bounds__(128)
 prepare_raster_kernel(const double* __restrict__ tri_src, const int n_tri, const double cx, const double cy, const double cz,
-                      R4<float>* __restrict__ tri_r, float* __restrict__ dmax_zero) {
+                      R4<float>* __restrict__ tri_r, float* __restrict__ dmax_zero, const ViewBasis view) {
     pdl_launch_dependents();
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j == 0 && dmax_zero) *dmax_zero = 0.f;
     if (j >= n_tri) return;
     const double cam[3] = {cx, cy, cz};
     R4<float> out[4];
-    prepare_raster(tri_src + (size_t)j * kTriSrcDoubles, cam, out);
+    prepare_raster(tri_src + (size_t)j * kTriSrcDoubles, cam, out, typename ViewOf<kView>::type(view));
 #pragma unroll
     for (int k = 0; k < 4; k++) tri_r[4 * j + k] = out[k];
 }
@@ -246,10 +250,13 @@ prepare_raster_kernel(const double* __restrict__ tri_src, const int n_tri, const
 // overlaps K1's launch thanks to the programmatic dependent launch.  No gain; not kept.)
 constexpr int kClassifyMaxTris = 256;
 constexpr int kClassifyBlock = 512, kClassifyLanes = 8;         // 8 lanes per tile: 64 tiles per block
+// (kView: the rotated records; the tile bounds are exact on them as they are, see rect_max)
+template <bool kView = false>
 __global__ void __launch_bounds__(kClassifyBlock)
 prepare_classify_kernel(const double* __restrict__ tri_src, const int n_tri, const double cx, const double cy, const double cz,
                         R4<float>* __restrict__ tri_r, const FrameParams<float> fp, const int tiles_x, const int n_tiles,
-                        int* __restrict__ order, int* __restrict__ order2, int* __restrict__ ctr, float* __restrict__ dmax_zero) {
+                        int* __restrict__ order, int* __restrict__ order2, int* __restrict__ ctr, float* __restrict__ dmax_zero,
+                        const ViewBasis view) {
     __shared__ R4<float> rec[4 * kClassifyMaxTris];
     __shared__ int cnt[3], base[3];
     const double cam[3] = {cx, cy, cz};
@@ -263,7 +270,7 @@ prepare_classify_kernel(const double* __restrict__ tri_src, const int n_tri, con
     if (threadIdx.x < 3) cnt[threadIdx.x] = 0;
     for (int j = threadIdx.x; j < n_tri; j += blockDim.x) {      // every block rebuilds the (few) records; block 0 publishes them
         R4<float> out[4];
-        prepare_raster(tri_src + (size_t)j * kTriSrcDoubles, cam, out);
+        prepare_raster(tri_src + (size_t)j * kTriSrcDoubles, cam, out, typename ViewOf<kView>::type(view));
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             rec[4 * j + k] = out[k];
@@ -352,14 +359,18 @@ constexpr int kWarpQueue = kFastTile * 4 + 32;                  // one strip of 
 template <int kPx> struct PxTag { static constexpr int value = kPx; };
 // kBvh (RmParams.accel): scene queries walk the hierarchy of rm_bvh.cuh (read through the read-only path; the nodes near
 // the root stay in L1) instead of every primitive; stage A then handles a thread's pixels one after the other.
-template <bool kSmem, int kBvhMode, int kGlass>
+// kView (rm_render_view): K0 wrote raster records rotated into the camera's basis `view` (the last argument, so that the
+// instantiations without it keep their code); stage A runs on them unchanged, and the world directions of the primary
+// rays -- spheres, n-gons, the hierarchy walk, shading -- are view.apply(D / |D|).
+template <bool kSmem, int kBvhMode, int kGlass, bool kView = false>
 __global__ void RM_K1_BOUNDS
 render_fast_kernel(const DeviceScene<float> ds, const FrameParams<float> fp, const int cull, const int tiles_x,
                    const int n_tiles, const float inv_tiles_x, float* __restrict__ rgb, int* __restrict__ prim_id,
                    float* __restrict__ dmax, int* __restrict__ ctr, const int* __restrict__ order, const int* __restrict__ order2,
                    unsigned char* rgb8, const PeerLink link, unsigned char* rgb8_out, const int normalise,
-                   unsigned char* rgb8_next, const int stage_mat) {
+                   unsigned char* rgb8_next, const int stage_mat, const ViewBasis view) {
     constexpr bool kBvh = kBvhMode != 0, kCount = kBvhMode == 2;    // 2: the counting instantiation (RmParams.accel = 2)
+    const typename ViewOf<kView>::type vw(view);
     const int zero_foreign = rgb8_next != nullptr;
     extern __shared__ __align__(32) unsigned char smem_raw[];
     __shared__ int cta_max;
@@ -450,7 +461,7 @@ render_fast_kernel(const DeviceScene<float> ds, const FrameParams<float> fp, con
     auto shade_entry = [&](const float4 e) {
         const unsigned xy = __float_as_uint(e.w);
         const int x = (int)(xy & 0xffffu), y = (int)(xy >> 16);
-        const Vec3<float> c = fast_shade<kGlass>(fv, fp, x, y, e.x, __float_as_int(e.y), __float_as_int(e.z));
+        const Vec3<float> c = fast_shade<kGlass>(fv, fp, x, y, e.x, __float_as_int(e.y), __float_as_int(e.z), vw);
         RM_CHECK(x >= 0 && x < fp.width && y >= fp.row_begin && y < fp.row_begin + (fp.n_bands - 1) * fp.row_step + 32 &&
                  (y - fp.row_begin) % fp.row_step < 32);
         float* dst = rgb + 3 * ((size_t)(y - fp.buf_row0) * fp.width + x);
@@ -531,7 +542,7 @@ render_fast_kernel(const DeviceScene<float> ds, const FrameParams<float> fp, con
                 PrimaryState<kPx> ps;
                 primary_begin<kPx>(ps, fp, x0 + lx, ys + ly);
                 if constexpr (kBvh) {
-                    primary_bvh<kPx, kCount>(ps, fv, fp);
+                    primary_bvh<kPx, kCount>(ps, fv, fp, vw);
                 } else {
                     // the strip: pixels [x0, x0 + 31] x [ys, ys + 3]
                     const float Xa = pixel_X(fp, x0), Xb = pixel_X(fp, x0 + kFastTile - 1);
@@ -547,7 +558,7 @@ render_fast_kernel(const DeviceScene<float> ds, const FrameParams<float> fp, con
                             primary_tri<kPx>(ps, tri_r[4 * jj], tri_r[4 * jj + 1], tri_r[4 * jj + 2], tri_r[4 * jj + 3], fv.n_sph + jj);
                         }
                     }
-                    if (rest) primary_rest<kPx>(ps, fv, fp);
+                    if (rest) primary_rest<kPx>(ps, fv, fp, vw);
                 }
                 if (prim_id) {
                     if (kPx == 4) __stcs(reinterpret_cast<int4*>(prim_id + px), make_int4(ps.id[0], ps.id[1], ps.id[kPx - 2], ps.id[kPx - 1]));
@@ -1203,7 +1214,9 @@ __global__ void __launch_bounds__(256) ffma_probe_kernel(float* __restrict__ sin
 
 namespace {
 cudaError_t launch_fast(const DeviceScene<float>& ds, const FrameParams<float>& fp, bool cull, float* rgb, int* prim_id,
-                        float* dmax, cudaStream_t stream, const double camera[3], int* launches, RenderExtras* ex) {
+                        float* dmax, cudaStream_t stream, const double camera[3], int* launches, RenderExtras* ex,
+                        const ViewBasis* view) {
+    const ViewBasis vb = view ? *view : ViewBasis{};
     unsigned char* rgb8 = ex ? ex->rgb8_zero : nullptr;
     if (ex && ex->ev_begin) cudaEventRecord(ex->ev_begin, stream);
     const int n_tri = tri_count(ds.lay, cull);
@@ -1211,12 +1224,14 @@ cudaError_t launch_fast(const DeviceScene<float>& ds, const FrameParams<float>& 
     const bool bvh = fp.accel != 0 && ds.bvh.n_nodes > 0 && ds.lay.n_lgt <= kBvhMaxLights;
     const bool classify = !bvh && ds.lay.n_sph + poly_count(ds.lay, cull) == 0 && n_tri <= kClassifyMaxTris && n_tiles <= ds.tile_order_cap / 2;
     if (classify)
-        prepare_classify_kernel<<<(n_tiles * kClassifyLanes + kClassifyBlock - 1) / kClassifyBlock, kClassifyBlock, 0, stream>>>(ds.tri_src, n_tri, camera[0], camera[1], camera[2], ds.tri_r,
+        (view ? prepare_classify_kernel<true> : prepare_classify_kernel<false>)
+            <<<(n_tiles * kClassifyLanes + kClassifyBlock - 1) / kClassifyBlock, kClassifyBlock, 0, stream>>>(ds.tri_src, n_tri, camera[0], camera[1], camera[2], ds.tri_r,
                                                                          fp, tiles_x, n_tiles, ds.tile_order, ds.tile_order + ds.tile_order_cap / 2, ds.ctr,
-                                                                         ex && ex->zero_dmax ? dmax : nullptr);
+                                                                         ex && ex->zero_dmax ? dmax : nullptr, vb);
     else
-        prepare_raster_kernel<<<(std::max(n_tri, 1) + 127) / 128, 128, 0, stream>>>(ds.tri_src, n_tri, camera[0], camera[1], camera[2], ds.tri_r,
-                                                                                     ex && ex->zero_dmax ? dmax : nullptr);
+        (view ? prepare_raster_kernel<true> : prepare_raster_kernel<false>)
+            <<<(std::max(n_tri, 1) + 127) / 128, 128, 0, stream>>>(ds.tri_src, n_tri, camera[0], camera[1], camera[2], ds.tri_r,
+                                                                    ex && ex->zero_dmax ? dmax : nullptr, vb);
     const PeerLink link = ex ? ex->link : PeerLink();
     const int* order = classify ? ds.tile_order : nullptr;
     if (ex) ex->scheduled = classify;
@@ -1242,6 +1257,9 @@ cudaError_t launch_fast(const DeviceScene<float>& ds, const FrameParams<float>& 
         if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_NONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
         if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
         if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_F64>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_NONE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_F32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_F64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
         if ((e = cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
     }
     const size_t smem_geo = (size_t)ds.lay.bytes + (size_t)ds.lay.n_tri * 64;
@@ -1287,19 +1305,24 @@ cudaError_t launch_fast(const DeviceScene<float>& ds, const FrameParams<float>& 
         {render_fast_kernel<false, 0, GLASS_NONE>, render_fast_kernel<false, 0, GLASS_F32>, render_fast_kernel<false, 0, GLASS_F64>},
         {render_fast_kernel<false, 1, GLASS_NONE>, render_fast_kernel<false, 1, GLASS_F32>, render_fast_kernel<false, 1, GLASS_F64>},
         {render_fast_kernel<false, 2, GLASS_NONE>, render_fast_kernel<false, 2, GLASS_F32>, render_fast_kernel<false, 2, GLASS_F64>}};
-    const K1 k = table[bvh ? (fp.accel == 2 ? 3 : 2) : use_smem ? 0 : 1][glass];
+    // under a view: no counting instantiation (accel = 2 renders as accel = 1)
+    static const K1 view_table[3][3] = {
+        {render_fast_kernel<true, 0, GLASS_NONE, true>, render_fast_kernel<true, 0, GLASS_F32, true>, render_fast_kernel<true, 0, GLASS_F64, true>},
+        {render_fast_kernel<false, 0, GLASS_NONE, true>, render_fast_kernel<false, 0, GLASS_F32, true>, render_fast_kernel<false, 0, GLASS_F64, true>},
+        {render_fast_kernel<false, 1, GLASS_NONE, true>, render_fast_kernel<false, 1, GLASS_F32, true>, render_fast_kernel<false, 1, GLASS_F64, true>}};
+    const K1 k = view ? view_table[bvh ? 2 : use_smem ? 0 : 1][glass] : table[bvh ? (fp.accel == 2 ? 3 : 2) : use_smem ? 0 : 1][glass];
     cfg.dynamicSmemBytes = use_smem ? smem : 0;
     int occ = 1;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, kFastBlock, cfg.dynamicSmemBytes)) != cudaSuccess) return e;
     cfg.gridDim = dim3(std::min(n_tiles, sm_count * std::max(occ, 1)));
     e = cudaLaunchKernelEx(&cfg, k, ds, fp, cull_i, tiles_x, n_tiles, inv_tiles_x, rgb, prim_id, dmax, ds.ctr, order, order2, rgb8,
-                           link, rgb8_out, normalise, rgb8_next, stage_mat);
+                           link, rgb8_out, normalise, rgb8_next, stage_mat, vb);
     if (e != cudaSuccess && want_coop) {                        // not available in this combination: the plain persistent launch
         cudaGetLastError();
         coop = 0;
         cfg.numAttrs = 1;
         e = cudaLaunchKernelEx(&cfg, k, ds, fp, cull_i, tiles_x, n_tiles, inv_tiles_x, rgb, prim_id, dmax, ds.ctr, order, order2, rgb8,
-                               link, rgb8_out, normalise, rgb8_next, stage_mat);
+                               link, rgb8_out, normalise, rgb8_next, stage_mat, vb);
     }
     if (e != cudaSuccess) return e;
     if (launches) (*launches)++;
@@ -1307,13 +1330,13 @@ cudaError_t launch_fast(const DeviceScene<float>& ds, const FrameParams<float>& 
     return cudaGetLastError();
 }
 cudaError_t launch_fast(const DeviceScene<double>&, const FrameParams<double>&, bool, double*, int*, double*, cudaStream_t,
-                        const double*, int*, RenderExtras*) { return cudaErrorInvalidValue; }
+                        const double*, int*, RenderExtras*, const ViewBasis*) { return cudaErrorInvalidValue; }
 }  // namespace
 
 template <typename R>
 cudaError_t launch_render(const DeviceScene<R>& ds, const FrameParams<R>& fp, bool cull, R* rgb, int* prim_id, R* dmax,
                           unsigned long long* counters, cudaStream_t stream, const double camera[3], int* launches,
-                          RenderExtras* ex) {
+                          RenderExtras* ex, const ViewBasis* view) {
     const int rows = fp.n_bands * 32;
     if (ex) ex->scheduled = false;
     if (rows <= 0 || fp.width <= 0) {                           // nothing to render: the profiling events still mark the (empty) frame
@@ -1325,22 +1348,17 @@ cudaError_t launch_render(const DeviceScene<R>& ds, const FrameParams<R>& fp, bo
     const dim3 grid((fp.width + kTileW - 1) / kTileW, (rows + kTileH - 1) / kTileH);
     // (a depth cap of 0 makes every pixel the background, hit or not -- renderer.rs:262-264 with n_recursion = 1: the generic
     // kernel follows cast_ray literally, the production kernel assumes at least the primary level)
-    if (sizeof(R) == 4 && !counters && camera && ds.tri_r && fp.max_depth >= 1) return launch_fast(ds, fp, cull, rgb, prim_id, dmax, stream, camera, launches, ex);
+    if (sizeof(R) == 4 && !counters && camera && ds.tri_r && fp.max_depth >= 1) return launch_fast(ds, fp, cull, rgb, prim_id, dmax, stream, camera, launches, ex, view);
     if (ex && ex->ev_begin) cudaEventRecord(ex->ev_begin, stream);
     if (ex && ex->ev_prepared) cudaEventRecord(ex->ev_prepared, stream);
     if (launches) (*launches)++;
     const int use_smem = ds.lay.bytes <= kSmemLimit;
     const size_t smem = use_smem ? (size_t)ds.lay.bytes : 0;
     cudaError_t e;
-    if (counters) {
-        auto k = render_kernel<R, true>;
-        if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
-        k<<<grid, kBlock, smem, stream>>>(ds, fp, cull ? 1 : 0, use_smem, rgb, prim_id, dmax, counters);
-    } else {
-        auto k = render_kernel<R, false>;
-        if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
-        k<<<grid, kBlock, smem, stream>>>(ds, fp, cull ? 1 : 0, use_smem, rgb, prim_id, dmax, nullptr);
-    }
+    const ViewBasis vb = view ? *view : ViewBasis{};
+    auto k = counters ? (view ? render_kernel<R, true, true> : render_kernel<R, true>) : (view ? render_kernel<R, false, true> : render_kernel<R, false>);
+    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+    k<<<grid, kBlock, smem, stream>>>(ds, fp, cull ? 1 : 0, use_smem, rgb, prim_id, dmax, counters, vb);
     if (ex && ex->ev_rendered) cudaEventRecord(ex->ev_rendered, stream);
     return cudaGetLastError();
 }
@@ -1495,8 +1513,8 @@ cudaError_t launch_ffma_probe(float* sink, int iters, int blocks, cudaStream_t s
     return cudaGetLastError();
 }
 
-template cudaError_t launch_render<float>(const DeviceScene<float>&, const FrameParams<float>&, bool, float*, int*, float*, unsigned long long*, cudaStream_t, const double*, int*, RenderExtras*);
-template cudaError_t launch_render<double>(const DeviceScene<double>&, const FrameParams<double>&, bool, double*, int*, double*, unsigned long long*, cudaStream_t, const double*, int*, RenderExtras*);
+template cudaError_t launch_render<float>(const DeviceScene<float>&, const FrameParams<float>&, bool, float*, int*, float*, unsigned long long*, cudaStream_t, const double*, int*, RenderExtras*, const ViewBasis*);
+template cudaError_t launch_render<double>(const DeviceScene<double>&, const FrameParams<double>&, bool, double*, int*, double*, unsigned long long*, cudaStream_t, const double*, int*, RenderExtras*, const ViewBasis*);
 template cudaError_t launch_tonemap<float>(const FrameParams<float>&, const float*, const float*, bool, unsigned char*, cudaStream_t);
 template cudaError_t launch_tonemap<double>(const FrameParams<double>&, const double*, const double*, bool, unsigned char*, cudaStream_t);
 

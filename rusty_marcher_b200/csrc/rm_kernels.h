@@ -80,10 +80,12 @@ struct RenderExtras {
 // (one thread per triangle, FP64) followed by render_fast_kernel; otherwise the generic kernel.
 // K1: render rows [fp.row_begin, fp.row_end).  rgb: H*W*3 of R; prim_id optional; dmax: scalar R that
 // receives max(old, tile max); counters: 17 x u64 (instrumented kernel) or null (production kernel).
+// view: the camera's orientation (rm_render_view), or null for the reference's camera looking down -z.  Under a view the
+// hierarchy kernel that counts its work (accel = 2) is not instantiated: accel = 2 renders as accel = 1.
 template <typename R>
 cudaError_t launch_render(const DeviceScene<R>& ds, const FrameParams<R>& fp, bool cull, R* rgb, int* prim_id, R* dmax,
                           unsigned long long* counters, cudaStream_t stream, const double camera[3] = nullptr,
-                          int* launches = nullptr, RenderExtras* extras = nullptr);
+                          int* launches = nullptr, RenderExtras* extras = nullptr, const ViewBasis* view = nullptr);
 
 // K4: FrameBuffer::normalize + to_vec (framebuffer.rs:40-82) over rows [fp.row_begin, fp.row_end).
 template <typename R>

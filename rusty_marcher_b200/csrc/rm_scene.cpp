@@ -535,4 +535,40 @@ template <typename R> FrameParams<R> make_frame_params(const RmParams& p) {
 template FrameParams<float> make_frame_params<float>(const RmParams&);
 template FrameParams<double> make_frame_params<double>(const RmParams&);
 
+// The normative construction of include/rm_b200.h (RmView), in f64 without contraction (-ffp-contract=off / -fmad=false):
+// geometry.rs's normalized is scale(1 / norm), norm = sqrt(x*x + y*y + z*z), and cross is geometry.rs:57-63.
+int view_basis(const RmView& view, double out[9], const char** err) {
+    const double* f = view.forward;
+    const double* up = view.up;
+    for (int a = 0; a < 3; a++)
+        if (!std::isfinite(f[a]) || !std::isfinite(up[a])) {
+            *err = "view: forward and up must be finite";
+            return RM_ERR_INVALID_ARGUMENT;
+        }
+    const double ff = f[0] * f[0] + f[1] * f[1] + f[2] * f[2];
+    if (ff == 0.) {
+        *err = "view: forward is the zero vector";
+        return RM_ERR_INVALID_ARGUMENT;
+    }
+    auto normalized = [](const double x, const double y, const double z, double* o) {
+        const double s = 1. / std::sqrt(x * x + y * y + z * z);
+        o[0] = x * s; o[1] = y * s; o[2] = z * s;
+    };
+    double* u = out;
+    double* v = out + 3;
+    double* w = out + 6;
+    normalized(-f[0], -f[1], -f[2], w);
+    const double cx = up[1] * w[2] - up[2] * w[1], cy = up[2] * w[0] - up[0] * w[2], cz = up[0] * w[1] - up[1] * w[0];
+    const double uu = up[0] * up[0] + up[1] * up[1] + up[2] * up[2];
+    if (cx * cx + cy * cy + cz * cz <= 1e-20 * uu) {
+        *err = "view: up is zero or parallel to forward";
+        return RM_ERR_INVALID_ARGUMENT;
+    }
+    normalized(cx, cy, cz, u);
+    v[0] = w[1] * u[2] - w[2] * u[1];
+    v[1] = w[2] * u[0] - w[0] * u[2];
+    v[2] = w[0] * u[1] - w[1] * u[0];
+    return RM_OK;
+}
+
 }  // namespace rm

@@ -117,4 +117,7 @@ int validate_scene(const RmFlatScene& fs, std::string& err);
 
 template <typename R> FrameParams<R> make_frame_params(const RmParams& p);
 
+// rm_view_basis (include/rm_b200.h): u, v, w of the view into out[0..8], or RM_ERR_INVALID_ARGUMENT with a reason in err.
+int view_basis(const RmView& view, double out[9], const char** err);
+
 }  // namespace rm

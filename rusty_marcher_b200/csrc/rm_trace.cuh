@@ -515,4 +515,35 @@ template <> RM_HD Vec3<double> backproject<double>(const FrameParams<double>& fp
     return normalized(v);
 }
 
+// Camera orientation (rm_render_view, include/rm_b200.h).  The orthonormal basis u, v, w (m[0..2], m[3..5], m[6..8]) takes
+// a camera-space direction d to the world direction ((u.x d.x + v.x d.y) + w.x d.z, ...); to_camera is the transpose,
+// (u.g, v.g, w.g), which K0 applies to the raster records so that stage A keeps its camera-space D = (X, Y, -1).
+// f: the basis rounded to FP32, for the production kernel's FP32 directions.
+struct ViewBasis {
+    double m[9];
+    float f[9];
+    RM_HD Vec3<double> apply(const Vec3<double> d) const {
+        return {(m[0] * d.x + m[3] * d.y) + m[6] * d.z, (m[1] * d.x + m[4] * d.y) + m[7] * d.z,
+                (m[2] * d.x + m[5] * d.y) + m[8] * d.z};
+    }
+    RM_HD Vec3<float> apply(const Vec3<float> d) const {
+        return {fmaf(f[6], d.z, fmaf(f[3], d.y, f[0] * d.x)), fmaf(f[7], d.z, fmaf(f[4], d.y, f[1] * d.x)),
+                fmaf(f[8], d.z, fmaf(f[5], d.y, f[2] * d.x))};
+    }
+    RM_HD Vec3<double> to_camera(const Vec3<double> g) const {
+        return {(m[0] * g.x + m[1] * g.y) + m[2] * g.z, (m[3] * g.x + m[4] * g.y) + m[5] * g.z,
+                (m[6] * g.x + m[7] * g.y) + m[8] * g.z};
+    }
+};
+// The reference's camera (u, v, w = x, y, z): every pre-existing kernel instantiates its code with this, which compiles
+// to exactly the code it had before the view existed.
+struct NoView {
+    NoView() = default;
+    RM_HD explicit NoView(const ViewBasis&) {}
+    template <typename R> RM_HD Vec3<R> apply(const Vec3<R> d) const { return d; }
+    RM_HD Vec3<double> to_camera(const Vec3<double> g) const { return g; }
+};
+template <bool kView> struct ViewOf { typedef NoView type; };
+template <> struct ViewOf<true> { typedef ViewBasis type; };
+
 }  // namespace rm

@@ -217,6 +217,70 @@ class Renderer:
         print(message)
         return message
 
+    def render_view(self, frame, scene, forward, up=(0., 1., 0.), prim_id=None, rgb8=None, patch_rows=(0, -1)):
+        """EXTENSION MODE (no reference counterpart): render() from the camera turned to look along `forward`, with `up`
+        (only its component orthogonal to forward matters) towards the top of the frame -- rm_render_view, or
+        rm_render_view_f64 with precision RM_FP64.  The basis is view_basis(forward, up); forward = (0, 0, -1) with up =
+        (0, 1, 0) is render()'s camera and frame.  Honours precision and accel like render(); fills frame.buffer (float32,
+        float64 for RM_FP64) over the rendered rows and the optional prim_id / rgb8 arrays, and returns the same kind of
+        status message.  Raises ValueError for an invalid view (see view_basis)."""
+        if int(self.width) != frame.width or int(self.height) != frame.height:
+            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
+        for name, a, dtype, shape in (("prim_id", prim_id, np.int32, (frame.height, frame.width)),
+                                      ("rgb8", rgb8, np.uint8, (frame.height, frame.width, 3))):
+            if a is not None and (not isinstance(a, np.ndarray) or a.dtype != dtype or a.shape != shape or not a.flags.c_contiguous
+                                  or not a.flags.writeable):
+                raise ValueError("%s must be a writeable C-contiguous %s array of shape %s" % (name, np.dtype(dtype).name, shape))
+        view = _view(forward, up)
+        view_basis(forward, up)                                 # ValueError for an invalid view, before any GPU work
+        L = _abi.load()
+        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
+        now = time.perf_counter()
+        p = self.params(frame, scene, patch_rows)
+        want64 = self.precision == _abi.RM_FP64
+        want_dtype = np.float64 if want64 else np.float32
+        if frame.buffer.dtype != want_dtype or not frame.buffer.flags.c_contiguous:
+            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=want_dtype)
+        stats = _abi.RmStats()
+        fn = L.rm_render_view_f64 if want64 else L.rm_render_view
+        _abi.check(fn(scene.device_handle(), C.byref(p), C.byref(view), frame.buffer.ctypes.data,
+                      prim_id.ctypes.data if prim_id is not None else None,
+                      rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
+        self.last_stats = stats
+        ms = int((time.perf_counter() - now) * 1000)
+        fps = 1000. / ms if ms > 0 else float("inf")
+        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
+        print(message)
+        return message
+
+
+def _view(forward, up):
+    fwd, u = [float(x) for x in forward], [float(x) for x in up]
+    if len(fwd) != 3 or len(u) != 3:
+        raise ValueError("forward and up must have three components")
+    v = _abi.RmView()
+    v.forward[:] = fwd
+    v.up[:] = u
+    return v
+
+
+def view_basis(forward, up=(0., 1., 0.)):
+    """The camera basis of a view (rm_view_basis, include/rm_b200.h): a (3, 3) float64 array whose rows are u (right), v
+    (up) and w (= -forward, normalised).  Raises ValueError for an invalid view: a component that is not finite, forward
+    = 0, or up zero or parallel to forward.  Needs no GPU."""
+    view = _view(forward, up)
+    out = np.zeros((3, 3), dtype=np.float64)
+    L = _abi.load()
+    rc = L.rm_view_basis(C.byref(view), out.ctypes.data_as(C.POINTER(C.c_double)))
+    if rc != _abi.RM_OK:
+        raise ValueError(L.rm_last_error().decode("utf-8", "replace"))
+    return out
+
+
+def look_at(eye, target):
+    """The `forward` of a camera at `eye` that looks at the point `target`: target - eye."""
+    return tuple(float(t) - float(e) for e, t in zip(Vec3f.of(eye), Vec3f.of(target)))
+
 
 def create_renderer(fov, height, width):
     return Renderer(fov, height, width)
