@@ -450,13 +450,28 @@ void fill_counters(RmStats* st, const unsigned long long* c) {
     for (int i = 0; i < rm::C_COUNT; i++) dst[i] = c[i];
 }
 
+// What a render_device_impl call asks for beyond the frame itself.  The defaults: K0 + K1 into rows indexed from frame
+// row 0, nothing reported back.
+template <typename R> struct RenderOptions {
+    bool buf_row0_is_tile = false;                  // rgb / prim rows indexed from the call's first row (buf_row0)
+    unsigned long long* counters = nullptr;         // the instrumented generic kernel's counters
+    rm::FrameParams<R>* out_fp = nullptr;           // out: the call's frame parameters
+    int* resident = nullptr;                        // out: RmStats::resident_prims
+    int* launches = nullptr;                        // incremented per kernel launch
+    unsigned char* rgb8_zero = nullptr;             // RenderExtras::rgb8_zero
+    bool* scheduled = nullptr;                      // out: rgb8_zero given and the frame got a tile schedule
+    const rm::PeerLink* link = nullptr;             // frame-level calls (rm_render_frame): the exchange, and with it
+    unsigned char* rgb8_out = nullptr;              //   RenderExtras::rgb8_out, normalise and rgb8_next
+    bool normalise = true;
+    unsigned char* rgb8_next = nullptr;
+    bool as_graph = false;                          // one graph launch if RM_B200_GRAPH=1
+    cudaEvent_t ev_after_k0 = nullptr;              // recorded between K0 and K1 unless profiling records one there
+    const rm::ViewBasis* view = nullptr;            // the camera's orientation (rm_render_view)
+};
+
 template <typename R>
 int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_prim, R* d_max, cudaStream_t stream,
-                       int buf_row0_is_tile, unsigned long long* d_counters, rm::FrameParams<R>* out_fp, int* resident,
-                       int* launches = nullptr, unsigned char* d_rgb8_zero = nullptr, bool* scheduled = nullptr,
-                       const rm::PeerLink* link = nullptr, unsigned char* d_rgb8_out = nullptr, bool normalise = true,
-                       unsigned char* d_rgb8_next = nullptr, bool as_graph = false, cudaEvent_t ev_after_k0 = nullptr,
-                       const rm::ViewBasis* view = nullptr) {
+                       const RenderOptions<R>& o = {}) {
     if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
     int rc = check_params(params);
     if (rc != RM_OK) return rc;
@@ -466,30 +481,30 @@ int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_p
     if ((rc = ensure_pack<R>(it->second, dp)) != RM_OK) return rc;
     if ((rc = order_scene_renders(it->second, stream)) != RM_OK) return rc;
     rm::FrameParams<R> fp = rm::make_frame_params<R>(*params);
-    fp.buf_row0 = buf_row0_is_tile ? fp.row_begin : 0;
-    if (out_fp) *out_fp = fp;
+    fp.buf_row0 = o.buf_row0_is_tile ? fp.row_begin : 0;
+    if (o.out_fp) *o.out_fp = fp;
     const bool cull = params->cull_backfacing != 0;
-    if (resident) *resident = dp.ds.lay.n_sph + rm::plane_count<R>(dp.ds.lay, cull);
+    if (o.resident) *o.resident = dp.ds.lay.n_sph + rm::plane_count<R>(dp.ds.lay, cull);
     rm::RenderExtras ex;
-    ex.rgb8_zero = d_rgb8_zero;
-    if (link) {
-        ex.link = *link;
+    ex.rgb8_zero = o.rgb8_zero;
+    if (o.link) {
+        ex.link = *o.link;
         ex.zero_dmax = true;
-        ex.rgb8_out = d_rgb8_out;
-        ex.normalise = normalise;
-        ex.rgb8_next = d_rgb8_next;
+        ex.rgb8_out = o.rgb8_out;
+        ex.normalise = o.normalise;
+        ex.rgb8_next = o.rgb8_next;
     }
     if (g.profiling && !g.prof.empty()) {
         g.prof_head = (g.prof_head + 1) % kProfRing;
         g.prof_frames++;
         ProfSlot& ps = g.prof[g.prof_head];
         ps.has_tone = false;
-        ps.split = link == nullptr;                             // frame-level calls keep K0 -> K1 a programmatic launch edge
+        ps.split = o.link == nullptr;                           // frame-level calls keep K0 -> K1 a programmatic launch edge
         ex.ev_begin = ps.e[0];
         ex.ev_prepared = ps.split ? ps.e[1] : nullptr;
         ex.ev_rendered = ps.e[2];
     }
-    if (ev_after_k0 && !ex.ev_prepared) ex.ev_prepared = ev_after_k0;      // recorded between K0 and K1 (host delivery reads the schedule early)
+    if (o.ev_after_k0 && !ex.ev_prepared) ex.ev_prepared = o.ev_after_k0;      // recorded between K0 and K1 (host delivery reads the schedule early)
     SceneEntry& se = it->second;
     // RM_B200_GRAPH=1 (read per call): frame-level calls go to the GPU as ONE graph launch from the scene's second frame on
     // (the first one runs the launchers' one-time set-up).  Opt-in, because on the device it is a wash: 4K cornell frame,
@@ -502,7 +517,7 @@ int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_p
     const char* genv = getenv("RM_B200_GRAPH");
     const int graph_mode = (!graph_broken && genv && genv[0] == '1') ? 1 : 0;
     bool launched = false;
-    if (as_graph && graph_mode == 1 && se.frames > 0 && fp.n_bands > 0) {
+    if (o.as_graph && graph_mode == 1 && se.frames > 0 && fp.n_bands > 0) {
         cudaEvent_t ev_begin = ex.ev_begin, ev_rendered = ex.ev_rendered;
         ex.ev_begin = ex.ev_prepared = ex.ev_rendered = nullptr;
         cudaGraph_t graph = nullptr;
@@ -512,7 +527,7 @@ int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_p
         if (!g.cap_stream) e = cudaStreamCreateWithFlags(&g.cap_stream, cudaStreamNonBlocking);
         if (e == cudaSuccess) e = cudaStreamBeginCapture(g.cap_stream, cudaStreamCaptureModeRelaxed);
         if (e == cudaSuccess) {
-            const cudaError_t el = rm::launch_render<R>(dp.ds, fp, cull, d_rgb, d_prim, d_max, d_counters, g.cap_stream, params->camera, launches, &ex, view);
+            const cudaError_t el = rm::launch_render<R>(dp.ds, fp, cull, d_rgb, d_prim, d_max, o.counters, g.cap_stream, params->camera, o.launches, &ex, o.view);
             e = cudaStreamEndCapture(g.cap_stream, &graph);
             if (el != cudaSuccess) e = el;
         }
@@ -543,14 +558,14 @@ int render_device_impl(RmScene scene, const RmParams* params, R* d_rgb, int* d_p
             ex.ev_rendered = ev_rendered;
         }
     }
-    if (!launched) CK(rm::launch_render<R>(dp.ds, fp, cull, d_rgb, d_prim, d_max, d_counters, stream, params->camera, launches, &ex, view));
+    if (!launched) CK(rm::launch_render<R>(dp.ds, fp, cull, d_rgb, d_prim, d_max, o.counters, stream, params->camera, o.launches, &ex, o.view));
     se.frames++;
     LastFrame& lf = it->second.last;
     lf.classified = sizeof(R) == 4 && ex.scheduled;
-    lf.scheduled = lf.classified && d_rgb8_zero != nullptr;
+    lf.scheduled = lf.classified && o.rgb8_zero != nullptr;
     lf.width = fp.width; lf.height = fp.height; lf.row_begin = fp.row_begin; lf.row_step = fp.row_step;
-    lf.n_bands = fp.n_bands; lf.buf_row0 = fp.buf_row0; lf.rgb8 = d_rgb8_zero;
-    if (scheduled) *scheduled = lf.scheduled;
+    lf.n_bands = fp.n_bands; lf.buf_row0 = fp.buf_row0; lf.rgb8 = o.rgb8_zero;
+    if (o.scheduled) *o.scheduled = lf.scheduled;
     return RM_OK;
 }
 
@@ -580,10 +595,13 @@ int render_host_impl(RmScene scene, const RmParams* params, R* out_rgb, int32_t*
     int resident = 0;
     int launches = 0;
     bool scheduled = false;
-    rc = render_device_impl<R>(scene, params, static_cast<R*>(g.rgb.p), out_prim ? static_cast<int*>(g.prim.p) : nullptr,
-                               d_max, s, 1, want_counters ? d_cnt : nullptr, &fp, &resident, &launches,
-                               out_rgb8 ? static_cast<unsigned char*>(g.rgb8.p) : nullptr, &scheduled, nullptr, nullptr, true, nullptr,
-                               false, nullptr, view);
+    RenderOptions<R> o;
+    o.buf_row0_is_tile = true;
+    o.counters = want_counters ? d_cnt : nullptr;
+    o.out_fp = &fp; o.resident = &resident; o.launches = &launches; o.scheduled = &scheduled;
+    o.rgb8_zero = out_rgb8 ? static_cast<unsigned char*>(g.rgb8.p) : nullptr;
+    o.view = view;
+    rc = render_device_impl<R>(scene, params, static_cast<R*>(g.rgb.p), out_prim ? static_cast<int*>(g.prim.p) : nullptr, d_max, s, o);
     if (rc != RM_OK) return rc;
     // a view call writes the caller's float frame itself: what the library delivered there before no longer holds
     if (view && out_rgb && rows) forget_deliveries(out_rgb + (size_t)fp.row_begin * fp.width * 3, rows * fp.width * 3 * sizeof(R));
@@ -712,8 +730,11 @@ int render_rows_impl(RmScene scene, const RmParams* params, const RowSink& sink,
         CK(cudaEventCreateWithFlags(&g.ev_early, cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&g.ev_list, cudaEventDisableTiming));
     }
-    rc = render_device_impl<float>(scene, params, static_cast<float*>(g.rgb.p), nullptr, d_max, s, 1, nullptr, &fp, &resident, &launches,
-                                   nullptr, nullptr, nullptr, nullptr, true, nullptr, false, early_wanted ? g.ev_k0 : nullptr);
+    RenderOptions<float> o;
+    o.buf_row0_is_tile = true;
+    o.out_fp = &fp; o.resident = &resident; o.launches = &launches;
+    o.ev_after_k0 = early_wanted ? g.ev_k0 : nullptr;
+    rc = render_device_impl<float>(scene, params, static_cast<float*>(g.rgb.p), nullptr, d_max, s, o);
     if (rc != RM_OK) return rc;
     CK(cudaEventRecord(g.ev[2], s));
     SceneEntry& se = g.scenes.find(scene)->second;
@@ -1206,11 +1227,14 @@ int rm_render_dispersive(const RmScene scenes[3], const RmParams* params, float*
     cudaStream_t s = g.stream;
     CK(cudaEventRecord(g.ev[0], s));
     int resident = 0, launches = 0;
+    RenderOptions<float> o;
+    o.buf_row0_is_tile = true;
+    o.resident = &resident; o.launches = &launches;
     for (int c = 0; c < 3; c++) {
         CK(cudaMemsetAsync(g.small.p, 0, 1024, s));
         // (the primary ray does not depend on the refractive index: the ids of the first pass are the frame's)
         rc = render_device_impl<float>(scenes[c], params, static_cast<float*>(g.rgb.p), (out_prim_id && c == 0) ? static_cast<int*>(g.prim.p) : nullptr,
-                                       d_max, s, 1, nullptr, nullptr, &resident, &launches);
+                                       d_max, s, o);
         if (rc != RM_OK) return rc;
         if (n_px)
             CK(cudaMemcpy2DAsync(static_cast<char*>(g.mix.p) + 4 * c, 12, static_cast<const char*>(g.rgb.p) + 4 * c, 12, 4, n_px,
@@ -1269,7 +1293,10 @@ int rm_render_supersampled(RmScene scene, const RmParams* params, int samples, f
     CK(cudaMemsetAsync(g.small.p, 0, 64, s));
     CK(cudaEventRecord(g.ev[1], s));
     int resident = 0, launches = 0;
-    rc = render_device_impl<float>(scene, &sp, static_cast<float*>(g.sub.p), nullptr, d_sub_max, s, 1, nullptr, nullptr, &resident, &launches);
+    RenderOptions<float> o;
+    o.buf_row0_is_tile = true;
+    o.resident = &resident; o.launches = &launches;
+    rc = render_device_impl<float>(scene, &sp, static_cast<float*>(g.sub.p), nullptr, d_sub_max, s, o);
     if (rc != RM_OK) return rc;
     CK(cudaEventRecord(g.ev[2], s));
     if (rows) {
@@ -1362,7 +1389,10 @@ int rm_render_adaptive(RmScene scene, const RmParams* params, int samples, doubl
     CK(cudaMemsetAsync(g.small.p, 0, 64, s));
     CK(cudaEventRecord(g.ev[1], s));
     int resident = 0, launches = 0;
-    rc = render_device_impl<float>(scene, &hp, d_rgb, static_cast<int*>(g.prim.p), d_max1, s, 1, nullptr, nullptr, &resident, &launches);
+    RenderOptions<float> o;
+    o.buf_row0_is_tile = true;
+    o.resident = &resident; o.launches = &launches;
+    rc = render_device_impl<float>(scene, &hp, d_rgb, static_cast<int*>(g.prim.p), d_max1, s, o);
     if (rc != RM_OK) return rc;
     if (rows) {
         CK(rm::launch_adaptive_mark(d_rgb, static_cast<const int*>(g.prim.p), fp.width, lo, hi, fp.row_begin, (int)rows, (float)contrast,
@@ -1412,9 +1442,9 @@ int rm_render_device(RmScene scene, const RmParams* params, void* d_rgb, int32_t
     if (!d_rgb || !d_max) return fail(RM_ERR_INVALID_ARGUMENT, "d_rgb and d_max must be device pointers");
     if (params && params->precision == RM_FP64)
         return render_device_impl<double>(scene, params, static_cast<double*>(d_rgb), d_prim_id, static_cast<double*>(d_max),
-                                          static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr);
+                                          static_cast<cudaStream_t>(stream));
     return render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max),
-                                     static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr);
+                                     static_cast<cudaStream_t>(stream));
 }
 
 int rm_render_view_device(RmScene scene, const RmParams* params, const RmView* view, void* d_rgb, int32_t* d_prim_id, void* d_max,
@@ -1426,24 +1456,32 @@ int rm_render_view_device(RmScene scene, const RmParams* params, const RmView* v
     if (identity) return rm_render_device(scene, params, d_rgb, d_prim_id, d_max, stream);
     std::lock_guard<std::mutex> lock(g.mu);
     if (!d_rgb || !d_max) return fail(RM_ERR_INVALID_ARGUMENT, "d_rgb and d_max must be device pointers");
-    if (params && params->precision == RM_FP64)
+    if (params && params->precision == RM_FP64) {
+        RenderOptions<double> o;
+        o.view = &vb;
         return render_device_impl<double>(scene, params, static_cast<double*>(d_rgb), d_prim_id, static_cast<double*>(d_max),
-                                          static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
-                                          nullptr, nullptr, true, nullptr, false, nullptr, &vb);
+                                          static_cast<cudaStream_t>(stream), o);
+    }
+    RenderOptions<float> o;
+    o.view = &vb;
     return render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max),
-                                     static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
-                                     nullptr, nullptr, true, nullptr, false, nullptr, &vb);
+                                     static_cast<cudaStream_t>(stream), o);
 }
 
 int rm_render_device_rgb8(RmScene scene, const RmParams* params, void* d_rgb, int32_t* d_prim_id, void* d_max, uint8_t* d_rgb8,
                           void* stream) {
     std::lock_guard<std::mutex> lock(g.mu);
     if (!d_rgb || !d_max || !d_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "d_rgb, d_max and d_rgb8 must be device pointers");
-    if (params && params->precision == RM_FP64)
+    if (params && params->precision == RM_FP64) {
+        RenderOptions<double> o;
+        o.rgb8_zero = d_rgb8;
         return render_device_impl<double>(scene, params, static_cast<double*>(d_rgb), d_prim_id, static_cast<double*>(d_max),
-                                          static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr, nullptr, d_rgb8);
+                                          static_cast<cudaStream_t>(stream), o);
+    }
+    RenderOptions<float> o;
+    o.rgb8_zero = d_rgb8;
     return render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max),
-                                     static_cast<cudaStream_t>(stream), 0, nullptr, nullptr, nullptr, nullptr, d_rgb8);
+                                     static_cast<cudaStream_t>(stream), o);
 }
 
 int rm_tonemap_device_busy(RmScene scene, const RmParams* params, const void* d_rgb, const void* d_max, int normalise,
@@ -1617,9 +1655,15 @@ int rm_render_frame(RmScene scene, const RmParams* params, void* d_rgb, int32_t*
     // K0 + K1; K1 ends with the exchange and the conversion to 8 bits (K4 fused).  Only rank 0 clears bytes of the 8-bit
     // frames (its own black pixels in this frame's buffer, the whole bands of the other ranks in the next frame's buffer):
     // zeros never travel over NVLink.
-    int rc = render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max), s, 0,
-                                       nullptr, &fp, nullptr, nullptr, x->rank == 0 ? frame8 : nullptr, nullptr, &link, frame8,
-                                       normalise != 0, frame8_next, true);
+    RenderOptions<float> o;
+    o.out_fp = &fp;
+    o.rgb8_zero = x->rank == 0 ? frame8 : nullptr;
+    o.link = &link;
+    o.rgb8_out = frame8;
+    o.normalise = normalise != 0;
+    o.rgb8_next = frame8_next;
+    o.as_graph = true;
+    int rc = render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max), s, o);
     if (rc != RM_OK) return rc;
     auto it = g.scenes.find(scene);
     const rm::DeviceScene<float>& ds = it->second.f32.ds;
@@ -1673,12 +1717,15 @@ int rm_render_device_stats(RmScene scene, const RmParams* params, void* d_rgb, i
     unsigned long long* d_cnt = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 64);
     CK(cudaMemsetAsync(d_cnt, 0, rm::C_COUNT * 8, s));
     int resident = 0;
-    if (params && params->precision == RM_FP64)
-        rc = render_device_impl<double>(scene, params, static_cast<double*>(d_rgb), d_prim_id, static_cast<double*>(d_max), s, 0,
-                                        d_cnt, nullptr, &resident);
-    else
-        rc = render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max), s, 0,
-                                       d_cnt, nullptr, &resident);
+    if (params && params->precision == RM_FP64) {
+        RenderOptions<double> o;
+        o.counters = d_cnt; o.resident = &resident;
+        rc = render_device_impl<double>(scene, params, static_cast<double*>(d_rgb), d_prim_id, static_cast<double*>(d_max), s, o);
+    } else {
+        RenderOptions<float> o;
+        o.counters = d_cnt; o.resident = &resident;
+        rc = render_device_impl<float>(scene, params, static_cast<float*>(d_rgb), d_prim_id, static_cast<float*>(d_max), s, o);
+    }
     if (rc != RM_OK) return rc;
     unsigned long long host[rm::C_COUNT];
     CK(cudaMemcpyAsync(host, d_cnt, sizeof host, cudaMemcpyDeviceToHost, s));

@@ -21,6 +21,7 @@
 #include <algorithm>
 #include <cassert>
 #include <cstdlib>
+#include <initializer_list>
 
 // -DRM_CHECKED: bounds and protocol checks inside the kernels (device assert: file, line, block and thread on stderr, then
 // the kernel traps and the next CUDA call fails).  compute-sanitizer is closed on this project's GPU pool, so this is the
@@ -357,6 +358,78 @@ constexpr int kWarpQueue = kFastTile * 4 + 32;                  // one strip of 
 #define RM_K1_MIN_BLOCKS_OPAQUE 2                               // the instantiation without recursion / f64 code (kGlass = false)
 #endif
 template <int kPx> struct PxTag { static constexpr int value = kPx; };
+
+// The scene in shared memory of K1 and adaptive_subpixel_kernel (kSmem): blob | raster records of every fast-path
+// triangle | materials mat_a | mat_b | mat_f (stage_mat: if they fit as well).  Both kernels stage and view it with these
+// helpers, so that a sub-pixel value of the adaptive kernel stays the value K1 writes for that pixel.
+// The static part, blob and materials, does not depend on K0.
+__device__ __forceinline__ void stage_static(const DeviceScene<float>& ds, const int stage_mat, unsigned char* smem_raw) {
+    const BlobLayout& L = ds.lay;
+    const uint4* src = reinterpret_cast<const uint4*>(ds.blob);
+    uint4* dst = reinterpret_cast<uint4*>(smem_raw);
+    const int n16 = L.bytes / 16;
+    for (int i = threadIdx.x; i < n16; i += kFastBlock) dst[i] = __ldg(src + i);
+    if (stage_mat) {                                            // materials behind the raster records: mat_a | mat_b | mat_f
+        uint4* m = dst + n16 + L.n_tri * 4;
+        const uint4* a = reinterpret_cast<const uint4*>(ds.mat_a);
+        const uint4* b = reinterpret_cast<const uint4*>(ds.mat_b);
+        for (int i = threadIdx.x; i < ds.n_mat; i += kFastBlock) {
+            m[i] = __ldg(a + i);
+            m[ds.n_mat + i] = __ldg(b + i);
+            reinterpret_cast<int*>(m + 2 * ds.n_mat)[i] = __ldg(ds.mat_f + i);
+        }
+    }
+}
+// The raster records K0 wrote; base and tri_r then point into shared memory.
+__device__ __forceinline__ void stage_raster(const DeviceScene<float>& ds, const int n_tri, unsigned char* smem_raw,
+                                             const unsigned char*& base, const R4<float>*& tri_r) {
+    uint4* dst = reinterpret_cast<uint4*>(smem_raw);
+    const int n16 = ds.lay.bytes / 16;
+    const uint4* rsrc = reinterpret_cast<const uint4*>(ds.tri_r);
+    for (int i = threadIdx.x; i < n_tri * 4; i += kFastBlock) dst[n16 + i] = rsrc[i];
+    base = smem_raw;
+    tri_r = reinterpret_cast<const R4<float>*>(smem_raw + ds.lay.bytes);
+}
+// The scene as the fast device functions read it: the blob's arrays from base (ds.blob or its staged copy), the n_tri
+// raster records from tri_r, the materials from shared memory if they were staged (smem_mat).  n_tri is the caller's
+// tri_count(): computed again here, it changes K1's machine code.
+template <bool kBvh, bool kCount>
+__device__ __forceinline__ FastViewT<kBvh, kCount> make_fast_view(const DeviceScene<float>& ds, const unsigned char* base,
+                                                                  const R4<float>* tri_r, const int n_tri, const int cull,
+                                                                  const bool smem_mat, const unsigned char* smem_raw) {
+    const BlobLayout& L = ds.lay;
+    FastViewT<kBvh, kCount> fv;
+    fv.bvh = ds.bvh;
+    fv.sph = reinterpret_cast<const R4<float>*>(base + L.off_sph);
+    fv.sph_id = reinterpret_cast<const int*>(base + L.off_sph_id);
+    fv.n_sph = L.n_sph;
+    fv.tri_g = reinterpret_cast<const R4<float>*>(base + L.off_tri_g);
+    fv.tri_r = tri_r;
+    fv.n_tri = n_tri;
+    fv.poly_slot = reinterpret_cast<const int*>(base + L.off_poly_slot);
+    fv.n_poly = poly_count(L, cull != 0);
+    fv.pln_n = reinterpret_cast<const R4<float>*>(base + L.off_pln_n);
+    fv.pln_c = reinterpret_cast<const R4<float>*>(base + L.off_pln_c);
+    fv.pln_v = reinterpret_cast<const I2*>(base + L.off_pln_v);
+    fv.pln_id = reinterpret_cast<const int*>(base + L.off_pln_id);
+    fv.vert = reinterpret_cast<const R4<float>*>(base + L.off_vert);
+    fv.mat_a = ds.mat_a;
+    fv.mat_b = ds.mat_b;
+    fv.mat_f = ds.mat_f;
+    if (smem_mat) {
+        fv.mat_a = reinterpret_cast<const R4<float>*>(smem_raw + L.bytes + (size_t)L.n_tri * 64);
+        fv.mat_b = fv.mat_a + ds.n_mat;
+        fv.mat_f = reinterpret_cast<const int*>(fv.mat_b + ds.n_mat);
+    }
+    fv.lgt_p = reinterpret_cast<const R4<float>*>(base + L.off_lgt_p);
+    fv.lgt_c = reinterpret_cast<const R4<float>*>(base + L.off_lgt_c);
+    fv.n_lgt = L.n_lgt;
+    fv.sph64 = ds.sph64;
+    fv.tri64 = ds.tri_src;
+    fv.pln64 = ds.pln64;
+    return fv;
+}
+
 // kBvh (RmParams.accel): scene queries walk the hierarchy of rm_bvh.cuh (read through the read-only path; the nodes near
 // the root stay in L1) instead of every primitive; stage A then handles a thread's pixels one after the other.
 // kView (rm_render_view): K0 wrote raster records rotated into the camera's basis `view` (the last argument, so that the
@@ -386,67 +459,17 @@ render_fast_kernel(const DeviceScene<float> ds, const FrameParams<float> fp, con
     const R4<float>* tri_r = ds.tri_r;
     if (threadIdx.x < 96) fill_off[threadIdx.x] = (threadIdx.x / 24) * fp.width * 3 + (threadIdx.x % 24) * 4;
     if (threadIdx.x == 0) cta_max = 0;
-    if (kSmem) {                                                // the static part of the scene: does not depend on K0
-        const uint4* src = reinterpret_cast<const uint4*>(ds.blob);
-        uint4* dst = reinterpret_cast<uint4*>(smem_raw);
-        const int n16 = L.bytes / 16;
-        for (int i = threadIdx.x; i < n16; i += kFastBlock) dst[i] = __ldg(src + i);
-        if (stage_mat) {                                        // materials behind the raster records: mat_a | mat_b | mat_f
-            uint4* m = dst + n16 + L.n_tri * 4;
-            const uint4* a = reinterpret_cast<const uint4*>(ds.mat_a);
-            const uint4* b = reinterpret_cast<const uint4*>(ds.mat_b);
-            for (int i = threadIdx.x; i < ds.n_mat; i += kFastBlock) {
-                m[i] = __ldg(a + i);
-                m[ds.n_mat + i] = __ldg(b + i);
-                reinterpret_cast<int*>(m + 2 * ds.n_mat)[i] = __ldg(ds.mat_f + i);
-            }
-        }
-    }
-    pdl_wait_primary();                                         // K0 has retired: raster records, schedule, zeroed maximum
+    if (kSmem) stage_static(ds, stage_mat, smem_raw);          // does not depend on K0
+    pdl_wait_primary();                                        // K0 has retired: raster records, schedule, zeroed maximum
     if (threadIdx.x == 0 && blockIdx.x == 0 && link.world > 0) {
         unsigned long long* const box = link.box[link.rank];
         box[56] = now_ns();                                     // stamp: start of the work
         box[61] = reinterpret_cast<const unsigned long long*>(ctr + 12)[0];     // K0's own stamps, for the phase breakdown
         box[62] = reinterpret_cast<const unsigned long long*>(ctr + 12)[1];     // (tile-scheduled scenes only)
     }
-    if (kSmem) {
-        uint4* dst = reinterpret_cast<uint4*>(smem_raw);
-        const int n16 = L.bytes / 16;
-        const uint4* rsrc = reinterpret_cast<const uint4*>(ds.tri_r);
-        for (int i = threadIdx.x; i < n_tri * 4; i += kFastBlock) dst[n16 + i] = rsrc[i];
-        base = smem_raw;
-        tri_r = reinterpret_cast<const R4<float>*>(smem_raw + L.bytes);
-    }
+    if (kSmem) stage_raster(ds, n_tri, smem_raw, base, tri_r);
     __syncthreads();
-    FastViewT<kBvh, kCount> fv;
-    fv.bvh = ds.bvh;
-    fv.sph = reinterpret_cast<const R4<float>*>(base + L.off_sph);
-    fv.sph_id = reinterpret_cast<const int*>(base + L.off_sph_id);
-    fv.n_sph = L.n_sph;
-    fv.tri_g = reinterpret_cast<const R4<float>*>(base + L.off_tri_g);
-    fv.tri_r = tri_r;
-    fv.n_tri = n_tri;
-    fv.poly_slot = reinterpret_cast<const int*>(base + L.off_poly_slot);
-    fv.n_poly = poly_count(L, cull != 0);
-    fv.pln_n = reinterpret_cast<const R4<float>*>(base + L.off_pln_n);
-    fv.pln_c = reinterpret_cast<const R4<float>*>(base + L.off_pln_c);
-    fv.pln_v = reinterpret_cast<const I2*>(base + L.off_pln_v);
-    fv.pln_id = reinterpret_cast<const int*>(base + L.off_pln_id);
-    fv.vert = reinterpret_cast<const R4<float>*>(base + L.off_vert);
-    fv.mat_a = ds.mat_a;
-    fv.mat_b = ds.mat_b;
-    fv.mat_f = ds.mat_f;
-    if (kSmem && stage_mat) {
-        fv.mat_a = reinterpret_cast<const R4<float>*>(smem_raw + L.bytes + (size_t)L.n_tri * 64);
-        fv.mat_b = fv.mat_a + ds.n_mat;
-        fv.mat_f = reinterpret_cast<const int*>(fv.mat_b + ds.n_mat);
-    }
-    fv.lgt_p = reinterpret_cast<const R4<float>*>(base + L.off_lgt_p);
-    fv.lgt_c = reinterpret_cast<const R4<float>*>(base + L.off_lgt_c);
-    fv.n_lgt = L.n_lgt;
-    fv.sph64 = ds.sph64;
-    fv.tri64 = ds.tri_src;
-    fv.pln64 = ds.pln64;
+    FastViewT<kBvh, kCount> fv = make_fast_view<kBvh, kCount>(ds, base, tri_r, n_tri, cull, kSmem && stage_mat, smem_raw);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const unsigned lane_lt = (1u << lane) - 1u;
@@ -1028,56 +1051,12 @@ adaptive_subpixel_kernel(const DeviceScene<float> ds, const FrameParams<float> f
     const int n_tri = tri_count(L, cull != 0);
     const unsigned char* base = ds.blob;
     const R4<float>* tri_r = ds.tri_r;
-    if (kSmem) {                                                // as K1: blob | raster records | materials (if they fit)
-        const uint4* src = reinterpret_cast<const uint4*>(ds.blob);
-        uint4* dst = reinterpret_cast<uint4*>(smem_raw);
-        const int n16 = L.bytes / 16;
-        for (int i = threadIdx.x; i < n16; i += kFastBlock) dst[i] = __ldg(src + i);
-        const uint4* rsrc = reinterpret_cast<const uint4*>(ds.tri_r);
-        for (int i = threadIdx.x; i < n_tri * 4; i += kFastBlock) dst[n16 + i] = rsrc[i];
-        if (stage_mat) {
-            uint4* m = dst + n16 + L.n_tri * 4;
-            const uint4* a = reinterpret_cast<const uint4*>(ds.mat_a);
-            const uint4* b = reinterpret_cast<const uint4*>(ds.mat_b);
-            for (int i = threadIdx.x; i < ds.n_mat; i += kFastBlock) {
-                m[i] = __ldg(a + i);
-                m[ds.n_mat + i] = __ldg(b + i);
-                reinterpret_cast<int*>(m + 2 * ds.n_mat)[i] = __ldg(ds.mat_f + i);
-            }
-        }
-        base = smem_raw;
-        tri_r = reinterpret_cast<const R4<float>*>(smem_raw + L.bytes);
+    if (kSmem) {                                                // as K1, which K0 has retired before
+        stage_static(ds, stage_mat, smem_raw);
+        stage_raster(ds, n_tri, smem_raw, base, tri_r);
     }
     __syncthreads();
-    FastViewT<kBvh, false> fv;
-    fv.bvh = ds.bvh;
-    fv.sph = reinterpret_cast<const R4<float>*>(base + L.off_sph);
-    fv.sph_id = reinterpret_cast<const int*>(base + L.off_sph_id);
-    fv.n_sph = L.n_sph;
-    fv.tri_g = reinterpret_cast<const R4<float>*>(base + L.off_tri_g);
-    fv.tri_r = tri_r;
-    fv.n_tri = n_tri;
-    fv.poly_slot = reinterpret_cast<const int*>(base + L.off_poly_slot);
-    fv.n_poly = poly_count(L, cull != 0);
-    fv.pln_n = reinterpret_cast<const R4<float>*>(base + L.off_pln_n);
-    fv.pln_c = reinterpret_cast<const R4<float>*>(base + L.off_pln_c);
-    fv.pln_v = reinterpret_cast<const I2*>(base + L.off_pln_v);
-    fv.pln_id = reinterpret_cast<const int*>(base + L.off_pln_id);
-    fv.vert = reinterpret_cast<const R4<float>*>(base + L.off_vert);
-    fv.mat_a = ds.mat_a;
-    fv.mat_b = ds.mat_b;
-    fv.mat_f = ds.mat_f;
-    if (kSmem && stage_mat) {
-        fv.mat_a = reinterpret_cast<const R4<float>*>(smem_raw + L.bytes + (size_t)L.n_tri * 64);
-        fv.mat_b = fv.mat_a + ds.n_mat;
-        fv.mat_f = reinterpret_cast<const int*>(fv.mat_b + ds.n_mat);
-    }
-    fv.lgt_p = reinterpret_cast<const R4<float>*>(base + L.off_lgt_p);
-    fv.lgt_c = reinterpret_cast<const R4<float>*>(base + L.off_lgt_c);
-    fv.n_lgt = L.n_lgt;
-    fv.sph64 = ds.sph64;
-    fv.tri64 = ds.tri_src;
-    fv.pln64 = ds.pln64;
+    FastViewT<kBvh, false> fv = make_fast_view<kBvh, false>(ds, base, tri_r, n_tri, cull, kSmem && stage_mat, smem_raw);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const unsigned lane_lt = (1u << lane) - 1u;
@@ -1213,16 +1192,75 @@ __global__ void __launch_bounds__(256) ffma_probe_kernel(float* __restrict__ sin
 }  // namespace
 
 namespace {
+// The launch plan of K1 and adaptive_subpixel_kernel: it picks the instantiation, and a sub-pixel value of the adaptive
+// kernel is the value K1 writes for that pixel only while both kernels pick alike.
+// Shared memory: scene blob | raster records of every fast-path triangle | materials (if they fit as well), next to the
+// kernel's static arrays (hit queues etc.) within dyn_limit.
+struct FastPlan {
+    bool bvh;                                                   // walk the hierarchy
+    bool use_smem;                                              // stage the scene in shared memory
+    int stage_mat;                                              // ... the materials as well
+    int glass;                                                  // GlassMode
+    size_t dyn_smem;                                            // dynamic shared memory of the launch
+    int row() const { return bvh ? 2 : use_smem ? 0 : 1; }      // of the instantiation tables: staged | global | hierarchy
+};
+
+FastPlan fast_plan(const DeviceScene<float>& ds, const FrameParams<float>& fp, const double camera[3], const int dyn_limit) {
+    FastPlan p;
+    p.bvh = fp.accel != 0 && ds.bvh.n_nodes > 0 && ds.lay.n_lgt <= kBvhMaxLights;
+    const size_t smem_geo = (size_t)ds.lay.bytes + (size_t)ds.lay.n_tri * 64;
+    const size_t smem_mat = (((size_t)ds.n_mat * 36) + 15) / 16 * 16;
+    p.stage_mat = smem_geo + smem_mat <= (size_t)dyn_limit ? 1 : 0;
+    const size_t smem = smem_geo + (p.stage_mat ? smem_mat : 0);
+    p.use_smem = !p.bvh && smem <= (size_t)dyn_limit;
+    // the reflect / refract recursion only where a frame can need it, its f64 ray geometry only where FP32 would not do
+    p.glass = glass_mode(ds.lay.any_glass != 0, ds.lay.n_sph, ds.lay.coord_max, ds.lay.r_min, camera);
+    p.dyn_smem = p.use_smem ? smem : 0;
+    return p;
+}
+
+// One-time set-up of a kernel family: the SM count, and the dynamic shared memory left next to the static arrays of its
+// widest instantiation (GLASS_F64 of the first row), opted in for its instantiations that stage the scene (`staged`: rows
+// indexed by GlassMode).  Each family has its own limit: K1's static arrays are larger than the adaptive kernel's.
+template <typename K>
+cudaError_t setup_family(std::initializer_list<const K*> staged, int& sm_count, int& dyn_limit) {
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa;
+    cudaError_t e;
+    if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+    if ((e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&fa, staged.begin()[0][GLASS_F64])) != cudaSuccess) return e;
+    dyn_limit = std::min(kSmemLimit, optin - (int)fa.sharedSizeBytes - 1024);
+    for (const K* row : staged)
+        for (int gm = GLASS_NONE; gm <= GLASS_F64; gm++)
+            if ((e = cudaFuncSetAttribute(row[gm], cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
+    return cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
+}
+
 cudaError_t launch_fast(const DeviceScene<float>& ds, const FrameParams<float>& fp, bool cull, float* rgb, int* prim_id,
                         float* dmax, cudaStream_t stream, const double camera[3], int* launches, RenderExtras* ex,
                         const ViewBasis* view) {
+    using K1 = decltype(&render_fast_kernel<true, 0, GLASS_NONE>);
+    static const K1 table[4][3] = {
+        {render_fast_kernel<true, 0, GLASS_NONE>, render_fast_kernel<true, 0, GLASS_F32>, render_fast_kernel<true, 0, GLASS_F64>},
+        {render_fast_kernel<false, 0, GLASS_NONE>, render_fast_kernel<false, 0, GLASS_F32>, render_fast_kernel<false, 0, GLASS_F64>},
+        {render_fast_kernel<false, 1, GLASS_NONE>, render_fast_kernel<false, 1, GLASS_F32>, render_fast_kernel<false, 1, GLASS_F64>},
+        {render_fast_kernel<false, 2, GLASS_NONE>, render_fast_kernel<false, 2, GLASS_F32>, render_fast_kernel<false, 2, GLASS_F64>}};
+    // under a view: no counting instantiation (accel = 2 renders as accel = 1)
+    static const K1 view_table[3][3] = {
+        {render_fast_kernel<true, 0, GLASS_NONE, true>, render_fast_kernel<true, 0, GLASS_F32, true>, render_fast_kernel<true, 0, GLASS_F64, true>},
+        {render_fast_kernel<false, 0, GLASS_NONE, true>, render_fast_kernel<false, 0, GLASS_F32, true>, render_fast_kernel<false, 0, GLASS_F64, true>},
+        {render_fast_kernel<false, 1, GLASS_NONE, true>, render_fast_kernel<false, 1, GLASS_F32, true>, render_fast_kernel<false, 1, GLASS_F64, true>}};
+    static int sm_count = 0, dyn_limit = 0;
+    cudaError_t e;
+    if (!sm_count && (e = setup_family<K1>({table[0], view_table[0]}, sm_count, dyn_limit)) != cudaSuccess) return e;
+    const FastPlan plan = fast_plan(ds, fp, camera, dyn_limit);
     const ViewBasis vb = view ? *view : ViewBasis{};
     unsigned char* rgb8 = ex ? ex->rgb8_zero : nullptr;
     if (ex && ex->ev_begin) cudaEventRecord(ex->ev_begin, stream);
     const int n_tri = tri_count(ds.lay, cull);
     const int tiles_x = fp.width / kFastTile, n_tiles = tiles_x * fp.n_bands;
-    const bool bvh = fp.accel != 0 && ds.bvh.n_nodes > 0 && ds.lay.n_lgt <= kBvhMaxLights;
-    const bool classify = !bvh && ds.lay.n_sph + poly_count(ds.lay, cull) == 0 && n_tri <= kClassifyMaxTris && n_tiles <= ds.tile_order_cap / 2;
+    const bool classify = !plan.bvh && ds.lay.n_sph + poly_count(ds.lay, cull) == 0 && n_tri <= kClassifyMaxTris && n_tiles <= ds.tile_order_cap / 2;
     if (classify)
         (view ? prepare_classify_kernel<true> : prepare_classify_kernel<false>)
             <<<(n_tiles * kClassifyLanes + kClassifyBlock - 1) / kClassifyBlock, kClassifyBlock, 0, stream>>>(ds.tri_src, n_tri, camera[0], camera[1], camera[2], ds.tri_r,
@@ -1243,29 +1281,6 @@ cudaError_t launch_fast(const DeviceScene<float>& ds, const FrameParams<float>& 
     unsigned char* rgb8_next = (rgb8_out && link.world > 1 && link.rank == 0) ? ex->rgb8_next : nullptr;
     if (ex && ex->ev_prepared) cudaEventRecord(ex->ev_prepared, stream);      // (an event here gives up the overlap of K1's launch with K0)
     if (launches) (*launches)++;
-    // shared memory: scene blob | raster records of every fast-path triangle | materials (if they fit as well), next to the
-    // kernel's static arrays (hit queues etc.) within the opt-in limit of the device
-    static int sm_count = 0, dyn_limit = 0;
-    cudaError_t e;
-    if (!sm_count) {
-        int dev = 0, optin = 0;
-        cudaFuncAttributes fa;
-        if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
-        if ((e = cudaFuncGetAttributes(&fa, render_fast_kernel<true, 0, GLASS_F64>)) != cudaSuccess) return e;
-        dyn_limit = std::min(kSmemLimit, optin - (int)fa.sharedSizeBytes - 1024);
-        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_NONE>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
-        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_F32>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
-        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_F64>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
-        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_NONE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
-        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_F32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
-        if ((e = cudaFuncSetAttribute(render_fast_kernel<true, 0, GLASS_F64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    }
-    const size_t smem_geo = (size_t)ds.lay.bytes + (size_t)ds.lay.n_tri * 64;
-    const size_t smem_mat = (((size_t)ds.n_mat * 36) + 15) / 16 * 16;
-    const int stage_mat = smem_geo + smem_mat <= (size_t)dyn_limit ? 1 : 0;
-    const size_t smem = smem_geo + (stage_mat ? smem_mat : 0);
     const float inv_tiles_x = 1.0f / (float)tiles_x;
     // launched with programmatic stream serialisation: the CTAs may become resident while K0 still runs (pdl_wait_primary)
     cudaLaunchAttribute attr[2];
@@ -1295,34 +1310,20 @@ cudaError_t launch_fast(const DeviceScene<float>& ds, const FrameParams<float>& 
     }
     const int cull_i = cull ? 1 : 0;
     const int* order2 = order ? ds.tile_order + ds.tile_order_cap / 2 : nullptr;
-    const bool use_smem = !bvh && smem <= (size_t)dyn_limit;
-    // the reflect / refract recursion only where a frame can need it, its f64 ray geometry only where FP32 would not do
-    const int glass = glass_mode(ds.lay.any_glass != 0, ds.lay.n_sph, ds.lay.coord_max, ds.lay.r_min, camera);
-    if (ex) ex->glass_mode = glass;
-    using K1 = decltype(&render_fast_kernel<true, 0, GLASS_NONE>);
-    static const K1 table[4][3] = {
-        {render_fast_kernel<true, 0, GLASS_NONE>, render_fast_kernel<true, 0, GLASS_F32>, render_fast_kernel<true, 0, GLASS_F64>},
-        {render_fast_kernel<false, 0, GLASS_NONE>, render_fast_kernel<false, 0, GLASS_F32>, render_fast_kernel<false, 0, GLASS_F64>},
-        {render_fast_kernel<false, 1, GLASS_NONE>, render_fast_kernel<false, 1, GLASS_F32>, render_fast_kernel<false, 1, GLASS_F64>},
-        {render_fast_kernel<false, 2, GLASS_NONE>, render_fast_kernel<false, 2, GLASS_F32>, render_fast_kernel<false, 2, GLASS_F64>}};
-    // under a view: no counting instantiation (accel = 2 renders as accel = 1)
-    static const K1 view_table[3][3] = {
-        {render_fast_kernel<true, 0, GLASS_NONE, true>, render_fast_kernel<true, 0, GLASS_F32, true>, render_fast_kernel<true, 0, GLASS_F64, true>},
-        {render_fast_kernel<false, 0, GLASS_NONE, true>, render_fast_kernel<false, 0, GLASS_F32, true>, render_fast_kernel<false, 0, GLASS_F64, true>},
-        {render_fast_kernel<false, 1, GLASS_NONE, true>, render_fast_kernel<false, 1, GLASS_F32, true>, render_fast_kernel<false, 1, GLASS_F64, true>}};
-    const K1 k = view ? view_table[bvh ? 2 : use_smem ? 0 : 1][glass] : table[bvh ? (fp.accel == 2 ? 3 : 2) : use_smem ? 0 : 1][glass];
-    cfg.dynamicSmemBytes = use_smem ? smem : 0;
+    if (ex) ex->glass_mode = plan.glass;
+    const K1 k = view ? view_table[plan.row()][plan.glass] : table[plan.bvh && fp.accel == 2 ? 3 : plan.row()][plan.glass];
+    cfg.dynamicSmemBytes = plan.dyn_smem;
     int occ = 1;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, kFastBlock, cfg.dynamicSmemBytes)) != cudaSuccess) return e;
     cfg.gridDim = dim3(std::min(n_tiles, sm_count * std::max(occ, 1)));
     e = cudaLaunchKernelEx(&cfg, k, ds, fp, cull_i, tiles_x, n_tiles, inv_tiles_x, rgb, prim_id, dmax, ds.ctr, order, order2, rgb8,
-                           link, rgb8_out, normalise, rgb8_next, stage_mat, vb);
+                           link, rgb8_out, normalise, rgb8_next, plan.stage_mat, vb);
     if (e != cudaSuccess && want_coop) {                        // not available in this combination: the plain persistent launch
         cudaGetLastError();
         coop = 0;
         cfg.numAttrs = 1;
         e = cudaLaunchKernelEx(&cfg, k, ds, fp, cull_i, tiles_x, n_tiles, inv_tiles_x, rgb, prim_id, dmax, ds.ctr, order, order2, rgb8,
-                               link, rgb8_out, normalise, rgb8_next, stage_mat, vb);
+                               link, rgb8_out, normalise, rgb8_next, plan.stage_mat, vb);
     }
     if (e != cudaSuccess) return e;
     if (launches) (*launches)++;
@@ -1422,7 +1423,6 @@ cudaError_t launch_adaptive_mark(const float* rgb, const int* id, int width, int
 cudaError_t launch_adaptive_subpixel(const DeviceScene<float>& ds, const FrameParams<float>& fp, bool cull, int samples,
                                      const unsigned* list, const unsigned* count, unsigned long long* next, float* sub,
                                      const double camera[3], cudaStream_t stream) {
-    // the instantiation launch_fast would pick for this scene and camera: hierarchy or not, glass mode, staged scene
     using K = decltype(&adaptive_subpixel_kernel<true, false, GLASS_NONE>);
     static const K table[3][3] = {
         {adaptive_subpixel_kernel<true, false, GLASS_NONE>, adaptive_subpixel_kernel<true, false, GLASS_F32>, adaptive_subpixel_kernel<true, false, GLASS_F64>},
@@ -1430,29 +1430,13 @@ cudaError_t launch_adaptive_subpixel(const DeviceScene<float>& ds, const FramePa
         {adaptive_subpixel_kernel<false, true, GLASS_NONE>, adaptive_subpixel_kernel<false, true, GLASS_F32>, adaptive_subpixel_kernel<false, true, GLASS_F64>}};
     static int sm_count = 0, dyn_limit = 0;
     cudaError_t e;
-    if (!sm_count) {
-        int dev = 0, optin = 0;
-        cudaFuncAttributes fa;
-        if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
-        if ((e = cudaFuncGetAttributes(&fa, table[0][GLASS_F64])) != cudaSuccess) return e;
-        dyn_limit = std::min(kSmemLimit, optin - (int)fa.sharedSizeBytes - 1024);
-        for (int gm = 0; gm < 3; gm++)
-            if ((e = cudaFuncSetAttribute(table[0][gm], cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_limit)) != cudaSuccess) return e;
-        if ((e = cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev)) != cudaSuccess) return e;
-    }
-    const bool bvh = fp.accel != 0 && ds.bvh.n_nodes > 0 && ds.lay.n_lgt <= kBvhMaxLights;
-    const size_t smem_geo = (size_t)ds.lay.bytes + (size_t)ds.lay.n_tri * 64;
-    const size_t smem_mat = (((size_t)ds.n_mat * 36) + 15) / 16 * 16;
-    const int stage_mat = smem_geo + smem_mat <= (size_t)dyn_limit ? 1 : 0;
-    const size_t smem = smem_geo + (stage_mat ? smem_mat : 0);
-    const bool use_smem = !bvh && smem <= (size_t)dyn_limit;
-    const int glass = glass_mode(ds.lay.any_glass != 0, ds.lay.n_sph, ds.lay.coord_max, ds.lay.r_min, camera);
-    const K k = table[bvh ? 2 : use_smem ? 0 : 1][glass];
-    const size_t dyn = use_smem ? smem : 0;
+    if (!sm_count && (e = setup_family<K>({table[0]}, sm_count, dyn_limit)) != cudaSuccess) return e;
+    const FastPlan plan = fast_plan(ds, fp, camera, dyn_limit);        // K1's plan for this scene and camera
+    const K k = table[plan.row()][plan.glass];
     int occ = 1;
-    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, kFastBlock, dyn)) != cudaSuccess) return e;
-    k<<<sm_count * std::max(occ, 1), kFastBlock, dyn, stream>>>(ds, fp, cull ? 1 : 0, samples, list, count, next, sub, stage_mat);
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, kFastBlock, plan.dyn_smem)) != cudaSuccess) return e;
+    k<<<sm_count * std::max(occ, 1), kFastBlock, plan.dyn_smem, stream>>>(ds, fp, cull ? 1 : 0, samples, list, count, next, sub,
+                                                                          plan.stage_mat);
     return cudaGetLastError();
 }
 
