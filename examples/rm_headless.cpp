@@ -15,6 +15,9 @@
 //   --look-at X,Y,Z                    the camera turned to look at that point (rm_render_view; an extension: the reference
 //                                      always looks down -z), --up X,Y,Z its up direction (default 0,1,0).  Combines with
 //                                      --camera, --accel, --f64 and --out; not with --samples, --contrast or --rows-f64
+//   --aperture A --focus F             depth of field: a thin lens of radius A focused at distance F, --samples S x S rays
+//                                      per pixel through it (rm_render_lens; an extension).  Combines with --samples,
+//                                      --look-at / --up, --camera and --accel; not with --contrast, --f64 or --rows-f64
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -43,6 +46,8 @@ int main(int argc, char** argv) {
     bool look = false;
     double target[3] = {0., 0., 0.};
     RmView view = {{0., 0., -1.}, {0., 1., 0.}};
+    bool use_lens = false, have_focus = false;
+    RmLens lens = {0., 1., 1};
     auto triple = [](const char* s, double v[3]) { char end = 0; return std::sscanf(s, "%lf,%lf,%lf%c", &v[0], &v[1], &v[2], &end) == 3; };
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
@@ -59,6 +64,8 @@ int main(int argc, char** argv) {
         else if (a == "--accel") accel = 1;
         else if (a == "--samples") { need(1); samples = std::atoi(argv[++i]); }
         else if (a == "--contrast") { need(1); contrast = std::strtod(argv[++i], nullptr); adaptive = true; }
+        else if (a == "--aperture") { need(1); lens.aperture = std::strtod(argv[++i], nullptr); use_lens = true; }
+        else if (a == "--focus") { need(1); lens.focus = std::strtod(argv[++i], nullptr); have_focus = true; }
         else if (a == "--look-at" || a == "--up") {
             need(1);
             if (!triple(argv[++i], a == "--up" ? view.up : target)) { std::fprintf(stderr, "rm_headless: %s takes X,Y,Z\n", a.c_str()); return 2; }
@@ -70,7 +77,12 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "rm_headless: --samples takes 1 to 8, with the FP32 kernels\n");
         return 2;
     }
-    if (look && (samples > 1 || adaptive || rows64)) {
+    if (use_lens != have_focus || (use_lens && (adaptive || f64 || rows64))) {
+        std::fprintf(stderr, "rm_headless: --aperture and --focus go together, and not with --contrast, --f64 or --rows-f64\n");
+        return 2;
+    }
+    lens.samples = samples;
+    if (look && !use_lens && (samples > 1 || adaptive || rows64)) {
         std::fprintf(stderr, "rm_headless: --look-at does not combine with --samples, --contrast or --rows-f64\n");
         return 2;
     }
@@ -129,7 +141,8 @@ int main(int argc, char** argv) {
     for (int f = 0; f < frames; f++) {
         const auto t0 = std::chrono::steady_clock::now();
         std::memset(&st, 0, sizeof st);
-        if (look && f64) rc = rm_render_view_f64(scene, &p, &view, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
+        if (use_lens) rc = rm_render_lens(scene, &p, look ? &view : nullptr, &lens, rgb32.data(), f == frames - 1 ? rgb8.data() : nullptr, &st);
+        else if (look && f64) rc = rm_render_view_f64(scene, &p, &view, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (look) rc = rm_render_view(scene, &p, &view, rgb32.data(), nullptr, nullptr, &st);
         else if (f64) rc = rm_render_f64(scene, &p, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (rows64) rc = rm_render_rows_f64(scene, &p, row_ptrs.data(), RM_ROWS_RETAINED, &st);
@@ -140,7 +153,9 @@ int main(int argc, char** argv) {
         std::printf("Scene rendered in %lld ms (%u fps, %.2f MP/s)\n", ms, ms > 0 ? (unsigned)fps : 4294967295u, fps * (double)n_px / 1e6);
     }
     // "Save to file": normalize + to_vec on the device (framebuffer.rs:40-82), then the P6 stream (framebuffer.rs:26-38)
-    if (adaptive) {
+    if (use_lens) {
+        // (the last frame above wrote the 8-bit frame)
+    } else if (adaptive) {
         std::vector<unsigned char> mask(n_px, 0);
         std::memset(&st, 0, sizeof st);
         if ((rc = rm_render_adaptive(scene, &p, samples, contrast, nullptr, rgb8.data(), mask.data(), &st)) != RM_OK) die("render (adaptive 8-bit frame)", rc);

@@ -324,6 +324,52 @@ int rm_render_view_f64(RmScene scene, const RmParams* params, const RmView* view
 int rm_render_view_device(RmScene scene, const RmParams* params, const RmView* view, void* d_rgb, int32_t* d_prim_id,
                           void* d_max, void* stream);
 
+/* ---- extension mode: depth of field -- a thin-lens camera with an aperture and a focus distance ---------------------------- *
+ * The reference's pinhole keeps every depth in focus; a thin lens blurs what lies off the plane in focus.
+ * Definition (normative; rm::lens_offset / rm::lens_ray in rm_trace.cuh are this, and the tests' restatement over the
+ * oracle is the same).  All in f64 without fused multiply-add.  s = samples; c the camera position; u, v, w the view's
+ * basis (rm_view_basis), or the identity without a view.  For output pixel (x, y) and sample (i, j), i, j in [0, s):
+ *   1. d = the reference's normalised backproject direction of sub-pixel (s x + j, s y + i) in the s W x s H frame
+ *      (rm_render_supersampled's sub-pixel ray).
+ *   2. Lens point: a = (i + j) mod s, b = j (the shift decorrelates lens strata from sub-pixel strata);
+ *      p = (2 a + 1) / s - 1, q = (2 b + 1) / s - 1;  lx = p * sqrt(1 - (q*q) * 0.5),  ly = q * sqrt(1 - (p*p) * 0.5)
+ *      (the elliptical grid-to-disc map: every point lies in the unit disc).
+ *   3. aperture = 0: the ray is (c, world(d)), the pinhole ray.  Otherwise
+ *        k = focus / (-d.z);  P = (d.x*k, d.y*k, d.z*k);  L = (aperture*lx, aperture*ly, 0);
+ *        e = normalized(P - L)  (geometry.rs's scale(1 / norm));
+ *        origin = c + ((u*L.x + v*L.y)), component by component in that order;  direction = world(e),
+ *      with world(e) = ((u.x*e.x + v.x*e.y) + w.x*e.z, ...) as for rm_render_view, not renormalised.
+ *   4. The sample's value is the reference's cast_ray from that ray (renderer.rs:254-309, levels 1..max_depth); everything
+ *      after the ray is unchanged, the world-z inside test of planar primitives included.
+ *   5. The pixel is the FP32 mean of its s^2 sample values in rm_render_supersampled's order (sub-rows i outer, j inner).
+ * Consequences:
+ *   - aperture = 0 without a view is rm_render_supersampled's frame bit for bit (the call is routed there); with s = 1 that
+ *     is also rm_render's frame.
+ *   - Points on the plane at distance `focus` (along the view axis) stay sharp: every sample of a pixel aims at the same P.
+ *   - At s = 1 the only lens point is the centre, so the lens has no effect.
+ *   - The lens pattern is the same for every pixel: out-of-focus objects show as s^2 overlapping copies, not as noise.  The
+ *     frame is deterministic by design.
+ * FP32 production path (lens_kernel): each sample ray is computed in f64 by rm::lens_ray and traced with the general FP32
+ * closest-hit query from level 1 on (brute force, or the hierarchy with accel != 0; accel = 2 renders as accel = 1), the rest
+ * as rm_render's shading stage; frames meet the FP32 parity criteria against the f64 definition.  cull_backfacing applies.
+ * Rows, outputs and stats as rm_render_supersampled: patch rows [b, e) with patch_row_stride <= 1, rows outside untouched;
+ * out_rgb (H*W*3 floats) and / or out_rgb8 (H*W*3 bytes: normalize() + to_vec() of the output rows by their own maximum);
+ * stats: max_value, ms_render (device time of the traced and resolved rows: no tone map, no copies), ms_total,
+ * kernel_launches, resident_prims, d2h_bytes.  Device memory: the output rows only (no s^2-sized scratch).  The call writes
+ * the caller's float frame, so the library forgets its previous deliveries into that memory (RM_ROWS_RETAINED).
+ * RM_ERR_INVALID_ARGUMENT: a NULL lens, samples outside [1, 8], aperture < 0, focus <= 0, a lens value that is not finite;
+ * an invalid view; precision other than RM_FP32; patch_row_stride > 1; max_depth < 1; an unknown scene; out_rgb and out_rgb8
+ * both NULL.  RM_ERR_DIMENSIONS: as for rm_render_supersampled.  Lens and parameter errors are reported without a device.
+ * Out of scope: random or per-pixel lens patterns and bokeh shapes; a lens for rm_render_adaptive, rm_render_dispersive,
+ * rm_render_rows_* and rm_render_frame; an FP64 entry point. */
+typedef struct RmLens {
+    double aperture;   /* lens radius in scene units, >= 0 */
+    double focus;      /* distance from the camera to the plane in focus, along the view axis, > 0 */
+    int32_t samples;   /* s: s x s sample rays per pixel, in [1, 8] */
+} RmLens;
+int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb,
+                   uint8_t* out_rgb8, RmStats* stats);
+
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device
  * scalar of the same type as d_rgb that receives max(previous value, tile max) -- zero it first.

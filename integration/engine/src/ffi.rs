@@ -168,6 +168,15 @@ pub struct RmView {
     pub up: [f64; 3],
 }
 
+/// thin-lens camera of rm_render_lens: lens radius (>= 0), distance of the plane in focus (> 0), s x s samples per pixel
+#[repr(C)]
+#[derive(Copy, Clone, Debug)]
+pub struct RmLens {
+    pub aperture: f64,
+    pub focus: f64,
+    pub samples: i32,
+}
+
 /// one frame on the GPUs of one box (one process per GPU)
 #[repr(C)]
 pub struct RmExchange {
@@ -218,6 +227,9 @@ extern "C" {
                               out_prim_id: *mut i32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
     pub fn rm_render_view_device(scene: RmScene, params: *const RmParams, view: *const RmView, d_rgb: *mut c_void,
                                  d_prim_id: *mut i32, d_max: *mut c_void, stream: *mut c_void) -> c_int;
+    /// depth of field: s x s sample rays per pixel through a thin lens, from the camera turned to `view` (null: down -z)
+    pub fn rm_render_lens(scene: RmScene, params: *const RmParams, view: *const RmView, lens: *const RmLens, out_rgb: *mut f32,
+                          out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
     // ---- the hot path, device buffers
     pub fn rm_render_device(scene: RmScene, params: *const RmParams, d_rgb: *mut c_void, d_prim_id: *mut i32,
                             d_max: *mut c_void, stream: *mut c_void) -> c_int;

@@ -78,6 +78,10 @@ class RmView(C.Structure):
     _fields_ = [("forward", d3), ("up", d3)]
 
 
+class RmLens(C.Structure):
+    _fields_ = [("aperture", C.c_double), ("focus", C.c_double), ("samples", C.c_int32)]
+
+
 RM_MAX_RANKS, RM_IPC_HANDLE_BYTES, RM_MAILBOX_BYTES = 16, 64, 512
 
 
@@ -123,6 +127,7 @@ SYMBOLS = {
     "rm_render_view": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), C.c_void_p, C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_render_view_f64": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), C.c_void_p, C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_render_view_device": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rm_render_lens": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), _P(RmLens), C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_scene_query_count": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),
     "rm_scene_accel_status": (C.c_int, [C.c_int64, _P(C.c_int32)]),
     "rm_scene_walk_stats": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),

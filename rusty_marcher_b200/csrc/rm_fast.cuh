@@ -801,6 +801,107 @@ RM_HD Vec3<float> cast_glass_impl(const FV& fv, const FrameParams<float>& fp, co
         }
     }
 }
+// renderer.rs:254-309 from a given ray (o, d) whose level-1 hit an FP32 query found: t1 (unit direction), slot1, id1 -- the
+// thin-lens camera's sample rays (lens_shade below).  The loop is cast_glass_impl's, kept as a copy of its own: sharing it
+// through one more inlined call changes the machine code of a pre-existing kernel instantiation.
+template <typename G, class FV>
+RM_HD Vec3<float> cast_glass_from(const FV& fv, const FrameParams<float>& fp, Vec3<G> o, Vec3<G> d, const float t1, const int slot1,
+                                  const int id1) {
+    struct Frame {
+        Vec3<float> c;
+        Vec3<G> ro, rd;
+        float k;
+        int state;   // bit0: a refracted ray is pending, bit1: the refracted ray is the one in flight
+    };
+    Frame fr[kMaxDepth];
+    int sp = 0;
+    const Vec3<float> bg = {fp.background, fp.background, fp.background};
+    Counters<false> st;
+    Vec3<float> v;
+    for (;;) {
+        const int level = sp + 1;                               // n_recursion
+        if (level > fp.max_depth) {
+            v = bg;                                             // renderer.rs:262-264
+        } else {
+            const Vec3<float> o32 = to_f32(o), d32 = to_f32(d);
+            HitRec<float> h;
+            bool got = true;
+            if (level == 1) {
+                h.dist = t1;
+                h.slot = slot1;
+                h.id = id1;
+            } else {
+                got = fv.template closest<false>(o32, d32, level, h, st);      // renderer.rs:266: the search, FP32
+            }
+            if (!got) {
+                v = bg;                                         // renderer.rs:300-306 (level > 1 here)
+            } else {
+                Vec3<G> p, n;
+                Vec3<float> p32, n32;
+                if constexpr (sizeof(G) == 8) {
+                    fv.refine(h.slot, o, d, (double)h.dist, p, n);
+                    p32 = to_f32(p);
+                    n32 = to_f32(n);
+                } else {
+                    fv.surface(h, o32, d32, n32);
+                    p32 = h.p;
+                    p = p32;
+                    n = n32;
+                }
+                const R4<float> ma = fv.mat_a[h.id];
+                const R4<float> mb = fv.mat_b[h.id];
+                Vec3<float> c = bg + fv.template direct<false>(o32, d32, p32, n32, ma, mb, st);   // renderer.rs:272-275
+                bool pushed = false;
+                if (fv.mat_f[h.id] & 1) {                       // renderer.rs:277
+                    Vec3<G> ro1, rd1, ro2, rd2;
+                    using N = typename std::conditional<sizeof(G) == 8, Fast64, Exact<float>>::type;
+                    const bool has_refl = reflect_ray<G, N>(d, p, n, (G)mb.w, ro1, rd1);  // renderer.rs:203-207
+                    const bool has_refr = refract_ray<G, N>(d, p, n, (G)mb.w, ro2, rd2);  // renderer.rs:235-239
+                    if (has_refl || has_refr) {
+                        RM_FAST_CHECK(sp < kMaxDepth);
+                        Frame& f = fr[sp];
+                        f.c = c;
+                        f.k = mb.z;
+                        if (has_refl) {
+                            f.state = has_refr ? 1 : 0;
+                            f.ro = ro2;
+                            f.rd = rd2;
+                            o = ro1;
+                            d = rd1;
+                        } else {
+                            f.state = 2;
+                            o = ro2;
+                            d = rd2;
+                        }
+                        sp++;
+                        pushed = true;
+                    }
+                }
+                if (pushed) continue;
+                v = c;
+            }
+        }
+        for (;;) {                                              // return v to the callers on the stack
+            if (sp == 0) return v;
+            Frame& f = fr[sp - 1];
+            if (f.state & 2) {
+                f.c = f.c + scaled(v, 1.f - f.k);               // renderer.rs:249
+                v = f.c;
+                sp--;
+            } else {
+                f.c = f.c + scaled(v, f.k);                     // renderer.rs:219
+                if (f.state & 1) {
+                    o = f.ro;
+                    d = f.rd;
+                    f.state = 2;
+                    break;
+                }
+                v = f.c;
+                sp--;
+            }
+        }
+    }
+}
 template <class FV, class VW = NoView>
 RM_GLASS_FN Vec3<float> cast_glass64(const FV& fv, const FrameParams<float>& fp, const int x, const int y, const float t1,
                                      const int slot1, const int id1, const VW& vw = VW()) {
@@ -833,6 +934,21 @@ RM_HD Vec3<float> fast_shade(FV& fv, const FrameParams<float>& fp, const int x, 
     Counters<false> st;
     const Vec3<float> bg = {fp.background, fp.background, fp.background};
     return bg + fv.template direct<false>(fp.camera, d, h.p, normal, fv.mat_a[id], fv.mat_b[id], st);   // renderer.rs:272-275
+}
+
+// A sample ray (o, d) of the thin-lens camera (rm_render_lens) whose level-1 closest-hit query found h (FP32, on the ray
+// rounded to FP32): renderer.rs:254-309 from there.  kGlass as for fast_shade: the recursion with the f64 ray (GLASS_F64)
+// or its FP32 rounding (GLASS_F32), or the direct lighting alone (GLASS_NONE).
+template <int kGlass, class FV>
+RM_HD Vec3<float> lens_shade(const FV& fv, const FrameParams<float>& fp, const Vec3<double> o, const Vec3<double> d, HitRec<float> h) {
+    if constexpr (kGlass == GLASS_F64) return cast_glass_from<double>(fv, fp, o, d, h.dist, h.slot, h.id);
+    const Vec3<float> o32 = to_f32(o), d32 = to_f32(d);
+    if constexpr (kGlass == GLASS_F32) return cast_glass_from<float>(fv, fp, o32, d32, h.dist, h.slot, h.id);
+    Vec3<float> normal;
+    fv.surface(h, o32, d32, normal);
+    Counters<false> st;
+    const Vec3<float> bg = {fp.background, fp.background, fp.background};
+    return bg + fv.template direct<false>(o32, d32, h.p, normal, fv.mat_a[h.id], fv.mat_b[h.id], st);   // renderer.rs:272-275
 }
 
 }  // namespace rm

@@ -123,6 +123,11 @@ cudaError_t launch_adaptive_mark(const float* rgb, const int* id, int width, int
 cudaError_t launch_adaptive_subpixel(const DeviceScene<float>& ds, const FrameParams<float>& fp, bool cull, int samples,
                                      const unsigned* list, const unsigned* count, unsigned long long* next, float* sub,
                                      const double camera[3], cudaStream_t stream);
+// lens_kernel (rm_lens.cu; rm_render_lens): the n_px output pixels from frame row fp.row_begin of the thin-lens camera lc, each the
+//   resolve_box mean of its lc.samples^2 sample rays (rgb: n_px * 3 floats), their maximum into *dmax; *next: a zeroed
+//   64-bit work counter.
+cudaError_t launch_lens(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, bool cull, long long n_px,
+                        unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
 // adaptive_resolve_kernel: every listed pixel's resolve_box of its sub-pixel values into rgb (rows from lo), their maximum into
 //   *dmax; max_entries bounds *count (sizes the grid).
 cudaError_t launch_adaptive_resolve(const float* sub, int samples, const unsigned* list, const unsigned* count, float* rgb, int width,

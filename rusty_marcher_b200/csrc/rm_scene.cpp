@@ -571,4 +571,22 @@ int view_basis(const RmView& view, double out[9], const char** err) {
     return RM_OK;
 }
 
+LensCamera make_lens_camera(const RmParams& p, const double* basis, const RmLens& lens) {
+    LensCamera lc;
+    const int s = lens.samples;
+    lc.width = (double)s * p.width;
+    lc.height = (double)s * p.height;
+    lc.half_fov = std::tan(p.fov / 2.);                         // renderer.rs:25-33, as make_frame_params
+    lc.ratio = lc.width / lc.height;
+    for (int a = 0; a < 3; a++) lc.cam[a] = p.camera[a];
+    for (int k = 0; k < 9; k++) {
+        lc.view.m[k] = basis ? basis[k] : (k % 4 == 0 ? 1. : 0.);
+        lc.view.f[k] = (float)lc.view.m[k];
+    }
+    lc.aperture = lens.aperture;
+    lc.focus = lens.focus;
+    lc.samples = s;
+    return lc;
+}
+
 }  // namespace rm

@@ -120,4 +120,8 @@ template <typename R> FrameParams<R> make_frame_params(const RmParams& p);
 // rm_view_basis (include/rm_b200.h): u, v, w of the view into out[0..8], or RM_ERR_INVALID_ARGUMENT with a reason in err.
 int view_basis(const RmView& view, double out[9], const char** err);
 
+// The thin-lens camera of rm_render_lens for the frame of p: the s x frame's backproject operands, the camera, the basis
+// (u, v, w in basis[0..8], or the identity for null) and the lens.  The lens is taken as given (rm_render_lens checks it).
+LensCamera make_lens_camera(const RmParams& p, const double* basis, const RmLens& lens);
+
 }  // namespace rm

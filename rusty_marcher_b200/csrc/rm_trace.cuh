@@ -546,4 +546,48 @@ struct NoView {
 template <bool kView> struct ViewOf { typedef NoView type; };
 template <> struct ViewOf<true> { typedef ViewBasis type; };
 
+// Thin-lens camera (rm_render_lens, include/rm_b200.h RmLens): the normative definition in f64 without fused multiply-add.
+// The kernel, the host code and the tests' host emulation all call these two functions.
+// Lens point of sample (i, j) of s x s: the stratum (a, b) = ((i + j) mod s, j) -- shifted so that lens strata do not follow
+// the sub-pixel strata -- taken from the square to the unit disc by the elliptical grid map.  Only sqrt, which is correctly
+// rounded on host and device, so every restatement gets the same bits.
+RM_HD void lens_offset(const int s, const int i, const int j, double* lx, double* ly) {
+    const int a = (i + j) % s, b = j;
+    const double p = (2. * a + 1.) / s - 1., q = (2. * b + 1.) / s - 1.;
+    *lx = p * sqrt(1. - (q * q) * 0.5);
+    *ly = q * sqrt(1. - (p * p) * 0.5);
+}
+
+struct LensCamera {
+    double width, height;     // of the s x frame: backproject's operands (renderer.rs:128-135)
+    double half_fov, ratio;   // tan(fov / 2) and width / height (renderer.rs:25-33)
+    double cam[3];
+    ViewBasis view;           // u, v, w; the identity without a view
+    double aperture, focus;   // lens radius (>= 0) and distance of the plane in focus along the view axis (> 0)
+    int samples;              // s
+};
+
+// The ray (o, d) of sample (i, j) of output pixel (x, y): d0 is the supersampled frame's sub-pixel (s x + j, s y + i)
+// direction; through a lens of radius > 0 the ray leaves the lens point L = aperture (lx, ly, 0) towards the point
+// P = d0 focus / -d0.z of the plane in focus, which every sample of the pixel shares.
+RM_HD void lens_ray(const LensCamera& lc, const int x, const int y, const int i, const int j, Vec3<double>& o, Vec3<double>& d) {
+    const int s = lc.samples;
+    const Vec3<double> d0 = normalized(Vec3<double>{2. * ((double)(s * x + j) / lc.width - 0.5) * lc.half_fov * lc.ratio,
+                                                    -2. * ((double)(s * y + i) / lc.height - 0.5) * lc.half_fov, -1.});
+    if (lc.aperture == 0.) {
+        o = {lc.cam[0], lc.cam[1], lc.cam[2]};
+        d = lc.view.apply(d0);
+        return;
+    }
+    double lx, ly;
+    lens_offset(s, i, j, &lx, &ly);
+    const double k = lc.focus / (-d0.z);
+    const Vec3<double> P = {d0.x * k, d0.y * k, d0.z * k};
+    const double Lx = lc.aperture * lx, Ly = lc.aperture * ly;
+    const Vec3<double> e = normalized(Vec3<double>{P.x - Lx, P.y - Ly, P.z});
+    const double* m = lc.view.m;
+    o = {lc.cam[0] + (m[0] * Lx + m[3] * Ly), lc.cam[1] + (m[1] * Lx + m[4] * Ly), lc.cam[2] + (m[2] * Lx + m[5] * Ly)};
+    d = lc.view.apply(e);
+}
+
 }  // namespace rm
