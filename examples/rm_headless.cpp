@@ -18,6 +18,10 @@
 //   --aperture A --focus F             depth of field: a thin lens of radius A focused at distance F, --samples S x S rays
 //                                      per pixel through it (rm_render_lens; an extension).  Combines with --samples,
 //                                      --look-at / --up, --camera and --accel; not with --contrast, --f64 or --rows-f64
+//   --light-radius R[,R...]            soft shadows: every light a sphere of radius R (one value for all lights, or one per
+//                                      light in the scene's order), sampled at --samples S x S points of its disc
+//                                      (rm_render_area_lights; an extension).  Combines with --samples, --camera and --accel;
+//                                      not with --look-at, --aperture, --contrast, --f64 or --rows-f64
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -48,6 +52,8 @@ int main(int argc, char** argv) {
     RmView view = {{0., 0., -1.}, {0., 1., 0.}};
     bool use_lens = false, have_focus = false;
     RmLens lens = {0., 1., 1};
+    bool area = false;
+    std::vector<double> radii;
     auto triple = [](const char* s, double v[3]) { char end = 0; return std::sscanf(s, "%lf,%lf,%lf%c", &v[0], &v[1], &v[2], &end) == 3; };
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
@@ -66,6 +72,18 @@ int main(int argc, char** argv) {
         else if (a == "--contrast") { need(1); contrast = std::strtod(argv[++i], nullptr); adaptive = true; }
         else if (a == "--aperture") { need(1); lens.aperture = std::strtod(argv[++i], nullptr); use_lens = true; }
         else if (a == "--focus") { need(1); lens.focus = std::strtod(argv[++i], nullptr); have_focus = true; }
+        else if (a == "--light-radius") {
+            need(1);
+            area = true;
+            radii.clear();
+            for (const char* q = argv[++i];;) {
+                char* end = nullptr;
+                radii.push_back(std::strtod(q, &end));
+                if (end == q || (*end != ',' && *end != 0)) { std::fprintf(stderr, "rm_headless: --light-radius takes R[,R...]\n"); return 2; }
+                if (*end == 0) break;
+                q = end + 1;
+            }
+        }
         else if (a == "--look-at" || a == "--up") {
             need(1);
             if (!triple(argv[++i], a == "--up" ? view.up : target)) { std::fprintf(stderr, "rm_headless: %s takes X,Y,Z\n", a.c_str()); return 2; }
@@ -82,6 +100,10 @@ int main(int argc, char** argv) {
         return 2;
     }
     lens.samples = samples;
+    if (area && (look || use_lens || adaptive || f64 || rows64)) {
+        std::fprintf(stderr, "rm_headless: --light-radius does not combine with --look-at, --aperture, --contrast, --f64 or --rows-f64\n");
+        return 2;
+    }
     if (look && !use_lens && (samples > 1 || adaptive || rows64)) {
         std::fprintf(stderr, "rm_headless: --look-at does not combine with --samples, --contrast or --rows-f64\n");
         return 2;
@@ -108,6 +130,18 @@ int main(int argc, char** argv) {
     rm_builder_offset_camera(b, cam);
     RmScene scene = 0;
     if ((rc = rm_builder_upload(b, &scene)) != RM_OK) die("rm_scene_upload", rc);
+
+    RmAreaLights area_lights = {0, nullptr, samples};
+    if (area) {
+        const int n_lights = rm_builder_flatten(b)->n_lights;
+        if (radii.size() == 1) radii.assign(n_lights, radii[0]);
+        if ((int)radii.size() != n_lights) {
+            std::fprintf(stderr, "rm_headless: --light-radius takes one radius or %d (one per light)\n", n_lights);
+            return 2;
+        }
+        area_lights.n_lights = n_lights;
+        area_lights.radius = radii.data();
+    }
 
     RmParams p;
     rm_params_default(&p, width, height);                                  // fov 1.5 (main.rs:368), depth cap 3, background 0.1
@@ -141,7 +175,8 @@ int main(int argc, char** argv) {
     for (int f = 0; f < frames; f++) {
         const auto t0 = std::chrono::steady_clock::now();
         std::memset(&st, 0, sizeof st);
-        if (use_lens) rc = rm_render_lens(scene, &p, look ? &view : nullptr, &lens, rgb32.data(), f == frames - 1 ? rgb8.data() : nullptr, &st);
+        if (area) rc = rm_render_area_lights(scene, &p, &area_lights, rgb32.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
+        else if (use_lens) rc = rm_render_lens(scene, &p, look ? &view : nullptr, &lens, rgb32.data(), f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (look && f64) rc = rm_render_view_f64(scene, &p, &view, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (look) rc = rm_render_view(scene, &p, &view, rgb32.data(), nullptr, nullptr, &st);
         else if (f64) rc = rm_render_f64(scene, &p, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
@@ -153,7 +188,7 @@ int main(int argc, char** argv) {
         std::printf("Scene rendered in %lld ms (%u fps, %.2f MP/s)\n", ms, ms > 0 ? (unsigned)fps : 4294967295u, fps * (double)n_px / 1e6);
     }
     // "Save to file": normalize + to_vec on the device (framebuffer.rs:40-82), then the P6 stream (framebuffer.rs:26-38)
-    if (use_lens) {
+    if (use_lens || area) {
         // (the last frame above wrote the 8-bit frame)
     } else if (adaptive) {
         std::vector<unsigned char> mask(n_px, 0);

@@ -370,6 +370,56 @@ typedef struct RmLens {
 int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb,
                    uint8_t* out_rgb8, RmStats* stats);
 
+/* ---- extension mode: soft shadows -- spherical area lights ------------------------------------------------------------------ *
+ * The reference's lights are points, so every shadow has a hard edge.  This call gives each of the scene's lights a radius
+ * for one frame (the uploaded scene and its format do not change); a light of radius r > 0 casts a penumbra.
+ * Definition (normative; rm::light_frame / rm::light_sample in rm_trace.cuh are this in f64, and the tests' restatement over
+ * the oracle is the same).  Light l has position c, colour k, intensity I, radius r >= 0; s = samples.  The reference's
+ * direct_lighting (renderer.rs:138-193) runs at every shading point p with unit normal n, at every recursion level; lights
+ * are visited in scene order, as in the reference.
+ *   - r = 0: the reference's point light: its own term, one shadow ray.
+ *   - r > 0: the light is replaced at p by s^2 point lights q_ab, visited a = 0..s-1 (outer), b = 0..s-1 (inner).  Each
+ *     contributes exactly the reference's per-light term with position q_ab and colour k * (1 / (s*s)): light_dir =
+ *     normalized(q - p), side, the +-1e-3 shadow origin, the any-hit query with no maximum distance (an occluder beyond q
+ *     still shadows, as in the reference), then diffuse and specular added to the running sum in that order.
+ *   - Sample points, in f64 without fused multiply-add (Duff et al. 2017, "Building an orthonormal basis, revisited":
+ *     branch-free and defined for every unit m):
+ *       m = normalized(c - p)  (the reference's light_dir towards the centre);
+ *       sigma = copysign(1, m.z);  alpha = -1 / (sigma + m.z);  beta = (m.x*m.y) * alpha;
+ *       t1 = (1 + ((sigma*m.x)*m.x) * alpha, sigma*beta, -sigma*m.x);  t2 = (beta, sigma + (m.y*m.y) * alpha, -m.y);
+ *       (lx, ly) = rm::lens_offset(s, a, b)  (RmLens's unit-disc points, as they are);
+ *       q = c + r * ((lx*t1) + (ly*t2)), component by component in that order.
+ *     The points lie on the disc of radius r through c that faces p: the silhouette of a spherical light.
+ * Consequences:
+ *   - At s = 1 the only point is (0, 0): q = c and the colour is k, both exactly -- the reference's frame.  A call whose
+ *     radii are all 0 is the reference's frame as well.  Both are routed to rm_render and give its frame, ids and 8-bit
+ *     frame bit for bit.
+ *   - Primary visibility does not depend on the lights: out_prim_id is rm_render's, and lights stay invisible.
+ * FP32 production path (area_light_kernel): primary hits as rm_render's kernel finds them (the same device functions);
+ * m, t1, t2, q and the colour scale in FP32 from the FP32 shading point, every shadow ray through the FP32 any-hit query
+ * (brute force, or the hierarchy with accel != 0 and at most 8 lights; accel = 2 renders as accel = 1); frames meet the FP32
+ * parity criteria against the f64 definition.  cull_backfacing applies.  The cost grows with s^2 times the area lights.
+ * Rows, outputs and stats as rm_render_lens: patch rows [b, e) with patch_row_stride <= 1, rows outside untouched; out_rgb
+ * (H*W*3 floats) and / or out_rgb8 (H*W*3 bytes: normalize() + to_vec() of the output rows by their own maximum); out_prim_id
+ * (H*W, optional): rm_render's primary ids; stats: max_value, ms_render (device time of K0 and the traced rows: no tone map,
+ * no copies), ms_total, kernel_launches, resident_prims, d2h_bytes; no event counters.  Device memory: the output rows (and
+ * 4 bytes per light).  The call writes the caller's float frame, so the library forgets its previous deliveries into that
+ * memory (RM_ROWS_RETAINED).
+ * RM_ERR_INVALID_ARGUMENT: a NULL lights; a NULL radius with n_lights > 0; a radius that is negative or not finite; samples
+ * outside [1, 8]; precision other than RM_FP32; patch_row_stride > 1; max_depth < 1; out_rgb and out_rgb8 both NULL (all
+ * reported without a device); n_lights different from the scene's light count; an unknown scene.  RM_ERR_DIMENSIONS: as
+ * for rm_render.
+ * Out of scope: area lights with a view, a lens, supersampling, rm_render_adaptive, rm_render_dispersive, rm_render_rows_*
+ * or rm_render_frame; an FP64 entry point; random or per-pixel sampling patterns; shapes other than the facing disc; a
+ * radius stored in the scene. */
+typedef struct RmAreaLights {
+    int32_t       n_lights;  /* must equal the scene's light count */
+    const double* radius;    /* n_lights radii in the scene's light order: finite, >= 0 (0 = the reference's point light) */
+    int32_t       samples;   /* s in [1, 8] */
+} RmAreaLights;
+int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLights* lights, float* out_rgb, int32_t* out_prim_id,
+                          uint8_t* out_rgb8, RmStats* stats);
+
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device
  * scalar of the same type as d_rgb that receives max(previous value, tile max) -- zero it first.

@@ -177,6 +177,15 @@ pub struct RmLens {
     pub samples: i32,
 }
 
+/// spherical area lights of rm_render_area_lights: one radius per scene light (0: the reference's point light), s x s samples
+#[repr(C)]
+#[derive(Copy, Clone, Debug)]
+pub struct RmAreaLights {
+    pub n_lights: i32,
+    pub radius: *const f64,
+    pub samples: i32,
+}
+
 /// one frame on the GPUs of one box (one process per GPU)
 #[repr(C)]
 pub struct RmExchange {
@@ -230,6 +239,9 @@ extern "C" {
     /// depth of field: s x s sample rays per pixel through a thin lens, from the camera turned to `view` (null: down -z)
     pub fn rm_render_lens(scene: RmScene, params: *const RmParams, view: *const RmView, lens: *const RmLens, out_rgb: *mut f32,
                           out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
+    /// soft shadows: every light of radius r > 0 as s x s points of the disc of radius r facing the shading point
+    pub fn rm_render_area_lights(scene: RmScene, params: *const RmParams, lights: *const RmAreaLights, out_rgb: *mut f32,
+                                 out_prim_id: *mut i32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
     // ---- the hot path, device buffers
     pub fn rm_render_device(scene: RmScene, params: *const RmParams, d_rgb: *mut c_void, d_prim_id: *mut i32,
                             d_max: *mut c_void, stream: *mut c_void) -> c_int;

@@ -12,6 +12,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -1517,6 +1518,114 @@ int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, co
         stats->kernel_launches = launches;
         stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
         stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
+    }
+    return RM_OK;
+}
+
+// Extension mode (include/rm_b200.h): K0 writes this camera's raster records, area_light_kernel traces and shades the output
+// rows, then, for the 8-bit frame, the tone-map kernel.  s = 1 and all radii 0 are rm_render's frame and go there.  The
+// argument checks need no device, except the light count, which needs the scene.
+int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLights* lights, float* out_rgb, int32_t* out_prim_id,
+                          uint8_t* out_rgb8, RmStats* stats) {
+    if (!lights) return fail(RM_ERR_INVALID_ARGUMENT, "lights is null");
+    if (lights->n_lights < 0) return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must be >= 0");
+    if (lights->n_lights > 0 && !lights->radius) return fail(RM_ERR_INVALID_ARGUMENT, "lights: radius is null");
+    bool any_area = false;
+    for (int l = 0; l < lights->n_lights; l++) {
+        const double r = lights->radius[l];
+        if (!std::isfinite(r) || r < 0.) return fail(RM_ERR_INVALID_ARGUMENT, "lights: every radius must be finite and >= 0");
+        any_area |= r > 0.;
+    }
+    if (lights->samples < 1 || lights->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "lights: samples must be in [1, 8]");
+    int rc = check_params(params);
+    if (rc != RM_OK) return rc;
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights needs max_depth >= 1");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    {
+        std::lock_guard<std::mutex> lock(g.mu);
+        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+        auto it = g.scenes.find(scene);
+        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+        if ((size_t)lights->n_lights != it->second.flat.lights.size())
+            return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must equal the scene's light count");
+    }
+    // one sample at the centre, or only point lights: the reference's lighting, rm_render's frame bit for bit
+    if (lights->samples == 1 || !any_area) return rm_render(scene, params, out_rgb, out_prim_id, out_rgb8, stats);
+    std::lock_guard<std::mutex> lock(g.mu);
+    auto it = g.scenes.find(scene);
+    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    DevicePack<float>& dp = it->second.f32;
+    cudaStream_t s = g.stream;
+    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
+    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
+    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
+    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
+    const bool cull = params->cull_backfacing != 0;
+    const int n_lgt = lights->n_lights, S = lights->samples;
+    rm::AreaLights al = {};
+    std::vector<float> radius(std::max(n_lgt, 1), 0.f);
+    for (int l = 0; l < n_lgt; l++) {
+        const double r = lights->radius[l];
+        radius[l] = r > 0. ? std::max((float)std::min(r, (double)FLT_MAX), 1e-30f) : 0.f;
+    }
+    for (int a = 0; a < S; a++)
+        for (int b = 0; b < S; b++) {
+            double lx, ly;
+            rm::lens_offset(S, a, b, &lx, &ly);
+            al.off[2 * (a * S + b)] = (float)lx;
+            al.off[2 * (a * S + b) + 1] = (float)ly;
+        }
+    al.samples = S;
+    al.inv_ss = 1.f / (float)(S * S);
+    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
+    if (out_prim_id && (rc = g.prim.ensure(std::max<size_t>(n_px * 4, 16))) != RM_OK) return rc;
+    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
+    float* d_max = static_cast<float*>(g.small.p);
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
+    float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
+    al.radius = d_radius;
+    CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaEventRecord(g.ev[0], s));
+    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
+    CK(cudaEventRecord(g.ev[1], s));
+    int launches = 0;
+    if (rows) {
+        CK(rm::launch_prepare(dp.ds, cull, params->camera, s));
+        CK(rm::launch_area_lights(dp.ds, fp, al, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p),
+                                  out_prim_id ? static_cast<int*>(g.prim.p) : nullptr, d_max, params->camera, s));
+        launches += 2;
+    }
+    CK(cudaEventRecord(g.ev[2], s));
+    if (out_rgb8 && rows) {
+        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
+        launches++;
+    }
+    const size_t host_px = (size_t)fp.row_begin * fp.width;
+    if (out_rgb && n_px) {
+        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
+        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
+    }
+    if (out_prim_id && n_px) CK(cudaMemcpyAsync(out_prim_id + host_px, g.prim.p, n_px * 4, cudaMemcpyDeviceToHost, s));
+    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
+    float h_max = 0.f;
+    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
+    CK(cudaEventRecord(g.ev[3], s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) {
+        std::memset(stats, 0, sizeof(*stats));
+        stats->max_value = (double)h_max;
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
+        stats->ms_render = ms;
+        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
+        stats->ms_total = ms;
+        stats->kernel_launches = launches;
+        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_prim_id ? 4 : 0) + (out_rgb8 ? 3 : 0));
     }
     return RM_OK;
 }

@@ -951,4 +951,89 @@ RM_HD Vec3<float> lens_shade(const FV& fv, const FrameParams<float>& fp, const V
     return bg + fv.template direct<false>(o32, d32, h.p, normal, fv.mat_a[h.id], fv.mat_b[h.id], st);   // renderer.rs:272-275
 }
 
+// ---- spherical area lights (rm_render_area_lights, include/rm_b200.h RmAreaLights) -----------------------------------------
+template <class FV> struct WalksHierarchy;
+template <bool kBvh, bool kCount> struct WalksHierarchy<FastViewT<kBvh, kCount>> { static constexpr bool value = kBvh; };
+
+// The view the shading code (fast_shade, cast_glass_impl) sees on an area-light frame: closest-hit queries, surfaces and
+// materials are the wrapped FastViewT's; direct() replaces every light of radius r > 0 by its s^2 sample points
+// (light_frame / light_sample in FP32 from the FP32 shading point), each with the colour scaled by 1 / s^2.  FastViewT's
+// own direct() is left as it is: the kernels that use it keep their machine code.
+template <class FV> struct AreaView {
+    const FV* fv;
+    const AreaLights* al;
+    const R4<float>* mat_a;
+    const R4<float>* mat_b;
+    const int* mat_f;
+
+    RM_HD AreaView(const FV& v, const AreaLights& a) : fv(&v), al(&a), mat_a(v.mat_a), mat_b(v.mat_b), mat_f(v.mat_f) {}
+
+    template <bool S> RM_HD bool closest(const Vec3<float> o, const Vec3<float> d, int level, HitRec<float>& h, Counters<S>& st) const {
+        return fv->template closest<S>(o, d, level, h, st);
+    }
+    RM_HD unsigned anyhit2(const Vec3<float> oA, const Vec3<float> dA, const Vec3<float> oB, const Vec3<float> dB, unsigned need) const {
+        return fv->anyhit2(oA, dA, oB, dB, need);
+    }
+    RM_HD void refine(const int slot, const Vec3<double> o, const Vec3<double> d, const double t32, Vec3<double>& p, Vec3<double>& n) const {
+        fv->refine(slot, o, d, t32, p, n);
+    }
+    RM_HD void surface(HitRec<float>& h, const Vec3<float> o, const Vec3<float> d, Vec3<float>& normal) const { fv->surface(h, o, d, normal); }
+
+    // renderer.rs:138-193 with area lights: lights in scene order; a light of radius 0 is the reference's point light (one
+    // shadow ray), one of radius r > 0 is s^2 point lights q_ab (a outer, b inner) of colour k / s^2.  Every point light
+    // contributes FastViewT::direct's term (the same arithmetic); its shadow rays go two at a time through anyhit2, and the
+    // contributions are added in the normative order.
+    template <bool S> RM_HD Vec3<float> direct(const Vec3<float> /*origin*/, const Vec3<float> dir, const Vec3<float> point,
+                                               const Vec3<float> normal, const R4<float> ma, const R4<float> mb, Counters<S>&) const {
+        Vec3<float> acc = {0.f, 0.f, 0.f};
+        const Vec3<float> to_viewer = -dir;                       // (as FastViewT::direct)
+        const Vec3<float> kd = {ma.x, ma.y, ma.z};
+        const int ss = al->samples * al->samples;
+        auto light = [&](const int l) {
+            const R4<float> lp = fv->lgt_p[l];
+            const Vec3<float> c = {lp.x, lp.y, lp.z};
+            const float r = al->radius[l];
+            const bool area = r > 0.f;
+            Vec3<float> lc = xyz(fv->lgt_c[l]);
+            Vec3<float> t1 = {0.f, 0.f, 0.f}, t2 = {0.f, 0.f, 0.f};
+            if (area) {
+                light_frame<float>(normalized(Vec3<float>{c.x - point.x, c.y - point.y, c.z - point.z}), t1, t2);
+                lc = scaled(lc, al->inv_ss);
+            }
+            const int n = area ? ss : 1;
+            auto at = [&](const int k) { return area ? light_sample<float>(c, r, t1, t2, al->off[2 * k], al->off[2 * k + 1]) : c; };
+            for (int k = 0; k < n; k += 2) {
+                const bool two = k + 1 < n;
+                const Vec3<float> qA = at(k), qB = at(two ? k + 1 : k);
+                const Vec3<float> ldA = normalized(Vec3<float>{qA.x - point.x, qA.y - point.y, qA.z - point.z});   // renderer.rs:166
+                const Vec3<float> ldB = normalized(Vec3<float>{qB.x - point.x, qB.y - point.y, qB.z - point.z});
+                const float sideA = dot(ldA, normal), sideB = dot(ldB, normal);
+                const float offA = sideA < 0.f ? -1e-3f : 1e-3f, offB = sideB < 0.f ? -1e-3f : 1e-3f;    // renderer.rs:168-172
+                const Vec3<float> soA = axpy(point, normal, offA), soB = axpy(point, normal, offB);
+                const unsigned blocked = fv->anyhit2(soA, ldA, soB, ldB, two ? 3u : 1u);                 // renderer.rs:174-177
+#pragma unroll
+                for (int e = 0; e < 2; e++) {
+                    if ((e && !two) || (blocked >> e & 1)) continue;
+                    const Vec3<float> ld = e ? ldB : ldA;
+                    const float side = e ? sideB : sideA;
+                    acc = acc + scaled(scaled(lc * kd, fmaxf(side, 0.f)), lp.w);                          // renderer.rs:138-140, 181-183
+                    const Vec3<float> reflected = reflect(-ld, normal);                                   // renderer.rs:144-145
+                    const float sf = fmaxf(dot(reflected, to_viewer), 0.f);                               // renderer.rs:150
+                    acc = acc + scaled(lc, pow_nonneg(sf * mb.x, mb.y));                                  // renderer.rs:186-189
+                }
+            }
+        };
+        if constexpr (WalksHierarchy<FV>::value) {
+            // as FastViewT::direct: the lights as unrolled, guarded calls (a scene with more than kBvhMaxLights lights stays
+            // on brute force)
+#pragma unroll
+            for (int l = 0; l < kBvhMaxLights; l++)
+                if (l < fv->n_lgt) light(l);
+        } else {
+            for (int l = 0; l < fv->n_lgt; l++) light(l);
+        }
+        return scaled(acc, ma.w);                                                                     // renderer.rs:192
+    }
+};
+
 }  // namespace rm

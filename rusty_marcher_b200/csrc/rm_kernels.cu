@@ -1221,6 +1221,13 @@ cudaError_t launch_render(const DeviceScene<R>& ds, const FrameParams<R>& fp, bo
     return cudaGetLastError();
 }
 
+cudaError_t launch_prepare(const DeviceScene<float>& ds, bool cull, const double camera[3], cudaStream_t stream) {
+    const int n_tri = tri_count(ds.lay, cull);
+    prepare_raster_kernel<false><<<(std::max(n_tri, 1) + 127) / 128, 128, 0, stream>>>(ds.tri_src, n_tri, camera[0], camera[1], camera[2],
+                                                                                    ds.tri_r, nullptr, ViewBasis{});
+    return cudaGetLastError();
+}
+
 cudaError_t launch_tonemap_busy(const DeviceScene<float>& ds, const FrameParams<float>& fp, const float* rgb, const float* dmax,
                                 bool normalise, unsigned char* rgb8, cudaStream_t stream) {
     const int tiles_x = fp.width / kFastTile, n_tiles = tiles_x * fp.n_bands;

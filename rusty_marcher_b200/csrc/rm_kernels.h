@@ -128,6 +128,13 @@ cudaError_t launch_adaptive_subpixel(const DeviceScene<float>& ds, const FramePa
 //   64-bit work counter.
 cudaError_t launch_lens(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, bool cull, long long n_px,
                         unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
+// K0 alone (prepare_raster_kernel, no view): the raster records of `camera` for the kernels that run stage A without K1.
+cudaError_t launch_prepare(const DeviceScene<float>& ds, bool cull, const double camera[3], cudaStream_t stream);
+// area_light_kernel (rm_area.cu; rm_render_area_lights): after launch_prepare for the same camera, the n_px pixels from frame row
+//   fp.row_begin (n_px a multiple of 32): K1's primary hits shaded with the area lights al (rgb: n_px * 3 floats, prim_id:
+//   n_px ids or null), their maximum into *dmax; *next: a zeroed 64-bit work counter.
+cudaError_t launch_area_lights(const DeviceScene<float>& ds, const FrameParams<float>& fp, const AreaLights& al, bool cull, long long n_px,
+                               unsigned long long* next, float* rgb, int* prim_id, float* dmax, const double camera[3], cudaStream_t stream);
 // adaptive_resolve_kernel: every listed pixel's resolve_box of its sub-pixel values into rgb (rows from lo), their maximum into
 //   *dmax; max_entries bounds *count (sizes the grid).
 cudaError_t launch_adaptive_resolve(const float* sub, int samples, const unsigned* list, const unsigned* count, float* rgb, int width,

@@ -590,4 +590,33 @@ RM_HD void lens_ray(const LensCamera& lc, const int x, const int y, const int i,
     d = lc.view.apply(e);
 }
 
+// Spherical area lights (rm_render_area_lights, include/rm_b200.h RmAreaLights).  R = double is the normative definition
+// (no fused multiply-add: the library is compiled with -fmad=false); R = float is the production path's FP32 restatement.
+// The kernel, the host emulation and the tests all call these two functions.
+// light_frame: an orthonormal basis (m, t1, t2) around the unit vector m, branch-free and defined for every unit m
+// (Duff et al. 2017, "Building an orthonormal basis, revisited").
+template <typename R> RM_HD void light_frame(const Vec3<R> m, Vec3<R>& t1, Vec3<R>& t2) {
+    const R sigma = copysign(R(1), m.z);
+    const R alpha = R(-1) / (sigma + m.z);
+    const R beta = (m.x * m.y) * alpha;
+    t1 = {R(1) + ((sigma * m.x) * m.x) * alpha, sigma * beta, -sigma * m.x};
+    t2 = {beta, sigma + (m.y * m.y) * alpha, -m.y};
+}
+// light_sample: the point q = c + r ((lx t1) + (ly t2)) of the disc of radius r through the light's centre c, facing the
+// shading point ((lx, ly) = lens_offset(s, a, b): a point of the unit disc).
+template <typename R> RM_HD Vec3<R> light_sample(const Vec3<R> c, const R r, const Vec3<R> t1, const Vec3<R> t2, const R lx, const R ly) {
+    return {c.x + r * ((lx * t1.x) + (ly * t2.x)), c.y + r * ((lx * t1.y) + (ly * t2.y)), c.z + r * ((lx * t1.z) + (ly * t2.z))};
+}
+
+constexpr int kAreaMaxSamples = 8;
+// The call's lights as the FP32 path reads them: radius[l] > 0 for an area light (a positive radius too small for FP32 is
+// kept at 1e-30, so the light stays one of s^2 points), 0 for the reference's point light; off: the unit-disc points
+// (lx, ly) = lens_offset(s, a, b) of sample a s + b, rounded to FP32; inv_ss = 1 / (s * s) in FP32.
+struct AreaLights {
+    const float* radius;
+    float off[2 * kAreaMaxSamples * kAreaMaxSamples];
+    int samples;
+    float inv_ss;
+};
+
 }  // namespace rm

@@ -296,6 +296,55 @@ class Renderer:
         print(message)
         return message
 
+    def render_area_lights(self, frame, scene, radii, samples=4, prim_id=None, rgb8=None, patch_rows=(0, -1)):
+        """EXTENSION MODE (no reference counterpart): soft shadows.  Each of the scene's lights gets a radius for this frame
+        (`radii`: one number for every light, or one per light in the scene's order; finite, >= 0, 0 = the reference's point
+        light), and a light of radius r > 0 is sampled at samples x samples points of the disc of radius r that faces the
+        shading point, each with 1 / samples^2 of its colour (rm_render_area_lights).  samples = 1, or every radius 0, is
+        render()'s frame.  Fills frame.buffer (float32) over the rendered rows and, if given, prim_id (H, W) int32 (render()'s
+        primary ids) and rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the same kind of status message
+        as render()."""
+        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
+            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
+        n = len(scene.lights)
+        r = np.asarray(radii, dtype=np.float64)
+        if r.ndim == 0:
+            r = np.full(n, float(r))
+        if r.shape != (n,):
+            raise ValueError("radii must be one number or %d (one per light of the scene), got shape %s" % (n, r.shape))
+        if not (np.all(np.isfinite(r)) and np.all(r >= 0.)):
+            raise ValueError("every radius must be finite and >= 0, got %r" % (r.tolist(),))
+        if self.precision != _abi.RM_FP32:
+            raise ValueError("render_area_lights computes in RM_FP32")
+        if int(self.width) != frame.width or int(self.height) != frame.height:
+            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
+        if len(patch_rows) > 2 and patch_rows[2] > 1:
+            raise ValueError("render_area_lights renders contiguous patch rows (stride <= 1)")
+        for name, a, dtype, shape in (("prim_id", prim_id, np.int32, (frame.height, frame.width)),
+                                      ("rgb8", rgb8, np.uint8, (frame.height, frame.width, 3))):
+            if a is not None and (not isinstance(a, np.ndarray) or a.dtype != dtype or a.shape != shape or not a.flags.c_contiguous
+                                  or not a.flags.writeable):
+                raise ValueError("%s must be a writeable C-contiguous %s array of shape %s" % (name, np.dtype(dtype).name, shape))
+        r = np.ascontiguousarray(r)
+        lights = _abi.RmAreaLights()
+        lights.n_lights, lights.radius, lights.samples = n, r.ctypes.data_as(C.POINTER(C.c_double)), int(samples)
+        L = _abi.load()
+        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
+        now = time.perf_counter()
+        p = self.params(frame, scene, patch_rows)
+        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
+            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
+        stats = _abi.RmStats()
+        _abi.check(L.rm_render_area_lights(scene.device_handle(), C.byref(p), C.byref(lights), frame.buffer.ctypes.data,
+                                           prim_id.ctypes.data if prim_id is not None else None,
+                                           rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
+        self.last_stats = stats
+        ms = int((time.perf_counter() - now) * 1000)
+        fps = 1000. / ms if ms > 0 else float("inf")
+        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
+        print(message)
+        return message
+
 
 def _view(forward, up):
     fwd, u = [float(x) for x in forward], [float(x) for x in up]
