@@ -22,6 +22,10 @@
 //                                      light in the scene's order), sampled at --samples S x S points of its disc
 //                                      (rm_render_area_lights; an extension).  Combines with --samples, --camera and --accel;
 //                                      not with --look-at, --aperture, --contrast, --f64 or --rows-f64
+//   --roughness G                      rough glass: every ray a glass-like hit spawns turned within atan(G) of its ideal
+//                                      direction, --samples S x S rays per pixel (rm_render_rough_glass; an extension; G for
+//                                      every primitive).  Combines with --samples, --aperture / --focus, --look-at / --up,
+//                                      --camera and --accel; not with --light-radius, --contrast, --f64 or --rows-f64
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -54,6 +58,8 @@ int main(int argc, char** argv) {
     RmLens lens = {0., 1., 1};
     bool area = false;
     std::vector<double> radii;
+    bool rough = false;
+    double roughness = 0.;
     auto triple = [](const char* s, double v[3]) { char end = 0; return std::sscanf(s, "%lf,%lf,%lf%c", &v[0], &v[1], &v[2], &end) == 3; };
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
@@ -72,6 +78,7 @@ int main(int argc, char** argv) {
         else if (a == "--contrast") { need(1); contrast = std::strtod(argv[++i], nullptr); adaptive = true; }
         else if (a == "--aperture") { need(1); lens.aperture = std::strtod(argv[++i], nullptr); use_lens = true; }
         else if (a == "--focus") { need(1); lens.focus = std::strtod(argv[++i], nullptr); have_focus = true; }
+        else if (a == "--roughness") { need(1); roughness = std::strtod(argv[++i], nullptr); rough = true; }
         else if (a == "--light-radius") {
             need(1);
             area = true;
@@ -104,7 +111,11 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "rm_headless: --light-radius does not combine with --look-at, --aperture, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (look && !use_lens && (samples > 1 || adaptive || rows64)) {
+    if (rough && (area || adaptive || f64 || rows64)) {
+        std::fprintf(stderr, "rm_headless: --roughness does not combine with --light-radius, --contrast, --f64 or --rows-f64\n");
+        return 2;
+    }
+    if (look && !use_lens && !rough && (samples > 1 || adaptive || rows64)) {
         std::fprintf(stderr, "rm_headless: --look-at does not combine with --samples, --contrast or --rows-f64\n");
         return 2;
     }
@@ -143,6 +154,14 @@ int main(int argc, char** argv) {
         area_lights.radius = radii.data();
     }
 
+    std::vector<double> rough_g;
+    RmRoughGlass rough_glass = {0, nullptr, samples};
+    if (rough) {
+        rough_g.assign(rm_scene_num_prims(scene), roughness);
+        rough_glass.n_prims = (int)rough_g.size();
+        rough_glass.roughness = rough_g.data();
+    }
+
     RmParams p;
     rm_params_default(&p, width, height);                                  // fov 1.5 (main.rs:368), depth cap 3, background 0.1
     rm_builder_get_camera(b, p.camera);
@@ -175,7 +194,9 @@ int main(int argc, char** argv) {
     for (int f = 0; f < frames; f++) {
         const auto t0 = std::chrono::steady_clock::now();
         std::memset(&st, 0, sizeof st);
-        if (area) rc = rm_render_area_lights(scene, &p, &area_lights, rgb32.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
+        if (rough) rc = rm_render_rough_glass(scene, &p, look ? &view : nullptr, use_lens ? &lens : nullptr, &rough_glass, rgb32.data(),
+                                              f == frames - 1 ? rgb8.data() : nullptr, &st);
+        else if (area) rc = rm_render_area_lights(scene, &p, &area_lights, rgb32.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (use_lens) rc = rm_render_lens(scene, &p, look ? &view : nullptr, &lens, rgb32.data(), f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (look && f64) rc = rm_render_view_f64(scene, &p, &view, rgb64.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (look) rc = rm_render_view(scene, &p, &view, rgb32.data(), nullptr, nullptr, &st);
@@ -188,7 +209,7 @@ int main(int argc, char** argv) {
         std::printf("Scene rendered in %lld ms (%u fps, %.2f MP/s)\n", ms, ms > 0 ? (unsigned)fps : 4294967295u, fps * (double)n_px / 1e6);
     }
     // "Save to file": normalize + to_vec on the device (framebuffer.rs:40-82), then the P6 stream (framebuffer.rs:26-38)
-    if (use_lens || area) {
+    if (use_lens || area || rough) {
         // (the last frame above wrote the 8-bit frame)
     } else if (adaptive) {
         std::vector<unsigned char> mask(n_px, 0);

@@ -420,6 +420,67 @@ typedef struct RmAreaLights {
 int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLights* lights, float* out_rgb, int32_t* out_prim_id,
                           uint8_t* out_rgb8, RmStats* stats);
 
+/* ---- extension mode: rough glass -- blurred refraction and reflection ------------------------------------------------------ *
+ * The reference's glass refracts and reflects along ideal directions (optics.rs:8-89).  This call gives each primitive a
+ * roughness for one frame (the uploaded scene and its format do not change): every ray a rough glass-like hit spawns is
+ * spread over a cone, sampled s x s per pixel -- frosted glass.  reflect_ray spawns a ray only at total internal reflection,
+ * so on glass the visible effect is mostly in the refracted ray; the roughness applies to both.
+ * Definition (normative; rm::rough_dir / rm::rough_reflect_origin / rm::rough_refract_origin / rm::rough_offset in
+ * rm_trace.cuh are this, and the tests' restatement over the oracle is the same).  All in f64 without fused multiply-add;
+ * s = samples.
+ *   1. Sample (i, j) of output pixel (x, y), i, j in [0, s), is rm_render_lens's sample ray: rm::lens_ray with the view's
+ *      basis (the identity without a view) and the lens (aperture 0 without one).
+ *   2. The sample's value is the reference's cast_ray from that ray (renderer.rs:254-309, levels 1..max_depth) with one
+ *      change.  At a hit of recursion level L (1 = the sample ray's own hit) on a glass-like primitive k with
+ *      g = roughness[k] > 0, let (lx, ly) = rm::lens_offset(s, (j + L) mod s, i) -- stratum ((i + j + L) mod s, i), a bijection
+ *      over the s^2 samples at every level, different from the lens's strata and shifted per level.  If (lx, ly) != (0, 0),
+ *      each ray the reference spawns there (reflect_ray's and refract_ray's, whichever exist) is changed:
+ *        (t1, t2) = the basis of rd by RmAreaLights's formula (Duff et al. 2017) with m = rd;
+ *        rd' = normalized(rd + g * ((lx*t1) + (ly*t2))), component by component in that order (geometry.rs's scale(1/norm));
+ *        the origin by the producing function's own rule applied to rd': a reflected ray leaves from point - hit_normal*1e-4
+ *        if dot(rd', hit_normal) < 0, else from point + hit_normal*1e-4; a refracted ray, with `normal` the hit normal turned
+ *        against the incident ray, from point + normal*1e-4 if dot(rd', normal) > 0, else from point - normal*1e-4.
+ *      Whether a ray exists (total internal reflection) and the weights k and 1 - k are decided before the change, exactly as
+ *      the reference decides them.
+ *   3. The pixel is the FP32 mean of its s^2 sample values in rm_render_supersampled's order (sub-rows i outer, j inner).
+ * Consequences:
+ *   - The offset is orthogonal to rd and at most 1 long, so rd' is always defined and lies within atan(g) of rd: g is the
+ *     tangent of the blur cone's half-angle.
+ *   - g = 0, or an offset of (0, 0), leaves the ray bit for bit as the reference spawns it; at s = 1 the only offset is (0, 0).
+ *   - s = 1, all roughness 0, and roughness on no glass-like primitive (decided on the host from the scene's materials) give
+ *     rm_render_lens's frame bit for bit and are routed there (which routes aperture 0 without a view to
+ *     rm_render_supersampled).
+ *   - Primary visibility does not depend on roughness: only rays spawned at glass-like hits turn.
+ *   - The pattern is fixed per pixel, not random: the frame is deterministic.
+ * FP32 production path (rough_glass_kernel): lens_kernel's schedule; each sample ray from rm::lens_ray in f64, traced with the
+ * general FP32 closest-hit query (brute force, or the hierarchy with accel != 0; accel = 2 renders as accel = 1), the
+ * recursion with a roughness per primitive id in FP32 (a positive value too small for FP32 is kept at 1e-30).  The turn is
+ * computed in f64 from the f64 ray where the scene takes f64 ray geometry, in FP32 otherwise; frames meet the FP32 parity
+ * criteria against the f64 definition.  cull_backfacing applies.
+ * Rows, outputs and stats as rm_render_lens: patch rows [b, e) with patch_row_stride <= 1, rows outside untouched; out_rgb
+ * (H*W*3 floats) and / or out_rgb8 (H*W*3 bytes: normalize() + to_vec() of the output rows by their own maximum); stats:
+ * max_value, ms_render, ms_total, kernel_launches, resident_prims, d2h_bytes.  Device memory: the output rows and 4 bytes per
+ * primitive.  The call writes the caller's float frame, so the library forgets its previous deliveries into that memory
+ * (RM_ROWS_RETAINED).
+ * RM_ERR_INVALID_ARGUMENT: a NULL rough; n_prims < 0, or a NULL roughness with n_prims > 0; a roughness that is negative or
+ * not finite; samples outside [1, 8]; an invalid view or lens by rm_render_lens's rules; lens->samples != rough->samples;
+ * precision other than RM_FP32; patch_row_stride > 1; max_depth < 1; out_rgb and out_rgb8 both NULL (all reported without
+ * a device); n_prims different from rm_scene_num_prims(scene); an unknown scene.  RM_ERR_DIMENSIONS: as for
+ * rm_render_supersampled.
+ * Out of scope: roughness with area lights, rm_render_adaptive, rm_render_dispersive, rm_render_rows_* or rm_render_frame;
+ * an FP64 entry point; random or per-pixel patterns and lobes other than the uniform-disc cone; roughness stored in the
+ * uploaded scene; per-channel roughness. */
+typedef struct RmRoughGlass {
+    int32_t       n_prims;    /* must equal rm_scene_num_prims(scene) */
+    const double* roughness;  /* n_prims values in primitive-id order (shapes in scene order, an Obj once per triangle):
+                                 finite, >= 0; 0 = the reference's ideal refraction / reflection.  Read only for glass-like
+                                 primitives: opaque hits spawn no ray (renderer.rs:277) */
+    int32_t       samples;    /* s in [1, 8] */
+} RmRoughGlass;
+int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* view /* NULL = the reference's camera */,
+                          const RmLens* lens /* NULL = pinhole */, const RmRoughGlass* rough, float* out_rgb,
+                          uint8_t* out_rgb8, RmStats* stats);
+
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device
  * scalar of the same type as d_rgb that receives max(previous value, tile max) -- zero it first.

@@ -186,6 +186,15 @@ pub struct RmAreaLights {
     pub samples: i32,
 }
 
+/// rough glass of rm_render_rough_glass: one roughness per primitive id (0: the reference's ideal optics), s x s samples
+#[repr(C)]
+#[derive(Copy, Clone, Debug)]
+pub struct RmRoughGlass {
+    pub n_prims: i32,
+    pub roughness: *const f64,
+    pub samples: i32,
+}
+
 /// one frame on the GPUs of one box (one process per GPU)
 #[repr(C)]
 pub struct RmExchange {
@@ -242,6 +251,9 @@ extern "C" {
     /// soft shadows: every light of radius r > 0 as s x s points of the disc of radius r facing the shading point
     pub fn rm_render_area_lights(scene: RmScene, params: *const RmParams, lights: *const RmAreaLights, out_rgb: *mut f32,
                                  out_prim_id: *mut i32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
+    /// rough glass: the rays a glass-like hit spawns spread over a cone of half-angle atan(roughness), s x s samples per pixel
+    pub fn rm_render_rough_glass(scene: RmScene, params: *const RmParams, view: *const RmView, lens: *const RmLens,
+                                 rough: *const RmRoughGlass, out_rgb: *mut f32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
     // ---- the hot path, device buffers
     pub fn rm_render_device(scene: RmScene, params: *const RmParams, d_rgb: *mut c_void, d_prim_id: *mut i32,
                             d_max: *mut c_void, stream: *mut c_void) -> c_int;

@@ -156,6 +156,7 @@ struct Context {
     Scratch sub;                      // rm_render_supersampled: the s x frame before the resolve; rm_render_adaptive: the
                                       // sub-pixel values of the refined pixels
     Scratch adapt;                    // rm_render_adaptive: the mask bytes and the list of refined pixels
+    Scratch rough;                    // rm_render_rough_glass: one FP32 roughness per primitive id
     Scratch pack;                     // host delivery: the busy tiles of a frame, packed in schedule order
     std::vector<Arena> arena_cache;   // device allocations of freed scenes, for the next upload
     // Host packs of the last few scenes by content (SURVEY.md 8f row 2, ingest): a caller that hands over the same scene
@@ -1030,6 +1031,7 @@ void rm_shutdown(void) {
     g.arena_cache.clear();
     g.pack_cache.clear();
     g.rgb.release(); g.prim.release(); g.rgb8.release(); g.small.release(); g.mix.release(); g.pack.release(); g.sub.release(); g.adapt.release();
+    g.rough.release();
     g.h_stage.release(); g.h_order.release(); g.h_upload.release(); g.h_early.release();
     if (g.side_stream) cudaStreamDestroy(g.side_stream);
     g.side_stream = nullptr;
@@ -1441,16 +1443,22 @@ int rm_render_adaptive(RmScene scene, const RmParams* params, int samples, doubl
 
 // Extension mode (include/rm_b200.h): lens_kernel traces and resolves the output rows, then, for the 8-bit frame, the
 // tone-map kernel.  The argument checks need no device.
-int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb, uint8_t* out_rgb8,
-                   RmStats* stats) {
+int check_lens(const RmLens* lens) {
     if (!lens) return fail(RM_ERR_INVALID_ARGUMENT, "lens is null");
     if (lens->samples < 1 || lens->samples > 8) return fail(RM_ERR_INVALID_ARGUMENT, "lens: samples must be in [1, 8]");
     if (!std::isfinite(lens->aperture) || !std::isfinite(lens->focus)) return fail(RM_ERR_INVALID_ARGUMENT, "lens: aperture and focus must be finite");
     if (lens->aperture < 0.) return fail(RM_ERR_INVALID_ARGUMENT, "lens: aperture must be >= 0");
     if (lens->focus <= 0.) return fail(RM_ERR_INVALID_ARGUMENT, "lens: focus must be > 0");
+    return RM_OK;
+}
+
+int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb, uint8_t* out_rgb8,
+                   RmStats* stats) {
+    int rc = check_lens(lens);
+    if (rc != RM_OK) return rc;
     rm::ViewBasis vb;
     bool identity = true;
-    int rc = view ? kernel_view(view, vb, &identity) : RM_OK;
+    rc = view ? kernel_view(view, vb, &identity) : RM_OK;
     if (rc != RM_OK) return rc;
     if ((rc = check_params(params)) != RM_OK) return rc;
     if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_lens computes in RM_FP32");
@@ -1626,6 +1634,126 @@ int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLig
         stats->kernel_launches = launches;
         stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
         stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_prim_id ? 4 : 0) + (out_rgb8 ? 3 : 0));
+    }
+    return RM_OK;
+}
+
+// is_glass_like of every primitive id (shapes in scene order, an Obj once per triangle)
+std::vector<unsigned char> glass_like_by_id(const rm::OwnedFlatScene& f) {
+    std::vector<unsigned char> out;
+    for (const RmShapeRef& sh : f.shapes) {
+        if (sh.kind == RM_SHAPE_SPHERE) out.push_back(f.spheres[sh.index].reflectance.is_glass_like != 0);
+        else if (sh.kind == RM_SHAPE_POLYGON) out.push_back(f.polygons[sh.index].reflectance.is_glass_like != 0);
+        else {
+            const RmObj& o = f.objs[sh.index];
+            for (int t = 0; t < o.n_triangles; t++) out.push_back(f.triangle_reflectances[o.first_triangle + t].is_glass_like != 0);
+        }
+    }
+    return out;
+}
+
+// Extension mode (include/rm_b200.h): rough_glass_kernel traces and resolves the output rows, then, for the 8-bit frame, the
+// tone-map kernel.  s = 1, and calls in which no glass-like primitive is rough, are rm_render_lens's frame and go there.  The
+// argument checks need no device, except the primitive count, which needs the scene.
+int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, const RmRoughGlass* rough,
+                          float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
+    if (!rough) return fail(RM_ERR_INVALID_ARGUMENT, "rough is null");
+    if (rough->n_prims < 0) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must be >= 0");
+    if (rough->n_prims > 0 && !rough->roughness) return fail(RM_ERR_INVALID_ARGUMENT, "rough: roughness is null");
+    for (int k = 0; k < rough->n_prims; k++) {
+        const double g = rough->roughness[k];
+        if (!std::isfinite(g) || g < 0.) return fail(RM_ERR_INVALID_ARGUMENT, "rough: every roughness must be finite and >= 0");
+    }
+    if (rough->samples < 1 || rough->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must be in [1, 8]");
+    const int S = rough->samples;
+    const RmLens pinhole = {0., 1., S};
+    int rc = check_lens(lens ? lens : &pinhole);
+    if (rc != RM_OK) return rc;
+    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must equal lens->samples");
+    rm::ViewBasis vb;
+    bool identity = true;
+    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
+    if ((rc = check_params(params)) != RM_OK) return rc;
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_rough_glass computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_rough_glass renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_rough_glass needs max_depth >= 1");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
+    RmParams sp = *params;
+    sp.width = S * params->width;
+    sp.height = S * params->height;
+    sp.patch_row_begin = 0;
+    sp.patch_row_end = -1;
+    if ((rc = check_params(&sp)) != RM_OK) return rc;
+    const RmLens& ln = lens ? *lens : pinhole;
+    bool any_rough = false;
+    {
+        std::lock_guard<std::mutex> lock(g.mu);
+        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+        auto it = g.scenes.find(scene);
+        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+        if (rough->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must equal the scene's primitive count");
+        const std::vector<unsigned char> glass = glass_like_by_id(it->second.flat);
+        for (int k = 0; k < rough->n_prims && !any_rough; k++) any_rough = glass[k] && rough->roughness[k] > 0.;
+    }
+    // one sample (its offset is (0, 0)), or no rough glass-like primitive: no ray is turned, rm_render_lens's frame bit for bit
+    if (S == 1 || !any_rough) return rm_render_lens(scene, params, view, &ln, out_rgb, out_rgb8, stats);
+    std::lock_guard<std::mutex> lock(g.mu);
+    auto it = g.scenes.find(scene);
+    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    DevicePack<float>& dp = it->second.f32;
+    cudaStream_t s = g.stream;
+    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
+    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
+    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
+    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const bool cull = params->cull_backfacing != 0;
+    std::vector<float> gf;
+    rm::RoughGlass rg = rm::make_rough_glass(S, rough->roughness, rough->n_prims, gf);
+    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
+    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
+    if ((rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
+    float* d_max = static_cast<float*>(g.small.p);
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
+    rg.g = static_cast<const float*>(g.rough.p);
+    CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaEventRecord(g.ev[0], s));
+    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
+    CK(cudaEventRecord(g.ev[1], s));
+    int launches = 0;
+    if (rows) {
+        CK(rm::launch_rough_glass(dp.ds, fp, lc, rg, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
+        launches++;
+    }
+    CK(cudaEventRecord(g.ev[2], s));
+    if (out_rgb8 && rows) {
+        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
+        launches++;
+    }
+    const size_t host_px = (size_t)fp.row_begin * fp.width;
+    if (out_rgb && n_px) {
+        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
+        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
+    }
+    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
+    float h_max = 0.f;
+    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
+    CK(cudaEventRecord(g.ev[3], s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) {
+        std::memset(stats, 0, sizeof(*stats));
+        stats->max_value = (double)h_max;
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
+        stats->ms_render = ms;
+        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
+        stats->ms_total = ms;
+        stats->kernel_launches = launches;
+        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
     }
     return RM_OK;
 }

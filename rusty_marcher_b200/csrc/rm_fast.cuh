@@ -951,6 +951,144 @@ RM_HD Vec3<float> lens_shade(const FV& fv, const FrameParams<float>& fp, const V
     return bg + fv.template direct<false>(o32, d32, h.p, normal, fv.mat_a[h.id], fv.mat_b[h.id], st);   // renderer.rs:272-275
 }
 
+// ---- rough glass (rm_render_rough_glass, include/rm_b200.h RmRoughGlass) --------------------------------------------------
+// cast_glass_from for sample (i, j) of the thin-lens camera with the call's roughness rg: at a glass-like hit of level L
+// whose primitive has g = rg.g[id] > 0, every ray the reference spawns is turned by rough_dir with the unit-disc point of
+// stratum ((i + j + L) mod s, i) and leaves from the origin its producing function picks for the new direction.  Whether a
+// ray exists and the weights k, 1 - k are the reference's, decided before the turn.  G = double: the turn in f64 from the f64
+// ray (rough_dir<double>, the normative definition); G = float: its FP32 restatement.  Kept apart from cast_glass_from so
+// that the lens kernel's machine code stays as it is.
+template <typename G, class FV>
+RM_HD Vec3<float> cast_glass_rough(const FV& fv, const FrameParams<float>& fp, const RoughGlass& rg, const int si, const int sj,
+                                   Vec3<G> o, Vec3<G> d, const float t1, const int slot1, const int id1) {
+    struct Frame {
+        Vec3<float> c;
+        Vec3<G> ro, rd;
+        float k;
+        int state;   // bit0: a refracted ray is pending, bit1: the refracted ray is the one in flight
+    };
+    Frame fr[kMaxDepth];
+    int sp = 0;
+    const Vec3<float> bg = {fp.background, fp.background, fp.background};
+    const int s = rg.samples;
+    Counters<false> st;
+    Vec3<float> v;
+    for (;;) {
+        const int level = sp + 1;                               // n_recursion
+        if (level > fp.max_depth) {
+            v = bg;                                             // renderer.rs:262-264
+        } else {
+            const Vec3<float> o32 = to_f32(o), d32 = to_f32(d);
+            HitRec<float> h;
+            bool got = true;
+            if (level == 1) {
+                h.dist = t1;
+                h.slot = slot1;
+                h.id = id1;
+            } else {
+                got = fv.template closest<false>(o32, d32, level, h, st);      // renderer.rs:266: the search, FP32
+            }
+            if (!got) {
+                v = bg;                                         // renderer.rs:300-306 (level > 1 here)
+            } else {
+                Vec3<G> p, n;
+                Vec3<float> p32, n32;
+                if constexpr (sizeof(G) == 8) {
+                    fv.refine(h.slot, o, d, (double)h.dist, p, n);
+                    p32 = to_f32(p);
+                    n32 = to_f32(n);
+                } else {
+                    fv.surface(h, o32, d32, n32);
+                    p32 = h.p;
+                    p = p32;
+                    n = n32;
+                }
+                const R4<float> ma = fv.mat_a[h.id];
+                const R4<float> mb = fv.mat_b[h.id];
+                Vec3<float> c = bg + fv.template direct<false>(o32, d32, p32, n32, ma, mb, st);   // renderer.rs:272-275
+                bool pushed = false;
+                if (fv.mat_f[h.id] & 1) {                       // renderer.rs:277
+                    Vec3<G> ro1, rd1, ro2, rd2;
+                    using N = typename std::conditional<sizeof(G) == 8, Fast64, Exact<float>>::type;
+                    const bool has_refl = reflect_ray<G, N>(d, p, n, (G)mb.w, ro1, rd1);  // renderer.rs:203-207
+                    const bool has_refr = refract_ray<G, N>(d, p, n, (G)mb.w, ro2, rd2);  // renderer.rs:235-239
+                    const float gf = rg.g[h.id];
+                    if (gf > 0.f && (has_refl || has_refr)) {
+                        const int k = ((sj + level) % s) * s + si;   // rough_offset(s, si, sj, level)
+                        G lx, ly;
+                        if constexpr (sizeof(G) == 8) {
+                            lx = rg.off[2 * k];
+                            ly = rg.off[2 * k + 1];
+                        } else {
+                            lx = rg.off32[2 * k];
+                            ly = rg.off32[2 * k + 1];
+                        }
+                        if (lx != G(0) || ly != G(0)) {
+                            if (has_refl) {
+                                rd1 = rough_dir<G>(rd1, (G)gf, lx, ly);
+                                ro1 = rough_reflect_origin<G>(p, n, rd1);
+                            }
+                            if (has_refr) {
+                                rd2 = rough_dir<G>(rd2, (G)gf, lx, ly);
+                                ro2 = rough_refract_origin<G>(p, n, d, rd2);
+                            }
+                        }
+                    }
+                    if (has_refl || has_refr) {
+                        RM_FAST_CHECK(sp < kMaxDepth);
+                        Frame& f = fr[sp];
+                        f.c = c;
+                        f.k = mb.z;
+                        if (has_refl) {
+                            f.state = has_refr ? 1 : 0;
+                            f.ro = ro2;
+                            f.rd = rd2;
+                            o = ro1;
+                            d = rd1;
+                        } else {
+                            f.state = 2;
+                            o = ro2;
+                            d = rd2;
+                        }
+                        sp++;
+                        pushed = true;
+                    }
+                }
+                if (pushed) continue;
+                v = c;
+            }
+        }
+        for (;;) {                                              // return v to the callers on the stack
+            if (sp == 0) return v;
+            Frame& f = fr[sp - 1];
+            if (f.state & 2) {
+                f.c = f.c + scaled(v, 1.f - f.k);               // renderer.rs:249
+                v = f.c;
+                sp--;
+            } else {
+                f.c = f.c + scaled(v, f.k);                     // renderer.rs:219
+                if (f.state & 1) {
+                    o = f.ro;
+                    d = f.rd;
+                    f.state = 2;
+                    break;
+                }
+                v = f.c;
+                sp--;
+            }
+        }
+    }
+}
+// Sample (i, j) of a rough-glass frame whose level-1 query found h: lens_shade with cast_glass_rough.  Every rough scene
+// has a glass-like primitive, so only the two glass modes exist.
+template <int kGlass, class FV>
+RM_HD Vec3<float> rough_shade(const FV& fv, const FrameParams<float>& fp, const RoughGlass& rg, const int i, const int j,
+                              const Vec3<double> o, const Vec3<double> d, HitRec<float> h) {
+    static_assert(kGlass == GLASS_F32 || kGlass == GLASS_F64, "rough glass is traced in a glass mode");
+    if constexpr (kGlass == GLASS_F64) return cast_glass_rough<double>(fv, fp, rg, i, j, o, d, h.dist, h.slot, h.id);
+    else return cast_glass_rough<float>(fv, fp, rg, i, j, to_f32(o), to_f32(d), h.dist, h.slot, h.id);
+}
+
 // ---- spherical area lights (rm_render_area_lights, include/rm_b200.h RmAreaLights) -----------------------------------------
 template <class FV> struct WalksHierarchy;
 template <bool kBvh, bool kCount> struct WalksHierarchy<FastViewT<kBvh, kCount>> { static constexpr bool value = kBvh; };

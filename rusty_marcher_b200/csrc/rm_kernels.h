@@ -128,6 +128,10 @@ cudaError_t launch_adaptive_subpixel(const DeviceScene<float>& ds, const FramePa
 //   64-bit work counter.
 cudaError_t launch_lens(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, bool cull, long long n_px,
                         unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
+// rough_glass_kernel (rm_rough.cu; rm_render_rough_glass): lens_kernel's frame with the reflect / refract recursion turned by the
+//   roughness rg (cast_glass_rough); rg.samples == lc.samples.
+cudaError_t launch_rough_glass(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const RoughGlass& rg,
+                               bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
 // K0 alone (prepare_raster_kernel, no view): the raster records of `camera` for the kernels that run stage A without K1.
 cudaError_t launch_prepare(const DeviceScene<float>& ds, bool cull, const double camera[3], cudaStream_t stream);
 // area_light_kernel (rm_area.cu; rm_render_area_lights): after launch_prepare for the same camera, the n_px pixels from frame row

@@ -2,6 +2,7 @@
 #include "rm_scene.h"
 
 #include <algorithm>
+#include <cfloat>
 #include <chrono>
 #include <cmath>
 #include <cstdio>
@@ -587,6 +588,27 @@ LensCamera make_lens_camera(const RmParams& p, const double* basis, const RmLens
     lc.focus = lens.focus;
     lc.samples = s;
     return lc;
+}
+
+RoughGlass make_rough_glass(const int samples, const double* roughness, const int n, std::vector<float>& g) {
+    g.assign(std::max(n, 1), 0.f);
+    for (int k = 0; k < n; k++) {
+        const double v = roughness[k];
+        g[k] = v > 0. ? std::max((float)std::min(v, (double)FLT_MAX), 1e-30f) : 0.f;
+    }
+    RoughGlass rg = {};
+    const int s = samples;
+    for (int a = 0; a < s; a++)
+        for (int b = 0; b < s; b++) {
+            double lx, ly;
+            lens_offset(s, a, b, &lx, &ly);
+            rg.off[2 * (a * s + b)] = lx;
+            rg.off[2 * (a * s + b) + 1] = ly;
+            rg.off32[2 * (a * s + b)] = (float)lx;
+            rg.off32[2 * (a * s + b) + 1] = (float)ly;
+        }
+    rg.samples = s;
+    return rg;
 }
 
 }  // namespace rm

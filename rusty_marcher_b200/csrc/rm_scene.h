@@ -124,4 +124,9 @@ int view_basis(const RmView& view, double out[9], const char** err);
 // (u, v, w in basis[0..8], or the identity for null) and the lens.  The lens is taken as given (rm_render_lens checks it).
 LensCamera make_lens_camera(const RmParams& p, const double* basis, const RmLens& lens);
 
+// The roughness of rm_render_rough_glass as the kernel reads it: g receives the n values in FP32 (a positive value too small
+// for FP32 kept at 1e-30, at least one entry), and the returned RoughGlass the unit-disc points of s x s; its g pointer is
+// left for the caller to set.  The values are taken as given (rm_render_rough_glass checks them).
+RoughGlass make_rough_glass(int samples, const double* roughness, int n, std::vector<float>& g);
+
 }  // namespace rm

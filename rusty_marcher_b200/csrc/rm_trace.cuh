@@ -619,4 +619,43 @@ struct AreaLights {
     float inv_ss;
 };
 
+// Rough glass (rm_render_rough_glass, include/rm_b200.h RmRoughGlass).  R = double is the normative definition (no fused
+// multiply-add); R = float is the GLASS_F32 path's FP32 restatement.  The kernel, the host emulation and the tests all call
+// these functions.
+// rough_dir: a ray direction rd spawned at a glass-like hit of roughness g, turned by the unit-disc point (lx, ly) in the
+// plane orthogonal to rd (light_frame's basis): normalized(rd + g ((lx t1) + (ly t2))).  The offset is orthogonal to rd and
+// at most 1 long, so the result lies within atan(g) of rd.  g = 0 or (lx, ly) = (0, 0) leave rd as it is, bit for bit.
+template <typename R> RM_HD Vec3<R> rough_dir(const Vec3<R> rd, const R g, const R lx, const R ly) {
+    if (!(g > R(0)) || (lx == R(0) && ly == R(0))) return rd;
+    Vec3<R> t1, t2;
+    light_frame<R>(rd, t1, t2);
+    return normalized(Vec3<R>{rd.x + g * ((lx * t1.x) + (ly * t2.x)), rd.y + g * ((lx * t1.y) + (ly * t2.y)),
+                              rd.z + g * ((lx * t1.z) + (ly * t2.z))});
+}
+// The origin of a turned ray, by the rule of the function that spawned it applied to the new direction rd:
+// reflect_ray's (optics.rs:41-45) against the hit normal, refract_ray's (optics.rs:82-86) against the normal turned against
+// the incident ray.
+template <typename R> RM_HD Vec3<R> rough_reflect_origin(const Vec3<R> point, const Vec3<R> hit_normal, const Vec3<R> rd) {
+    return dot(rd, hit_normal) < R(0) ? axmy(point, hit_normal, R(1e-4)) : axpy(point, hit_normal, R(1e-4));
+}
+template <typename R>
+RM_HD Vec3<R> rough_refract_origin(const Vec3<R> point, const Vec3<R> hit_normal, const Vec3<R> incident, const Vec3<R> rd) {
+    const Vec3<R> normal = -dot(hit_normal, incident) < R(0) ? -hit_normal : hit_normal;
+    return dot(rd, normal) > R(0) ? axpy(point, normal, R(1e-4)) : axmy(point, normal, R(1e-4));
+}
+// The unit-disc point of sample (i, j) of s x s at recursion level L (1 = the sample ray's own hit): lens_offset(s,
+// (j + L) mod s, i), the stratum ((i + j + L) mod s, i) -- a bijection over the s^2 samples at every level, shifted per
+// level and different from the lens's strata.
+RM_HD void rough_offset(const int s, const int i, const int j, const int level, double* lx, double* ly) {
+    lens_offset(s, (j + level) % s, i, lx, ly);
+}
+// The call's roughness as the kernel reads it: g[id] per primitive id in FP32 (a positive value too small for FP32 is kept
+// at 1e-30, so that it stays positive); off: lens_offset(s, a, b) of stratum a s + b in f64, and rounded to FP32 in off32.
+struct RoughGlass {
+    const float* g;
+    double off[2 * kAreaMaxSamples * kAreaMaxSamples];
+    float off32[2 * kAreaMaxSamples * kAreaMaxSamples];
+    int samples;
+};
+
 }  // namespace rm
