@@ -26,6 +26,11 @@
 //                                      direction, --samples S x S rays per pixel (rm_render_rough_glass; an extension; G for
 //                                      every primitive).  Combines with --samples, --aperture / --focus, --look-at / --up,
 //                                      --camera and --accel; not with --light-radius, --contrast, --f64 or --rows-f64
+//   --move K,X,Y,Z                     motion blur: shape K of the scene (in scene order; every triangle of an Obj) moves by
+//                                      (X, Y, Z) over the shutter, --samples S x S rays per pixel at S^2 times
+//                                      (rm_render_motion; an extension).  Combines with --samples, --aperture / --focus,
+//                                      --look-at / --up, --camera and --accel; not with --roughness, --light-radius,
+//                                      --contrast, --f64 or --rows-f64
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -60,6 +65,9 @@ int main(int argc, char** argv) {
     std::vector<double> radii;
     bool rough = false;
     double roughness = 0.;
+    bool moving = false;
+    int move_shape = -1;
+    double move_by[3] = {0., 0., 0.};
     auto triple = [](const char* s, double v[3]) { char end = 0; return std::sscanf(s, "%lf,%lf,%lf%c", &v[0], &v[1], &v[2], &end) == 3; };
     for (int i = 1; i < argc; i++) {
         const std::string a = argv[i];
@@ -79,6 +87,15 @@ int main(int argc, char** argv) {
         else if (a == "--aperture") { need(1); lens.aperture = std::strtod(argv[++i], nullptr); use_lens = true; }
         else if (a == "--focus") { need(1); lens.focus = std::strtod(argv[++i], nullptr); have_focus = true; }
         else if (a == "--roughness") { need(1); roughness = std::strtod(argv[++i], nullptr); rough = true; }
+        else if (a == "--move") {
+            need(1);
+            char end = 0;
+            if (std::sscanf(argv[++i], "%d,%lf,%lf,%lf%c", &move_shape, &move_by[0], &move_by[1], &move_by[2], &end) != 4) {
+                std::fprintf(stderr, "rm_headless: --move takes K,X,Y,Z\n");
+                return 2;
+            }
+            moving = true;
+        }
         else if (a == "--light-radius") {
             need(1);
             area = true;
@@ -115,7 +132,11 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "rm_headless: --roughness does not combine with --light-radius, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (look && !use_lens && !rough && (samples > 1 || adaptive || rows64)) {
+    if (moving && (rough || area || adaptive || f64 || rows64)) {
+        std::fprintf(stderr, "rm_headless: --move does not combine with --roughness, --light-radius, --contrast, --f64 or --rows-f64\n");
+        return 2;
+    }
+    if (look && !use_lens && !rough && !moving && (samples > 1 || adaptive || rows64)) {
         std::fprintf(stderr, "rm_headless: --look-at does not combine with --samples, --contrast or --rows-f64\n");
         return 2;
     }
@@ -162,6 +183,27 @@ int main(int argc, char** argv) {
         rough_glass.roughness = rough_g.data();
     }
 
+    std::vector<double> disp;
+    RmMotion motion = {0, nullptr, samples};
+    if (moving) {
+        const RmFlatScene* fs = rm_builder_flatten(b);
+        if (move_shape < 0 || move_shape >= fs->n_shapes) {
+            std::fprintf(stderr, "rm_headless: --move: the scene has shapes 0 to %d\n", fs->n_shapes - 1);
+            return 2;
+        }
+        disp.assign(3 * (size_t)rm_scene_num_prims(scene), 0.);
+        size_t first = 0;                                                  // primitive ids: shapes in order, an Obj per triangle
+        for (int k = 0; k <= move_shape; k++) {
+            const int n = fs->shapes[k].kind == RM_SHAPE_OBJ ? fs->objs[fs->shapes[k].index].n_triangles : 1;
+            if (k == move_shape)
+                for (int t = 0; t < n; t++)
+                    for (int c = 0; c < 3; c++) disp[3 * (first + t) + c] = move_by[c];
+            first += n;
+        }
+        motion.n_prims = rm_scene_num_prims(scene);
+        motion.displacement = disp.data();
+    }
+
     RmParams p;
     rm_params_default(&p, width, height);                                  // fov 1.5 (main.rs:368), depth cap 3, background 0.1
     rm_builder_get_camera(b, p.camera);
@@ -194,7 +236,9 @@ int main(int argc, char** argv) {
     for (int f = 0; f < frames; f++) {
         const auto t0 = std::chrono::steady_clock::now();
         std::memset(&st, 0, sizeof st);
-        if (rough) rc = rm_render_rough_glass(scene, &p, look ? &view : nullptr, use_lens ? &lens : nullptr, &rough_glass, rgb32.data(),
+        if (moving) rc = rm_render_motion(scene, &p, look ? &view : nullptr, use_lens ? &lens : nullptr, &motion, rgb32.data(),
+                                          f == frames - 1 ? rgb8.data() : nullptr, &st);
+        else if (rough) rc = rm_render_rough_glass(scene, &p, look ? &view : nullptr, use_lens ? &lens : nullptr, &rough_glass, rgb32.data(),
                                               f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (area) rc = rm_render_area_lights(scene, &p, &area_lights, rgb32.data(), nullptr, f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (use_lens) rc = rm_render_lens(scene, &p, look ? &view : nullptr, &lens, rgb32.data(), f == frames - 1 ? rgb8.data() : nullptr, &st);
@@ -209,7 +253,7 @@ int main(int argc, char** argv) {
         std::printf("Scene rendered in %lld ms (%u fps, %.2f MP/s)\n", ms, ms > 0 ? (unsigned)fps : 4294967295u, fps * (double)n_px / 1e6);
     }
     // "Save to file": normalize + to_vec on the device (framebuffer.rs:40-82), then the P6 stream (framebuffer.rs:26-38)
-    if (use_lens || area || rough) {
+    if (use_lens || area || rough || moving) {
         // (the last frame above wrote the 8-bit frame)
     } else if (adaptive) {
         std::vector<unsigned char> mask(n_px, 0);

@@ -481,6 +481,60 @@ int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* v
                           const RmLens* lens /* NULL = pinhole */, const RmRoughGlass* rough, float* out_rgb,
                           uint8_t* out_rgb8, RmStats* stats);
 
+/* ---- extension mode: motion blur -- primitives that move over the shutter interval ------------------------------------------ *
+ * The reference renders one instant.  This call gives each primitive a displacement for one frame (the uploaded scene and its
+ * format do not change): over the shutter it moves by that much, and the s x s samples of a pixel see it at s^2 different
+ * times -- moving objects smear along their path.  Translation only; lights and the camera do not move.
+ * Definition (normative; rm::motion_time in rm_trace.cuh is this, and the tests' restatement over the oracle is the same).  All
+ * in f64 without fused multiply-add; s = samples.
+ *   1. Motion.  Primitive k (primitive-id order: shapes in scene order, an Obj once per triangle) has the displacement v_k
+ *      (3 doubles): how far it moves over the whole shutter.  The uploaded scene is its pose at shutter time tau = 0.
+ *   2. Time of a sample.  Sample (i, j), i, j in [0, s), of output pixel (x, y) has the time stratum
+ *      m = s*((2i + j) mod s) + ((i + j) mod s) -- a bijection onto [0, s^2) for every s, since (a - b) mod s = i -- and the time
+ *      tau = (m + 0.5) / s^2 - 0.5, in (-1/2, 1/2) and symmetric about 0.  Every pixel uses the same pattern.
+ *   3. Scene at tau.  Primitive k is translated by tau*v_k, component by component: a sphere's centre becomes c + tau*v; a
+ *      triangle's or polygon's vertices (and its plane point) become each vertex + tau*v, its normal unchanged.  Translation
+ *      leaves normals alone, so the reference's world-z inside test and the hittable / back-facing / degenerate classes of a
+ *      planar primitive do not change.
+ *   4. The sample's value is the reference's cast_ray (renderer.rs:254-309, levels 1..max_depth) from rm_render_lens's sample
+ *      ray (rm::lens_ray with the view's basis -- the identity without a view -- and the lens -- aperture 0 without one), in the
+ *      scene at tau: the whole recursion and every shadow ray of the sample see the same tau.
+ *   5. The pixel is the FP32 mean of its s^2 sample values in rm_render_supersampled's order (sub-rows i outer, j inner).
+ * Consequences:
+ *   - At s = 1, tau = 0; with every displacement zero nothing moves.  Both give rm_render_lens's frame bit for bit and are
+ *     routed there (which routes aperture 0 without a view to rm_render_supersampled).
+ *   - A pixel none of whose samples meets a swept primitive -- directly, through the recursion or through a shadow ray -- is
+ *     rm_render_lens's pixel.
+ *   - The pattern is fixed, not random: the frame is deterministic.
+ * FP32 production path (motion_kernel): lens_kernel's schedule; each sample ray from rm::lens_ray in f64, each query at the
+ * sample's tau: primitive k is tested against the ray with its origin shifted to o - tau*v_k (v_k rounded to FP32) -- the same
+ * ray parameter t, and the unchanged per-primitive routines.  Brute force, or with accel != 0 a hierarchy over swept boxes
+ * (each primitive's box at tau = -1/2 united with its box at tau = +1/2), built on the host once per scene and displacements
+ * and kept (accel = 2 renders as accel = 1).  Frames meet the FP32 parity criteria against the f64 definition.
+ * cull_backfacing applies.
+ * Rows, outputs and stats as rm_render_lens: patch rows [b, e) with patch_row_stride <= 1, rows outside untouched; out_rgb
+ * (H*W*3 floats) and / or out_rgb8 (H*W*3 bytes: normalize() + to_vec() of the output rows by their own maximum); stats:
+ * max_value, ms_render, ms_total, kernel_launches, resident_prims, d2h_bytes.  Device memory: the output rows, 16 bytes per
+ * primitive and, with accel != 0, the swept hierarchy.  The call writes the caller's float frame, so the library forgets its
+ * previous deliveries into that memory (RM_ROWS_RETAINED).
+ * RM_ERR_INVALID_ARGUMENT: a NULL motion; n_prims < 0, or a NULL displacement with n_prims > 0; a displacement that is not
+ * finite; samples outside [1, 8]; an invalid view or lens by rm_render_lens's rules; lens->samples != motion->samples;
+ * precision other than RM_FP32; patch_row_stride > 1; max_depth < 1; out_rgb and out_rgb8 both NULL (all reported without a
+ * device); n_prims different from rm_scene_num_prims(scene); an unknown scene.  RM_ERR_DIMENSIONS: as for
+ * rm_render_supersampled.
+ * Out of scope: motion with rough glass, area lights, rm_render_adaptive, rm_render_dispersive, rm_render_rows_* or
+ * rm_render_frame; moving lights or a moving camera; rotation, scaling or curved paths; motion stored in the uploaded scene;
+ * an FP64 entry point; random or per-pixel time patterns. */
+typedef struct RmMotion {
+    int32_t       n_prims;       /* must equal rm_scene_num_prims(scene) */
+    const double* displacement;  /* 3 * n_prims values, x y z per primitive id (shapes in scene order, an Obj once per
+                                    triangle): finite; how far the primitive moves over the shutter */
+    int32_t       samples;       /* s in [1, 8] */
+} RmMotion;
+int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view /* NULL = the reference's camera */,
+                     const RmLens* lens /* NULL = pinhole */, const RmMotion* motion, float* out_rgb, uint8_t* out_rgb8,
+                     RmStats* stats);
+
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device
  * scalar of the same type as d_rgb that receives max(previous value, tile max) -- zero it first.

@@ -195,6 +195,15 @@ pub struct RmRoughGlass {
     pub samples: i32,
 }
 
+/// motion blur of rm_render_motion: one displacement (x, y, z) per primitive id over the shutter, s x s samples in time
+#[repr(C)]
+#[derive(Copy, Clone, Debug)]
+pub struct RmMotion {
+    pub n_prims: i32,
+    pub displacement: *const f64,
+    pub samples: i32,
+}
+
 /// one frame on the GPUs of one box (one process per GPU)
 #[repr(C)]
 pub struct RmExchange {
@@ -254,6 +263,9 @@ extern "C" {
     /// rough glass: the rays a glass-like hit spawns spread over a cone of half-angle atan(roughness), s x s samples per pixel
     pub fn rm_render_rough_glass(scene: RmScene, params: *const RmParams, view: *const RmView, lens: *const RmLens,
                                  rough: *const RmRoughGlass, out_rgb: *mut f32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
+    /// motion blur: every primitive translated by tau * displacement, the s x s samples of a pixel at s^2 times tau in (-1/2, 1/2)
+    pub fn rm_render_motion(scene: RmScene, params: *const RmParams, view: *const RmView, lens: *const RmLens,
+                            motion: *const RmMotion, out_rgb: *mut f32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
     // ---- the hot path, device buffers
     pub fn rm_render_device(scene: RmScene, params: *const RmParams, d_rgb: *mut c_void, d_prim_id: *mut i32,
                             d_max: *mut c_void, stream: *mut c_void) -> c_int;

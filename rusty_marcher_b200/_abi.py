@@ -90,6 +90,10 @@ class RmRoughGlass(C.Structure):
     _fields_ = [("n_prims", C.c_int32), ("roughness", C.POINTER(C.c_double)), ("samples", C.c_int32)]
 
 
+class RmMotion(C.Structure):
+    _fields_ = [("n_prims", C.c_int32), ("displacement", C.POINTER(C.c_double)), ("samples", C.c_int32)]
+
+
 RM_MAX_RANKS, RM_IPC_HANDLE_BYTES, RM_MAILBOX_BYTES = 16, 64, 512
 
 
@@ -139,6 +143,8 @@ SYMBOLS = {
     "rm_render_area_lights": (C.c_int, [C.c_int64, _P(RmParams), _P(RmAreaLights), C.c_void_p, C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_render_rough_glass": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), _P(RmLens), _P(RmRoughGlass), C.c_void_p, C.c_void_p,
                                         _P(RmStats)]),
+    "rm_render_motion": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), _P(RmLens), _P(RmMotion), C.c_void_p, C.c_void_p,
+                                   _P(RmStats)]),
     "rm_scene_query_count": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),
     "rm_scene_accel_status": (C.c_int, [C.c_int64, _P(C.c_int32)]),
     "rm_scene_walk_stats": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),

@@ -87,6 +87,8 @@ struct SceneEntry {
     // sequence number and buffers are kernel parameters -- and pushed into the instantiated graph with cudaGraphExecUpdate
     cudaGraphExec_t graph_exec = nullptr;
     long long frames = 0;
+    uint64_t hash[2] = {0, 0};        // the content key of its FP32 pack (pack_for), and with it of its motions
+    size_t hash_bytes = 0;
 };
 
 struct Scratch {
@@ -157,6 +159,23 @@ struct Context {
                                       // sub-pixel values of the refined pixels
     Scratch adapt;                    // rm_render_adaptive: the mask bytes and the list of refined pixels
     Scratch rough;                    // rm_render_rough_glass: one FP32 roughness per primitive id
+    // rm_render_motion: per (scene, displacements) by content -- the FP32 displacement of every primitive by the kernel's
+    // indices and, once a call walks the hierarchy, the swept hierarchy (a loop over frames with unchanged motion builds it
+    // once); the last few, most recent last.  Device copy of one of them in `motion`, [v | nodes | prims].
+    struct MotionEntry {
+        uint64_t key[4] = {0, 0, 0, 0};
+        size_t bytes = 0;
+        std::vector<rm::R4<float>> v;
+        double reach = 0.;
+        bool swept = false;
+        std::vector<rm::R4<float>> nodes;
+        std::vector<int> prims;
+        uint64_t serial = 0;
+    };
+    std::vector<MotionEntry> motion_cache;
+    uint64_t motion_serial = 0, motion_on_device = 0;
+    bool motion_on_device_swept = false;
+    Scratch motion;
     Scratch pack;                     // host delivery: the busy tiles of a frame, packed in schedule order
     std::vector<Arena> arena_cache;   // device allocations of freed scenes, for the next upload
     // Host packs of the last few scenes by content (SURVEY.md 8f row 2, ingest): a caller that hands over the same scene
@@ -333,6 +352,9 @@ template <> int pack_for<float>(SceneEntry& se, std::shared_ptr<rm::PackedScene<
     size_t bytes = 0;
     uint64_t h = 0, h2 = 0;
     hash_scene(se.flat, bytes, h, h2);
+    se.hash[0] = h;
+    se.hash[1] = h2;
+    se.hash_bytes = bytes;
     for (size_t i = 0; i < g.pack_cache.size(); i++)
         if (g.pack_cache[i].hash == h && g.pack_cache[i].hash2 == h2 && g.pack_cache[i].bytes == bytes) {
             out = g.pack_cache[i].pack;
@@ -1031,7 +1053,9 @@ void rm_shutdown(void) {
     g.arena_cache.clear();
     g.pack_cache.clear();
     g.rgb.release(); g.prim.release(); g.rgb8.release(); g.small.release(); g.mix.release(); g.pack.release(); g.sub.release(); g.adapt.release();
-    g.rough.release();
+    g.rough.release(); g.motion.release();
+    g.motion_cache.clear();
+    g.motion_on_device = 0;
     g.h_stage.release(); g.h_order.release(); g.h_upload.release(); g.h_early.release();
     if (g.side_stream) cudaStreamDestroy(g.side_stream);
     g.side_stream = nullptr;
@@ -1753,6 +1777,163 @@ int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* v
         stats->ms_total = ms;
         stats->kernel_launches = launches;
         stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
+    }
+    return RM_OK;
+}
+
+// Extension mode (include/rm_b200.h): motion_kernel traces and resolves the output rows, then, for the 8-bit frame, the
+// tone-map kernel.  s = 1 (every sample at tau = 0) and calls in which nothing moves are rm_render_lens's frame and go there.
+// The argument checks need no device, except the primitive count, which needs the scene.
+int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, const RmMotion* motion,
+                     float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
+    if (!motion) return fail(RM_ERR_INVALID_ARGUMENT, "motion is null");
+    if (motion->n_prims < 0) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must be >= 0");
+    if (motion->n_prims > 0 && !motion->displacement) return fail(RM_ERR_INVALID_ARGUMENT, "motion: displacement is null");
+    bool any_motion = false;
+    for (size_t k = 0; k < 3 * (size_t)motion->n_prims; k++) {
+        const double v = motion->displacement[k];
+        if (!std::isfinite(v)) return fail(RM_ERR_INVALID_ARGUMENT, "motion: every displacement must be finite");
+        any_motion |= v != 0.;
+    }
+    if (motion->samples < 1 || motion->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must be in [1, 8]");
+    const int S = motion->samples;
+    const RmLens pinhole = {0., 1., S};
+    int rc = check_lens(lens ? lens : &pinhole);
+    if (rc != RM_OK) return rc;
+    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal lens->samples");
+    rm::ViewBasis vb;
+    bool identity = true;
+    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
+    if ((rc = check_params(params)) != RM_OK) return rc;
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_motion computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_motion renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_motion needs max_depth >= 1");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
+    RmParams sp = *params;
+    sp.width = S * params->width;
+    sp.height = S * params->height;
+    sp.patch_row_begin = 0;
+    sp.patch_row_end = -1;
+    if ((rc = check_params(&sp)) != RM_OK) return rc;
+    const RmLens& ln = lens ? *lens : pinhole;
+    {
+        std::lock_guard<std::mutex> lock(g.mu);
+        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+        auto it = g.scenes.find(scene);
+        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+        if (motion->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must equal the scene's primitive count");
+    }
+    // one sample (its time is 0), or nothing moves: the scene is its uploaded pose, rm_render_lens's frame bit for bit
+    if (S == 1 || !any_motion) return rm_render_lens(scene, params, view, &ln, out_rgb, out_rgb8, stats);
+    std::lock_guard<std::mutex> lock(g.mu);
+    auto it = g.scenes.find(scene);
+    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    SceneEntry& se = it->second;
+    DevicePack<float>& dp = se.f32;
+    cudaStream_t s = g.stream;
+    if ((rc = ensure_pack<float>(se, dp)) != RM_OK) return rc;
+    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
+    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
+    const bool walk = fp.accel != 0 && dp.ds.bvh.n_nodes > 0 && dp.ds.lay.n_lgt <= rm::kBvhMaxLights;
+    // the motion's per-primitive data by content: found in the cache, or made now (the swept hierarchy only once a call walks)
+    const size_t disp_bytes = 3 * sizeof(double) * (size_t)motion->n_prims;
+    const uint64_t key[4] = {se.hash[0], se.hash[1], hash_bytes(motion->displacement, disp_bytes, 0x452821E638D01377ull),
+                             hash_bytes(motion->displacement, disp_bytes, 0xBE5466CF34E90C6Cull)};
+    const size_t key_bytes = se.hash_bytes + disp_bytes;
+    Context::MotionEntry* me = nullptr;
+    for (size_t i = 0; i < g.motion_cache.size(); i++)
+        if (std::equal(key, key + 4, g.motion_cache[i].key) && g.motion_cache[i].bytes == key_bytes) {
+            std::rotate(g.motion_cache.begin() + i, g.motion_cache.begin() + i + 1, g.motion_cache.end());   // most recent last
+            me = &g.motion_cache.back();
+            break;
+        }
+    std::shared_ptr<rm::PackedScene<float>> pack;
+    if (!me || (walk && !me->swept)) {
+        if ((rc = pack_for<float>(se, pack)) != RM_OK) return rc;
+    }
+    if (!me) {
+        if (g.motion_cache.size() >= 4) g.motion_cache.erase(g.motion_cache.begin());
+        g.motion_cache.emplace_back();
+        me = &g.motion_cache.back();
+        std::copy(key, key + 4, me->key);
+        me->bytes = key_bytes;
+        rm::motion_displacements(*pack, motion->displacement, me->v, me->reach);
+        me->serial = ++g.motion_serial;
+    }
+    if (walk && !me->swept) {
+        rm::build_swept_bvh(*pack, me->v, me->nodes, me->prims, &host_pool());
+        me->swept = true;
+    }
+    rm::Motion mo = rm::make_motion(S);
+    const rm::BlobLayout& L = dp.ds.lay;
+    const size_t v_bytes = me->v.size() * sizeof(rm::R4<float>);
+    const size_t n_bytes = me->nodes.size() * sizeof(rm::R4<float>), p_bytes = me->prims.size() * sizeof(int);
+    const size_t o_nodes = align256(v_bytes), o_prims = o_nodes + align256(n_bytes);
+    // the previous call has finished with the device copy (every call ends in a stream synchronisation)
+    if (g.motion_on_device != me->serial || (walk && !g.motion_on_device_swept)) {
+        if ((rc = g.motion.ensure(o_prims + std::max<size_t>(p_bytes, 16))) != RM_OK) return rc;
+        CK(cudaMemcpyAsync(g.motion.p, me->v.data(), v_bytes, cudaMemcpyHostToDevice, s));
+        if (me->swept) {
+            CK(cudaMemcpyAsync(static_cast<char*>(g.motion.p) + o_nodes, me->nodes.data(), n_bytes, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(static_cast<char*>(g.motion.p) + o_prims, me->prims.data(), p_bytes, cudaMemcpyHostToDevice, s));
+        }
+        g.motion_on_device = me->serial;
+        g.motion_on_device_swept = me->swept;
+    }
+    if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
+    const rm::R4<float>* dv = static_cast<const rm::R4<float>*>(g.motion.p);
+    mo.v_sph = dv;
+    mo.v_tri = dv + L.n_sph;
+    mo.v_pln = dv + L.n_sph + L.n_tri;
+    rm::DeviceScene<float> ds = dp.ds;                          // the scene's pack with the swept hierarchy
+    if (walk) {
+        ds.bvh.nodes = reinterpret_cast<const rm::R4<float>*>(static_cast<const char*>(g.motion.p) + o_nodes);
+        ds.bvh.prims = reinterpret_cast<const int*>(static_cast<const char*>(g.motion.p) + o_prims);
+        ds.bvh.n_nodes = (int)(me->nodes.size() / 4);
+    }
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const bool cull = params->cull_backfacing != 0;
+    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
+    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
+    float* d_max = static_cast<float*>(g.small.p);
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
+    CK(cudaEventRecord(g.ev[0], s));
+    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
+    CK(cudaEventRecord(g.ev[1], s));
+    int launches = 0;
+    if (rows) {
+        CK(rm::launch_motion(ds, fp, lc, mo, me->reach, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
+        launches++;
+    }
+    CK(cudaEventRecord(g.ev[2], s));
+    if (out_rgb8 && rows) {
+        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
+        launches++;
+    }
+    const size_t host_px = (size_t)fp.row_begin * fp.width;
+    if (out_rgb && n_px) {
+        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
+        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
+    }
+    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
+    float h_max = 0.f;
+    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
+    CK(cudaEventRecord(g.ev[3], s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) {
+        std::memset(stats, 0, sizeof(*stats));
+        stats->max_value = (double)h_max;
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
+        stats->ms_render = ms;
+        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
+        stats->ms_total = ms;
+        stats->kernel_launches = launches;
+        stats->resident_prims = L.n_sph + rm::plane_count<float>(L, cull);
         stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
     }
     return RM_OK;

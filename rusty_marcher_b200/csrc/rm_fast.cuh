@@ -1174,4 +1174,146 @@ template <class FV> struct AreaView {
     }
 };
 
+// ---- motion blur (rm_render_motion, include/rm_b200.h RmMotion) -------------------------------------------------------------
+// Primitive k at time tau is its uploaded pose translated by tau v_k.  A ray (o, d) meets it at parameter t exactly where the
+// ray (o - tau v_k, d) meets the unmoved primitive, so every per-primitive routine runs unchanged on the shifted origin.  A
+// zero displacement leaves the origin's bits as they are (o - tau * 0 would turn a -0 into +0 for tau < 0).
+template <typename R> RM_HD R motion_shift(const R o, const R tau, const float v) { return v != 0.f ? o - tau * (R)v : o; }
+template <typename R> RM_HD Vec3<R> motion_shift(const Vec3<R> o, const R tau, const R4<float> v) {
+    return {motion_shift<R>(o.x, tau, v.x), motion_shift<R>(o.y, tau, v.y), motion_shift<R>(o.z, tau, v.z)};
+}
+template <typename R> RM_HD Vec3<R> motion_unshift(const Vec3<R> p, const R tau, const R4<float> v) {
+    return {v.x != 0.f ? p.x + tau * (R)v.x : p.x, v.y != 0.f ? p.y + tau * (R)v.y : p.y, v.z != 0.f ? p.z + tau * (R)v.z : p.z};
+}
+
+// The view the shading code (lens_shade, cast_glass_from) sees on a motion frame at one sample's time tau: the wrapped
+// FastViewT's arrays, and every primitive tested with the ray origin shifted by its own displacement (FastViewT::tri_hit,
+// sphere_intersect, plane_intersect and, through the swept hierarchy, FastViewT::leaf_hit, all unchanged).  Surfaces and the
+// f64 refinement run FastViewT's own code on the shifted origin and shift the point back.  direct() is FastViewT::direct's
+// arithmetic with the shadow rays traced at the same tau, light by light (the same decisions and the same sums as its pairs).
+template <bool kBvh> struct MotionView {
+    using FV = FastViewT<kBvh, false>;
+    const FV* fv;
+    const Motion* mo;
+    float tau;
+    double tau64;
+    const R4<float>* mat_a;
+    const R4<float>* mat_b;
+    const int* mat_f;
+
+    RM_HD MotionView(const FV& v, const Motion& m, const int q)
+        : fv(&v), mo(&m), tau(m.tau32[q]), tau64(m.tau[q]), mat_a(v.mat_a), mat_b(v.mat_b), mat_f(v.mat_f) {}
+
+    RM_HD R4<float> vel_of_slot(const int slot) const {
+        if (slot < fv->n_sph) return mo->v_sph[slot];
+        if (slot < fv->n_sph + fv->n_tri) return mo->v_tri[slot - fv->n_sph];
+        return mo->v_pln[slot - fv->n_sph - fv->n_tri];
+    }
+    RM_HD R4<float> vel_of_entry(const int e) const {
+        const unsigned kind = (unsigned)e >> 30;
+        const int i = e & 0x3fffffff;
+        return kind == BVH_SPHERE ? mo->v_sph[i] : kind == BVH_TRI ? mo->v_tri[i] : mo->v_pln[i];
+    }
+
+    template <bool S> RM_HD bool closest(const Vec3<float> o, const Vec3<float> d, int /*level*/, HitRec<float>& h, Counters<S>& st) const {
+        bool hit = false;
+        if constexpr (kBvh) {
+            h.dist = INFINITY;
+            bvh_walk<false>(fv->bvh, o, d,
+                            [&](const int e) {
+                                float t;
+                                int slot, id;
+                                if (fv->leaf_hit(e, motion_shift(o, tau, vel_of_entry(e)), d, t, slot, id)) FV::keep(h, hit, t, slot, id);
+                                return false;
+                            },
+                            [&]() { return h.dist * 1.00001f; });
+            return hit;
+        }
+        for (int i = 0; i < fv->n_sph; i++) {
+            Cand<float> c;
+            if (sphere_intersect<S>(fv->sph[i], motion_shift(o, tau, mo->v_sph[i]), d, c, st)) FV::keep(h, hit, c.key, i, fv->sph_id[i]);
+        }
+        const R4<float>* g = fv->tri_g;
+        for (int j = 0; j < fv->n_tri; j++, g += 4) {
+            float t;
+            if (FV::tri_hit(g, motion_shift(o, tau, mo->v_tri[j]), d, t)) FV::keep(h, hit, t, fv->n_sph + j, FV::as_int(g[3].z));
+        }
+        for (int k = 0; k < fv->n_poly; k++) {
+            const int i = fv->poly_slot[k];
+            Cand<float> c;
+            if (plane_intersect<S>(fv->pln_n[i], fv->pln_c[i], fv->pln_v[i], fv->vert, motion_shift(o, tau, mo->v_pln[i]), d, c, st))
+                FV::keep(h, hit, c.key, fv->n_sph + fv->n_tri + i, fv->pln_id[i]);
+        }
+        return hit;
+    }
+
+    RM_HD bool anyhit(const Vec3<float> o, const Vec3<float> d) const {
+        if constexpr (kBvh) {
+            return bvh_walk<false>(fv->bvh, o, d,
+                                   [&](const int e) {
+                                       float t;
+                                       int slot, id;
+                                       return fv->leaf_hit(e, motion_shift(o, tau, vel_of_entry(e)), d, t, slot, id);
+                                   },
+                                   []() { return INFINITY; });
+        }
+        Counters<false> st;
+        Cand<float> c;
+        for (int i = 0; i < fv->n_sph; i++)
+            if (sphere_intersect<false>(fv->sph[i], motion_shift(o, tau, mo->v_sph[i]), d, c, st)) return true;
+        const R4<float>* g = fv->tri_g;
+        for (int j = 0; j < fv->n_tri; j++, g += 4) {
+            float t;
+            if (FV::tri_hit(g, motion_shift(o, tau, mo->v_tri[j]), d, t)) return true;
+        }
+        for (int k = 0; k < fv->n_poly; k++) {
+            const int i = fv->poly_slot[k];
+            if (plane_intersect<false>(fv->pln_n[i], fv->pln_c[i], fv->pln_v[i], fv->vert, motion_shift(o, tau, mo->v_pln[i]), d, c, st))
+                return true;
+        }
+        return false;
+    }
+
+    // renderer.rs:138-193: FastViewT::direct's terms, added in the same order
+    template <bool S> RM_HD Vec3<float> direct(const Vec3<float> /*origin*/, const Vec3<float> dir, const Vec3<float> point,
+                                               const Vec3<float> normal, const R4<float> ma, const R4<float> mb, Counters<S>&) const {
+        Vec3<float> acc = {0.f, 0.f, 0.f};
+        const Vec3<float> to_viewer = -dir;                       // (as FastViewT::direct)
+        const Vec3<float> kd = {ma.x, ma.y, ma.z};
+        auto light = [&](const int l) {
+            const R4<float> lp = fv->lgt_p[l];
+            const Vec3<float> ld = normalized(Vec3<float>{lp.x - point.x, lp.y - point.y, lp.z - point.z});   // renderer.rs:166
+            const float side = dot(ld, normal);
+            const float off = side < 0.f ? -1e-3f : 1e-3f;                                                 // renderer.rs:168-172
+            if (anyhit(axpy(point, normal, off), ld)) return;                                             // renderer.rs:174-177
+            const Vec3<float> lc = xyz(fv->lgt_c[l]);
+            acc = acc + scaled(scaled(lc * kd, fmaxf(side, 0.f)), lp.w);                                  // renderer.rs:138-140, 181-183
+            const Vec3<float> reflected = reflect(-ld, normal);                                           // renderer.rs:144-145
+            const float sf = fmaxf(dot(reflected, to_viewer), 0.f);                                       // renderer.rs:150
+            acc = acc + scaled(lc, pow_nonneg(sf * mb.x, mb.y));                                          // renderer.rs:186-189
+        };
+        if constexpr (kBvh) {
+            // as FastViewT::direct: the lights as unrolled, guarded calls (a scene with more than kBvhMaxLights lights stays on
+            // brute force)
+#pragma unroll
+            for (int l = 0; l < kBvhMaxLights; l++)
+                if (l < fv->n_lgt) light(l);
+        } else {
+            for (int l = 0; l < fv->n_lgt; l++) light(l);
+        }
+        return scaled(acc, ma.w);                                                                     // renderer.rs:192
+    }
+
+    RM_HD void surface(HitRec<float>& h, const Vec3<float> o, const Vec3<float> d, Vec3<float>& normal) const {
+        const R4<float> v = vel_of_slot(h.slot);
+        fv->surface(h, motion_shift(o, tau, v), d, normal);
+        h.p = motion_unshift(h.p, tau, v);
+    }
+    RM_HD void refine(const int slot, const Vec3<double> o, const Vec3<double> d, const double t32, Vec3<double>& p, Vec3<double>& n) const {
+        const R4<float> v = vel_of_slot(slot);
+        fv->refine(slot, motion_shift(o, tau64, v), d, t32, p, n);
+        p = motion_unshift(p, tau64, v);
+    }
+};
+
 }  // namespace rm

@@ -132,6 +132,12 @@ cudaError_t launch_lens(const DeviceScene<float>& ds, const FrameParams<float>& 
 //   roughness rg (cast_glass_rough); rg.samples == lc.samples.
 cudaError_t launch_rough_glass(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const RoughGlass& rg,
                                bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
+// motion_kernel (rm_motion.cu; rm_render_motion): lens_kernel's frame with every query of sample q at its time mo.tau[q]
+//   (MotionView); mo.samples == lc.samples.  ds carries the swept hierarchy; reach = the largest displacement component / 2,
+//   by which the primitives leave their uploaded pose (the glass mode's coordinate bound).
+cudaError_t launch_motion(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const Motion& mo,
+                          double reach, bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax,
+                          cudaStream_t stream);
 // K0 alone (prepare_raster_kernel, no view): the raster records of `camera` for the kernels that run stage A without K1.
 cudaError_t launch_prepare(const DeviceScene<float>& ds, bool cull, const double camera[3], cudaStream_t stream);
 // area_light_kernel (rm_area.cu; rm_render_area_lights): after launch_prepare for the same camera, the n_px pixels from frame row

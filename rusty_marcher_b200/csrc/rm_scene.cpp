@@ -267,6 +267,7 @@ template <> void write_fast<float>(const Buf<PlaneTmp>& pln, BlobLayout& L, unsi
     const auto t0 = std::chrono::steady_clock::now();
     out.bvh_depth = build_bvh(boxes, out.bvh_nodes, out.bvh_prims, &pool);
     out.hierarchy_build_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    out.bvh_boxes = std::move(boxes);
 }
 
 }  // namespace
@@ -609,6 +610,59 @@ RoughGlass make_rough_glass(const int samples, const double* roughness, const in
         }
     rg.samples = s;
     return rg;
+}
+
+void motion_displacements(const PackedScene<float>& ps, const double* disp, std::vector<R4<float>>& v, double& reach) {
+    const BlobLayout& L = ps.lay;
+    const unsigned char* b = ps.blob_data();
+    const int* sph_id = reinterpret_cast<const int*>(b + L.off_sph_id);
+    const R4<float>* tri_g = reinterpret_cast<const R4<float>*>(b + L.off_tri_g);
+    const int* pln_id = reinterpret_cast<const int*>(b + L.off_pln_id);
+    v.assign((size_t)L.n_sph + L.n_tri + L.n_pln + 1, R4<float>{0.f, 0.f, 0.f, 0.f});
+    reach = 0.;
+    auto put = [&](const size_t at, const int id) {
+        const double* q = disp + 3 * (size_t)id;
+        v[at] = {(float)q[0], (float)q[1], (float)q[2], 0.f};
+        for (int a = 0; a < 3; a++) reach = std::fmax(reach, 0.5 * std::fabs((double)(&v[at].x)[a]));
+    };
+    for (int i = 0; i < L.n_sph; i++) put((size_t)i, sph_id[i]);
+    for (int j = 0; j < L.n_tri; j++) {
+        int id;
+        std::memcpy(&id, &tri_g[4 * (size_t)j + 3].z, 4);
+        put((size_t)L.n_sph + j, id);
+    }
+    for (int i = 0; i < L.n_pln; i++) put((size_t)L.n_sph + L.n_tri + i, pln_id[i]);
+}
+
+Motion make_motion(const int samples) {
+    Motion mo = {};
+    const int s = samples;
+    for (int i = 0; i < s; i++)
+        for (int j = 0; j < s; j++) {
+            mo.tau[i * s + j] = motion_time(s, i, j);
+            mo.tau32[i * s + j] = (float)mo.tau[i * s + j];
+        }
+    mo.samples = s;
+    return mo;
+}
+
+int build_swept_bvh(const PackedScene<float>& ps, const std::vector<R4<float>>& v, std::vector<R4<float>>& nodes, std::vector<int>& prims,
+                    HostPool* pool) {
+    const BlobLayout& L = ps.lay;
+    Buf<BvhPrimBox> boxes(ps.bvh_boxes.size());
+    for (size_t k = 0; k < boxes.size(); k++) {
+        BvhPrimBox bx = ps.bvh_boxes[k];
+        const unsigned kind = (unsigned)bx.code >> 30;
+        const size_t i = (size_t)(bx.code & 0x3fffffff);
+        const R4<float>& d = v[kind == BVH_SPHERE ? i : kind == BVH_TRI ? L.n_sph + i : (size_t)L.n_sph + L.n_tri + i];
+        for (int a = 0; a < 3; a++) {
+            const double h = 0.5 * std::fabs((double)(&d.x)[a]);     // tau v for tau in [-1/2, 1/2]: at most |v| / 2 either way
+            bx.lo[a] -= h;
+            bx.hi[a] += h;
+        }
+        boxes[k] = bx;
+    }
+    return build_bvh(boxes, nodes, prims, pool);
 }
 
 }  // namespace rm

@@ -66,6 +66,12 @@ template <typename R> RM_HD int plane_count(const BlobLayout& L, bool cull) {
 RM_HD int tri_count(const BlobLayout& L, bool cull) { return cull ? L.n_tri_live : L.n_tri; }
 RM_HD int poly_count(const BlobLayout& L, bool cull) { return cull ? L.n_poly_live : L.n_poly; }
 
+// Bounds of one hittable primitive (f64, unpadded) and its entry code kind << 30 | index for the hierarchy's leaves.
+struct BvhPrimBox {
+    double lo[3], hi[3];
+    int code;
+};
+
 template <typename R> struct PackedScene {
     BlobLayout lay;
     Buf<BlobChunk> blob;              // lay.bytes bytes, 32-byte aligned
@@ -81,15 +87,11 @@ template <typename R> struct PackedScene {
     // FP32 pack only: hierarchy over the hittable primitives (rm_bvh.cuh), used when RmParams.accel is set
     std::vector<R4<float>> bvh_nodes;
     std::vector<int> bvh_prims;
+    Buf<BvhPrimBox> bvh_boxes;        // ... and the boxes it was built from (rm_render_motion sweeps them)
     int bvh_depth = 0;
     double hierarchy_build_ms = 0.;
 };
 
-// Bounds of one hittable primitive (f64, unpadded) and its entry code kind << 30 | index for the hierarchy's leaves.
-struct BvhPrimBox {
-    double lo[3], hi[3];
-    int code;
-};
 // Builds the hierarchy of rm_bvh.cuh (nodes: 4 x R4<float> each; prims: leaf entries).  Returns its depth.
 // `pool`: threads to build on (large scenes); none = threads of the call's own.
 int build_bvh(const Buf<BvhPrimBox>& boxes, std::vector<R4<float>>& nodes, std::vector<int>& prims, HostPool* pool = nullptr);
@@ -128,5 +130,18 @@ LensCamera make_lens_camera(const RmParams& p, const double* basis, const RmLens
 // for FP32 kept at 1e-30, at least one entry), and the returned RoughGlass the unit-disc points of s x s; its g pointer is
 // left for the caller to set.  The values are taken as given (rm_render_rough_glass checks them).
 RoughGlass make_rough_glass(int samples, const double* roughness, int n, std::vector<float>& g);
+
+// The motion of rm_render_motion as the kernel reads it: v receives the FP32 displacement {v, 0} of every primitive of the
+// FP32 pack ps by the kernel's indices (Motion's layout: spheres | fast-path triangles | plane slots, from the ids in the
+// blob), disp holding 3 doubles per primitive id; reach receives the largest |component| of those FP32 values over 2.  The
+// values are taken as given (rm_render_motion checks them).
+void motion_displacements(const PackedScene<float>& ps, const double* disp, std::vector<R4<float>>& v, double& reach);
+// The samples' times of s x s (motion_time in f64 and rounded to FP32); the pointers are left for the caller to set.
+Motion make_motion(int samples);
+// The swept hierarchy of a motion frame: build_bvh over the pack's boxes, each grown by |v| / 2 per axis of its primitive's
+// displacement in v (make_motion's layout) -- the union of its boxes at tau = -1/2 and +1/2.  With every displacement zero
+// it is the pack's own hierarchy, byte for byte.
+int build_swept_bvh(const PackedScene<float>& ps, const std::vector<R4<float>>& v, std::vector<R4<float>>& nodes, std::vector<int>& prims,
+                    HostPool* pool = nullptr);
 
 }  // namespace rm

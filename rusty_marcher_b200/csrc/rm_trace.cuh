@@ -658,4 +658,24 @@ struct RoughGlass {
     int samples;
 };
 
+// Motion blur (rm_render_motion, include/rm_b200.h RmMotion).  The time of sample (i, j) of s x s: stratum
+// m = s ((2i + j) mod s) + ((i + j) mod s) -- a bijection onto [0, s^2), since (a - b) mod s = i -- and
+// tau = (m + 0.5) / s^2 - 0.5, in (-1/2, 1/2), symmetric about 0, and 0 at s = 1.  f64 without fused multiply-add; the
+// kernel, the host emulation and the tests all call it.
+RM_HD double motion_time(const int s, const int i, const int j) {
+    const int m = s * ((2 * i + j) % s) + (i + j) % s;
+    return ((double)m + 0.5) / (double)(s * s) - 0.5;
+}
+// The call's motion as the kernel reads it: the FP32 displacement {v, 0} of every primitive by the kernel's own indices --
+// sphere i, fast-path triangle j, plane slot i of the generic arrays (the layout's full lists, so that culling changes no
+// index) -- and the time of sample q = i s + j in f64 and rounded to FP32.
+struct Motion {
+    const R4<float>* v_sph;
+    const R4<float>* v_tri;
+    const R4<float>* v_pln;
+    double tau[kAreaMaxSamples * kAreaMaxSamples];
+    float tau32[kAreaMaxSamples * kAreaMaxSamples];
+    int samples;
+};
+
 }  // namespace rm

@@ -407,6 +407,66 @@ class Renderer:
         print(message)
         return message
 
+    def render_motion(self, frame, scene, displacement, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., rgb8=None,
+                      patch_rows=(0, -1)):
+        """EXTENSION MODE (no reference counterpart): motion blur.  Each shape moves by a displacement over the shutter
+        (`displacement`: one 3-vector for every shape, or one per entry of scene.shapes, an Obj's value covering all its
+        triangles; finite), the scene as given being its pose at mid-shutter; the samples x samples rays of a pixel see the
+        scene at as many different times, and the pixel is their mean (rm_render_motion).  forward / up turn the camera as
+        render_view() does, aperture / focus add render_lens()'s thin lens (aperture 0: the pinhole).  samples = 1, or no
+        displacement at all, is render_lens()'s frame.  Fills frame.buffer (float32) over the rendered rows and, if given,
+        rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the same kind of status message as render()."""
+        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
+            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
+        n = len(scene.shapes)
+        v = np.asarray(displacement, dtype=np.float64)
+        if v.shape == (3,):
+            v = np.tile(v, (n, 1))
+        if v.shape != (n, 3):
+            raise ValueError("displacement must be one 3-vector or %d (one per shape of the scene), got shape %s" % (n, v.shape))
+        if not np.all(np.isfinite(v)):
+            raise ValueError("every displacement must be finite, got %r" % (v.tolist(),))
+        aperture, focus = float(aperture), float(focus)
+        if not (np.isfinite(aperture) and aperture >= 0.):
+            raise ValueError("aperture must be finite and >= 0, got %r" % (aperture,))
+        if not (np.isfinite(focus) and focus > 0.):
+            raise ValueError("focus must be finite and > 0, got %r" % (focus,))
+        if self.precision != _abi.RM_FP32:
+            raise ValueError("render_motion computes in RM_FP32")
+        if int(self.width) != frame.width or int(self.height) != frame.height:
+            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
+        if len(patch_rows) > 2 and patch_rows[2] > 1:
+            raise ValueError("render_motion renders contiguous patch rows (stride <= 1)")
+        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
+                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
+            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
+        view = None
+        if forward is not None:
+            view = _view(forward, up)
+            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
+        # primitive ids: shapes in scene order, an Obj once per triangle
+        per_prim = np.ascontiguousarray(np.repeat(v, [s.triangles.shape[0] if isinstance(s, Obj) else 1 for s in scene.shapes], axis=0))
+        lens = _abi.RmLens()
+        lens.aperture, lens.focus, lens.samples = aperture, focus, int(samples)
+        motion = _abi.RmMotion()
+        motion.n_prims, motion.displacement, motion.samples = per_prim.shape[0], per_prim.ctypes.data_as(C.POINTER(C.c_double)), int(samples)
+        L = _abi.load()
+        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
+        now = time.perf_counter()
+        p = self.params(frame, scene, patch_rows)
+        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
+            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
+        stats = _abi.RmStats()
+        _abi.check(L.rm_render_motion(scene.device_handle(), C.byref(p), C.byref(view) if view is not None else None, C.byref(lens),
+                                      C.byref(motion), frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None,
+                                      C.byref(stats)))
+        self.last_stats = stats
+        ms = int((time.perf_counter() - now) * 1000)
+        fps = 1000. / ms if ms > 0 else float("inf")
+        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
+        print(message)
+        return message
+
 
 def _view(forward, up):
     fwd, u = [float(x) for x in forward], [float(x) for x in up]

@@ -1,0 +1,185 @@
+"""Cost of motion blur (rm_render_motion) on one GPU, next to rm_render_lens at the same s and view.
+
+    python tools/motion_bench.py [--out FILE] [--calls N]
+
+For demo (1600x1280) and stress_4k through the hierarchy (1024 spheres + 8192 triangles, 3840x2160, accel = 1; f64 ray
+geometry), at s = 2 and 4, under a camera turned 10 degrees to the left (so that rm_render_lens runs lens_kernel rather than
+routing to rm_render_supersampled) and without a lens:
+  * rm_render_lens, and rm_render_motion with every shape moving by a seeded displacement of length 0.5 and 2 (one direction
+    per shape): call time (host wall time around the synchronous call), the call's ms_render (device time of the traced and
+    resolved rows) and ms_total (device time of the whole call, copies included), medians of N calls after 2 warm-up calls;
+  * in a separate pass under torch.profiler (CUDA activities): the mean time of lens_kernel / motion_kernel.
+Then the one-off cost of the swept hierarchy on BASELINE.json configs[4]'s scene (4096 spheres + 100,352 triangles, accel =
+1): the wall time of the first rm_render_motion call with a new motion (which builds it), of the second with the same motion
+(which finds it in the cache), and of rm_render_lens, each on a small 640x384 frame at s = 2 so that the frame itself costs
+little.  Outputs: float + 8-bit frame into pinned host memory (rm_host_alloc).  The card's name and power limit are read in the
+same run (nvidia-smi --query-gpu, read-only)."""
+import argparse
+import ctypes as C
+import math
+import os
+import sys
+import time
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+import numpy as np  # noqa: E402
+
+import rusty_marcher_b200 as rm  # noqa: E402
+from rusty_marcher_b200 import _abi, workloads  # noqa: E402
+from rusty_marcher_b200.obj import Obj  # noqa: E402
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+from supersample_bench import card  # noqa: E402
+
+# (label, description, width, height, accel)
+CASES = [("demo", workloads.describe("demo"), 1600, 1280, 0),
+         ("stress_4k_bvh", workloads.describe("stress", n_spheres=1024, grid=64), 3840, 2160, 1)]
+SAMPLES = (2, 4)
+LENGTHS = (0.5, 2.)
+YAW = math.radians(10.)
+
+
+def displacement(scene, length, seed=11):
+    """one seeded direction per shape, scaled to `length`, expanded to primitive ids: (n_prims, 3)"""
+    d = np.random.default_rng(seed).normal(size=(len(scene.shapes), 3))
+    d *= length / np.linalg.norm(d, axis=1, keepdims=True)
+    return np.ascontiguousarray(np.repeat(d, [s.triangles.shape[0] if isinstance(s, Obj) else 1 for s in scene.shapes], axis=0))
+
+
+def motion_of(v, s):
+    m = _abi.RmMotion()
+    m.n_prims, m.displacement, m.samples = v.shape[0], v.ctypes.data_as(C.POINTER(C.c_double)), s
+    return m
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", default=None)
+    ap.add_argument("--calls", type=int, default=10)
+    args = ap.parse_args()
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+
+    rm.init(0)
+    L = _abi.load()
+    lines = []
+
+    def say(s=""):
+        print(s, flush=True)
+        lines.append(s)
+
+    say("motion blur (rm_render_motion), one GPU: %s" % torch.cuda.get_device_name(0))
+    say("card: %s" % card())
+    say("calls per point: %d (median), after 2 warm-up calls; outputs: float + 8-bit frame into pinned host memory" % args.calls)
+    view = _abi.RmView()
+    view.forward[:] = [-math.sin(YAW), 0., -math.cos(YAW)]
+    view.up[:] = [0., 1., 0.]
+
+    def timed(fn):
+        st = _abi.RmStats()
+        walls, ren, tot = [], [], []
+        for i in range(2 + args.calls):
+            t0 = time.perf_counter()
+            _abi.check(fn(st))
+            t1 = time.perf_counter()
+            if i >= 2:
+                walls.append(1e3 * (t1 - t0))
+                ren.append(st.ms_render)
+                tot.append(st.ms_total)
+        return float(np.median(walls)), float(np.median(ren)), float(np.median(tot))
+
+    def kernel_ms(fn, name):
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for _ in range(3):
+                _abi.check(fn(None))
+            torch.cuda.synchronize()
+        ks = [e.time_range.elapsed_us() for e in prof.events() if name in e.name and e.device_type.name == "CUDA"]
+        if not ks:                                              # (kernels attached to a host-side event instead)
+            ks = [k.duration for e in prof.events() for k in getattr(e, "kernels", []) if name in k.name]
+        if len(ks) != 3:
+            raise RuntimeError("torch.profiler recorded %d %s launches, expected 3" % (len(ks), name))
+        return 1e-3 * float(np.mean(ks))
+
+    for label, desc, w, h, accel in CASES:
+        scene = workloads.build_scene(desc)
+        r = rm.create_renderer(1.5, h, w)
+        r.accel = bool(accel)
+        fb = rm.create_frame_buffer(32, 32)
+        fb.width, fb.height = w, h
+        p = r.params(fb, scene)
+        hd = scene.device_handle()
+        out = L.rm_host_alloc(h * w * 12)
+        out8 = L.rm_host_alloc(h * w * 3)
+        say()
+        say("%s (%dx%d, accel %d, %d primitives, view: yaw 10 degrees, no lens)" % (label, w, h, accel, scene.num_prims))
+        say("  %2s %-24s %9s %10s %10s %10s %8s" % ("s", "call", "wall ms", "ms_render", "ms_total", "kernel ms", "x lens"))
+        try:
+            for s in SAMPLES:
+                ln = _abi.RmLens()
+                ln.aperture, ln.focus, ln.samples = 0., 1., s
+
+                def lens_call(st):
+                    return L.rm_render_lens(hd, C.byref(p), C.byref(view), C.byref(ln), out, out8, C.byref(st) if st is not None else None)
+                wall, ren0, tot = timed(lens_call)
+                km = kernel_ms(lens_call, "lens_kernel")
+                say("  %2d %-24s %9.3f %10.3f %10.3f %10.3f %8s" % (s, "rm_render_lens", wall, ren0, tot, km, "1.00"))
+                for length in LENGTHS:
+                    v = displacement(scene, length)
+                    mo = motion_of(v, s)
+
+                    def motion_call(st, mo=mo):
+                        return L.rm_render_motion(hd, C.byref(p), C.byref(view), None, C.byref(mo), out, out8,
+                                                  C.byref(st) if st is not None else None)
+                    wall, ren, tot = timed(motion_call)
+                    km = kernel_ms(motion_call, "motion_kernel")
+                    say("  %2d %-24s %9.3f %10.3f %10.3f %10.3f %8.2f" % (s, "motion, |v| = %g" % length, wall, ren, tot, km, ren / ren0))
+        finally:
+            L.rm_host_free(out)
+            L.rm_host_free(out8)
+            scene.release()
+
+    # the swept hierarchy's one-off cost on configs[4]'s scene
+    w, h, s = 640, 384, 2
+    scene = workloads.scene("stress", n_spheres=4096, grid=224)
+    r = rm.create_renderer(1.5, h, w)
+    r.accel = True
+    fb = rm.create_frame_buffer(32, 32)
+    fb.width, fb.height = w, h
+    p = r.params(fb, scene)
+    hd = scene.device_handle()
+    out = L.rm_host_alloc(h * w * 12)
+    out8 = L.rm_host_alloc(h * w * 3)
+    say()
+    say("swept hierarchy, configs[4] scene (%d primitives, accel 1), %dx%d, s = %d, view: yaw 10 degrees" % (scene.num_prims, w, h, s))
+    try:
+        ln = _abi.RmLens()
+        ln.aperture, ln.focus, ln.samples = 0., 1., s
+        st = _abi.RmStats()
+        for _ in range(2):
+            _abi.check(L.rm_render_lens(hd, C.byref(p), C.byref(view), C.byref(ln), out, out8, C.byref(st)))
+        t0 = time.perf_counter()
+        _abi.check(L.rm_render_lens(hd, C.byref(p), C.byref(view), C.byref(ln), out, out8, C.byref(st)))
+        say("  rm_render_lens:                                wall %9.3f ms, ms_render %8.3f" % (1e3 * (time.perf_counter() - t0), st.ms_render))
+        for length in LENGTHS:
+            mo = motion_of(displacement(scene, length), s)
+            for k, what in enumerate(("first call (builds the hierarchy)", "second call, same motion")):
+                t0 = time.perf_counter()
+                _abi.check(L.rm_render_motion(hd, C.byref(p), C.byref(view), None, C.byref(mo), out, out8, C.byref(st)))
+                say("  |v| = %-4g %-36s wall %9.3f ms, ms_render %8.3f" % (length, what + ":", 1e3 * (time.perf_counter() - t0), st.ms_render))
+    finally:
+        L.rm_host_free(out)
+        L.rm_host_free(out8)
+        scene.release()
+    say()
+    say("ms_render: device time of the traced and resolved rows (lens_kernel / motion_kernel); ms_total: the whole call,")
+    say("copies included; kernel ms: the kernel's mean time under torch.profiler; x lens: ms_render over rm_render_lens's at the")
+    say("same s.  Every shape moves, each in its own seeded direction; the hierarchy frames walk the swept hierarchy.")
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            f.write("\n".join(lines) + "\n")
+
+
+if __name__ == "__main__":
+    main()
