@@ -31,6 +31,10 @@
 //                                      (rm_render_motion; an extension).  Combines with --samples, --aperture / --focus,
 //                                      --look-at / --up, --camera and --accel; not with --roughness, --light-radius,
 //                                      --contrast, --f64 or --rows-f64
+//   --combine                          distributed ray tracing: --light-radius, --roughness, --move, --aperture / --focus and
+//                                      --look-at / --up all together, --samples S x S rays per pixel each sampling every
+//                                      effect at once (rm_render_distributed; an extension; an area light is one point per
+//                                      ray).  Not with --contrast, --f64 or --rows-f64
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -66,6 +70,7 @@ int main(int argc, char** argv) {
     bool rough = false;
     double roughness = 0.;
     bool moving = false;
+    bool combine = false;
     int move_shape = -1;
     double move_by[3] = {0., 0., 0.};
     auto triple = [](const char* s, double v[3]) { char end = 0; return std::sscanf(s, "%lf,%lf,%lf%c", &v[0], &v[1], &v[2], &end) == 3; };
@@ -82,6 +87,7 @@ int main(int argc, char** argv) {
         else if (a == "--f64") f64 = true;              // the validation kernels: the reference's own f64 arithmetic
         else if (a == "--rows-f64") rows64 = true;      // FP32 kernels into the reference's frame type (one allocation per row, f64)
         else if (a == "--accel") accel = 1;
+        else if (a == "--combine") combine = true;
         else if (a == "--samples") { need(1); samples = std::atoi(argv[++i]); }
         else if (a == "--contrast") { need(1); contrast = std::strtod(argv[++i], nullptr); adaptive = true; }
         else if (a == "--aperture") { need(1); lens.aperture = std::strtod(argv[++i], nullptr); use_lens = true; }
@@ -124,19 +130,23 @@ int main(int argc, char** argv) {
         return 2;
     }
     lens.samples = samples;
-    if (area && (look || use_lens || adaptive || f64 || rows64)) {
+    if (combine && (adaptive || f64 || rows64)) {
+        std::fprintf(stderr, "rm_headless: --combine does not combine with --contrast, --f64 or --rows-f64\n");
+        return 2;
+    }
+    if (area && !combine && (look || use_lens || adaptive || f64 || rows64)) {
         std::fprintf(stderr, "rm_headless: --light-radius does not combine with --look-at, --aperture, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (rough && (area || adaptive || f64 || rows64)) {
+    if (rough && !combine && (area || adaptive || f64 || rows64)) {
         std::fprintf(stderr, "rm_headless: --roughness does not combine with --light-radius, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (moving && (rough || area || adaptive || f64 || rows64)) {
+    if (moving && !combine && (rough || area || adaptive || f64 || rows64)) {
         std::fprintf(stderr, "rm_headless: --move does not combine with --roughness, --light-radius, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (look && !use_lens && !rough && !moving && (samples > 1 || adaptive || rows64)) {
+    if (look && !combine && !use_lens && !rough && !moving && (samples > 1 || adaptive || rows64)) {
         std::fprintf(stderr, "rm_headless: --look-at does not combine with --samples, --contrast or --rows-f64\n");
         return 2;
     }
@@ -236,7 +246,10 @@ int main(int argc, char** argv) {
     for (int f = 0; f < frames; f++) {
         const auto t0 = std::chrono::steady_clock::now();
         std::memset(&st, 0, sizeof st);
-        if (moving) rc = rm_render_motion(scene, &p, look ? &view : nullptr, use_lens ? &lens : nullptr, &motion, rgb32.data(),
+        if (combine) rc = rm_render_distributed(scene, &p, samples, look ? &view : nullptr, use_lens ? &lens : nullptr, area ? &area_lights : nullptr,
+                                                rough ? &rough_glass : nullptr, moving ? &motion : nullptr, rgb32.data(),
+                                                f == frames - 1 ? rgb8.data() : nullptr, &st);
+        else if (moving) rc = rm_render_motion(scene, &p, look ? &view : nullptr, use_lens ? &lens : nullptr, &motion, rgb32.data(),
                                           f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (rough) rc = rm_render_rough_glass(scene, &p, look ? &view : nullptr, use_lens ? &lens : nullptr, &rough_glass, rgb32.data(),
                                               f == frames - 1 ? rgb8.data() : nullptr, &st);
@@ -253,7 +266,7 @@ int main(int argc, char** argv) {
         std::printf("Scene rendered in %lld ms (%u fps, %.2f MP/s)\n", ms, ms > 0 ? (unsigned)fps : 4294967295u, fps * (double)n_px / 1e6);
     }
     // "Save to file": normalize + to_vec on the device (framebuffer.rs:40-82), then the P6 stream (framebuffer.rs:26-38)
-    if (use_lens || area || rough || moving) {
+    if (combine || use_lens || area || rough || moving) {
         // (the last frame above wrote the 8-bit frame)
     } else if (adaptive) {
         std::vector<unsigned char> mask(n_px, 0);

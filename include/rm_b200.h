@@ -361,7 +361,8 @@ int rm_render_view_device(RmScene scene, const RmParams* params, const RmView* v
  * an invalid view; precision other than RM_FP32; patch_row_stride > 1; max_depth < 1; an unknown scene; out_rgb and out_rgb8
  * both NULL.  RM_ERR_DIMENSIONS: as for rm_render_supersampled.  Lens and parameter errors are reported without a device.
  * Out of scope: random or per-pixel lens patterns and bokeh shapes; a lens for rm_render_adaptive, rm_render_dispersive,
- * rm_render_rows_* and rm_render_frame; an FP64 entry point. */
+ * rm_render_rows_* and rm_render_frame; an FP64 entry point.  A lens together with area lights, rough glass and motion:
+ * rm_render_distributed. */
 typedef struct RmLens {
     double aperture;   /* lens radius in scene units, >= 0 */
     double focus;      /* distance from the camera to the plane in focus, along the view axis, > 0 */
@@ -411,7 +412,8 @@ int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, co
  * for rm_render.
  * Out of scope: area lights with a view, a lens, supersampling, rm_render_adaptive, rm_render_dispersive, rm_render_rows_*
  * or rm_render_frame; an FP64 entry point; random or per-pixel sampling patterns; shapes other than the facing disc; a
- * radius stored in the scene. */
+ * radius stored in the scene.  Area lights with a view, a lens, rough glass or motion, sampled one point per sample ray:
+ * rm_render_distributed. */
 typedef struct RmAreaLights {
     int32_t       n_lights;  /* must equal the scene's light count */
     const double* radius;    /* n_lights radii in the scene's light order: finite, >= 0 (0 = the reference's point light) */
@@ -467,9 +469,9 @@ int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLig
  * precision other than RM_FP32; patch_row_stride > 1; max_depth < 1; out_rgb and out_rgb8 both NULL (all reported without
  * a device); n_prims different from rm_scene_num_prims(scene); an unknown scene.  RM_ERR_DIMENSIONS: as for
  * rm_render_supersampled.
- * Out of scope: roughness with area lights, rm_render_adaptive, rm_render_dispersive, rm_render_rows_* or rm_render_frame;
- * an FP64 entry point; random or per-pixel patterns and lobes other than the uniform-disc cone; roughness stored in the
- * uploaded scene; per-channel roughness. */
+ * Out of scope: rm_render_adaptive, rm_render_dispersive, rm_render_rows_* or rm_render_frame; an FP64 entry point; random
+ * or per-pixel patterns and lobes other than the uniform-disc cone; roughness stored in the uploaded scene; per-channel
+ * roughness.  Roughness with area lights or motion: rm_render_distributed. */
 typedef struct RmRoughGlass {
     int32_t       n_prims;    /* must equal rm_scene_num_prims(scene) */
     const double* roughness;  /* n_prims values in primitive-id order (shapes in scene order, an Obj once per triangle):
@@ -522,9 +524,9 @@ int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* v
  * precision other than RM_FP32; patch_row_stride > 1; max_depth < 1; out_rgb and out_rgb8 both NULL (all reported without a
  * device); n_prims different from rm_scene_num_prims(scene); an unknown scene.  RM_ERR_DIMENSIONS: as for
  * rm_render_supersampled.
- * Out of scope: motion with rough glass, area lights, rm_render_adaptive, rm_render_dispersive, rm_render_rows_* or
- * rm_render_frame; moving lights or a moving camera; rotation, scaling or curved paths; motion stored in the uploaded scene;
- * an FP64 entry point; random or per-pixel time patterns. */
+ * Out of scope: rm_render_adaptive, rm_render_dispersive, rm_render_rows_* or rm_render_frame; moving lights or a moving
+ * camera; rotation, scaling or curved paths; motion stored in the uploaded scene; an FP64 entry point; random or per-pixel
+ * time patterns.  Motion with rough glass or area lights: rm_render_distributed. */
 typedef struct RmMotion {
     int32_t       n_prims;       /* must equal rm_scene_num_prims(scene) */
     const double* displacement;  /* 3 * n_prims values, x y z per primitive id (shapes in scene order, an Obj once per
@@ -534,6 +536,57 @@ typedef struct RmMotion {
 int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view /* NULL = the reference's camera */,
                      const RmLens* lens /* NULL = pinhole */, const RmMotion* motion, float* out_rgb, uint8_t* out_rgb8,
                      RmStats* stats);
+
+/* ---- extension mode: distributed ray tracing -- depth of field, soft shadows, rough glass and motion blur at once ---------- *
+ * Cook, Porter and Carpenter (1984): every sample ray samples every dimension at once -- the lens point, the time, a point
+ * of each area light and the direction of every ray rough glass scatters -- and the pixel is the mean over its samples.  This
+ * call takes the structs of rm_render_lens, rm_render_area_lights, rm_render_rough_glass and rm_render_motion together; none
+ * changes, and the ABI version stays 5.
+ * Definition (normative; rm::area_offset in rm_trace.cuh holds rule 4's stratum, and the tests' restatement over the oracle is
+ * the same).  All in f64 without fused multiply-add; s = samples, and every struct given has samples == s.
+ *   1. Sample (i, j), i, j in [0, s), of output pixel (x, y) is rm_render_lens's sample ray: rm::lens_ray with the view's basis
+ *      (the identity without a view) and the lens (aperture 0 without one).
+ *   2. Time.  tau = rm::motion_time(s, i, j), and the sample sees the scene at tau as RmMotion defines it (without motion tau
+ *      plays no role).  The whole recursion and every shadow ray of the sample see the same tau; lights and the camera do not
+ *      move.
+ *   3. Rough glass.  At a hit of level L, the rays a glass-like hit spawns are turned as RmRoughGlass defines it, with
+ *      rm::rough_offset(s, i, j, L) and the same side rules for the origin; hit points and normals are the scene's at tau.
+ *   4. Area lights, one point per sample.  At a shading point p of level L, a light of radius 0 is the reference's point
+ *      light.  A light of centre c, colour k and radius r > 0 is ONE point light of colour k (not k / s^2) at
+ *      q = rm::light_sample(c, r, t1, t2, lx, ly), with (t1, t2) = rm::light_frame(normalized(c - p)) and (lx, ly) the
+ *      elliptical grid-to-disc map (rm::lens_offset's) of the stratum (a, b) = ((i + 2j + L) mod s, (i + 3j) mod s):
+ *      rm::area_offset(s, i, j, L).  Its shadow ray is traced in the scene at tau; otherwise the term is the reference's
+ *      per-light term, with the +-1e-3 origin and no maximum distance.  The stratum map has determinant 1 over Z_s, a bijection
+ *      over the s^2 samples for every s and L; for s >= 4 neither coordinate is a shifted copy of a coordinate of the
+ *      sub-pixel, lens, rough or time strata (at s = 2 and 3 some sharing cannot be avoided).
+ *      This is NOT rm_render_area_lights' frame: there each pixel traces one primary ray and every area light is s^2 point
+ *      lights of colour k / s^2 at each shading point.  Here the pixel's s^2 samples do the averaging, at s^2 shadow rays per
+ *      area light and pixel instead of s^4.
+ *   5. The pixel is the FP32 mean of its s^2 sample values in rm::resolve_box's order (sub-rows i outer, j inner).
+ * Routing -- each routed case is that call, and gives its frame bit for bit.  An area light is active when its radius is
+ * > 0; rough glass when some glass-like primitive has roughness > 0 (decided on the host, as rm_render_rough_glass does);
+ * motion when some displacement is != 0.
+ *   - s = 1, or no active effect: rm_render_lens (with the pinhole when no lens is given);
+ *   - rough glass alone: rm_render_rough_glass;  motion alone: rm_render_motion;
+ *   - an active area light, or rough glass together with motion: distributed_kernel.
+ * FP32 production path (distributed_kernel): motion_kernel's schedule; queries at the sample's tau as rm_render_motion makes
+ * them (over the swept hierarchy with accel != 0) when motion is active, and over the scene's own otherwise (brute force for
+ * scenes of more than 8 lights); rough_glass_kernel's turn; the light point of rule 4 in FP32 from the FP32 shading point.
+ * Frames meet the FP32 parity criteria against the f64 definition.  cull_backfacing applies.
+ * Rows, outputs and stats as rm_render_lens: patch rows [b, e) with patch_row_stride <= 1, rows outside untouched; out_rgb
+ * and / or out_rgb8; stats: max_value, ms_render, ms_total, kernel_launches, resident_prims, d2h_bytes.  The call writes the
+ * caller's float frame, so the library forgets its previous deliveries into that memory (RM_ROWS_RETAINED).
+ * RM_ERR_INVALID_ARGUMENT: samples outside [1, 8]; a given struct whose samples differs from s; a struct that is invalid by
+ * its own call's rules (a radius, a roughness, a displacement, the view, the lens); precision other than RM_FP32;
+ * patch_row_stride > 1; max_depth < 1; out_rgb and out_rgb8 both NULL (all reported without a device); n_lights different
+ * from the scene's light count, n_prims different from rm_scene_num_prims(scene); an unknown scene.  RM_ERR_DIMENSIONS: as
+ * for rm_render_supersampled.
+ * Out of scope: random or per-pixel patterns; an FP64 entry point; combining with rm_render_adaptive, rm_render_dispersive,
+ * rm_render_rows_* or rm_render_frame; moving lights. */
+int rm_render_distributed(RmScene scene, const RmParams* params, int samples,
+                          const RmView* view /* NULL = the reference's camera */, const RmLens* lens /* NULL = pinhole */,
+                          const RmAreaLights* lights /* NULL = point lights */, const RmRoughGlass* rough /* NULL = ideal optics */,
+                          const RmMotion* motion /* NULL = nothing moves */, float* out_rgb, uint8_t* out_rgb8, RmStats* stats);
 
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device

@@ -266,6 +266,11 @@ extern "C" {
     /// motion blur: every primitive translated by tau * displacement, the s x s samples of a pixel at s^2 times tau in (-1/2, 1/2)
     pub fn rm_render_motion(scene: RmScene, params: *const RmParams, view: *const RmView, lens: *const RmLens,
                             motion: *const RmMotion, out_rgb: *mut f32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
+    /// distributed ray tracing: lens, area lights (one point per sample ray), rough glass and motion together, s x s samples per
+    /// pixel; every struct may be null, and every one given has samples == s
+    pub fn rm_render_distributed(scene: RmScene, params: *const RmParams, samples: c_int, view: *const RmView, lens: *const RmLens,
+                                 lights: *const RmAreaLights, rough: *const RmRoughGlass, motion: *const RmMotion,
+                                 out_rgb: *mut f32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
     // ---- the hot path, device buffers
     pub fn rm_render_device(scene: RmScene, params: *const RmParams, d_rgb: *mut c_void, d_prim_id: *mut i32,
                             d_max: *mut c_void, stream: *mut c_void) -> c_int;

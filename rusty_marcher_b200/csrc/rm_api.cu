@@ -1476,6 +1476,50 @@ int check_lens(const RmLens* lens) {
     return RM_OK;
 }
 
+namespace {
+
+// The argument checks of the effect structs, shared by their own calls and rm_render_distributed; none needs a device.
+// any_*: whether the struct asks for an effect at all (a radius > 0, a displacement != 0).
+int check_area_lights(const RmAreaLights* lights, bool* any_area) {
+    if (!lights) return fail(RM_ERR_INVALID_ARGUMENT, "lights is null");
+    if (lights->n_lights < 0) return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must be >= 0");
+    if (lights->n_lights > 0 && !lights->radius) return fail(RM_ERR_INVALID_ARGUMENT, "lights: radius is null");
+    *any_area = false;
+    for (int l = 0; l < lights->n_lights; l++) {
+        const double r = lights->radius[l];
+        if (!std::isfinite(r) || r < 0.) return fail(RM_ERR_INVALID_ARGUMENT, "lights: every radius must be finite and >= 0");
+        *any_area |= r > 0.;
+    }
+    if (lights->samples < 1 || lights->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "lights: samples must be in [1, 8]");
+    return RM_OK;
+}
+int check_rough(const RmRoughGlass* rough) {
+    if (!rough) return fail(RM_ERR_INVALID_ARGUMENT, "rough is null");
+    if (rough->n_prims < 0) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must be >= 0");
+    if (rough->n_prims > 0 && !rough->roughness) return fail(RM_ERR_INVALID_ARGUMENT, "rough: roughness is null");
+    for (int k = 0; k < rough->n_prims; k++) {
+        const double g = rough->roughness[k];
+        if (!std::isfinite(g) || g < 0.) return fail(RM_ERR_INVALID_ARGUMENT, "rough: every roughness must be finite and >= 0");
+    }
+    if (rough->samples < 1 || rough->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must be in [1, 8]");
+    return RM_OK;
+}
+int check_motion(const RmMotion* motion, bool* any_motion) {
+    if (!motion) return fail(RM_ERR_INVALID_ARGUMENT, "motion is null");
+    if (motion->n_prims < 0) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must be >= 0");
+    if (motion->n_prims > 0 && !motion->displacement) return fail(RM_ERR_INVALID_ARGUMENT, "motion: displacement is null");
+    *any_motion = false;
+    for (size_t k = 0; k < 3 * (size_t)motion->n_prims; k++) {
+        const double v = motion->displacement[k];
+        if (!std::isfinite(v)) return fail(RM_ERR_INVALID_ARGUMENT, "motion: every displacement must be finite");
+        *any_motion |= v != 0.;
+    }
+    if (motion->samples < 1 || motion->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must be in [1, 8]");
+    return RM_OK;
+}
+
+}  // namespace
+
 int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb, uint8_t* out_rgb8,
                    RmStats* stats) {
     int rc = check_lens(lens);
@@ -1559,17 +1603,10 @@ int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, co
 // argument checks need no device, except the light count, which needs the scene.
 int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLights* lights, float* out_rgb, int32_t* out_prim_id,
                           uint8_t* out_rgb8, RmStats* stats) {
-    if (!lights) return fail(RM_ERR_INVALID_ARGUMENT, "lights is null");
-    if (lights->n_lights < 0) return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must be >= 0");
-    if (lights->n_lights > 0 && !lights->radius) return fail(RM_ERR_INVALID_ARGUMENT, "lights: radius is null");
     bool any_area = false;
-    for (int l = 0; l < lights->n_lights; l++) {
-        const double r = lights->radius[l];
-        if (!std::isfinite(r) || r < 0.) return fail(RM_ERR_INVALID_ARGUMENT, "lights: every radius must be finite and >= 0");
-        any_area |= r > 0.;
-    }
-    if (lights->samples < 1 || lights->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "lights: samples must be in [1, 8]");
-    int rc = check_params(params);
+    int rc = check_area_lights(lights, &any_area);
+    if (rc != RM_OK) return rc;
+    if ((rc = check_params(params)) != RM_OK) return rc;
     if (rc != RM_OK) return rc;
     if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights computes in RM_FP32");
     if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights renders contiguous patch rows (patch_row_stride <= 1)");
@@ -1681,18 +1718,11 @@ std::vector<unsigned char> glass_like_by_id(const rm::OwnedFlatScene& f) {
 // argument checks need no device, except the primitive count, which needs the scene.
 int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, const RmRoughGlass* rough,
                           float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
-    if (!rough) return fail(RM_ERR_INVALID_ARGUMENT, "rough is null");
-    if (rough->n_prims < 0) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must be >= 0");
-    if (rough->n_prims > 0 && !rough->roughness) return fail(RM_ERR_INVALID_ARGUMENT, "rough: roughness is null");
-    for (int k = 0; k < rough->n_prims; k++) {
-        const double g = rough->roughness[k];
-        if (!std::isfinite(g) || g < 0.) return fail(RM_ERR_INVALID_ARGUMENT, "rough: every roughness must be finite and >= 0");
-    }
-    if (rough->samples < 1 || rough->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must be in [1, 8]");
+    int rc = check_rough(rough);
+    if (rc != RM_OK) return rc;
     const int S = rough->samples;
     const RmLens pinhole = {0., 1., S};
-    int rc = check_lens(lens ? lens : &pinhole);
-    if (rc != RM_OK) return rc;
+    if ((rc = check_lens(lens ? lens : &pinhole)) != RM_OK) return rc;
     if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must equal lens->samples");
     rm::ViewBasis vb;
     bool identity = true;
@@ -1782,25 +1812,86 @@ int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* v
     return RM_OK;
 }
 
+namespace {
+
+// The motion of a frame on the device (rm_render_motion, rm_render_distributed; g.mu held, the scene's FP32 pack ensured): the
+// per-primitive data by content, from the cache or made now (the swept hierarchy only once a call walks), copied to g.motion
+// unless it is there already.  mo receives the displacement pointers, ds the scene's pack with the swept hierarchy when
+// `walk`, reach the motion's reach (the glass mode's coordinate bound).
+int stage_motion(SceneEntry& se, const DevicePack<float>& dp, const RmMotion* motion, const bool walk, cudaStream_t s, rm::Motion& mo,
+                 rm::DeviceScene<float>& ds, double& reach) {
+    int rc;
+    // the motion's per-primitive data by content: found in the cache, or made now (the swept hierarchy only once a call walks)
+    const size_t disp_bytes = 3 * sizeof(double) * (size_t)motion->n_prims;
+    const uint64_t key[4] = {se.hash[0], se.hash[1], hash_bytes(motion->displacement, disp_bytes, 0x452821E638D01377ull),
+                             hash_bytes(motion->displacement, disp_bytes, 0xBE5466CF34E90C6Cull)};
+    const size_t key_bytes = se.hash_bytes + disp_bytes;
+    Context::MotionEntry* me = nullptr;
+    for (size_t i = 0; i < g.motion_cache.size(); i++)
+        if (std::equal(key, key + 4, g.motion_cache[i].key) && g.motion_cache[i].bytes == key_bytes) {
+            std::rotate(g.motion_cache.begin() + i, g.motion_cache.begin() + i + 1, g.motion_cache.end());   // most recent last
+            me = &g.motion_cache.back();
+            break;
+        }
+    std::shared_ptr<rm::PackedScene<float>> pack;
+    if (!me || (walk && !me->swept)) {
+        if ((rc = pack_for<float>(se, pack)) != RM_OK) return rc;
+    }
+    if (!me) {
+        if (g.motion_cache.size() >= 4) g.motion_cache.erase(g.motion_cache.begin());
+        g.motion_cache.emplace_back();
+        me = &g.motion_cache.back();
+        std::copy(key, key + 4, me->key);
+        me->bytes = key_bytes;
+        rm::motion_displacements(*pack, motion->displacement, me->v, me->reach);
+        me->serial = ++g.motion_serial;
+    }
+    if (walk && !me->swept) {
+        rm::build_swept_bvh(*pack, me->v, me->nodes, me->prims, &host_pool());
+        me->swept = true;
+    }
+    const rm::BlobLayout& L = dp.ds.lay;
+    const size_t v_bytes = me->v.size() * sizeof(rm::R4<float>);
+    const size_t n_bytes = me->nodes.size() * sizeof(rm::R4<float>), p_bytes = me->prims.size() * sizeof(int);
+    const size_t o_nodes = align256(v_bytes), o_prims = o_nodes + align256(n_bytes);
+    // the previous call has finished with the device copy (every call ends in a stream synchronisation)
+    if (g.motion_on_device != me->serial || (walk && !g.motion_on_device_swept)) {
+        if ((rc = g.motion.ensure(o_prims + std::max<size_t>(p_bytes, 16))) != RM_OK) return rc;
+        CK(cudaMemcpyAsync(g.motion.p, me->v.data(), v_bytes, cudaMemcpyHostToDevice, s));
+        if (me->swept) {
+            CK(cudaMemcpyAsync(static_cast<char*>(g.motion.p) + o_nodes, me->nodes.data(), n_bytes, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(static_cast<char*>(g.motion.p) + o_prims, me->prims.data(), p_bytes, cudaMemcpyHostToDevice, s));
+        }
+        g.motion_on_device = me->serial;
+        g.motion_on_device_swept = me->swept;
+    }
+    const rm::R4<float>* dv = static_cast<const rm::R4<float>*>(g.motion.p);
+    mo.v_sph = dv;
+    mo.v_tri = dv + L.n_sph;
+    mo.v_pln = dv + L.n_sph + L.n_tri;
+    ds = dp.ds;
+    if (walk) {
+        ds.bvh.nodes = reinterpret_cast<const rm::R4<float>*>(static_cast<const char*>(g.motion.p) + o_nodes);
+        ds.bvh.prims = reinterpret_cast<const int*>(static_cast<const char*>(g.motion.p) + o_prims);
+        ds.bvh.n_nodes = (int)(me->nodes.size() / 4);
+    }
+    reach = me->reach;
+    return RM_OK;
+}
+
+}  // namespace
+
 // Extension mode (include/rm_b200.h): motion_kernel traces and resolves the output rows, then, for the 8-bit frame, the
 // tone-map kernel.  s = 1 (every sample at tau = 0) and calls in which nothing moves are rm_render_lens's frame and go there.
 // The argument checks need no device, except the primitive count, which needs the scene.
 int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, const RmMotion* motion,
                      float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
-    if (!motion) return fail(RM_ERR_INVALID_ARGUMENT, "motion is null");
-    if (motion->n_prims < 0) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must be >= 0");
-    if (motion->n_prims > 0 && !motion->displacement) return fail(RM_ERR_INVALID_ARGUMENT, "motion: displacement is null");
     bool any_motion = false;
-    for (size_t k = 0; k < 3 * (size_t)motion->n_prims; k++) {
-        const double v = motion->displacement[k];
-        if (!std::isfinite(v)) return fail(RM_ERR_INVALID_ARGUMENT, "motion: every displacement must be finite");
-        any_motion |= v != 0.;
-    }
-    if (motion->samples < 1 || motion->samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must be in [1, 8]");
+    int rc = check_motion(motion, &any_motion);
+    if (rc != RM_OK) return rc;
     const int S = motion->samples;
     const RmLens pinhole = {0., 1., S};
-    int rc = check_lens(lens ? lens : &pinhole);
-    if (rc != RM_OK) return rc;
+    if ((rc = check_lens(lens ? lens : &pinhole)) != RM_OK) return rc;
     if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal lens->samples");
     rm::ViewBasis vb;
     bool identity = true;
@@ -1837,62 +1928,11 @@ int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, 
     rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
     fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
     const bool walk = fp.accel != 0 && dp.ds.bvh.n_nodes > 0 && dp.ds.lay.n_lgt <= rm::kBvhMaxLights;
-    // the motion's per-primitive data by content: found in the cache, or made now (the swept hierarchy only once a call walks)
-    const size_t disp_bytes = 3 * sizeof(double) * (size_t)motion->n_prims;
-    const uint64_t key[4] = {se.hash[0], se.hash[1], hash_bytes(motion->displacement, disp_bytes, 0x452821E638D01377ull),
-                             hash_bytes(motion->displacement, disp_bytes, 0xBE5466CF34E90C6Cull)};
-    const size_t key_bytes = se.hash_bytes + disp_bytes;
-    Context::MotionEntry* me = nullptr;
-    for (size_t i = 0; i < g.motion_cache.size(); i++)
-        if (std::equal(key, key + 4, g.motion_cache[i].key) && g.motion_cache[i].bytes == key_bytes) {
-            std::rotate(g.motion_cache.begin() + i, g.motion_cache.begin() + i + 1, g.motion_cache.end());   // most recent last
-            me = &g.motion_cache.back();
-            break;
-        }
-    std::shared_ptr<rm::PackedScene<float>> pack;
-    if (!me || (walk && !me->swept)) {
-        if ((rc = pack_for<float>(se, pack)) != RM_OK) return rc;
-    }
-    if (!me) {
-        if (g.motion_cache.size() >= 4) g.motion_cache.erase(g.motion_cache.begin());
-        g.motion_cache.emplace_back();
-        me = &g.motion_cache.back();
-        std::copy(key, key + 4, me->key);
-        me->bytes = key_bytes;
-        rm::motion_displacements(*pack, motion->displacement, me->v, me->reach);
-        me->serial = ++g.motion_serial;
-    }
-    if (walk && !me->swept) {
-        rm::build_swept_bvh(*pack, me->v, me->nodes, me->prims, &host_pool());
-        me->swept = true;
-    }
     rm::Motion mo = rm::make_motion(S);
-    const rm::BlobLayout& L = dp.ds.lay;
-    const size_t v_bytes = me->v.size() * sizeof(rm::R4<float>);
-    const size_t n_bytes = me->nodes.size() * sizeof(rm::R4<float>), p_bytes = me->prims.size() * sizeof(int);
-    const size_t o_nodes = align256(v_bytes), o_prims = o_nodes + align256(n_bytes);
-    // the previous call has finished with the device copy (every call ends in a stream synchronisation)
-    if (g.motion_on_device != me->serial || (walk && !g.motion_on_device_swept)) {
-        if ((rc = g.motion.ensure(o_prims + std::max<size_t>(p_bytes, 16))) != RM_OK) return rc;
-        CK(cudaMemcpyAsync(g.motion.p, me->v.data(), v_bytes, cudaMemcpyHostToDevice, s));
-        if (me->swept) {
-            CK(cudaMemcpyAsync(static_cast<char*>(g.motion.p) + o_nodes, me->nodes.data(), n_bytes, cudaMemcpyHostToDevice, s));
-            CK(cudaMemcpyAsync(static_cast<char*>(g.motion.p) + o_prims, me->prims.data(), p_bytes, cudaMemcpyHostToDevice, s));
-        }
-        g.motion_on_device = me->serial;
-        g.motion_on_device_swept = me->swept;
-    }
+    rm::DeviceScene<float> ds;
+    double reach = 0.;
+    if ((rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
     if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
-    const rm::R4<float>* dv = static_cast<const rm::R4<float>*>(g.motion.p);
-    mo.v_sph = dv;
-    mo.v_tri = dv + L.n_sph;
-    mo.v_pln = dv + L.n_sph + L.n_tri;
-    rm::DeviceScene<float> ds = dp.ds;                          // the scene's pack with the swept hierarchy
-    if (walk) {
-        ds.bvh.nodes = reinterpret_cast<const rm::R4<float>*>(static_cast<const char*>(g.motion.p) + o_nodes);
-        ds.bvh.prims = reinterpret_cast<const int*>(static_cast<const char*>(g.motion.p) + o_prims);
-        ds.bvh.n_nodes = (int)(me->nodes.size() / 4);
-    }
     const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
     const bool cull = params->cull_backfacing != 0;
     const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
@@ -1906,7 +1946,7 @@ int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, 
     CK(cudaEventRecord(g.ev[1], s));
     int launches = 0;
     if (rows) {
-        CK(rm::launch_motion(ds, fp, lc, mo, me->reach, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
+        CK(rm::launch_motion(ds, fp, lc, mo, reach, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
         launches++;
     }
     CK(cudaEventRecord(g.ev[2], s));
@@ -1933,7 +1973,140 @@ int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, 
         CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
         stats->ms_total = ms;
         stats->kernel_launches = launches;
-        stats->resident_prims = L.n_sph + rm::plane_count<float>(L, cull);
+        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
+    }
+    return RM_OK;
+}
+
+// Extension mode (include/rm_b200.h): distributed_kernel traces and resolves the output rows with every given effect at once,
+// then, for the 8-bit frame, the tone-map kernel.  A call whose only active effect is rough glass or motion is that effect's
+// own call, and s = 1 or no active effect is rm_render_lens's: those go there and give their frames bit for bit.  The
+// argument checks need no device, except the light and primitive counts, which need the scene.
+int rm_render_distributed(RmScene scene, const RmParams* params, int samples, const RmView* view, const RmLens* lens,
+                          const RmAreaLights* lights, const RmRoughGlass* rough, const RmMotion* motion, float* out_rgb,
+                          uint8_t* out_rgb8, RmStats* stats) {
+    if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_distributed: samples must be in [1, 8]");
+    const int S = samples;
+    bool any_area = false, any_motion = false;
+    int rc;
+    if (lights) {
+        if ((rc = check_area_lights(lights, &any_area)) != RM_OK) return rc;
+        if (lights->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lights: samples must equal the call's samples");
+    }
+    if (rough) {
+        if ((rc = check_rough(rough)) != RM_OK) return rc;
+        if (rough->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must equal the call's samples");
+    }
+    if (motion) {
+        if ((rc = check_motion(motion, &any_motion)) != RM_OK) return rc;
+        if (motion->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal the call's samples");
+    }
+    const RmLens pinhole = {0., 1., S};
+    if ((rc = check_lens(lens ? lens : &pinhole)) != RM_OK) return rc;
+    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lens: samples must equal the call's samples");
+    rm::ViewBasis vb;
+    bool identity = true;
+    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
+    if ((rc = check_params(params)) != RM_OK) return rc;
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_distributed computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_distributed renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_distributed needs max_depth >= 1");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
+    RmParams sp = *params;
+    sp.width = S * params->width;
+    sp.height = S * params->height;
+    sp.patch_row_begin = 0;
+    sp.patch_row_end = -1;
+    if ((rc = check_params(&sp)) != RM_OK) return rc;
+    const RmLens& ln = lens ? *lens : pinhole;
+    bool any_rough = false;
+    {
+        std::lock_guard<std::mutex> lock(g.mu);
+        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+        auto it = g.scenes.find(scene);
+        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+        if (lights && (size_t)lights->n_lights != it->second.flat.lights.size())
+            return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must equal the scene's light count");
+        if (rough && rough->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must equal the scene's primitive count");
+        if (motion && motion->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must equal the scene's primitive count");
+        if (rough) {
+            const std::vector<unsigned char> glass = glass_like_by_id(it->second.flat);
+            for (int k = 0; k < rough->n_prims && !any_rough; k++) any_rough = glass[k] && rough->roughness[k] > 0.;
+        }
+    }
+    // one sample (every offset (0, 0), every time 0), or a single effect that has a call of its own: that call's frame
+    if (S == 1 || (!any_area && !any_rough && !any_motion)) return rm_render_lens(scene, params, view, &ln, out_rgb, out_rgb8, stats);
+    if (!any_area && !any_motion) return rm_render_rough_glass(scene, params, view, lens, rough, out_rgb, out_rgb8, stats);
+    if (!any_area && !any_rough) return rm_render_motion(scene, params, view, lens, motion, out_rgb, out_rgb8, stats);
+    std::lock_guard<std::mutex> lock(g.mu);
+    auto it = g.scenes.find(scene);
+    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    SceneEntry& se = it->second;
+    DevicePack<float>& dp = se.f32;
+    cudaStream_t s = g.stream;
+    if ((rc = ensure_pack<float>(se, dp)) != RM_OK) return rc;
+    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
+    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
+    const bool walk = fp.accel != 0 && dp.ds.bvh.n_nodes > 0 && dp.ds.lay.n_lgt <= rm::kBvhMaxLights;
+    rm::Motion mo = rm::make_motion(S);
+    rm::DeviceScene<float> ds = dp.ds;
+    double reach = 0.;
+    if (any_motion && (rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
+    if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const bool cull = params->cull_backfacing != 0;
+    std::vector<float> radius, gf;
+    rm::AreaPoints ap = rm::make_area_points(S, lights ? lights->radius : nullptr, lights ? lights->n_lights : 0, radius);
+    radius.resize(std::max<size_t>(radius.size(), se.flat.lights.size()), 0.f);   // no lights given: every light a point
+    rm::RoughGlass rg = rm::make_rough_glass(S, any_rough ? rough->roughness : nullptr, any_rough ? rough->n_prims : 0, gf);
+    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
+    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
+    if (any_rough && (rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
+    float* d_max = static_cast<float*>(g.small.p);
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
+    float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
+    ap.radius = d_radius;
+    rg.g = any_rough ? static_cast<const float*>(g.rough.p) : nullptr;
+    CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
+    if (any_rough) CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaEventRecord(g.ev[0], s));
+    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
+    CK(cudaEventRecord(g.ev[1], s));
+    int launches = 0;
+    if (rows) {
+        CK(rm::launch_distributed(ds, fp, lc, ap, rg, mo, any_motion, reach, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p),
+                                  d_max, s));
+        launches++;
+    }
+    CK(cudaEventRecord(g.ev[2], s));
+    if (out_rgb8 && rows) {
+        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
+        launches++;
+    }
+    const size_t host_px = (size_t)fp.row_begin * fp.width;
+    if (out_rgb && n_px) {
+        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
+        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
+    }
+    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
+    float h_max = 0.f;
+    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
+    CK(cudaEventRecord(g.ev[3], s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) {
+        std::memset(stats, 0, sizeof(*stats));
+        stats->max_value = (double)h_max;
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
+        stats->ms_render = ms;
+        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
+        stats->ms_total = ms;
+        stats->kernel_launches = launches;
+        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
         stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
     }
     return RM_OK;

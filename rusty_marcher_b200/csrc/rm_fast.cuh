@@ -1316,4 +1316,240 @@ template <bool kBvh> struct MotionView {
     }
 };
 
+// ---- distributed ray tracing (rm_render_distributed, include/rm_b200.h) ----------------------------------------------------
+// The view the shading code (cast_glass_distributed, distributed_shade) sees for sample (i, j) of a distributed frame:
+// closest-hit queries, surfaces and the f64 refinement are MotionView's at the sample's time when kMotion, and the wrapped
+// FastViewT's otherwise (no per-primitive displacement loads).  direct() takes the recursion level L and replaces every light
+// of radius r > 0 by ONE point light of its full colour, on the disc facing the shading point at the point of stratum
+// area_offset(s, i, j, L); a light of radius 0 is the reference's point light.  The shadow rays go two at a time (anyhit2 of
+// FastViewT, or two MotionView::anyhit at the sample's time), and the terms are FastViewT::direct's, added in its order.
+template <bool kBvh, bool kMotion> struct DistributedView {
+    using FV = FastViewT<kBvh, false>;
+    const FV* fv;
+    MotionView<kBvh> mv;
+    const AreaPoints* ap;
+    int si, sj;
+    const R4<float>* mat_a;
+    const R4<float>* mat_b;
+    const int* mat_f;
+
+    RM_HD DistributedView(const FV& v, const Motion& m, const AreaPoints& a, const int q)
+        : fv(&v), mv(v, m, q), ap(&a), si(q / a.samples), sj(q % a.samples), mat_a(v.mat_a), mat_b(v.mat_b), mat_f(v.mat_f) {}
+
+    template <bool S> RM_HD bool closest(const Vec3<float> o, const Vec3<float> d, int level, HitRec<float>& h, Counters<S>& st) const {
+        if constexpr (kMotion) return mv.template closest<S>(o, d, level, h, st);
+        else return fv->template closest<S>(o, d, level, h, st);
+    }
+    RM_HD unsigned anyhit2(const Vec3<float> oA, const Vec3<float> dA, const Vec3<float> oB, const Vec3<float> dB, unsigned need) const {
+        if constexpr (kMotion) {
+            unsigned blocked = 0;
+            if ((need & 1u) && mv.anyhit(oA, dA)) blocked |= 1u;
+            if ((need & 2u) && mv.anyhit(oB, dB)) blocked |= 2u;
+            return blocked;
+        } else {
+            return fv->anyhit2(oA, dA, oB, dB, need);
+        }
+    }
+    RM_HD void refine(const int slot, const Vec3<double> o, const Vec3<double> d, const double t32, Vec3<double>& p, Vec3<double>& n) const {
+        if constexpr (kMotion) mv.refine(slot, o, d, t32, p, n);
+        else fv->refine(slot, o, d, t32, p, n);
+    }
+    RM_HD void surface(HitRec<float>& h, const Vec3<float> o, const Vec3<float> d, Vec3<float>& normal) const {
+        if constexpr (kMotion) mv.surface(h, o, d, normal);
+        else fv->surface(h, o, d, normal);
+    }
+
+    // renderer.rs:138-193 at a shading point of level `level`, the lights in pairs as FastViewT::direct takes them
+    template <bool S> RM_HD Vec3<float> direct(const int level, const Vec3<float> dir, const Vec3<float> point, const Vec3<float> normal,
+                                               const R4<float> ma, const R4<float> mb, Counters<S>&) const {
+        Vec3<float> acc = {0.f, 0.f, 0.f};
+        const Vec3<float> to_viewer = -dir;                       // (as FastViewT::direct)
+        const Vec3<float> kd = {ma.x, ma.y, ma.z};
+        const int s = ap->samples;
+        const int k = ((si + 2 * sj + level) % s) * s + (si + 3 * sj) % s;   // area_offset(s, i, j, level)
+        const float lx = ap->off[2 * k], ly = ap->off[2 * k + 1];
+        const int n_lgt = fv->n_lgt;
+        auto at = [&](const int l) {                              // the light's point for this sample and level
+            const R4<float> lp = fv->lgt_p[l];
+            const Vec3<float> c = {lp.x, lp.y, lp.z};
+            const float r = ap->radius[l];
+            if (!(r > 0.f)) return c;
+            Vec3<float> t1, t2;
+            light_frame<float>(normalized(Vec3<float>{c.x - point.x, c.y - point.y, c.z - point.z}), t1, t2);
+            return light_sample<float>(c, r, t1, t2, lx, ly);
+        };
+        auto pair = [&](const int l0) {
+            const bool two = l0 + 1 < n_lgt;
+            const Vec3<float> qA = at(l0), qB = at(two ? l0 + 1 : l0);
+            const Vec3<float> ldA = normalized(Vec3<float>{qA.x - point.x, qA.y - point.y, qA.z - point.z});   // renderer.rs:166
+            const Vec3<float> ldB = normalized(Vec3<float>{qB.x - point.x, qB.y - point.y, qB.z - point.z});
+            const float sideA = dot(ldA, normal), sideB = dot(ldB, normal);
+            const float offA = sideA < 0.f ? -1e-3f : 1e-3f, offB = sideB < 0.f ? -1e-3f : 1e-3f;    // renderer.rs:168-172
+            const Vec3<float> soA = axpy(point, normal, offA), soB = axpy(point, normal, offB);
+            const unsigned blocked = anyhit2(soA, ldA, soB, ldB, two ? 3u : 1u);                     // renderer.rs:174-177
+#pragma unroll
+            for (int r = 0; r < 2; r++) {
+                if ((r && !two) || (blocked >> r & 1)) continue;
+                const float w = fv->lgt_p[l0 + r].w;
+                const Vec3<float> ld = r ? ldB : ldA;
+                const float side = r ? sideB : sideA;
+                const Vec3<float> lc = xyz(fv->lgt_c[l0 + r]);
+                acc = acc + scaled(scaled(lc * kd, fmaxf(side, 0.f)), w);                             // renderer.rs:138-140, 181-183
+                const Vec3<float> reflected = reflect(-ld, normal);                                   // renderer.rs:144-145
+                const float sf = fmaxf(dot(reflected, to_viewer), 0.f);                               // renderer.rs:150
+                acc = acc + scaled(lc, pow_nonneg(sf * mb.x, mb.y));                                  // renderer.rs:186-189
+            }
+        };
+        if constexpr (kBvh) {
+            // as FastViewT::direct: the lights as unrolled, guarded pairs (a scene with more than kBvhMaxLights lights stays on
+            // brute force)
+#pragma unroll
+            for (int p = 0; p < kBvhMaxLights / 2; p++)
+                if (2 * p < n_lgt) pair(2 * p);
+        } else {
+            for (int l0 = 0; l0 < n_lgt; l0 += 2) pair(l0);
+        }
+        return scaled(acc, ma.w);                                                                     // renderer.rs:192
+    }
+};
+
+// cast_glass_rough for a DistributedView: the same recursion, the same turn of the rays a rough glass-like hit spawns (rg.g
+// null: no primitive is rough), with the level passed to direct().  A copy of its own, so that the rough-glass kernel keeps its
+// machine code.
+template <typename G, class DV>
+RM_HD Vec3<float> cast_glass_distributed(const DV& fv, const FrameParams<float>& fp, const RoughGlass& rg, Vec3<G> o, Vec3<G> d,
+                                         const float t1, const int slot1, const int id1) {
+    struct Frame {
+        Vec3<float> c;
+        Vec3<G> ro, rd;
+        float k;
+        int state;   // bit0: a refracted ray is pending, bit1: the refracted ray is the one in flight
+    };
+    Frame fr[kMaxDepth];
+    int sp = 0;
+    const Vec3<float> bg = {fp.background, fp.background, fp.background};
+    const int s = rg.samples, si = fv.si, sj = fv.sj;
+    Counters<false> st;
+    Vec3<float> v;
+    for (;;) {
+        const int level = sp + 1;                               // n_recursion
+        if (level > fp.max_depth) {
+            v = bg;                                             // renderer.rs:262-264
+        } else {
+            const Vec3<float> o32 = to_f32(o), d32 = to_f32(d);
+            HitRec<float> h;
+            bool got = true;
+            if (level == 1) {
+                h.dist = t1;
+                h.slot = slot1;
+                h.id = id1;
+            } else {
+                got = fv.template closest<false>(o32, d32, level, h, st);      // renderer.rs:266: the search, FP32
+            }
+            if (!got) {
+                v = bg;                                         // renderer.rs:300-306 (level > 1 here)
+            } else {
+                Vec3<G> p, n;
+                Vec3<float> p32, n32;
+                if constexpr (sizeof(G) == 8) {
+                    fv.refine(h.slot, o, d, (double)h.dist, p, n);
+                    p32 = to_f32(p);
+                    n32 = to_f32(n);
+                } else {
+                    fv.surface(h, o32, d32, n32);
+                    p32 = h.p;
+                    p = p32;
+                    n = n32;
+                }
+                const R4<float> ma = fv.mat_a[h.id];
+                const R4<float> mb = fv.mat_b[h.id];
+                Vec3<float> c = bg + fv.template direct<false>(level, d32, p32, n32, ma, mb, st);   // renderer.rs:272-275
+                bool pushed = false;
+                if (fv.mat_f[h.id] & 1) {                       // renderer.rs:277
+                    Vec3<G> ro1, rd1, ro2, rd2;
+                    using N = typename std::conditional<sizeof(G) == 8, Fast64, Exact<float>>::type;
+                    const bool has_refl = reflect_ray<G, N>(d, p, n, (G)mb.w, ro1, rd1);  // renderer.rs:203-207
+                    const bool has_refr = refract_ray<G, N>(d, p, n, (G)mb.w, ro2, rd2);  // renderer.rs:235-239
+                    const float gf = rg.g ? rg.g[h.id] : 0.f;
+                    if (gf > 0.f && (has_refl || has_refr)) {
+                        const int k = ((sj + level) % s) * s + si;   // rough_offset(s, si, sj, level)
+                        G lx, ly;
+                        if constexpr (sizeof(G) == 8) {
+                            lx = rg.off[2 * k];
+                            ly = rg.off[2 * k + 1];
+                        } else {
+                            lx = rg.off32[2 * k];
+                            ly = rg.off32[2 * k + 1];
+                        }
+                        if (lx != G(0) || ly != G(0)) {
+                            if (has_refl) {
+                                rd1 = rough_dir<G>(rd1, (G)gf, lx, ly);
+                                ro1 = rough_reflect_origin<G>(p, n, rd1);
+                            }
+                            if (has_refr) {
+                                rd2 = rough_dir<G>(rd2, (G)gf, lx, ly);
+                                ro2 = rough_refract_origin<G>(p, n, d, rd2);
+                            }
+                        }
+                    }
+                    if (has_refl || has_refr) {
+                        RM_FAST_CHECK(sp < kMaxDepth);
+                        Frame& f = fr[sp];
+                        f.c = c;
+                        f.k = mb.z;
+                        if (has_refl) {
+                            f.state = has_refr ? 1 : 0;
+                            f.ro = ro2;
+                            f.rd = rd2;
+                            o = ro1;
+                            d = rd1;
+                        } else {
+                            f.state = 2;
+                            o = ro2;
+                            d = rd2;
+                        }
+                        sp++;
+                        pushed = true;
+                    }
+                }
+                if (pushed) continue;
+                v = c;
+            }
+        }
+        for (;;) {                                              // return v to the callers on the stack
+            if (sp == 0) return v;
+            Frame& f = fr[sp - 1];
+            if (f.state & 2) {
+                f.c = f.c + scaled(v, 1.f - f.k);               // renderer.rs:249
+                v = f.c;
+                sp--;
+            } else {
+                f.c = f.c + scaled(v, f.k);                     // renderer.rs:219
+                if (f.state & 1) {
+                    o = f.ro;
+                    d = f.rd;
+                    f.state = 2;
+                    break;
+                }
+                v = f.c;
+                sp--;
+            }
+        }
+    }
+}
+// A sample ray (o, d) of a distributed frame whose level-1 query found h: lens_shade with cast_glass_distributed, and in
+// GLASS_NONE the direct lighting alone at level 1.
+template <int kGlass, class DV>
+RM_HD Vec3<float> distributed_shade(const DV& fv, const FrameParams<float>& fp, const RoughGlass& rg, const Vec3<double> o,
+                                    const Vec3<double> d, HitRec<float> h) {
+    if constexpr (kGlass == GLASS_F64) return cast_glass_distributed<double>(fv, fp, rg, o, d, h.dist, h.slot, h.id);
+    const Vec3<float> o32 = to_f32(o), d32 = to_f32(d);
+    if constexpr (kGlass == GLASS_F32) return cast_glass_distributed<float>(fv, fp, rg, o32, d32, h.dist, h.slot, h.id);
+    Vec3<float> normal;
+    fv.surface(h, o32, d32, normal);
+    Counters<false> st;
+    const Vec3<float> bg = {fp.background, fp.background, fp.background};
+    return bg + fv.template direct<false>(1, d32, h.p, normal, fv.mat_a[h.id], fv.mat_b[h.id], st);   // renderer.rs:272-275
+}
+
 }  // namespace rm

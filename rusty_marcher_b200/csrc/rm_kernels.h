@@ -138,6 +138,12 @@ cudaError_t launch_rough_glass(const DeviceScene<float>& ds, const FrameParams<f
 cudaError_t launch_motion(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const Motion& mo,
                           double reach, bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax,
                           cudaStream_t stream);
+// distributed_kernel (rm_distributed.cu; rm_render_distributed): lens_kernel's frame with the area lights' one point per sample
+//   and level (ap), the rough turn (rg; rg.g null: nothing is rough) and, when `motion`, every query of sample q at its time
+//   mo.tau[q] (ds then carries the swept hierarchy, and reach is as for launch_motion); ap, rg and mo have lc.samples.
+cudaError_t launch_distributed(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const AreaPoints& ap,
+                               const RoughGlass& rg, const Motion& mo, bool motion, double reach, bool cull, long long n_px,
+                               unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
 // K0 alone (prepare_raster_kernel, no view): the raster records of `camera` for the kernels that run stage A without K1.
 cudaError_t launch_prepare(const DeviceScene<float>& ds, bool cull, const double camera[3], cudaStream_t stream);
 // area_light_kernel (rm_area.cu; rm_render_area_lights): after launch_prepare for the same camera, the n_px pixels from frame row

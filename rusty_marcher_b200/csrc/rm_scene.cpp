@@ -634,6 +634,26 @@ void motion_displacements(const PackedScene<float>& ps, const double* disp, std:
     for (int i = 0; i < L.n_pln; i++) put((size_t)L.n_sph + L.n_tri + i, pln_id[i]);
 }
 
+AreaPoints make_area_points(const int samples, const double* radius, const int n, std::vector<float>& r) {
+    r.assign(std::max(n, 1), 0.f);
+    for (int l = 0; l < n; l++) {
+        const double v = radius[l];
+        r[l] = v > 0. ? std::max((float)std::min(v, (double)FLT_MAX), 1e-30f) : 0.f;
+    }
+    AreaPoints ap = {};
+    const int s = samples;
+    for (int i = 0; i < s; i++)                                 // level 0: every stratum once, the map being a bijection
+        for (int j = 0; j < s; j++) {
+            double lx, ly;
+            area_offset(s, i, j, 0, &lx, &ly);
+            const int k = ((i + 2 * j) % s) * s + (i + 3 * j) % s;
+            ap.off[2 * k] = (float)lx;
+            ap.off[2 * k + 1] = (float)ly;
+        }
+    ap.samples = s;
+    return ap;
+}
+
 Motion make_motion(const int samples) {
     Motion mo = {};
     const int s = samples;

@@ -138,6 +138,10 @@ RoughGlass make_rough_glass(int samples, const double* roughness, int n, std::ve
 void motion_displacements(const PackedScene<float>& ps, const double* disp, std::vector<R4<float>>& v, double& reach);
 // The samples' times of s x s (motion_time in f64 and rounded to FP32); the pointers are left for the caller to set.
 Motion make_motion(int samples);
+// The area lights of rm_render_distributed as the kernel reads them: r receives the n radii in FP32 (as rm_render_area_lights
+// keeps them: a positive radius too small for FP32 at 1e-30, at least one entry), and the returned AreaPoints the unit-disc
+// point of every stratum of area_offset; its radius pointer is left for the caller to set.  The radii are taken as given.
+AreaPoints make_area_points(int samples, const double* radius, int n, std::vector<float>& r);
 // The swept hierarchy of a motion frame: build_bvh over the pack's boxes, each grown by |v| / 2 per axis of its primitive's
 // displacement in v (make_motion's layout) -- the union of its boxes at tau = -1/2 and +1/2.  With every displacement zero
 // it is the pack's own hierarchy, byte for byte.

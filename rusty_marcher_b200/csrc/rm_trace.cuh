@@ -678,4 +678,21 @@ struct Motion {
     int samples;
 };
 
+// Distributed ray tracing (rm_render_distributed, include/rm_b200.h).  The light point of sample (i, j) of s x s at a shading
+// point of recursion level L: the unit-disc point (lens_offset's elliptical grid map) of the stratum
+// (a, b) = ((i + 2j + L) mod s, (i + 3j) mod s).  The map (i, j) -> (a, b) has determinant 1 over Z_s, a bijection over the s^2
+// samples at every level; (0, 0) at s = 1.  f64 without fused multiply-add; the kernel, the host emulation and the tests all
+// call it.
+RM_HD void area_offset(const int s, const int i, const int j, const int level, double* lx, double* ly) {
+    const int a = (i + 2 * j + level) % s, b = (i + 3 * j) % s;
+    lens_offset(s, (a - b + s) % s, b, lx, ly);                // lens_offset's stratum ((a - b) + b, b) mod s = (a, b)
+}
+// The call's area lights as the distributed kernel reads them: radius[l] as AreaLights has it; off[2 (a s + b)]: the unit-disc
+// point of stratum (a, b) rounded to FP32.
+struct AreaPoints {
+    const float* radius;
+    float off[2 * kAreaMaxSamples * kAreaMaxSamples];
+    int samples;
+};
+
 }  // namespace rm

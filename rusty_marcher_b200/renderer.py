@@ -263,11 +263,7 @@ class Renderer:
         uint8 with normalize + to_vec of that frame; returns the same kind of status message as render()."""
         if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
             raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        aperture, focus = float(aperture), float(focus)
-        if not (np.isfinite(aperture) and aperture >= 0.):
-            raise ValueError("aperture must be finite and >= 0, got %r" % (aperture,))
-        if not (np.isfinite(focus) and focus > 0.):
-            raise ValueError("focus must be finite and > 0, got %r" % (focus,))
+        aperture, focus = _lens_values(aperture, focus)
         if self.precision != _abi.RM_FP32:
             raise ValueError("render_lens computes in RM_FP32")
         if int(self.width) != frame.width or int(self.height) != frame.height:
@@ -307,14 +303,8 @@ class Renderer:
         as render()."""
         if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
             raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        n = len(scene.lights)
-        r = np.asarray(radii, dtype=np.float64)
-        if r.ndim == 0:
-            r = np.full(n, float(r))
-        if r.shape != (n,):
-            raise ValueError("radii must be one number or %d (one per light of the scene), got shape %s" % (n, r.shape))
-        if not (np.all(np.isfinite(r)) and np.all(r >= 0.)):
-            raise ValueError("every radius must be finite and >= 0, got %r" % (r.tolist(),))
+        r = _light_radii(scene, radii)
+        n = r.shape[0]
         if self.precision != _abi.RM_FP32:
             raise ValueError("render_area_lights computes in RM_FP32")
         if int(self.width) != frame.width or int(self.height) != frame.height:
@@ -326,7 +316,6 @@ class Renderer:
             if a is not None and (not isinstance(a, np.ndarray) or a.dtype != dtype or a.shape != shape or not a.flags.c_contiguous
                                   or not a.flags.writeable):
                 raise ValueError("%s must be a writeable C-contiguous %s array of shape %s" % (name, np.dtype(dtype).name, shape))
-        r = np.ascontiguousarray(r)
         lights = _abi.RmAreaLights()
         lights.n_lights, lights.radius, lights.samples = n, r.ctypes.data_as(C.POINTER(C.c_double)), int(samples)
         L = _abi.load()
@@ -358,19 +347,8 @@ class Renderer:
         frame; returns the same kind of status message as render()."""
         if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
             raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        n = len(scene.shapes)
-        g = np.asarray(roughness, dtype=np.float64)
-        if g.ndim == 0:
-            g = np.full(n, float(g))
-        if g.shape != (n,):
-            raise ValueError("roughness must be one number or %d (one per shape of the scene), got shape %s" % (n, g.shape))
-        if not (np.all(np.isfinite(g)) and np.all(g >= 0.)):
-            raise ValueError("every roughness must be finite and >= 0, got %r" % (g.tolist(),))
-        aperture, focus = float(aperture), float(focus)
-        if not (np.isfinite(aperture) and aperture >= 0.):
-            raise ValueError("aperture must be finite and >= 0, got %r" % (aperture,))
-        if not (np.isfinite(focus) and focus > 0.):
-            raise ValueError("focus must be finite and > 0, got %r" % (focus,))
+        per_prim = _roughness_by_prim(scene, roughness)
+        aperture, focus = _lens_values(aperture, focus)
         if self.precision != _abi.RM_FP32:
             raise ValueError("render_rough_glass computes in RM_FP32")
         if int(self.width) != frame.width or int(self.height) != frame.height:
@@ -384,8 +362,6 @@ class Renderer:
         if forward is not None:
             view = _view(forward, up)
             view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
-        # primitive ids: shapes in scene order, an Obj once per triangle
-        per_prim = np.ascontiguousarray(np.repeat(g, [s.triangles.shape[0] if isinstance(s, Obj) else 1 for s in scene.shapes]))
         lens = _abi.RmLens()
         lens.aperture, lens.focus, lens.samples = aperture, focus, int(samples)
         rough = _abi.RmRoughGlass()
@@ -418,19 +394,8 @@ class Renderer:
         rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the same kind of status message as render()."""
         if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
             raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        n = len(scene.shapes)
-        v = np.asarray(displacement, dtype=np.float64)
-        if v.shape == (3,):
-            v = np.tile(v, (n, 1))
-        if v.shape != (n, 3):
-            raise ValueError("displacement must be one 3-vector or %d (one per shape of the scene), got shape %s" % (n, v.shape))
-        if not np.all(np.isfinite(v)):
-            raise ValueError("every displacement must be finite, got %r" % (v.tolist(),))
-        aperture, focus = float(aperture), float(focus)
-        if not (np.isfinite(aperture) and aperture >= 0.):
-            raise ValueError("aperture must be finite and >= 0, got %r" % (aperture,))
-        if not (np.isfinite(focus) and focus > 0.):
-            raise ValueError("focus must be finite and > 0, got %r" % (focus,))
+        per_prim = _displacement_by_prim(scene, displacement)
+        aperture, focus = _lens_values(aperture, focus)
         if self.precision != _abi.RM_FP32:
             raise ValueError("render_motion computes in RM_FP32")
         if int(self.width) != frame.width or int(self.height) != frame.height:
@@ -444,8 +409,6 @@ class Renderer:
         if forward is not None:
             view = _view(forward, up)
             view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
-        # primitive ids: shapes in scene order, an Obj once per triangle
-        per_prim = np.ascontiguousarray(np.repeat(v, [s.triangles.shape[0] if isinstance(s, Obj) else 1 for s in scene.shapes], axis=0))
         lens = _abi.RmLens()
         lens.aperture, lens.focus, lens.samples = aperture, focus, int(samples)
         motion = _abi.RmMotion()
@@ -466,6 +429,120 @@ class Renderer:
         message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
         print(message)
         return message
+
+    def render_distributed(self, frame, scene, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., light_radii=None,
+                           roughness=None, displacement=None, rgb8=None, patch_rows=(0, -1)):
+        """EXTENSION MODE (no reference counterpart): distributed ray tracing.  Depth of field (forward / up, aperture / focus
+        as render_lens() takes them), soft shadows (light_radii as render_area_lights() takes its radii), rough glass
+        (roughness as render_rough_glass() takes it) and motion blur (displacement as render_motion() takes it) in one frame:
+        every one of the samples x samples rays of a pixel samples the lens, the time, one point of each area light and the
+        turn of every ray rough glass spawns, and the pixel is their mean (rm_render_distributed).  None leaves an effect out.
+        An area light here is one point per sample ray with the light's full colour -- not render_area_lights()'s frame.
+        samples = 1, or no active effect, is render_lens()'s frame; rough glass alone is render_rough_glass()'s and motion
+        alone render_motion()'s.  Fills frame.buffer (float32) over the rendered rows and, if given, rgb8 (H, W, 3) uint8 with
+        normalize + to_vec of that frame; returns the same kind of status message as render()."""
+        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
+            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
+        radii = None if light_radii is None else _light_radii(scene, light_radii)
+        rough_by_prim = None if roughness is None else _roughness_by_prim(scene, roughness)
+        disp_by_prim = None if displacement is None else _displacement_by_prim(scene, displacement)
+        aperture, focus = _lens_values(aperture, focus)
+        if self.precision != _abi.RM_FP32:
+            raise ValueError("render_distributed computes in RM_FP32")
+        if int(self.width) != frame.width or int(self.height) != frame.height:
+            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
+        if len(patch_rows) > 2 and patch_rows[2] > 1:
+            raise ValueError("render_distributed renders contiguous patch rows (stride <= 1)")
+        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
+                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
+            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
+        view = None
+        if forward is not None:
+            view = _view(forward, up)
+            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
+        s = int(samples)
+        lens = _abi.RmLens()
+        lens.aperture, lens.focus, lens.samples = aperture, focus, s
+        lights = rough = motion = None
+        if radii is not None:
+            lights = _abi.RmAreaLights()
+            lights.n_lights, lights.radius, lights.samples = radii.shape[0], radii.ctypes.data_as(C.POINTER(C.c_double)), s
+        if rough_by_prim is not None:
+            rough = _abi.RmRoughGlass()
+            rough.n_prims, rough.roughness, rough.samples = rough_by_prim.shape[0], rough_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s
+        if disp_by_prim is not None:
+            motion = _abi.RmMotion()
+            motion.n_prims, motion.displacement, motion.samples = disp_by_prim.shape[0], disp_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s
+        L = _abi.load()
+        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
+        now = time.perf_counter()
+        p = self.params(frame, scene, patch_rows)
+        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
+            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
+        stats = _abi.RmStats()
+        ref = lambda x: C.byref(x) if x is not None else None     # noqa: E731
+        _abi.check(L.rm_render_distributed(scene.device_handle(), C.byref(p), s, ref(view), C.byref(lens), ref(lights), ref(rough),
+                                           ref(motion), frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None,
+                                           C.byref(stats)))
+        self.last_stats = stats
+        ms = int((time.perf_counter() - now) * 1000)
+        fps = 1000. / ms if ms > 0 else float("inf")
+        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
+        print(message)
+        return message
+
+
+def _light_radii(scene, radii):
+    """One radius per light of the scene (one number for every light, or one per light), float64, checked."""
+    n = len(scene.lights)
+    r = np.asarray(radii, dtype=np.float64)
+    if r.ndim == 0:
+        r = np.full(n, float(r))
+    if r.shape != (n,):
+        raise ValueError("radii must be one number or %d (one per light of the scene), got shape %s" % (n, r.shape))
+    if not (np.all(np.isfinite(r)) and np.all(r >= 0.)):
+        raise ValueError("every radius must be finite and >= 0, got %r" % (r.tolist(),))
+    return np.ascontiguousarray(r)
+
+
+def _per_prim(scene, per_shape):
+    # primitive ids: shapes in scene order, an Obj once per triangle
+    return np.ascontiguousarray(np.repeat(per_shape, [s.triangles.shape[0] if isinstance(s, Obj) else 1 for s in scene.shapes], axis=0))
+
+
+def _roughness_by_prim(scene, roughness):
+    """The roughness of every primitive id (one number for every shape, or one per shape), float64, checked."""
+    n = len(scene.shapes)
+    g = np.asarray(roughness, dtype=np.float64)
+    if g.ndim == 0:
+        g = np.full(n, float(g))
+    if g.shape != (n,):
+        raise ValueError("roughness must be one number or %d (one per shape of the scene), got shape %s" % (n, g.shape))
+    if not (np.all(np.isfinite(g)) and np.all(g >= 0.)):
+        raise ValueError("every roughness must be finite and >= 0, got %r" % (g.tolist(),))
+    return _per_prim(scene, g)
+
+
+def _displacement_by_prim(scene, displacement):
+    """The displacement of every primitive id (one 3-vector for every shape, or one per shape), (n_prims, 3) float64, checked."""
+    n = len(scene.shapes)
+    v = np.asarray(displacement, dtype=np.float64)
+    if v.shape == (3,):
+        v = np.tile(v, (n, 1))
+    if v.shape != (n, 3):
+        raise ValueError("displacement must be one 3-vector or %d (one per shape of the scene), got shape %s" % (n, v.shape))
+    if not np.all(np.isfinite(v)):
+        raise ValueError("every displacement must be finite, got %r" % (v.tolist(),))
+    return _per_prim(scene, v)
+
+
+def _lens_values(aperture, focus):
+    aperture, focus = float(aperture), float(focus)
+    if not (np.isfinite(aperture) and aperture >= 0.):
+        raise ValueError("aperture must be finite and >= 0, got %r" % (aperture,))
+    if not (np.isfinite(focus) and focus > 0.):
+        raise ValueError("focus must be finite and > 0, got %r" % (focus,))
+    return aperture, focus
 
 
 def _view(forward, up):
