@@ -588,6 +588,59 @@ int rm_render_distributed(RmScene scene, const RmParams* params, int samples,
                           const RmAreaLights* lights /* NULL = point lights */, const RmRoughGlass* rough /* NULL = ideal optics */,
                           const RmMotion* motion /* NULL = nothing moves */, float* out_rgb, uint8_t* out_rgb8, RmStats* stats);
 
+/* ---- extension mode: diffuse interreflection -- light that bounces off opaque surfaces ------------------------------------- *
+ * The reference's opaque hits add background + direct lighting and spawn no ray (renderer.rs:277), so a surface receives
+ * light only from the lights it sees.  This call lets every opaque hit spawn one cosine-weighted diffuse ray per sample
+ * (Kajiya 1986): colour bleeds from one surface onto its neighbours, and corners that see less of the scene darken.  No
+ * scene data is added: the bounce's weight is the material's own diffusion * diffuse_color, the factor direct_lighting
+ * applies (renderer.rs:181-183,192).  The ABI version stays 5.
+ * Definition (normative; rm::diffuse_offset / rm::diffuse_point / rm::diffuse_stratum / rm::diffuse_normal / rm::diffuse_dir /
+ * rm::diffuse_origin in rm_trace.cuh are this, and the tests' restatement over the oracle is the same).  All in f64 without
+ * fused multiply-add; s = samples.
+ *   1. Sample (i, j), i, j in [0, s), of output pixel (x, y) is rm_render_lens's sample ray: rm::lens_ray with the view's basis
+ *      (the identity without a view) and the lens (aperture 0 without one).
+ *   2. The sample's value is the reference's cast_ray from that ray (renderer.rs:254-309, levels 1..max_depth, the reference's
+ *      order of additions) with one change.  At a hit of level L < max_depth on a primitive that is not glass-like, whose
+ *      diffusion is > 0 and some of whose diffuse_color components are > 0, the sample spawns one diffuse ray:
+ *        stratum: (a, b) = ((2i + 3j + L) mod s, (3i + 5j) mod s) -- determinant 2*5 - 3*3 = 1 over Z_s, a bijection over the
+ *          s^2 samples for every s and L; for s >= 4 neither coordinate is a shifted copy of a coordinate of the sub-pixel,
+ *          lens, rough, area or time strata (at s = 2 and 3 some sharing cannot be avoided);
+ *        disc point: the Shirley-Chiu concentric map of the stratum centre, p = (2a + 1)/s - 1, q = (2b + 1)/s - 1: (0, 0) if
+ *          p = q = 0; else if |p| > |q|, r = p and phi = (pi/4)(q/p); otherwise r = q and phi = pi/2 - (pi/4)(p/q);
+ *          (lx, ly) = (r cos phi, r sin phi).  The map is equal-area, so Malley's lift below is cosine-weighted (the elliptical
+ *          map of rm::lens_offset is not, and would weight the hemisphere wrongly);
+ *        direction: n_f = the hit normal turned against the incident ray d (n if dot(n, d) < 0, else -n); (t1, t2) =
+ *          rm::light_frame(n_f); z = sqrt(1 - ((lx lx) + (ly ly))), > 0 since r <= 1 - 1/s;
+ *          rd = normalized(((lx t1) + (ly t2)) + z n_f), component by component in that order;
+ *        origin: point + n_f 1e-4, reflect_ray's offset (optics.rs:41-45);
+ *        addition: c = background + direct as the reference has it, then c += scaled(v * diffuse_color, diffusion), with v the
+ *          value of the diffuse ray at level L + 1 (a miss there is the background, as for every level > 1).
+ *      Glass-like hits keep the reference's optics and spawn no diffuse ray, so a level pushes at most one frame and max_depth
+ *      caps the whole path, bounces included.
+ *   3. The pixel is the FP32 mean of its s^2 sample values in rm::resolve_box's order (sub-rows i outer, j inner).
+ * Consequences:
+ *   - Primary visibility is rm_render_lens's.  At s = 1 every hit bounces once, along n_f.
+ *   - The pattern is fixed per pixel, not random: the frame is deterministic, and under-sampled indirect light shows as
+ *     structure, not noise.
+ *   - max_depth = 1, and scenes in which no primitive meets the bounce condition (decided on the host from the scene's
+ *     materials), give rm_render_lens's frame bit for bit and are routed there.  s = 1 is not routed.
+ * FP32 production path (indirect_kernel): lens_kernel's schedule; each sample ray from rm::lens_ray in f64, traced with the
+ * general FP32 closest-hit query (brute force, or the hierarchy with accel != 0 for scenes of at most 8 lights; accel = 2
+ * renders as accel = 1).  The disc points are computed on the host (cos and sin) and read from a table; the bounce is computed
+ * in f64 from the refined f64 point and normal where the scene takes f64 ray geometry, in FP32 otherwise.  Frames meet the FP32
+ * parity criteria against the f64 definition.  cull_backfacing applies.
+ * Rows, outputs and stats as rm_render_lens: patch rows [b, e) with patch_row_stride <= 1, rows outside untouched; out_rgb
+ * and / or out_rgb8; stats: max_value, ms_render, ms_total, kernel_launches, resident_prims, d2h_bytes.  The call writes the
+ * caller's float frame, so the library forgets its previous deliveries into that memory (RM_ROWS_RETAINED).
+ * RM_ERR_INVALID_ARGUMENT: samples outside [1, 8]; an invalid view or lens by rm_render_lens's rules; lens->samples !=
+ * samples; precision other than RM_FP32; patch_row_stride > 1; max_depth < 1; out_rgb and out_rgb8 both NULL (all reported
+ * without a device); an unknown scene.  RM_ERR_DIMENSIONS: as for rm_render_supersampled.
+ * Out of scope: combining with rm_render_distributed (area lights, rough glass, motion); bounces from glass-like hits;
+ * emissive materials; random or per-pixel patterns and progressive accumulation; an FP64 entry point; rm_render_rows_*,
+ * rm_render_frame, rm_render_adaptive or rm_render_dispersive. */
+int rm_render_indirect(RmScene scene, const RmParams* params, const RmView* view /* NULL = the reference's camera */,
+                       const RmLens* lens /* NULL = pinhole */, int samples, float* out_rgb, uint8_t* out_rgb8, RmStats* stats);
+
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device
  * scalar of the same type as d_rgb that receives max(previous value, tile max) -- zero it first.

@@ -1713,6 +1713,25 @@ std::vector<unsigned char> glass_like_by_id(const rm::OwnedFlatScene& f) {
     return out;
 }
 
+// Whether some primitive spawns rm_render_indirect's diffuse ray: not glass-like, diffusion > 0 and a diffuse_color component > 0.
+bool any_diffuse_bounce(const rm::OwnedFlatScene& f) {
+    auto bounces = [](const RmReflectance& r) {
+        return !r.is_glass_like && r.diffusion > 0. && (r.diffuse_color[0] > 0. || r.diffuse_color[1] > 0. || r.diffuse_color[2] > 0.);
+    };
+    for (const RmShapeRef& sh : f.shapes) {
+        if (sh.kind == RM_SHAPE_SPHERE) {
+            if (bounces(f.spheres[sh.index].reflectance)) return true;
+        } else if (sh.kind == RM_SHAPE_POLYGON) {
+            if (bounces(f.polygons[sh.index].reflectance)) return true;
+        } else {
+            const RmObj& o = f.objs[sh.index];
+            for (int t = 0; t < o.n_triangles; t++)
+                if (bounces(f.triangle_reflectances[o.first_triangle + t])) return true;
+        }
+    }
+    return false;
+}
+
 // Extension mode (include/rm_b200.h): rough_glass_kernel traces and resolves the output rows, then, for the 8-bit frame, the
 // tone-map kernel.  s = 1, and calls in which no glass-like primitive is rough, are rm_render_lens's frame and go there.  The
 // argument checks need no device, except the primitive count, which needs the scene.
@@ -1780,6 +1799,99 @@ int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* v
     int launches = 0;
     if (rows) {
         CK(rm::launch_rough_glass(dp.ds, fp, lc, rg, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
+        launches++;
+    }
+    CK(cudaEventRecord(g.ev[2], s));
+    if (out_rgb8 && rows) {
+        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
+        launches++;
+    }
+    const size_t host_px = (size_t)fp.row_begin * fp.width;
+    if (out_rgb && n_px) {
+        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
+        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
+    }
+    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
+    float h_max = 0.f;
+    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
+    CK(cudaEventRecord(g.ev[3], s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) {
+        std::memset(stats, 0, sizeof(*stats));
+        stats->max_value = (double)h_max;
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
+        stats->ms_render = ms;
+        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
+        stats->ms_total = ms;
+        stats->kernel_launches = launches;
+        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
+    }
+    return RM_OK;
+}
+
+// Extension mode (include/rm_b200.h): indirect_kernel traces and resolves the output rows, then, for the 8-bit frame, the
+// tone-map kernel.  max_depth = 1, and scenes in which no primitive bounces, are rm_render_lens's frame and go there.  The
+// argument checks need no device.
+int rm_render_indirect(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, int samples, float* out_rgb,
+                       uint8_t* out_rgb8, RmStats* stats) {
+    if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect: samples must be in [1, 8]");
+    const int S = samples;
+    const RmLens pinhole = {0., 1., S};
+    int rc = check_lens(lens ? lens : &pinhole);
+    if (rc != RM_OK) return rc;
+    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lens: samples must equal the call's samples");
+    rm::ViewBasis vb;
+    bool identity = true;
+    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
+    if ((rc = check_params(params)) != RM_OK) return rc;
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect needs max_depth >= 1");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
+    RmParams sp = *params;
+    sp.width = S * params->width;
+    sp.height = S * params->height;
+    sp.patch_row_begin = 0;
+    sp.patch_row_end = -1;
+    if ((rc = check_params(&sp)) != RM_OK) return rc;
+    const RmLens& ln = lens ? *lens : pinhole;
+    bool any_bounce = false;
+    {
+        std::lock_guard<std::mutex> lock(g.mu);
+        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+        auto it = g.scenes.find(scene);
+        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+        any_bounce = any_diffuse_bounce(it->second.flat);
+    }
+    // one level, or no primitive that bounces: no diffuse ray is spawned, rm_render_lens's frame bit for bit
+    if (params->max_depth == 1 || !any_bounce) return rm_render_lens(scene, params, view, &ln, out_rgb, out_rgb8, stats);
+    std::lock_guard<std::mutex> lock(g.mu);
+    auto it = g.scenes.find(scene);
+    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    DevicePack<float>& dp = it->second.f32;
+    cudaStream_t s = g.stream;
+    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
+    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
+    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
+    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const bool cull = params->cull_backfacing != 0;
+    const rm::Diffuse df = rm::make_diffuse(S);
+    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
+    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
+    float* d_max = static_cast<float*>(g.small.p);
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
+    CK(cudaEventRecord(g.ev[0], s));
+    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
+    CK(cudaEventRecord(g.ev[1], s));
+    int launches = 0;
+    if (rows) {
+        CK(rm::launch_indirect(dp.ds, fp, lc, df, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
         launches++;
     }
     CK(cudaEventRecord(g.ev[2], s));

@@ -144,6 +144,10 @@ cudaError_t launch_motion(const DeviceScene<float>& ds, const FrameParams<float>
 cudaError_t launch_distributed(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const AreaPoints& ap,
                                const RoughGlass& rg, const Motion& mo, bool motion, double reach, bool cull, long long n_px,
                                unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
+// indirect_kernel (rm_indirect.cu; rm_render_indirect): lens_kernel's frame with one diffuse bounce per qualifying opaque hit
+//   (cast_indirect) at the disc points df; df.samples == lc.samples.
+cudaError_t launch_indirect(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const Diffuse& df,
+                            bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
 // K0 alone (prepare_raster_kernel, no view): the raster records of `camera` for the kernels that run stage A without K1.
 cudaError_t launch_prepare(const DeviceScene<float>& ds, bool cull, const double camera[3], cudaStream_t stream);
 // area_light_kernel (rm_area.cu; rm_render_area_lights): after launch_prepare for the same camera, the n_px pixels from frame row

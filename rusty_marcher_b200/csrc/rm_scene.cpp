@@ -685,4 +685,20 @@ int build_swept_bvh(const PackedScene<float>& ps, const std::vector<R4<float>>& 
     return build_bvh(boxes, nodes, prims, pool);
 }
 
+Diffuse make_diffuse(const int samples) {
+    Diffuse df = {};
+    const int s = samples;
+    for (int a = 0; a < s; a++)
+        for (int b = 0; b < s; b++) {
+            double lx, ly;
+            diffuse_point(s, a, b, &lx, &ly);
+            df.off[2 * (a * s + b)] = lx;
+            df.off[2 * (a * s + b) + 1] = ly;
+            df.off32[2 * (a * s + b)] = (float)lx;
+            df.off32[2 * (a * s + b) + 1] = (float)ly;
+        }
+    df.samples = s;
+    return df;
+}
+
 }  // namespace rm

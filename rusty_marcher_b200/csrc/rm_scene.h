@@ -131,6 +131,9 @@ LensCamera make_lens_camera(const RmParams& p, const double* basis, const RmLens
 // left for the caller to set.  The values are taken as given (rm_render_rough_glass checks them).
 RoughGlass make_rough_glass(int samples, const double* roughness, int n, std::vector<float>& g);
 
+// The disc points of rm_render_indirect's bounces as the kernel reads them: diffuse_point of every stratum of s x s.
+Diffuse make_diffuse(int samples);
+
 // The motion of rm_render_motion as the kernel reads it: v receives the FP32 displacement {v, 0} of every primitive of the
 // FP32 pack ps by the kernel's indices (Motion's layout: spheres | fast-path triangles | plane slots, from the ids in the
 // blob), disp holding 3 doubles per primitive id; reach receives the largest |component| of those FP32 values over 2.  The

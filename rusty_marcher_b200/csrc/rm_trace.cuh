@@ -695,4 +695,58 @@ struct AreaPoints {
     int samples;
 };
 
+// Diffuse interreflection (rm_render_indirect, include/rm_b200.h).  The normative definition in f64 without fused
+// multiply-add; the kernel, the host emulation and the tests all call these functions.
+// diffuse_point: the Shirley-Chiu concentric map (1997) of the centre of stratum (a, b) of s x s, (p, q) = ((2a + 1) / s - 1,
+// (2b + 1) / s - 1), to the unit disc.  Equal-area, so Malley's lift of the points to the hemisphere is cosine-weighted.  It
+// needs cos and sin, whose host and device results may differ, so it is evaluated on the host only (the kernel reads a table).
+inline void diffuse_point(const int s, const int a, const int b, double* lx, double* ly) {
+    const double p = (2. * a + 1.) / s - 1., q = (2. * b + 1.) / s - 1.;
+    const double quarter_pi = 3.14159265358979323846 / 4.;
+    if (p == 0. && q == 0.) {
+        *lx = 0.;
+        *ly = 0.;
+        return;
+    }
+    double r, phi;
+    if (fabs(p) > fabs(q)) {
+        r = p;
+        phi = quarter_pi * (q / p);
+    } else {
+        r = q;
+        phi = 3.14159265358979323846 / 2. - quarter_pi * (p / q);
+    }
+    *lx = r * cos(phi);
+    *ly = r * sin(phi);
+}
+// The stratum of sample (i, j) of s x s at recursion level L (1 = the sample ray's own hit): (a, b) = ((2i + 3j + L) mod s,
+// (3i + 5j) mod s), a map of determinant 1 over Z_s, so a bijection over the s^2 samples at every level.
+RM_HD int diffuse_stratum(const int s, const int i, const int j, const int level) {
+    return ((2 * i + 3 * j + level) % s) * s + (3 * i + 5 * j) % s;
+}
+inline void diffuse_offset(const int s, const int i, const int j, const int level, double* lx, double* ly) {
+    const int k = diffuse_stratum(s, i, j, level);
+    diffuse_point(s, k / s, k % s, lx, ly);
+}
+// The hit normal turned against the incident ray d: n if dot(n, d) < 0, else -n.
+template <typename R> RM_HD Vec3<R> diffuse_normal(const Vec3<R> n, const Vec3<R> d) { return dot(n, d) < R(0) ? n : -n; }
+// The bounce direction around the facing normal nf: Malley's lift of the disc point (lx, ly) in light_frame's basis,
+// normalized(((lx t1) + (ly t2)) + z nf) with z = sqrt(1 - ((lx lx) + (ly ly))), component by component in that order.
+template <typename R> RM_HD Vec3<R> diffuse_dir(const Vec3<R> nf, const R lx, const R ly) {
+    Vec3<R> t1, t2;
+    light_frame<R>(nf, t1, t2);
+    const R z = Num<R>::sqrt_(R(1) - ((lx * lx) + (ly * ly)));
+    return normalized(Vec3<R>{((lx * t1.x) + (ly * t2.x)) + z * nf.x, ((lx * t1.y) + (ly * t2.y)) + z * nf.y,
+                              ((lx * t1.z) + (ly * t2.z)) + z * nf.z});
+}
+// The bounce ray's origin: point + nf 1e-4, reflect_ray's offset (optics.rs:41-45).
+template <typename R> RM_HD Vec3<R> diffuse_origin(const Vec3<R> point, const Vec3<R> nf) { return axpy(point, nf, R(1e-4)); }
+// The call's bounce points as the kernel reads them: off[2 (a s + b)] = diffuse_point(s, a, b) in f64, and rounded to FP32
+// in off32.
+struct Diffuse {
+    double off[2 * kAreaMaxSamples * kAreaMaxSamples];
+    float off32[2 * kAreaMaxSamples * kAreaMaxSamples];
+    int samples;
+};
+
 }  // namespace rm

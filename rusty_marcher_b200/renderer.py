@@ -491,6 +491,51 @@ class Renderer:
         print(message)
         return message
 
+    def render_indirect(self, frame, scene, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., rgb8=None,
+                        patch_rows=(0, -1)):
+        """EXTENSION MODE (no reference counterpart): diffuse interreflection.  Every opaque hit whose material has diffusion > 0
+        and a non-black diffuse_color spawns one cosine-weighted diffuse ray, a different one for each of the samples x samples
+        rays of a pixel, and adds what it sees weighted by diffusion * diffuse_color: colour bleeds between surfaces and
+        corners darken (rm_render_indirect).  The scene's max_depth caps the whole path, bounces included.  forward / up turn
+        the camera as render_view() does, aperture / focus add render_lens()'s thin lens (aperture 0: the pinhole).
+        max_depth = 1, or a scene in which nothing bounces, is render_lens()'s frame.  Fills frame.buffer (float32) over the
+        rendered rows and, if given, rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the same kind of
+        status message as render()."""
+        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
+            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
+        aperture, focus = _lens_values(aperture, focus)
+        if self.precision != _abi.RM_FP32:
+            raise ValueError("render_indirect computes in RM_FP32")
+        if int(self.width) != frame.width or int(self.height) != frame.height:
+            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
+        if len(patch_rows) > 2 and patch_rows[2] > 1:
+            raise ValueError("render_indirect renders contiguous patch rows (stride <= 1)")
+        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
+                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
+            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
+        view = None
+        if forward is not None:
+            view = _view(forward, up)
+            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
+        s = int(samples)
+        lens = _abi.RmLens()
+        lens.aperture, lens.focus, lens.samples = aperture, focus, s
+        L = _abi.load()
+        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
+        now = time.perf_counter()
+        p = self.params(frame, scene, patch_rows)
+        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
+            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
+        stats = _abi.RmStats()
+        _abi.check(L.rm_render_indirect(scene.device_handle(), C.byref(p), C.byref(view) if view is not None else None, C.byref(lens), s,
+                                        frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
+        self.last_stats = stats
+        ms = int((time.perf_counter() - now) * 1000)
+        fps = 1000. / ms if ms > 0 else float("inf")
+        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
+        print(message)
+        return message
+
 
 def _light_radii(scene, radii):
     """One radius per light of the scene (one number for every light, or one per light), float64, checked."""
