@@ -40,6 +40,12 @@
 //                                      an extension).  Combines with --samples, --aperture / --focus, --look-at / --up,
 //                                      --camera and --accel; not with --light-radius, --roughness, --move, --combine,
 //                                      --contrast, --f64 or --rows-f64
+//   --path                             path-traced frames: --indirect's diffuse bounce with --combine's --light-radius,
+//                                      --roughness, --move and --aperture / --focus, --samples S x S rays per pixel each
+//                                      sampling every effect and every bounce at once, --depth capping the whole path
+//                                      (rm_render_path; an extension).  Combines with --samples, --depth, --light-radius,
+//                                      --roughness, --move, --aperture / --focus, --look-at / --up, --camera and --accel; not
+//                                      with --combine, --indirect, --contrast, --f64 or --rows-f64
 //
 //   g++ -std=c++17 -Iinclude examples/rm_headless.cpp -o examples/rm_headless -Lrusty_marcher_b200 -lrm_b200 -Wl,-rpath,'$ORIGIN/../rusty_marcher_b200'
 #include <chrono>
@@ -77,6 +83,7 @@ int main(int argc, char** argv) {
     bool moving = false;
     bool combine = false;
     bool indirect = false;
+    bool path = false;
     int move_shape = -1;
     double move_by[3] = {0., 0., 0.};
     auto triple = [](const char* s, double v[3]) { char end = 0; return std::sscanf(s, "%lf,%lf,%lf%c", &v[0], &v[1], &v[2], &end) == 3; };
@@ -95,6 +102,7 @@ int main(int argc, char** argv) {
         else if (a == "--accel") accel = 1;
         else if (a == "--combine") combine = true;
         else if (a == "--indirect") indirect = true;
+        else if (a == "--path") path = true;
         else if (a == "--samples") { need(1); samples = std::atoi(argv[++i]); }
         else if (a == "--contrast") { need(1); contrast = std::strtod(argv[++i], nullptr); adaptive = true; }
         else if (a == "--aperture") { need(1); lens.aperture = std::strtod(argv[++i], nullptr); use_lens = true; }
@@ -141,23 +149,27 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "rm_headless: --combine does not combine with --contrast, --f64 or --rows-f64\n");
         return 2;
     }
+    if (path && (combine || indirect || adaptive || f64 || rows64)) {
+        std::fprintf(stderr, "rm_headless: --path does not combine with --combine, --indirect, --contrast, --f64 or --rows-f64\n");
+        return 2;
+    }
     if (indirect && (area || rough || moving || combine || adaptive || f64 || rows64)) {
         std::fprintf(stderr, "rm_headless: --indirect does not combine with --light-radius, --roughness, --move, --combine, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (area && !combine && (look || use_lens || adaptive || f64 || rows64)) {
+    if (area && !combine && !path && (look || use_lens || adaptive || f64 || rows64)) {
         std::fprintf(stderr, "rm_headless: --light-radius does not combine with --look-at, --aperture, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (rough && !combine && (area || adaptive || f64 || rows64)) {
+    if (rough && !combine && !path && (area || adaptive || f64 || rows64)) {
         std::fprintf(stderr, "rm_headless: --roughness does not combine with --light-radius, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (moving && !combine && (rough || area || adaptive || f64 || rows64)) {
+    if (moving && !combine && !path && (rough || area || adaptive || f64 || rows64)) {
         std::fprintf(stderr, "rm_headless: --move does not combine with --roughness, --light-radius, --contrast, --f64 or --rows-f64\n");
         return 2;
     }
-    if (look && !combine && !indirect && !use_lens && !rough && !moving && (samples > 1 || adaptive || rows64)) {
+    if (look && !combine && !path && !indirect && !use_lens && !rough && !moving && (samples > 1 || adaptive || rows64)) {
         std::fprintf(stderr, "rm_headless: --look-at does not combine with --samples, --contrast or --rows-f64\n");
         return 2;
     }
@@ -257,7 +269,10 @@ int main(int argc, char** argv) {
     for (int f = 0; f < frames; f++) {
         const auto t0 = std::chrono::steady_clock::now();
         std::memset(&st, 0, sizeof st);
-        if (combine) rc = rm_render_distributed(scene, &p, samples, look ? &view : nullptr, use_lens ? &lens : nullptr, area ? &area_lights : nullptr,
+        if (path) rc = rm_render_path(scene, &p, samples, look ? &view : nullptr, use_lens ? &lens : nullptr, area ? &area_lights : nullptr,
+                                      rough ? &rough_glass : nullptr, moving ? &motion : nullptr, rgb32.data(),
+                                      f == frames - 1 ? rgb8.data() : nullptr, &st);
+        else if (combine) rc = rm_render_distributed(scene, &p, samples, look ? &view : nullptr, use_lens ? &lens : nullptr, area ? &area_lights : nullptr,
                                                 rough ? &rough_glass : nullptr, moving ? &motion : nullptr, rgb32.data(),
                                                 f == frames - 1 ? rgb8.data() : nullptr, &st);
         else if (indirect) rc = rm_render_indirect(scene, &p, look ? &view : nullptr, use_lens ? &lens : nullptr, samples, rgb32.data(),
@@ -279,7 +294,7 @@ int main(int argc, char** argv) {
         std::printf("Scene rendered in %lld ms (%u fps, %.2f MP/s)\n", ms, ms > 0 ? (unsigned)fps : 4294967295u, fps * (double)n_px / 1e6);
     }
     // "Save to file": normalize + to_vec on the device (framebuffer.rs:40-82), then the P6 stream (framebuffer.rs:26-38)
-    if (combine || indirect || use_lens || area || rough || moving) {
+    if (path || combine || indirect || use_lens || area || rough || moving) {
         // (the last frame above wrote the 8-bit frame)
     } else if (adaptive) {
         std::vector<unsigned char> mask(n_px, 0);

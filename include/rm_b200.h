@@ -582,7 +582,7 @@ int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view /
  * from the scene's light count, n_prims different from rm_scene_num_prims(scene); an unknown scene.  RM_ERR_DIMENSIONS: as
  * for rm_render_supersampled.
  * Out of scope: random or per-pixel patterns; an FP64 entry point; combining with rm_render_adaptive, rm_render_dispersive,
- * rm_render_rows_* or rm_render_frame; moving lights. */
+ * rm_render_rows_* or rm_render_frame; moving lights.  Diffuse interreflection with these effects: rm_render_path. */
 int rm_render_distributed(RmScene scene, const RmParams* params, int samples,
                           const RmView* view /* NULL = the reference's camera */, const RmLens* lens /* NULL = pinhole */,
                           const RmAreaLights* lights /* NULL = point lights */, const RmRoughGlass* rough /* NULL = ideal optics */,
@@ -637,9 +637,60 @@ int rm_render_distributed(RmScene scene, const RmParams* params, int samples,
  * without a device); an unknown scene.  RM_ERR_DIMENSIONS: as for rm_render_supersampled.
  * Out of scope: combining with rm_render_distributed (area lights, rough glass, motion); bounces from glass-like hits;
  * emissive materials; random or per-pixel patterns and progressive accumulation; an FP64 entry point; rm_render_rows_*,
- * rm_render_frame, rm_render_adaptive or rm_render_dispersive. */
+ * rm_render_frame, rm_render_adaptive or rm_render_dispersive.  The bounce with area lights, rough glass and motion:
+ * rm_render_path. */
 int rm_render_indirect(RmScene scene, const RmParams* params, const RmView* view /* NULL = the reference's camera */,
                        const RmLens* lens /* NULL = pinhole */, int samples, float* out_rgb, uint8_t* out_rgb8, RmStats* stats);
+
+/* ---- extension mode: path-traced frames -- diffuse interreflection with depth of field, soft shadows, rough glass and
+ * motion blur at once ------------------------------------------------------------------------------------------------------ *
+ * rm_render_indirect's diffuse bounce inside rm_render_distributed's frame: every sample ray samples the lens point, the time,
+ * a point of each area light, the turn of every ray rough glass spawns and the direction of every diffuse ray, and the pixel
+ * is the mean over its samples (Cook 1984 with Kajiya 1986's bounce).  The signature is rm_render_distributed's; no struct is
+ * added or changed, and the ABI version stays 5.
+ * Definition (normative; every rule is already stated above for rm_render_lens, rm_render_motion, rm_render_rough_glass,
+ * rm_render_distributed and rm_render_indirect, and the tests' restatement over the oracle is the same).  All in f64 without
+ * fused multiply-add; s = samples, and every struct given has samples == s.
+ *   1. Sample ray.  Sample (i, j), i, j in [0, s), of output pixel (x, y) is rm_render_lens's sample ray: rm::lens_ray with the
+ *      view's basis (the identity without a view) and the lens (aperture 0 without one).
+ *   2. Time.  tau = rm::motion_time(s, i, j), and the sample sees the scene at tau as RmMotion defines it.  Every query of the
+ *      sample's path sees the same tau: primary, glass, diffuse and shadow rays alike.  Lights and the camera do not move.
+ *   3. Rough glass.  The rays a rough glass-like hit of level L spawns are turned with rm::rough_offset(s, i, j, L), as in
+ *      rm_render_distributed rule 3.
+ *   4. Area lights.  At every shading point of level L, a light of radius r > 0 is one point light of its full colour at the
+ *      point of stratum rm::area_offset(s, i, j, L), as in rm_render_distributed rule 4.  The hit of a diffuse ray spawned at
+ *      level L is a shading point of level L + 1, so it samples its lights at rm::area_offset(s, i, j, L + 1).
+ *   5. Diffuse bounce.  rm_render_indirect rule 2, unchanged: at a hit of level L < max_depth on a primitive that is not
+ *      glass-like, whose diffusion is > 0 and some of whose diffuse_color components are > 0, one diffuse ray of stratum
+ *      rm::diffuse_stratum(s, i, j, L), through the concentric disc map and rm::diffuse_dir, from rm::diffuse_origin; the point
+ *      and normal are the scene's at tau.  The additions are, in this order: c = background + direct(L); then, if glass-like,
+ *      the reference's reflect / refract terms; otherwise c += scaled(v * diffuse_color, diffusion).
+ *   6. The pixel is the FP32 mean of its s^2 sample values in rm::resolve_box's order (sub-rows i outer, j inner).
+ * Glass-like hits spawn no diffuse ray, so a level pushes at most one frame and max_depth caps the whole path.
+ * Routing -- each routed case is that call, and gives its frame bit for bit.  "Active" is as rm_render_distributed has it: a
+ * radius > 0, roughness > 0 on a glass-like primitive, a displacement != 0.
+ *   - max_depth = 1, or no primitive meets the bounce condition (decided on the host from the scene's materials):
+ *     rm_render_distributed with the same arguments (which routes further by itself);
+ *   - otherwise s = 1 (area_offset, rough_offset and motion_time are then the identity), or no active effect:
+ *     rm_render_indirect(scene, params, view, lens, s, ...);
+ *   - otherwise path_kernel.
+ * FP32 production path (path_kernel): distributed_kernel's schedule, with rm_render_distributed's queries (at the sample's tau
+ * over the swept hierarchy with accel != 0 when motion is active, over the scene's own otherwise; brute force for scenes of
+ * more than 8 lights), its light points and its rough turn, and rm_render_indirect's bounce: read from the host's disc-point
+ * table, computed in f64 from the refined f64 point (at tau with motion) and normal where the scene takes f64 ray geometry, in
+ * FP32 otherwise.  Frames meet the FP32 parity criteria against the f64 definition.  cull_backfacing applies.
+ * Rows, outputs and stats as rm_render_distributed: patch rows [b, e) with patch_row_stride <= 1, rows outside untouched;
+ * out_rgb and / or out_rgb8; stats: max_value, ms_render, ms_total, kernel_launches, resident_prims, d2h_bytes.  The call
+ * writes the caller's float frame, so the library forgets its previous deliveries into that memory (RM_ROWS_RETAINED).
+ * RM_ERR_INVALID_ARGUMENT: as for rm_render_distributed, with the same messages for the structs (reported without a device,
+ * except the light and primitive counts); an unknown scene.  RM_ERR_DIMENSIONS: as for rm_render_supersampled.
+ * Out of scope: bounces from glass-like hits; emissive materials and sampling emitters by their geometry; random, per-pixel or
+ * progressive sample patterns and s > 8; an FP64 entry point; rm_render_rows_*, rm_render_frame, rm_render_adaptive or
+ * rm_render_dispersive; moving lights. */
+int rm_render_path(RmScene scene, const RmParams* params, int samples, const RmView* view /* NULL = the reference's camera */,
+                   const RmLens* lens /* NULL = pinhole */, const RmAreaLights* lights /* NULL = point lights */,
+                   const RmRoughGlass* rough /* NULL = ideal optics */, const RmMotion* motion /* NULL = nothing moves */,
+                   float* out_rgb, uint8_t* out_rgb8, RmStats* stats);
 
 /* ---- the hot path, device buffers (no copies; for callers that keep frames in HBM) ----------- *
  * d_rgb: device float (RM_FP32) or double (RM_FP64) H*W*3; d_prim_id optional; d_max: device

@@ -15,7 +15,7 @@ fn main() {
         ])
         .arg(&lib)
         .args(
-            ["rm_api.cu", "rm_kernels.cu", "rm_lens.cu", "rm_area.cu", "rm_rough.cu", "rm_motion.cu", "rm_distributed.cu", "rm_indirect.cu", "rm_scene.cpp", "rm_bvh.cpp", "rm_host.cpp"]
+            ["rm_api.cu", "rm_kernels.cu", "rm_lens.cu", "rm_area.cu", "rm_rough.cu", "rm_motion.cu", "rm_distributed.cu", "rm_indirect.cu", "rm_path.cu", "rm_scene.cpp", "rm_bvh.cpp", "rm_host.cpp"]
                 .iter()
                 .map(|f| src.join(f)),
         )

@@ -275,6 +275,11 @@ extern "C" {
     /// pixel through the thin lens (null: pinhole) from the camera turned to `view` (null: down -z)
     pub fn rm_render_indirect(scene: RmScene, params: *const RmParams, view: *const RmView, lens: *const RmLens, samples: c_int,
                               out_rgb: *mut f32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
+    /// path-traced frames: rm_render_indirect's diffuse bounce with rm_render_distributed's lens, area lights, rough glass and
+    /// motion (each null: left out), s x s samples per pixel
+    pub fn rm_render_path(scene: RmScene, params: *const RmParams, samples: c_int, view: *const RmView, lens: *const RmLens,
+                          lights: *const RmAreaLights, rough: *const RmRoughGlass, motion: *const RmMotion,
+                          out_rgb: *mut f32, out_rgb8: *mut u8, stats: *mut RmStats) -> c_int;
     // ---- the hot path, device buffers
     pub fn rm_render_device(scene: RmScene, params: *const RmParams, d_rgb: *mut c_void, d_prim_id: *mut i32,
                             d_max: *mut c_void, stream: *mut c_void) -> c_int;

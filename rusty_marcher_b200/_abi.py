@@ -148,6 +148,8 @@ SYMBOLS = {
     "rm_render_distributed": (C.c_int, [C.c_int64, _P(RmParams), C.c_int, _P(RmView), _P(RmLens), _P(RmAreaLights), _P(RmRoughGlass),
                                         _P(RmMotion), C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_render_indirect": (C.c_int, [C.c_int64, _P(RmParams), _P(RmView), _P(RmLens), C.c_int, C.c_void_p, C.c_void_p, _P(RmStats)]),
+    "rm_render_path": (C.c_int, [C.c_int64, _P(RmParams), C.c_int, _P(RmView), _P(RmLens), _P(RmAreaLights), _P(RmRoughGlass), _P(RmMotion),
+                                 C.c_void_p, C.c_void_p, _P(RmStats)]),
     "rm_scene_query_count": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),
     "rm_scene_accel_status": (C.c_int, [C.c_int64, _P(C.c_int32)]),
     "rm_scene_walk_stats": (C.c_int, [C.c_int64, _P(C.c_uint64), C.c_int]),

@@ -2224,6 +2224,141 @@ int rm_render_distributed(RmScene scene, const RmParams* params, int samples, co
     return RM_OK;
 }
 
+// Extension mode (include/rm_b200.h): path_kernel traces and resolves the output rows with the diffuse bounce and every given
+// effect at once, then, for the 8-bit frame, the tone-map kernel.  max_depth = 1, or a scene in which no primitive bounces, is
+// rm_render_distributed's frame; s = 1, or no active effect, is rm_render_indirect's: those go there and give their frames bit
+// for bit.  The argument checks need no device, except the light and primitive counts, which need the scene.
+int rm_render_path(RmScene scene, const RmParams* params, int samples, const RmView* view, const RmLens* lens, const RmAreaLights* lights,
+                   const RmRoughGlass* rough, const RmMotion* motion, float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
+    if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_path: samples must be in [1, 8]");
+    const int S = samples;
+    bool any_area = false, any_motion = false;
+    int rc;
+    if (lights) {
+        if ((rc = check_area_lights(lights, &any_area)) != RM_OK) return rc;
+        if (lights->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lights: samples must equal the call's samples");
+    }
+    if (rough) {
+        if ((rc = check_rough(rough)) != RM_OK) return rc;
+        if (rough->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must equal the call's samples");
+    }
+    if (motion) {
+        if ((rc = check_motion(motion, &any_motion)) != RM_OK) return rc;
+        if (motion->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal the call's samples");
+    }
+    const RmLens pinhole = {0., 1., S};
+    if ((rc = check_lens(lens ? lens : &pinhole)) != RM_OK) return rc;
+    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lens: samples must equal the call's samples");
+    rm::ViewBasis vb;
+    bool identity = true;
+    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
+    if ((rc = check_params(params)) != RM_OK) return rc;
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_path computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_path renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_path needs max_depth >= 1");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
+    RmParams sp = *params;
+    sp.width = S * params->width;
+    sp.height = S * params->height;
+    sp.patch_row_begin = 0;
+    sp.patch_row_end = -1;
+    if ((rc = check_params(&sp)) != RM_OK) return rc;
+    const RmLens& ln = lens ? *lens : pinhole;
+    bool any_rough = false, any_bounce = false;
+    {
+        std::lock_guard<std::mutex> lock(g.mu);
+        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+        auto it = g.scenes.find(scene);
+        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+        if (lights && (size_t)lights->n_lights != it->second.flat.lights.size())
+            return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must equal the scene's light count");
+        if (rough && rough->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must equal the scene's primitive count");
+        if (motion && motion->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must equal the scene's primitive count");
+        if (rough) {
+            const std::vector<unsigned char> glass = glass_like_by_id(it->second.flat);
+            for (int k = 0; k < rough->n_prims && !any_rough; k++) any_rough = glass[k] && rough->roughness[k] > 0.;
+        }
+        any_bounce = any_diffuse_bounce(it->second.flat);
+    }
+    // one level, or no primitive that bounces: no diffuse ray is spawned, rm_render_distributed's frame (routed further there)
+    if (params->max_depth == 1 || !any_bounce)
+        return rm_render_distributed(scene, params, samples, view, lens, lights, rough, motion, out_rgb, out_rgb8, stats);
+    // one sample (every area, rough and time offset the identity), or no active effect: rm_render_indirect's frame
+    if (S == 1 || (!any_area && !any_rough && !any_motion)) return rm_render_indirect(scene, params, view, lens, S, out_rgb, out_rgb8, stats);
+    std::lock_guard<std::mutex> lock(g.mu);
+    auto it = g.scenes.find(scene);
+    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    SceneEntry& se = it->second;
+    DevicePack<float>& dp = se.f32;
+    cudaStream_t s = g.stream;
+    if ((rc = ensure_pack<float>(se, dp)) != RM_OK) return rc;
+    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
+    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
+    const bool walk = fp.accel != 0 && dp.ds.bvh.n_nodes > 0 && dp.ds.lay.n_lgt <= rm::kBvhMaxLights;
+    rm::Motion mo = rm::make_motion(S);
+    rm::DeviceScene<float> ds = dp.ds;
+    double reach = 0.;
+    if (any_motion && (rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
+    if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const bool cull = params->cull_backfacing != 0;
+    std::vector<float> radius, gf;
+    rm::AreaPoints ap = rm::make_area_points(S, lights ? lights->radius : nullptr, lights ? lights->n_lights : 0, radius);
+    radius.resize(std::max<size_t>(radius.size(), se.flat.lights.size()), 0.f);   // no lights given: every light a point
+    rm::RoughGlass rg = rm::make_rough_glass(S, any_rough ? rough->roughness : nullptr, any_rough ? rough->n_prims : 0, gf);
+    const rm::Diffuse df = rm::make_diffuse(S);
+    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
+    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
+    if (any_rough && (rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
+    float* d_max = static_cast<float*>(g.small.p);
+    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
+    float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
+    ap.radius = d_radius;
+    rg.g = any_rough ? static_cast<const float*>(g.rough.p) : nullptr;
+    CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
+    if (any_rough) CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaEventRecord(g.ev[0], s));
+    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
+    CK(cudaEventRecord(g.ev[1], s));
+    int launches = 0;
+    if (rows) {
+        CK(rm::launch_path(ds, fp, lc, ap, rg, mo, df, any_motion, reach, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p),
+                           d_max, s));
+        launches++;
+    }
+    CK(cudaEventRecord(g.ev[2], s));
+    if (out_rgb8 && rows) {
+        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
+        launches++;
+    }
+    const size_t host_px = (size_t)fp.row_begin * fp.width;
+    if (out_rgb && n_px) {
+        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
+        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
+    }
+    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
+    float h_max = 0.f;
+    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
+    CK(cudaEventRecord(g.ev[3], s));
+    CK(cudaStreamSynchronize(s));
+    if (stats) {
+        std::memset(stats, 0, sizeof(*stats));
+        stats->max_value = (double)h_max;
+        float ms = 0.f;
+        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
+        stats->ms_render = ms;
+        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
+        stats->ms_total = ms;
+        stats->kernel_launches = launches;
+        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
+    }
+    return RM_OK;
+}
+
 int rm_render_device(RmScene scene, const RmParams* params, void* d_rgb, int32_t* d_prim_id, void* d_max, void* stream) {
     std::lock_guard<std::mutex> lock(g.mu);
     if (!d_rgb || !d_max) return fail(RM_ERR_INVALID_ARGUMENT, "d_rgb and d_max must be device pointers");

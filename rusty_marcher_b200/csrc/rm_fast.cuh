@@ -1695,4 +1695,172 @@ RM_HD Vec3<float> indirect_shade(const FV& fv, const FrameParams<float>& fp, con
     else return cast_indirect<float, kGlass == GLASS_F32>(fv, fp, df, i, j, to_f32(o), to_f32(d), h.dist, h.slot, h.id);
 }
 
+// ---- path-traced frames (rm_render_path, include/rm_b200.h) ---------------------------------------------------------------
+// cast_glass_distributed with cast_indirect's bounce: every query, surface and shadow ray on the DistributedView of sample
+// (i, j) = (fv.si, fv.sj) (the scene at the sample's time, the area lights' point of area_offset(s, i, j, L) at level L),
+// rough glass-like hits turn the rays they spawn by rough_offset(s, i, j, L), and at a hit of level L < max_depth on a
+// primitive that is not glass-like, with diffusion > 0 and some diffuse_color component > 0, one diffuse ray leaves from
+// diffuse_origin along diffuse_dir with the disc point of stratum diffuse_stratum(s, i, j, L); its value v (background on a
+// miss) is added as c + scaled(v * kd, diffusion), and its hit, a shading point of level L + 1, samples its lights at
+// area_offset(s, i, j, L + 1).  A level pushes at most one frame, so the stack holds at most max_depth - 1.  G = double: the
+// bounce in f64 from the refined point and normal (with motion, MotionView::refine's point at the sample's time); G = float:
+// from the FP32 table.  kGlassOps = false (GLASS_NONE) leaves out the reflect / refract branch.  A copy of its own, so that
+// the distributed and indirect kernels keep their machine code.
+template <typename G, bool kGlassOps, class DV>
+RM_HD Vec3<float> cast_path(const DV& fv, const FrameParams<float>& fp, const RoughGlass& rg, const Diffuse& df, Vec3<G> o, Vec3<G> d,
+                            const float t1, const int slot1, const int id1) {
+    struct Frame {
+        Vec3<float> c;
+        Vec3<G> ro, rd;
+        float k;
+        int state;   // bit0: a refracted ray is pending, bit1: the refracted ray is the one in flight, bit2: a diffuse ray is
+        int id;      // in flight from primitive id
+    };
+    Frame fr[kMaxDepth];
+    int sp = 0;
+    const Vec3<float> bg = {fp.background, fp.background, fp.background};
+    const int s = df.samples, si = fv.si, sj = fv.sj;
+    Counters<false> st;
+    Vec3<float> v;
+    for (;;) {
+        const int level = sp + 1;                               // n_recursion
+        if (level > fp.max_depth) {
+            v = bg;                                             // renderer.rs:262-264
+        } else {
+            const Vec3<float> o32 = to_f32(o), d32 = to_f32(d);
+            HitRec<float> h;
+            bool got = true;
+            if (level == 1) {
+                h.dist = t1;
+                h.slot = slot1;
+                h.id = id1;
+            } else {
+                got = fv.template closest<false>(o32, d32, level, h, st);      // renderer.rs:266: the search, FP32
+            }
+            if (!got) {
+                v = bg;                                         // renderer.rs:300-306 (level > 1 here)
+            } else {
+                Vec3<G> p, n;
+                Vec3<float> p32, n32;
+                if constexpr (sizeof(G) == 8) {
+                    fv.refine(h.slot, o, d, (double)h.dist, p, n);
+                    p32 = to_f32(p);
+                    n32 = to_f32(n);
+                } else {
+                    fv.surface(h, o32, d32, n32);
+                    p32 = h.p;
+                    p = p32;
+                    n = n32;
+                }
+                const R4<float> ma = fv.mat_a[h.id];
+                const R4<float> mb = fv.mat_b[h.id];
+                Vec3<float> c = bg + fv.template direct<false>(level, d32, p32, n32, ma, mb, st);   // renderer.rs:272-275
+                bool pushed = false;
+                const bool glass = kGlassOps && (fv.mat_f[h.id] & 1);
+                if (glass) {                                    // renderer.rs:277
+                    Vec3<G> ro1, rd1, ro2, rd2;
+                    using N = typename std::conditional<sizeof(G) == 8, Fast64, Exact<float>>::type;
+                    const bool has_refl = reflect_ray<G, N>(d, p, n, (G)mb.w, ro1, rd1);  // renderer.rs:203-207
+                    const bool has_refr = refract_ray<G, N>(d, p, n, (G)mb.w, ro2, rd2);  // renderer.rs:235-239
+                    const float gf = rg.g ? rg.g[h.id] : 0.f;
+                    if (gf > 0.f && (has_refl || has_refr)) {
+                        const int k = ((sj + level) % s) * s + si;   // rough_offset(s, si, sj, level)
+                        G lx, ly;
+                        if constexpr (sizeof(G) == 8) {
+                            lx = rg.off[2 * k];
+                            ly = rg.off[2 * k + 1];
+                        } else {
+                            lx = rg.off32[2 * k];
+                            ly = rg.off32[2 * k + 1];
+                        }
+                        if (lx != G(0) || ly != G(0)) {
+                            if (has_refl) {
+                                rd1 = rough_dir<G>(rd1, (G)gf, lx, ly);
+                                ro1 = rough_reflect_origin<G>(p, n, rd1);
+                            }
+                            if (has_refr) {
+                                rd2 = rough_dir<G>(rd2, (G)gf, lx, ly);
+                                ro2 = rough_refract_origin<G>(p, n, d, rd2);
+                            }
+                        }
+                    }
+                    if (has_refl || has_refr) {
+                        RM_FAST_CHECK(sp < kMaxDepth);
+                        Frame& f = fr[sp];
+                        f.c = c;
+                        f.k = mb.z;
+                        if (has_refl) {
+                            f.state = has_refr ? 1 : 0;
+                            f.ro = ro2;
+                            f.rd = rd2;
+                            o = ro1;
+                            d = rd1;
+                        } else {
+                            f.state = 2;
+                            o = ro2;
+                            d = rd2;
+                        }
+                        sp++;
+                        pushed = true;
+                    }
+                } else if (level < fp.max_depth && ma.w > 0.f && (ma.x > 0.f || ma.y > 0.f || ma.z > 0.f)) {
+                    const int k = diffuse_stratum(s, si, sj, level);
+                    G lx, ly;
+                    if constexpr (sizeof(G) == 8) {
+                        lx = df.off[2 * k];
+                        ly = df.off[2 * k + 1];
+                    } else {
+                        lx = df.off32[2 * k];
+                        ly = df.off32[2 * k + 1];
+                    }
+                    const Vec3<G> nf = diffuse_normal<G>(n, d);
+                    RM_FAST_CHECK(sp < kMaxDepth);
+                    Frame& f = fr[sp];
+                    f.c = c;
+                    f.state = 4;
+                    f.id = h.id;
+                    o = diffuse_origin<G>(p, nf);
+                    d = diffuse_dir<G>(nf, lx, ly);
+                    sp++;
+                    pushed = true;
+                }
+                if (pushed) continue;
+                v = c;
+            }
+        }
+        for (;;) {                                              // return v to the callers on the stack
+            if (sp == 0) return v;
+            Frame& f = fr[sp - 1];
+            if (f.state & 4) {
+                const R4<float> ma = fv.mat_a[f.id];
+                v = f.c + scaled(v * Vec3<float>{ma.x, ma.y, ma.z}, ma.w);     // renderer.rs:181-183,192's lc * kd, diffusion
+                sp--;
+            } else if (f.state & 2) {
+                f.c = f.c + scaled(v, 1.f - f.k);               // renderer.rs:249
+                v = f.c;
+                sp--;
+            } else {
+                f.c = f.c + scaled(v, f.k);                     // renderer.rs:219
+                if (f.state & 1) {
+                    o = f.ro;
+                    d = f.rd;
+                    f.state = 2;
+                    break;
+                }
+                v = f.c;
+                sp--;
+            }
+        }
+    }
+}
+// A sample ray (o, d) of a path-traced frame whose level-1 query found h: distributed_shade with cast_path.  Opaque hits
+// recurse here, so GLASS_NONE traces the same loop in FP32 without the glass branch (distributed_shade's level-1 shortcut
+// would drop the bounces).
+template <int kGlass, class DV>
+RM_HD Vec3<float> path_shade(const DV& fv, const FrameParams<float>& fp, const RoughGlass& rg, const Diffuse& df, const Vec3<double> o,
+                             const Vec3<double> d, HitRec<float> h) {
+    if constexpr (kGlass == GLASS_F64) return cast_path<double, true>(fv, fp, rg, df, o, d, h.dist, h.slot, h.id);
+    else return cast_path<float, kGlass == GLASS_F32>(fv, fp, rg, df, to_f32(o), to_f32(d), h.dist, h.slot, h.id);
+}
+
 }  // namespace rm

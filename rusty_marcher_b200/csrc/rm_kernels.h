@@ -148,6 +148,11 @@ cudaError_t launch_distributed(const DeviceScene<float>& ds, const FrameParams<f
 //   (cast_indirect) at the disc points df; df.samples == lc.samples.
 cudaError_t launch_indirect(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const Diffuse& df,
                             bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
+// path_kernel (rm_path.cu; rm_render_path): distributed_kernel's frame with one diffuse bounce per qualifying opaque hit
+//   (cast_path) at the disc points df; ap, rg, mo and df have lc.samples, and ds, motion and reach are as for launch_distributed.
+cudaError_t launch_path(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const AreaPoints& ap,
+                        const RoughGlass& rg, const Motion& mo, const Diffuse& df, bool motion, double reach, bool cull, long long n_px,
+                        unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
 // K0 alone (prepare_raster_kernel, no view): the raster records of `camera` for the kernels that run stage A without K1.
 cudaError_t launch_prepare(const DeviceScene<float>& ds, bool cull, const double camera[3], cudaStream_t stream);
 // area_light_kernel (rm_area.cu; rm_render_area_lights): after launch_prepare for the same camera, the n_px pixels from frame row

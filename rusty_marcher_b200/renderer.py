@@ -536,6 +536,66 @@ class Renderer:
         print(message)
         return message
 
+    def render_path(self, frame, scene, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., light_radii=None,
+                    roughness=None, displacement=None, rgb8=None, patch_rows=(0, -1)):
+        """EXTENSION MODE (no reference counterpart): path-traced frames.  render_indirect()'s diffuse bounce together with
+        render_distributed()'s depth of field (forward / up, aperture / focus), soft shadows (light_radii), rough glass
+        (roughness) and motion blur (displacement), each taken as render_distributed() takes it and None leaving it out: every
+        one of the samples x samples rays of a pixel samples the lens, the time, one point of each area light, the turn of every
+        ray rough glass spawns and the direction of every diffuse ray, and the pixel is their mean (rm_render_path).  The
+        scene's max_depth caps the whole path, bounces included.  max_depth = 1, or a scene in which nothing bounces, is
+        render_distributed()'s frame; otherwise samples = 1, or no active effect, is render_indirect()'s.  Fills frame.buffer
+        (float32) over the rendered rows and, if given, rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the
+        same kind of status message as render()."""
+        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
+            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
+        radii = None if light_radii is None else _light_radii(scene, light_radii)
+        rough_by_prim = None if roughness is None else _roughness_by_prim(scene, roughness)
+        disp_by_prim = None if displacement is None else _displacement_by_prim(scene, displacement)
+        aperture, focus = _lens_values(aperture, focus)
+        if self.precision != _abi.RM_FP32:
+            raise ValueError("render_path computes in RM_FP32")
+        if int(self.width) != frame.width or int(self.height) != frame.height:
+            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
+        if len(patch_rows) > 2 and patch_rows[2] > 1:
+            raise ValueError("render_path renders contiguous patch rows (stride <= 1)")
+        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
+                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
+            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
+        view = None
+        if forward is not None:
+            view = _view(forward, up)
+            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
+        s = int(samples)
+        lens = _abi.RmLens()
+        lens.aperture, lens.focus, lens.samples = aperture, focus, s
+        lights = rough = motion = None
+        if radii is not None:
+            lights = _abi.RmAreaLights()
+            lights.n_lights, lights.radius, lights.samples = radii.shape[0], radii.ctypes.data_as(C.POINTER(C.c_double)), s
+        if rough_by_prim is not None:
+            rough = _abi.RmRoughGlass()
+            rough.n_prims, rough.roughness, rough.samples = rough_by_prim.shape[0], rough_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s
+        if disp_by_prim is not None:
+            motion = _abi.RmMotion()
+            motion.n_prims, motion.displacement, motion.samples = disp_by_prim.shape[0], disp_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s
+        L = _abi.load()
+        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
+        now = time.perf_counter()
+        p = self.params(frame, scene, patch_rows)
+        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
+            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
+        stats = _abi.RmStats()
+        ref = lambda x: C.byref(x) if x is not None else None     # noqa: E731
+        _abi.check(L.rm_render_path(scene.device_handle(), C.byref(p), s, ref(view), C.byref(lens), ref(lights), ref(rough), ref(motion),
+                                    frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
+        self.last_stats = stats
+        ms = int((time.perf_counter() - now) * 1000)
+        fps = 1000. / ms if ms > 0 else float("inf")
+        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
+        print(message)
+        return message
+
 
 def _light_radii(scene, radii):
     """One radius per light of the scene (one number for every light, or one per light), float64, checked."""
