@@ -1518,55 +1518,60 @@ int check_motion(const RmMotion* motion, bool* any_motion) {
     return RM_OK;
 }
 
-}  // namespace
-
-int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb, uint8_t* out_rgb8,
-                   RmStats* stats) {
-    int rc = check_lens(lens);
-    if (rc != RM_OK) return rc;
+// The argument checks the sampled-frame calls share, in this order: the lens (the pinhole of S samples where lens is null) and
+// its samples (samples_msg where they are not S), the view, params, the outputs and the S x frame.  `name` is the call, as its
+// messages name it; none of the checks needs a device.  Out: the lens in effect, the view's basis and whether it is the
+// identity.
+struct SampledCall {
+    RmLens lens;
     rm::ViewBasis vb;
     bool identity = true;
-    rc = view ? kernel_view(view, vb, &identity) : RM_OK;
+};
+int check_sampled_call(const std::string& name, const RmParams* params, const RmView* view, const RmLens* lens, const int S,
+                       const char* samples_msg, const float* out_rgb, const uint8_t* out_rgb8, SampledCall& c) {
+    c.lens = lens ? *lens : RmLens{0., 1., S};
+    int rc = check_lens(&c.lens);
     if (rc != RM_OK) return rc;
+    if (c.lens.samples != S) return fail(RM_ERR_INVALID_ARGUMENT, samples_msg);
+    if ((rc = view ? kernel_view(view, c.vb, &c.identity) : RM_OK) != RM_OK) return rc;
     if ((rc = check_params(params)) != RM_OK) return rc;
-    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_lens computes in RM_FP32");
-    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_lens renders contiguous patch rows (patch_row_stride <= 1)");
-    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_lens needs max_depth >= 1");
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, name + " computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, name + " renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, name + " needs max_depth >= 1");
     if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
-    const int samples = lens->samples;
     // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
     RmParams sp = *params;
-    sp.width = samples * params->width;
-    sp.height = samples * params->height;
+    sp.width = S * params->width;
+    sp.height = S * params->height;
     sp.patch_row_begin = 0;
     sp.patch_row_end = -1;
-    if ((rc = check_params(&sp)) != RM_OK) return rc;
-    if (lens->aperture == 0. && identity) return rm_render_supersampled(scene, params, samples, out_rgb, out_rgb8, stats);
-    std::lock_guard<std::mutex> lock(g.mu);
-    if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
-    auto it = g.scenes.find(scene);
-    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-    DevicePack<float>& dp = it->second.f32;
-    cudaStream_t s = g.stream;
-    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
-    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
-    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
-    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, *lens);
-    const bool cull = params->cull_backfacing != 0;
+    return check_params(&sp);
+}
+
+// The frame delivery of the sampled-frame calls and rm_render_area_lights (g.mu held, the effect's uploads already queued, so
+// that they stay outside ms_total): render(n_px, next, rgb, dmax) makes `launches` launches that write the output rows of fp
+// into rgb (g.rgb; g.prim for out_prim_id) and their maximum into *dmax, from the zeroed 64-bit work counter *next.  Then the
+// tone map for the 8-bit frame, the copies to the caller and the stats.  ms_render times the render launches alone.
+extern "C++" {                                                 // a template: C++ linkage inside the C ABI block
+template <typename Render>
+int deliver_sampled_frame(const DevicePack<float>& dp, const rm::FrameParams<float>& fp, const bool cull, float* out_rgb,
+                          int32_t* out_prim_id, uint8_t* out_rgb8, RmStats* stats, const int launches_render, Render render) {
     const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
+    int rc;
     if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
+    if (out_prim_id && (rc = g.prim.ensure(std::max<size_t>(n_px * 4, 16))) != RM_OK) return rc;
     if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
     if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
     float* d_max = static_cast<float*>(g.small.p);
     unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
+    cudaStream_t s = g.stream;
     CK(cudaEventRecord(g.ev[0], s));
     CK(cudaMemsetAsync(g.small.p, 0, 64, s));
     CK(cudaEventRecord(g.ev[1], s));
     int launches = 0;
     if (rows) {
-        CK(rm::launch_lens(dp.ds, fp, lc, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
-        launches++;
+        CK(render((long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max));
+        launches += launches_render;
     }
     CK(cudaEventRecord(g.ev[2], s));
     if (out_rgb8 && rows) {
@@ -1578,6 +1583,7 @@ int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, co
         forget_deliveries(out_rgb + host_px * 3, n_px * 12);
         CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
     }
+    if (out_prim_id && n_px) CK(cudaMemcpyAsync(out_prim_id + host_px, g.prim.p, n_px * 4, cudaMemcpyDeviceToHost, s));
     if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
     float h_max = 0.f;
     if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
@@ -1593,9 +1599,37 @@ int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, co
         stats->ms_total = ms;
         stats->kernel_launches = launches;
         stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
-        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
+        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_prim_id ? 4 : 0) + (out_rgb8 ? 3 : 0));
     }
     return RM_OK;
+}
+}  // extern "C++"
+
+}  // namespace
+
+int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb, uint8_t* out_rgb8,
+                   RmStats* stats) {
+    int rc = check_lens(lens);
+    if (rc != RM_OK) return rc;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_lens", params, view, lens, lens->samples, "", out_rgb, out_rgb8, c)) != RM_OK) return rc;
+    if (lens->aperture == 0. && c.identity) return rm_render_supersampled(scene, params, lens->samples, out_rgb, out_rgb8, stats);
+    std::lock_guard<std::mutex> lock(g.mu);
+    if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
+    auto it = g.scenes.find(scene);
+    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
+    DevicePack<float>& dp = it->second.f32;
+    cudaStream_t s = g.stream;
+    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
+    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
+    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
+    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, *lens);
+    const bool cull = params->cull_backfacing != 0;
+    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
+                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
+                                     return rm::launch_lens(dp.ds, fp, lc, cull, n_px, next, rgb, dmax, s);
+                                 });
 }
 
 // Extension mode (include/rm_b200.h): K0 writes this camera's raster records, area_light_kernel traces and shades the output
@@ -1648,55 +1682,19 @@ int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLig
         }
     al.samples = S;
     al.inv_ss = 1.f / (float)(S * S);
-    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
-    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
-    if (out_prim_id && (rc = g.prim.ensure(std::max<size_t>(n_px * 4, 16))) != RM_OK) return rc;
-    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    // the radius table behind the 64 bytes the delivery zeroes
     if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
-    float* d_max = static_cast<float*>(g.small.p);
-    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
     float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
     al.radius = d_radius;
     CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaEventRecord(g.ev[0], s));
-    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
-    CK(cudaEventRecord(g.ev[1], s));
-    int launches = 0;
-    if (rows) {
-        CK(rm::launch_prepare(dp.ds, cull, params->camera, s));
-        CK(rm::launch_area_lights(dp.ds, fp, al, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p),
-                                  out_prim_id ? static_cast<int*>(g.prim.p) : nullptr, d_max, params->camera, s));
-        launches += 2;
-    }
-    CK(cudaEventRecord(g.ev[2], s));
-    if (out_rgb8 && rows) {
-        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
-        launches++;
-    }
-    const size_t host_px = (size_t)fp.row_begin * fp.width;
-    if (out_rgb && n_px) {
-        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
-        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
-    }
-    if (out_prim_id && n_px) CK(cudaMemcpyAsync(out_prim_id + host_px, g.prim.p, n_px * 4, cudaMemcpyDeviceToHost, s));
-    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
-    float h_max = 0.f;
-    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
-    CK(cudaEventRecord(g.ev[3], s));
-    CK(cudaStreamSynchronize(s));
-    if (stats) {
-        std::memset(stats, 0, sizeof(*stats));
-        stats->max_value = (double)h_max;
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
-        stats->ms_render = ms;
-        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
-        stats->ms_total = ms;
-        stats->kernel_launches = launches;
-        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
-        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_prim_id ? 4 : 0) + (out_rgb8 ? 3 : 0));
-    }
-    return RM_OK;
+    return deliver_sampled_frame(dp, fp, cull, out_rgb, out_prim_id, out_rgb8, stats, 2,
+                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
+                                     const cudaError_t e = rm::launch_prepare(dp.ds, cull, params->camera, s);
+                                     if (e != cudaSuccess) return e;
+                                     return rm::launch_area_lights(dp.ds, fp, al, cull, n_px, next, rgb,
+                                                                   out_prim_id ? static_cast<int*>(g.prim.p) : nullptr, dmax,
+                                                                   params->camera, s);
+                                 });
 }
 
 // is_glass_like of every primitive id (shapes in scene order, an Obj once per triangle)
@@ -1740,25 +1738,8 @@ int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* v
     int rc = check_rough(rough);
     if (rc != RM_OK) return rc;
     const int S = rough->samples;
-    const RmLens pinhole = {0., 1., S};
-    if ((rc = check_lens(lens ? lens : &pinhole)) != RM_OK) return rc;
-    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must equal lens->samples");
-    rm::ViewBasis vb;
-    bool identity = true;
-    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
-    if ((rc = check_params(params)) != RM_OK) return rc;
-    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_rough_glass computes in RM_FP32");
-    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_rough_glass renders contiguous patch rows (patch_row_stride <= 1)");
-    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_rough_glass needs max_depth >= 1");
-    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
-    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
-    RmParams sp = *params;
-    sp.width = S * params->width;
-    sp.height = S * params->height;
-    sp.patch_row_begin = 0;
-    sp.patch_row_end = -1;
-    if ((rc = check_params(&sp)) != RM_OK) return rc;
-    const RmLens& ln = lens ? *lens : pinhole;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_rough_glass", params, view, lens, S, "rough: samples must equal lens->samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
     bool any_rough = false;
     {
         std::lock_guard<std::mutex> lock(g.mu);
@@ -1770,7 +1751,7 @@ int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* v
         for (int k = 0; k < rough->n_prims && !any_rough; k++) any_rough = glass[k] && rough->roughness[k] > 0.;
     }
     // one sample (its offset is (0, 0)), or no rough glass-like primitive: no ray is turned, rm_render_lens's frame bit for bit
-    if (S == 1 || !any_rough) return rm_render_lens(scene, params, view, &ln, out_rgb, out_rgb8, stats);
+    if (S == 1 || !any_rough) return rm_render_lens(scene, params, view, &c.lens, out_rgb, out_rgb8, stats);
     std::lock_guard<std::mutex> lock(g.mu);
     auto it = g.scenes.find(scene);
     if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
@@ -1780,55 +1761,17 @@ int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* v
     if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
     rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
     fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
     const bool cull = params->cull_backfacing != 0;
     std::vector<float> gf;
     rm::RoughGlass rg = rm::make_rough_glass(S, rough->roughness, rough->n_prims, gf);
-    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
-    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
-    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
-    if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
     if ((rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
-    float* d_max = static_cast<float*>(g.small.p);
-    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
     rg.g = static_cast<const float*>(g.rough.p);
     CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaEventRecord(g.ev[0], s));
-    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
-    CK(cudaEventRecord(g.ev[1], s));
-    int launches = 0;
-    if (rows) {
-        CK(rm::launch_rough_glass(dp.ds, fp, lc, rg, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
-        launches++;
-    }
-    CK(cudaEventRecord(g.ev[2], s));
-    if (out_rgb8 && rows) {
-        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
-        launches++;
-    }
-    const size_t host_px = (size_t)fp.row_begin * fp.width;
-    if (out_rgb && n_px) {
-        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
-        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
-    }
-    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
-    float h_max = 0.f;
-    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
-    CK(cudaEventRecord(g.ev[3], s));
-    CK(cudaStreamSynchronize(s));
-    if (stats) {
-        std::memset(stats, 0, sizeof(*stats));
-        stats->max_value = (double)h_max;
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
-        stats->ms_render = ms;
-        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
-        stats->ms_total = ms;
-        stats->kernel_launches = launches;
-        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
-        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
-    }
-    return RM_OK;
+    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
+                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
+                                     return rm::launch_rough_glass(dp.ds, fp, lc, rg, cull, n_px, next, rgb, dmax, s);
+                                 });
 }
 
 // Extension mode (include/rm_b200.h): indirect_kernel traces and resolves the output rows, then, for the 8-bit frame, the
@@ -1838,26 +1781,9 @@ int rm_render_indirect(RmScene scene, const RmParams* params, const RmView* view
                        uint8_t* out_rgb8, RmStats* stats) {
     if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect: samples must be in [1, 8]");
     const int S = samples;
-    const RmLens pinhole = {0., 1., S};
-    int rc = check_lens(lens ? lens : &pinhole);
-    if (rc != RM_OK) return rc;
-    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lens: samples must equal the call's samples");
-    rm::ViewBasis vb;
-    bool identity = true;
-    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
-    if ((rc = check_params(params)) != RM_OK) return rc;
-    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect computes in RM_FP32");
-    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect renders contiguous patch rows (patch_row_stride <= 1)");
-    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect needs max_depth >= 1");
-    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
-    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
-    RmParams sp = *params;
-    sp.width = S * params->width;
-    sp.height = S * params->height;
-    sp.patch_row_begin = 0;
-    sp.patch_row_end = -1;
-    if ((rc = check_params(&sp)) != RM_OK) return rc;
-    const RmLens& ln = lens ? *lens : pinhole;
+    int rc;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_indirect", params, view, lens, S, "lens: samples must equal the call's samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
     bool any_bounce = false;
     {
         std::lock_guard<std::mutex> lock(g.mu);
@@ -1867,7 +1793,7 @@ int rm_render_indirect(RmScene scene, const RmParams* params, const RmView* view
         any_bounce = any_diffuse_bounce(it->second.flat);
     }
     // one level, or no primitive that bounces: no diffuse ray is spawned, rm_render_lens's frame bit for bit
-    if (params->max_depth == 1 || !any_bounce) return rm_render_lens(scene, params, view, &ln, out_rgb, out_rgb8, stats);
+    if (params->max_depth == 1 || !any_bounce) return rm_render_lens(scene, params, view, &c.lens, out_rgb, out_rgb8, stats);
     std::lock_guard<std::mutex> lock(g.mu);
     auto it = g.scenes.find(scene);
     if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
@@ -1877,51 +1803,13 @@ int rm_render_indirect(RmScene scene, const RmParams* params, const RmView* view
     if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
     rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
     fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
     const bool cull = params->cull_backfacing != 0;
     const rm::Diffuse df = rm::make_diffuse(S);
-    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
-    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
-    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
-    if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
-    float* d_max = static_cast<float*>(g.small.p);
-    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
-    CK(cudaEventRecord(g.ev[0], s));
-    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
-    CK(cudaEventRecord(g.ev[1], s));
-    int launches = 0;
-    if (rows) {
-        CK(rm::launch_indirect(dp.ds, fp, lc, df, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
-        launches++;
-    }
-    CK(cudaEventRecord(g.ev[2], s));
-    if (out_rgb8 && rows) {
-        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
-        launches++;
-    }
-    const size_t host_px = (size_t)fp.row_begin * fp.width;
-    if (out_rgb && n_px) {
-        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
-        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
-    }
-    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
-    float h_max = 0.f;
-    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
-    CK(cudaEventRecord(g.ev[3], s));
-    CK(cudaStreamSynchronize(s));
-    if (stats) {
-        std::memset(stats, 0, sizeof(*stats));
-        stats->max_value = (double)h_max;
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
-        stats->ms_render = ms;
-        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
-        stats->ms_total = ms;
-        stats->kernel_launches = launches;
-        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
-        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
-    }
-    return RM_OK;
+    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
+                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
+                                     return rm::launch_indirect(dp.ds, fp, lc, df, cull, n_px, next, rgb, dmax, s);
+                                 });
 }
 
 namespace {
@@ -2002,25 +1890,8 @@ int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, 
     int rc = check_motion(motion, &any_motion);
     if (rc != RM_OK) return rc;
     const int S = motion->samples;
-    const RmLens pinhole = {0., 1., S};
-    if ((rc = check_lens(lens ? lens : &pinhole)) != RM_OK) return rc;
-    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal lens->samples");
-    rm::ViewBasis vb;
-    bool identity = true;
-    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
-    if ((rc = check_params(params)) != RM_OK) return rc;
-    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_motion computes in RM_FP32");
-    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_motion renders contiguous patch rows (patch_row_stride <= 1)");
-    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_motion needs max_depth >= 1");
-    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
-    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
-    RmParams sp = *params;
-    sp.width = S * params->width;
-    sp.height = S * params->height;
-    sp.patch_row_begin = 0;
-    sp.patch_row_end = -1;
-    if ((rc = check_params(&sp)) != RM_OK) return rc;
-    const RmLens& ln = lens ? *lens : pinhole;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_motion", params, view, lens, S, "motion: samples must equal lens->samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
     {
         std::lock_guard<std::mutex> lock(g.mu);
         if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
@@ -2029,7 +1900,7 @@ int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, 
         if (motion->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must equal the scene's primitive count");
     }
     // one sample (its time is 0), or nothing moves: the scene is its uploaded pose, rm_render_lens's frame bit for bit
-    if (S == 1 || !any_motion) return rm_render_lens(scene, params, view, &ln, out_rgb, out_rgb8, stats);
+    if (S == 1 || !any_motion) return rm_render_lens(scene, params, view, &c.lens, out_rgb, out_rgb8, stats);
     std::lock_guard<std::mutex> lock(g.mu);
     auto it = g.scenes.find(scene);
     if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
@@ -2045,50 +1916,12 @@ int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, 
     double reach = 0.;
     if ((rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
     if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
     const bool cull = params->cull_backfacing != 0;
-    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
-    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
-    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
-    if ((rc = g.small.ensure(1024)) != RM_OK) return rc;
-    float* d_max = static_cast<float*>(g.small.p);
-    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
-    CK(cudaEventRecord(g.ev[0], s));
-    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
-    CK(cudaEventRecord(g.ev[1], s));
-    int launches = 0;
-    if (rows) {
-        CK(rm::launch_motion(ds, fp, lc, mo, reach, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p), d_max, s));
-        launches++;
-    }
-    CK(cudaEventRecord(g.ev[2], s));
-    if (out_rgb8 && rows) {
-        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
-        launches++;
-    }
-    const size_t host_px = (size_t)fp.row_begin * fp.width;
-    if (out_rgb && n_px) {
-        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
-        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
-    }
-    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
-    float h_max = 0.f;
-    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
-    CK(cudaEventRecord(g.ev[3], s));
-    CK(cudaStreamSynchronize(s));
-    if (stats) {
-        std::memset(stats, 0, sizeof(*stats));
-        stats->max_value = (double)h_max;
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
-        stats->ms_render = ms;
-        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
-        stats->ms_total = ms;
-        stats->kernel_launches = launches;
-        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
-        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
-    }
-    return RM_OK;
+    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
+                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
+                                     return rm::launch_motion(ds, fp, lc, mo, reach, cull, n_px, next, rgb, dmax, s);
+                                 });
 }
 
 // Extension mode (include/rm_b200.h): distributed_kernel traces and resolves the output rows with every given effect at once,
@@ -2114,25 +1947,8 @@ int rm_render_distributed(RmScene scene, const RmParams* params, int samples, co
         if ((rc = check_motion(motion, &any_motion)) != RM_OK) return rc;
         if (motion->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal the call's samples");
     }
-    const RmLens pinhole = {0., 1., S};
-    if ((rc = check_lens(lens ? lens : &pinhole)) != RM_OK) return rc;
-    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lens: samples must equal the call's samples");
-    rm::ViewBasis vb;
-    bool identity = true;
-    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
-    if ((rc = check_params(params)) != RM_OK) return rc;
-    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_distributed computes in RM_FP32");
-    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_distributed renders contiguous patch rows (patch_row_stride <= 1)");
-    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_distributed needs max_depth >= 1");
-    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
-    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
-    RmParams sp = *params;
-    sp.width = S * params->width;
-    sp.height = S * params->height;
-    sp.patch_row_begin = 0;
-    sp.patch_row_end = -1;
-    if ((rc = check_params(&sp)) != RM_OK) return rc;
-    const RmLens& ln = lens ? *lens : pinhole;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_distributed", params, view, lens, S, "lens: samples must equal the call's samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
     bool any_rough = false;
     {
         std::lock_guard<std::mutex> lock(g.mu);
@@ -2149,7 +1965,7 @@ int rm_render_distributed(RmScene scene, const RmParams* params, int samples, co
         }
     }
     // one sample (every offset (0, 0), every time 0), or a single effect that has a call of its own: that call's frame
-    if (S == 1 || (!any_area && !any_rough && !any_motion)) return rm_render_lens(scene, params, view, &ln, out_rgb, out_rgb8, stats);
+    if (S == 1 || (!any_area && !any_rough && !any_motion)) return rm_render_lens(scene, params, view, &c.lens, out_rgb, out_rgb8, stats);
     if (!any_area && !any_motion) return rm_render_rough_glass(scene, params, view, lens, rough, out_rgb, out_rgb8, stats);
     if (!any_area && !any_rough) return rm_render_motion(scene, params, view, lens, motion, out_rgb, out_rgb8, stats);
     std::lock_guard<std::mutex> lock(g.mu);
@@ -2167,61 +1983,24 @@ int rm_render_distributed(RmScene scene, const RmParams* params, int samples, co
     double reach = 0.;
     if (any_motion && (rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
     if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
     const bool cull = params->cull_backfacing != 0;
     std::vector<float> radius, gf;
     rm::AreaPoints ap = rm::make_area_points(S, lights ? lights->radius : nullptr, lights ? lights->n_lights : 0, radius);
     radius.resize(std::max<size_t>(radius.size(), se.flat.lights.size()), 0.f);   // no lights given: every light a point
     rm::RoughGlass rg = rm::make_rough_glass(S, any_rough ? rough->roughness : nullptr, any_rough ? rough->n_prims : 0, gf);
-    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
-    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
-    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    // the radius table behind the 64 bytes the delivery zeroes
     if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
     if (any_rough && (rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
-    float* d_max = static_cast<float*>(g.small.p);
-    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
     float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
     ap.radius = d_radius;
     rg.g = any_rough ? static_cast<const float*>(g.rough.p) : nullptr;
     CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
     if (any_rough) CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaEventRecord(g.ev[0], s));
-    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
-    CK(cudaEventRecord(g.ev[1], s));
-    int launches = 0;
-    if (rows) {
-        CK(rm::launch_distributed(ds, fp, lc, ap, rg, mo, any_motion, reach, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p),
-                                  d_max, s));
-        launches++;
-    }
-    CK(cudaEventRecord(g.ev[2], s));
-    if (out_rgb8 && rows) {
-        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
-        launches++;
-    }
-    const size_t host_px = (size_t)fp.row_begin * fp.width;
-    if (out_rgb && n_px) {
-        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
-        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
-    }
-    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
-    float h_max = 0.f;
-    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
-    CK(cudaEventRecord(g.ev[3], s));
-    CK(cudaStreamSynchronize(s));
-    if (stats) {
-        std::memset(stats, 0, sizeof(*stats));
-        stats->max_value = (double)h_max;
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
-        stats->ms_render = ms;
-        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
-        stats->ms_total = ms;
-        stats->kernel_launches = launches;
-        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
-        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
-    }
-    return RM_OK;
+    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
+                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
+                                     return rm::launch_distributed(ds, fp, lc, ap, rg, mo, any_motion, reach, cull, n_px, next, rgb, dmax, s);
+                                 });
 }
 
 // Extension mode (include/rm_b200.h): path_kernel traces and resolves the output rows with the diffuse bounce and every given
@@ -2246,25 +2025,8 @@ int rm_render_path(RmScene scene, const RmParams* params, int samples, const RmV
         if ((rc = check_motion(motion, &any_motion)) != RM_OK) return rc;
         if (motion->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal the call's samples");
     }
-    const RmLens pinhole = {0., 1., S};
-    if ((rc = check_lens(lens ? lens : &pinhole)) != RM_OK) return rc;
-    if (lens && lens->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lens: samples must equal the call's samples");
-    rm::ViewBasis vb;
-    bool identity = true;
-    if ((rc = view ? kernel_view(view, vb, &identity) : RM_OK) != RM_OK) return rc;
-    if ((rc = check_params(params)) != RM_OK) return rc;
-    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_path computes in RM_FP32");
-    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_path renders contiguous patch rows (patch_row_stride <= 1)");
-    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_path needs max_depth >= 1");
-    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
-    // the s x frame's parameters must make a valid frame, as for rm_render_supersampled
-    RmParams sp = *params;
-    sp.width = S * params->width;
-    sp.height = S * params->height;
-    sp.patch_row_begin = 0;
-    sp.patch_row_end = -1;
-    if ((rc = check_params(&sp)) != RM_OK) return rc;
-    const RmLens& ln = lens ? *lens : pinhole;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_path", params, view, lens, S, "lens: samples must equal the call's samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
     bool any_rough = false, any_bounce = false;
     {
         std::lock_guard<std::mutex> lock(g.mu);
@@ -2301,62 +2063,25 @@ int rm_render_path(RmScene scene, const RmParams* params, int samples, const RmV
     double reach = 0.;
     if (any_motion && (rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
     if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? vb.m : nullptr, ln);
+    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
     const bool cull = params->cull_backfacing != 0;
     std::vector<float> radius, gf;
     rm::AreaPoints ap = rm::make_area_points(S, lights ? lights->radius : nullptr, lights ? lights->n_lights : 0, radius);
     radius.resize(std::max<size_t>(radius.size(), se.flat.lights.size()), 0.f);   // no lights given: every light a point
     rm::RoughGlass rg = rm::make_rough_glass(S, any_rough ? rough->roughness : nullptr, any_rough ? rough->n_prims : 0, gf);
     const rm::Diffuse df = rm::make_diffuse(S);
-    const size_t rows = (size_t)fp.n_bands * 32, n_px = rows * (size_t)fp.width;
-    if ((rc = g.rgb.ensure(std::max<size_t>(n_px * 12, 16))) != RM_OK) return rc;
-    if (out_rgb8 && (rc = g.rgb8.ensure(std::max<size_t>(n_px * 3, 16))) != RM_OK) return rc;
+    // the radius table behind the 64 bytes the delivery zeroes
     if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
     if (any_rough && (rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
-    float* d_max = static_cast<float*>(g.small.p);
-    unsigned long long* d_next = reinterpret_cast<unsigned long long*>(static_cast<char*>(g.small.p) + 24);
     float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
     ap.radius = d_radius;
     rg.g = any_rough ? static_cast<const float*>(g.rough.p) : nullptr;
     CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
     if (any_rough) CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaEventRecord(g.ev[0], s));
-    CK(cudaMemsetAsync(g.small.p, 0, 64, s));
-    CK(cudaEventRecord(g.ev[1], s));
-    int launches = 0;
-    if (rows) {
-        CK(rm::launch_path(ds, fp, lc, ap, rg, mo, df, any_motion, reach, cull, (long long)n_px, d_next, static_cast<float*>(g.rgb.p),
-                           d_max, s));
-        launches++;
-    }
-    CK(cudaEventRecord(g.ev[2], s));
-    if (out_rgb8 && rows) {
-        CK(rm::launch_tonemap<float>(fp, static_cast<const float*>(g.rgb.p), d_max, true, static_cast<unsigned char*>(g.rgb8.p), s));
-        launches++;
-    }
-    const size_t host_px = (size_t)fp.row_begin * fp.width;
-    if (out_rgb && n_px) {
-        forget_deliveries(out_rgb + host_px * 3, n_px * 12);
-        CK(cudaMemcpyAsync(out_rgb + host_px * 3, g.rgb.p, n_px * 12, cudaMemcpyDeviceToHost, s));
-    }
-    if (out_rgb8 && n_px) CK(cudaMemcpyAsync(out_rgb8 + host_px * 3, g.rgb8.p, n_px * 3, cudaMemcpyDeviceToHost, s));
-    float h_max = 0.f;
-    if (stats) CK(cudaMemcpyAsync(&h_max, d_max, sizeof(float), cudaMemcpyDeviceToHost, s));
-    CK(cudaEventRecord(g.ev[3], s));
-    CK(cudaStreamSynchronize(s));
-    if (stats) {
-        std::memset(stats, 0, sizeof(*stats));
-        stats->max_value = (double)h_max;
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, g.ev[1], g.ev[2]));
-        stats->ms_render = ms;
-        CK(cudaEventElapsedTime(&ms, g.ev[0], g.ev[3]));
-        stats->ms_total = ms;
-        stats->kernel_launches = launches;
-        stats->resident_prims = dp.ds.lay.n_sph + rm::plane_count<float>(dp.ds.lay, cull);
-        stats->d2h_bytes = (uint64_t)n_px * ((out_rgb ? 12 : 0) + (out_rgb8 ? 3 : 0));
-    }
-    return RM_OK;
+    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
+                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
+                                     return rm::launch_path(ds, fp, lc, ap, rg, mo, df, any_motion, reach, cull, n_px, next, rgb, dmax, s);
+                                 });
 }
 
 int rm_render_device(RmScene scene, const RmParams* params, void* d_rgb, int32_t* d_prim_id, void* d_max, void* stream) {

@@ -1,5 +1,5 @@
-// rm_fast_setup.cuh -- what the kernels over FastViewT share (rm_kernels.cu: K1 and the adaptive sub-pixel kernel; rm_lens.cu:
-// the thin-lens camera's kernel): the CTA shape, the staging of the scene in shared memory and the view of it, and on the host
+// rm_fast_setup.cuh -- what the kernels over FastViewT share (rm_kernels.cu: K1 and the adaptive sub-pixel kernel; rm_sampled.cuh:
+// the sampled-frame kernel): the CTA shape, the staging of the scene in shared memory and the view of it, and on the host
 // the launch plan and the one-time set-up of a kernel family.
 #pragma once
 
@@ -43,10 +43,10 @@ __device__ __forceinline__ void atomic_max_nonneg(double* addr, double v) {
 #endif
 constexpr int kFastBlock = RM_K1_BLOCK;
 
-// The scene in shared memory of K1, adaptive_subpixel_kernel and lens_kernel (kSmem): blob | raster records of every
+// The scene in shared memory of K1, adaptive_subpixel_kernel and sampled_kernel (kSmem): blob | raster records of every
 // fast-path triangle | materials mat_a | mat_b | mat_f (stage_mat: if they fit as well).  The kernels stage and view it with
 // these helpers, so that a sub-pixel value of the adaptive kernel stays the value K1 writes for that pixel.
-// The static part, blob and materials, does not depend on K0 (lens_kernel stages only this part).
+// The static part, blob and materials, does not depend on K0 (sampled_kernel stages only this part).
 __device__ __forceinline__ void stage_static(const DeviceScene<float>& ds, const int stage_mat, unsigned char* smem_raw) {
     const BlobLayout& L = ds.lay;
     const uint4* src = reinterpret_cast<const uint4*>(ds.blob);
@@ -114,7 +114,7 @@ __device__ __forceinline__ FastViewT<kBvh, kCount> make_fast_view(const DeviceSc
     return fv;
 }
 
-// The launch plan of K1, adaptive_subpixel_kernel and lens_kernel: it picks the instantiation, and a sub-pixel value of the
+// The launch plan of K1, adaptive_subpixel_kernel and sampled_kernel: it picks the instantiation, and a sub-pixel value of the
 // adaptive kernel is the value K1 writes for that pixel only while both kernels pick alike.
 // Shared memory: scene blob | raster records of every fast-path triangle | materials (if they fit as well), next to the
 // kernel's static arrays (hit queues etc.) within dyn_limit.

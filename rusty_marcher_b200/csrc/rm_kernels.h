@@ -123,33 +123,34 @@ cudaError_t launch_adaptive_mark(const float* rgb, const int* id, int width, int
 cudaError_t launch_adaptive_subpixel(const DeviceScene<float>& ds, const FrameParams<float>& fp, bool cull, int samples,
                                      const unsigned* list, const unsigned* count, unsigned long long* next, float* sub,
                                      const double camera[3], cudaStream_t stream);
-// lens_kernel (rm_lens.cu; rm_render_lens): the n_px output pixels from frame row fp.row_begin of the thin-lens camera lc, each the
-//   resolve_box mean of its lc.samples^2 sample rays (rgb: n_px * 3 floats), their maximum into *dmax; *next: a zeroed
-//   64-bit work counter.
+// The sampled-frame kernel (rm_sampled.cuh: sampled_kernel<E>), one launcher per effect type E, each in its own translation unit.
+// launch_lens (rm_lens.cu, lens_kernel::Effect; rm_render_lens): the n_px output pixels from frame row fp.row_begin of the thin-lens
+//   camera lc, each the resolve_box mean of its lc.samples^2 sample rays (rgb: n_px * 3 floats), their maximum into *dmax;
+//   *next: a zeroed 64-bit work counter.
 cudaError_t launch_lens(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, bool cull, long long n_px,
                         unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
-// rough_glass_kernel (rm_rough.cu; rm_render_rough_glass): lens_kernel's frame with the reflect / refract recursion turned by the
-//   roughness rg (cast_glass_rough); rg.samples == lc.samples.
+// launch_rough_glass (rm_rough.cu, rough_glass_kernel::Effect; rm_render_rough_glass): launch_lens's frame with the reflect / refract
+//   recursion turned by the roughness rg (cast_glass_rough); rg.samples == lc.samples.
 cudaError_t launch_rough_glass(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const RoughGlass& rg,
                                bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
-// motion_kernel (rm_motion.cu; rm_render_motion): lens_kernel's frame with every query of sample q at its time mo.tau[q]
-//   (MotionView); mo.samples == lc.samples.  ds carries the swept hierarchy; reach = the largest displacement component / 2,
+// launch_motion (rm_motion.cu, motion_kernel::Effect; rm_render_motion): launch_lens's frame with every query of sample q at its time
+//   mo.tau[q] (MotionView); mo.samples == lc.samples.  ds carries the swept hierarchy; reach = the largest displacement component / 2,
 //   by which the primitives leave their uploaded pose (the glass mode's coordinate bound).
 cudaError_t launch_motion(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const Motion& mo,
                           double reach, bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax,
                           cudaStream_t stream);
-// distributed_kernel (rm_distributed.cu; rm_render_distributed): lens_kernel's frame with the area lights' one point per sample
-//   and level (ap), the rough turn (rg; rg.g null: nothing is rough) and, when `motion`, every query of sample q at its time
+// launch_distributed (rm_distributed.cu, distributed_kernel::Effect; rm_render_distributed): launch_lens's frame with the area lights'
+//   one point per sample and level (ap), the rough turn (rg; rg.g null: nothing is rough) and, when `motion`, every query of sample q at its time
 //   mo.tau[q] (ds then carries the swept hierarchy, and reach is as for launch_motion); ap, rg and mo have lc.samples.
 cudaError_t launch_distributed(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const AreaPoints& ap,
                                const RoughGlass& rg, const Motion& mo, bool motion, double reach, bool cull, long long n_px,
                                unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
-// indirect_kernel (rm_indirect.cu; rm_render_indirect): lens_kernel's frame with one diffuse bounce per qualifying opaque hit
-//   (cast_indirect) at the disc points df; df.samples == lc.samples.
+// launch_indirect (rm_indirect.cu, indirect_kernel::Effect; rm_render_indirect): launch_lens's frame with one diffuse bounce per
+//   qualifying opaque hit (cast_indirect) at the disc points df; df.samples == lc.samples.
 cudaError_t launch_indirect(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const Diffuse& df,
                             bool cull, long long n_px, unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
-// path_kernel (rm_path.cu; rm_render_path): distributed_kernel's frame with one diffuse bounce per qualifying opaque hit
-//   (cast_path) at the disc points df; ap, rg, mo and df have lc.samples, and ds, motion and reach are as for launch_distributed.
+// launch_path (rm_path.cu, path_kernel::Effect; rm_render_path): launch_distributed's frame with one diffuse bounce per qualifying
+//   opaque hit (cast_path) at the disc points df; ap, rg, mo and df have lc.samples, and ds, motion and reach are as for launch_distributed.
 cudaError_t launch_path(const DeviceScene<float>& ds, const FrameParams<float>& fp, const LensCamera& lc, const AreaPoints& ap,
                         const RoughGlass& rg, const Motion& mo, const Diffuse& df, bool motion, double reach, bool cull, long long n_px,
                         unsigned long long* next, float* rgb, float* dmax, cudaStream_t stream);
