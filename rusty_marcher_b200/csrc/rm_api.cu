@@ -1465,8 +1465,7 @@ int rm_render_adaptive(RmScene scene, const RmParams* params, int samples, doubl
     return RM_OK;
 }
 
-// Extension mode (include/rm_b200.h): lens_kernel traces and resolves the output rows, then, for the 8-bit frame, the
-// tone-map kernel.  The argument checks need no device.
+// The checks of a lens (rm_render_lens and the sampled-frame calls that take one); none needs a device.
 int check_lens(const RmLens* lens) {
     if (!lens) return fail(RM_ERR_INVALID_ARGUMENT, "lens is null");
     if (lens->samples < 1 || lens->samples > 8) return fail(RM_ERR_INVALID_ARGUMENT, "lens: samples must be in [1, 8]");
@@ -1607,96 +1606,6 @@ int deliver_sampled_frame(const DevicePack<float>& dp, const rm::FrameParams<flo
 
 }  // namespace
 
-int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb, uint8_t* out_rgb8,
-                   RmStats* stats) {
-    int rc = check_lens(lens);
-    if (rc != RM_OK) return rc;
-    SampledCall c;
-    if ((rc = check_sampled_call("rm_render_lens", params, view, lens, lens->samples, "", out_rgb, out_rgb8, c)) != RM_OK) return rc;
-    if (lens->aperture == 0. && c.identity) return rm_render_supersampled(scene, params, lens->samples, out_rgb, out_rgb8, stats);
-    std::lock_guard<std::mutex> lock(g.mu);
-    if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
-    auto it = g.scenes.find(scene);
-    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-    DevicePack<float>& dp = it->second.f32;
-    cudaStream_t s = g.stream;
-    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
-    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
-    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
-    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, *lens);
-    const bool cull = params->cull_backfacing != 0;
-    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
-                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
-                                     return rm::launch_lens(dp.ds, fp, lc, cull, n_px, next, rgb, dmax, s);
-                                 });
-}
-
-// Extension mode (include/rm_b200.h): K0 writes this camera's raster records, area_light_kernel traces and shades the output
-// rows, then, for the 8-bit frame, the tone-map kernel.  s = 1 and all radii 0 are rm_render's frame and go there.  The
-// argument checks need no device, except the light count, which needs the scene.
-int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLights* lights, float* out_rgb, int32_t* out_prim_id,
-                          uint8_t* out_rgb8, RmStats* stats) {
-    bool any_area = false;
-    int rc = check_area_lights(lights, &any_area);
-    if (rc != RM_OK) return rc;
-    if ((rc = check_params(params)) != RM_OK) return rc;
-    if (rc != RM_OK) return rc;
-    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights computes in RM_FP32");
-    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights renders contiguous patch rows (patch_row_stride <= 1)");
-    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights needs max_depth >= 1");
-    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
-    {
-        std::lock_guard<std::mutex> lock(g.mu);
-        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
-        auto it = g.scenes.find(scene);
-        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-        if ((size_t)lights->n_lights != it->second.flat.lights.size())
-            return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must equal the scene's light count");
-    }
-    // one sample at the centre, or only point lights: the reference's lighting, rm_render's frame bit for bit
-    if (lights->samples == 1 || !any_area) return rm_render(scene, params, out_rgb, out_prim_id, out_rgb8, stats);
-    std::lock_guard<std::mutex> lock(g.mu);
-    auto it = g.scenes.find(scene);
-    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-    DevicePack<float>& dp = it->second.f32;
-    cudaStream_t s = g.stream;
-    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
-    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
-    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
-    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const bool cull = params->cull_backfacing != 0;
-    const int n_lgt = lights->n_lights, S = lights->samples;
-    rm::AreaLights al = {};
-    std::vector<float> radius(std::max(n_lgt, 1), 0.f);
-    for (int l = 0; l < n_lgt; l++) {
-        const double r = lights->radius[l];
-        radius[l] = r > 0. ? std::max((float)std::min(r, (double)FLT_MAX), 1e-30f) : 0.f;
-    }
-    for (int a = 0; a < S; a++)
-        for (int b = 0; b < S; b++) {
-            double lx, ly;
-            rm::lens_offset(S, a, b, &lx, &ly);
-            al.off[2 * (a * S + b)] = (float)lx;
-            al.off[2 * (a * S + b) + 1] = (float)ly;
-        }
-    al.samples = S;
-    al.inv_ss = 1.f / (float)(S * S);
-    // the radius table behind the 64 bytes the delivery zeroes
-    if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
-    float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
-    al.radius = d_radius;
-    CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
-    return deliver_sampled_frame(dp, fp, cull, out_rgb, out_prim_id, out_rgb8, stats, 2,
-                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
-                                     const cudaError_t e = rm::launch_prepare(dp.ds, cull, params->camera, s);
-                                     if (e != cudaSuccess) return e;
-                                     return rm::launch_area_lights(dp.ds, fp, al, cull, n_px, next, rgb,
-                                                                   out_prim_id ? static_cast<int*>(g.prim.p) : nullptr, dmax,
-                                                                   params->camera, s);
-                                 });
-}
-
 // is_glass_like of every primitive id (shapes in scene order, an Obj once per triangle)
 std::vector<unsigned char> glass_like_by_id(const rm::OwnedFlatScene& f) {
     std::vector<unsigned char> out;
@@ -1730,91 +1639,9 @@ bool any_diffuse_bounce(const rm::OwnedFlatScene& f) {
     return false;
 }
 
-// Extension mode (include/rm_b200.h): rough_glass_kernel traces and resolves the output rows, then, for the 8-bit frame, the
-// tone-map kernel.  s = 1, and calls in which no glass-like primitive is rough, are rm_render_lens's frame and go there.  The
-// argument checks need no device, except the primitive count, which needs the scene.
-int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, const RmRoughGlass* rough,
-                          float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
-    int rc = check_rough(rough);
-    if (rc != RM_OK) return rc;
-    const int S = rough->samples;
-    SampledCall c;
-    if ((rc = check_sampled_call("rm_render_rough_glass", params, view, lens, S, "rough: samples must equal lens->samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
-    bool any_rough = false;
-    {
-        std::lock_guard<std::mutex> lock(g.mu);
-        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
-        auto it = g.scenes.find(scene);
-        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-        if (rough->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must equal the scene's primitive count");
-        const std::vector<unsigned char> glass = glass_like_by_id(it->second.flat);
-        for (int k = 0; k < rough->n_prims && !any_rough; k++) any_rough = glass[k] && rough->roughness[k] > 0.;
-    }
-    // one sample (its offset is (0, 0)), or no rough glass-like primitive: no ray is turned, rm_render_lens's frame bit for bit
-    if (S == 1 || !any_rough) return rm_render_lens(scene, params, view, &c.lens, out_rgb, out_rgb8, stats);
-    std::lock_guard<std::mutex> lock(g.mu);
-    auto it = g.scenes.find(scene);
-    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-    DevicePack<float>& dp = it->second.f32;
-    cudaStream_t s = g.stream;
-    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
-    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
-    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
-    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
-    const bool cull = params->cull_backfacing != 0;
-    std::vector<float> gf;
-    rm::RoughGlass rg = rm::make_rough_glass(S, rough->roughness, rough->n_prims, gf);
-    if ((rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
-    rg.g = static_cast<const float*>(g.rough.p);
-    CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
-    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
-                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
-                                     return rm::launch_rough_glass(dp.ds, fp, lc, rg, cull, n_px, next, rgb, dmax, s);
-                                 });
-}
-
-// Extension mode (include/rm_b200.h): indirect_kernel traces and resolves the output rows, then, for the 8-bit frame, the
-// tone-map kernel.  max_depth = 1, and scenes in which no primitive bounces, are rm_render_lens's frame and go there.  The
-// argument checks need no device.
-int rm_render_indirect(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, int samples, float* out_rgb,
-                       uint8_t* out_rgb8, RmStats* stats) {
-    if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect: samples must be in [1, 8]");
-    const int S = samples;
-    int rc;
-    SampledCall c;
-    if ((rc = check_sampled_call("rm_render_indirect", params, view, lens, S, "lens: samples must equal the call's samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
-    bool any_bounce = false;
-    {
-        std::lock_guard<std::mutex> lock(g.mu);
-        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
-        auto it = g.scenes.find(scene);
-        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-        any_bounce = any_diffuse_bounce(it->second.flat);
-    }
-    // one level, or no primitive that bounces: no diffuse ray is spawned, rm_render_lens's frame bit for bit
-    if (params->max_depth == 1 || !any_bounce) return rm_render_lens(scene, params, view, &c.lens, out_rgb, out_rgb8, stats);
-    std::lock_guard<std::mutex> lock(g.mu);
-    auto it = g.scenes.find(scene);
-    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-    DevicePack<float>& dp = it->second.f32;
-    cudaStream_t s = g.stream;
-    if ((rc = ensure_pack<float>(it->second, dp)) != RM_OK) return rc;
-    if ((rc = order_scene_renders(it->second, s)) != RM_OK) return rc;
-    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
-    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
-    const bool cull = params->cull_backfacing != 0;
-    const rm::Diffuse df = rm::make_diffuse(S);
-    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
-                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
-                                     return rm::launch_indirect(dp.ds, fp, lc, df, cull, n_px, next, rgb, dmax, s);
-                                 });
-}
-
 namespace {
 
-// The motion of a frame on the device (rm_render_motion, rm_render_distributed; g.mu held, the scene's FP32 pack ensured): the
+// The motion of a frame on the device (render_sampled; g.mu held, the scene's FP32 pack ensured): the
 // per-primitive data by content, from the cache or made now (the swept hierarchy only once a call walks), copied to g.motion
 // unless it is there already.  mo receives the displacement pointers, ds the scene's pack with the swept hierarchy when
 // `walk`, reach the motion's reach (the glass mode's coordinate bound).
@@ -1879,208 +1706,279 @@ int stage_motion(SceneEntry& se, const DevicePack<float>& dp, const RmMotion* mo
     return RM_OK;
 }
 
-}  // namespace
-
-// Extension mode (include/rm_b200.h): motion_kernel traces and resolves the output rows, then, for the 8-bit frame, the
-// tone-map kernel.  s = 1 (every sample at tau = 0) and calls in which nothing moves are rm_render_lens's frame and go there.
-// The argument checks need no device, except the primitive count, which needs the scene.
-int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, const RmMotion* motion,
-                     float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
-    bool any_motion = false;
-    int rc = check_motion(motion, &any_motion);
-    if (rc != RM_OK) return rc;
-    const int S = motion->samples;
-    SampledCall c;
-    if ((rc = check_sampled_call("rm_render_motion", params, view, lens, S, "motion: samples must equal lens->samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
-    {
-        std::lock_guard<std::mutex> lock(g.mu);
-        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
-        auto it = g.scenes.find(scene);
-        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-        if (motion->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must equal the scene's primitive count");
-    }
-    // one sample (its time is 0), or nothing moves: the scene is its uploaded pose, rm_render_lens's frame bit for bit
-    if (S == 1 || !any_motion) return rm_render_lens(scene, params, view, &c.lens, out_rgb, out_rgb8, stats);
-    std::lock_guard<std::mutex> lock(g.mu);
+// The lock-held start of a sampled-frame call's render (g.mu held): the ready check, the scene, its FP32 pack, its renders
+// ordered on the library's stream and the call's frame parameters, whose scratch frames are indexed from the call's first row.
+struct SceneFrame {
+    SceneEntry* se = nullptr;
+    rm::FrameParams<float> fp;
+    bool cull = false;
+};
+int acquire_scene(RmScene scene, const RmParams* params, SceneFrame& f) {
+    if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
     auto it = g.scenes.find(scene);
     if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-    SceneEntry& se = it->second;
+    f.se = &it->second;
+    int rc;
+    if ((rc = ensure_pack<float>(*f.se, f.se->f32)) != RM_OK) return rc;
+    if ((rc = order_scene_renders(*f.se, g.stream)) != RM_OK) return rc;
+    f.fp = rm::make_frame_params<float>(*params);
+    f.fp.buf_row0 = f.fp.row_begin;
+    f.cull = params->cull_backfacing != 0;
+    return RM_OK;
+}
+
+// The kernel that renders a sampled-frame call, from the effects active in it (include/rm_b200.h has the rules; each routed
+// case gives the frame of the call it is routed to, bit for bit):
+//   A  an area light of radius > 0,                     with s > 1;
+//   R  roughness > 0 on a glass-like primitive,         with s > 1;
+//   M  a displacement != 0,                             with s > 1;
+//   B  max_depth > 1 and a primitive that bounces,      rm_render_indirect and rm_render_path only.
+// The rows are checked in this order:
+//   B and (A or R or M)   path_kernel (its motion variant with M)
+//   B                     indirect_kernel
+//   A, or R and M         distributed_kernel (its motion variant with M)
+//   R                     rough_glass_kernel
+//   M                     motion_kernel
+//   none                  rm_render_supersampled for aperture 0 without a turned view, lens_kernel otherwise
+enum class Route { kSupersampled, kLens, kRoughGlass, kMotion, kDistributed, kIndirect, kPath };
+Route route_of(const bool A, const bool R, const bool M, const bool B, const bool pinhole) {
+    if (B) return A || R || M ? Route::kPath : Route::kIndirect;
+    if (A || (R && M)) return Route::kDistributed;
+    if (R) return Route::kRoughGlass;
+    if (M) return Route::kMotion;
+    return pinhole ? Route::kSupersampled : Route::kLens;
+}
+
+// The effect structs of a sampled-frame call, checked (null: not given), and whether it has the diffuse bounce.
+struct Effects {
+    const RmAreaLights* lights = nullptr;
+    const RmRoughGlass* rough = nullptr;
+    const RmMotion* motion = nullptr;
+    bool any_area = false, any_motion = false;   // check_area_lights' and check_motion's verdicts
+    bool bounce = false;
+};
+
+// The render of the six sampled-frame calls after their device-free checks (c from check_sampled_call).  One hold of g.mu
+// covers the scene's light and primitive counts, the route and the render: the uploads the routed kernel reads, then the
+// delivery.  The pinhole frame goes to rm_render_supersampled, which takes g.mu itself.
+int render_sampled(RmScene scene, const RmParams* params, const RmView* view, const SampledCall& c, const Effects& e, float* out_rgb,
+                   uint8_t* out_rgb8, RmStats* stats) {
+    const int S = c.lens.samples;
+    std::unique_lock<std::mutex> lock(g.mu);
+    SceneFrame f;
+    int rc = acquire_scene(scene, params, f);
+    if (rc != RM_OK) return rc;
+    SceneEntry& se = *f.se;
+    if (e.lights && (size_t)e.lights->n_lights != se.flat.lights.size())
+        return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must equal the scene's light count");
+    if (e.rough && e.rough->n_prims != se.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must equal the scene's primitive count");
+    if (e.motion && e.motion->n_prims != se.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must equal the scene's primitive count");
+    bool any_rough = false;
+    if (e.rough && S > 1) {
+        const std::vector<unsigned char> glass = glass_like_by_id(se.flat);
+        for (int k = 0; k < e.rough->n_prims && !any_rough; k++) any_rough = glass[k] && e.rough->roughness[k] > 0.;
+    }
+    // s = 1: every lens, area, rough and time offset is the identity
+    const bool A = S > 1 && e.any_area, R = S > 1 && any_rough, M = S > 1 && e.any_motion;
+    const bool B = e.bounce && params->max_depth > 1 && any_diffuse_bounce(se.flat);
+    const Route route = route_of(A, R, M, B, c.lens.aperture == 0. && c.identity);
+    if (route == Route::kSupersampled) {
+        lock.unlock();
+        return rm_render_supersampled(scene, params, S, out_rgb, out_rgb8, stats);
+    }
     DevicePack<float>& dp = se.f32;
     cudaStream_t s = g.stream;
-    if ((rc = ensure_pack<float>(se, dp)) != RM_OK) return rc;
-    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
-    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const bool walk = fp.accel != 0 && dp.ds.bvh.n_nodes > 0 && dp.ds.lay.n_lgt <= rm::kBvhMaxLights;
-    rm::Motion mo = rm::make_motion(S);
-    rm::DeviceScene<float> ds;
-    double reach = 0.;
-    if ((rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
-    if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
     const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
-    const bool cull = params->cull_backfacing != 0;
+    rm::DeviceScene<float> ds = dp.ds;
+    rm::Motion mo = rm::make_motion(S);
+    double reach = 0.;
+    if (M) {
+        const bool walk = f.fp.accel != 0 && dp.ds.bvh.n_nodes > 0 && dp.ds.lay.n_lgt <= rm::kBvhMaxLights;
+        if ((rc = stage_motion(se, dp, e.motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
+    }
+    std::vector<float> radius, gf;                              // read by copies the delivery waits for
+    rm::AreaPoints ap = {};
+    if (route == Route::kDistributed || route == Route::kPath) {
+        ap = rm::make_area_points(S, e.lights ? e.lights->radius : nullptr, e.lights ? e.lights->n_lights : 0, radius);
+        radius.resize(std::max<size_t>(radius.size(), se.flat.lights.size()), 0.f);   // no lights given: every light a point
+        // the radius table behind the 64 bytes the delivery zeroes
+        if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
+        float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
+        ap.radius = d_radius;
+        CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
+    }
+    rm::RoughGlass rg = rm::make_rough_glass(S, R ? e.rough->roughness : nullptr, R ? e.rough->n_prims : 0, gf);
+    if (R) {
+        if ((rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
+        rg.g = static_cast<const float*>(g.rough.p);
+        CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
+    }
+    const rm::Diffuse df = B ? rm::make_diffuse(S) : rm::Diffuse{};
+    const rm::FrameParams<float>& fp = f.fp;
+    const bool cull = f.cull;
     return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
                                  [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
-                                     return rm::launch_motion(ds, fp, lc, mo, reach, cull, n_px, next, rgb, dmax, s);
+                                     switch (route) {
+                                     case Route::kLens: return rm::launch_lens(ds, fp, lc, cull, n_px, next, rgb, dmax, s);
+                                     case Route::kRoughGlass: return rm::launch_rough_glass(ds, fp, lc, rg, cull, n_px, next, rgb, dmax, s);
+                                     case Route::kMotion: return rm::launch_motion(ds, fp, lc, mo, reach, cull, n_px, next, rgb, dmax, s);
+                                     case Route::kDistributed:
+                                         return rm::launch_distributed(ds, fp, lc, ap, rg, mo, M, reach, cull, n_px, next, rgb, dmax, s);
+                                     case Route::kIndirect: return rm::launch_indirect(ds, fp, lc, df, cull, n_px, next, rgb, dmax, s);
+                                     default: return rm::launch_path(ds, fp, lc, ap, rg, mo, df, M, reach, cull, n_px, next, rgb, dmax, s);
+                                     }
                                  });
 }
 
-// Extension mode (include/rm_b200.h): distributed_kernel traces and resolves the output rows with every given effect at once,
-// then, for the 8-bit frame, the tone-map kernel.  A call whose only active effect is rough glass or motion is that effect's
-// own call, and s = 1 or no active effect is rm_render_lens's: those go there and give their frames bit for bit.  The
-// argument checks need no device, except the light and primitive counts, which need the scene.
+// rm_render_distributed and rm_render_path: the same arguments and checks; the path call adds the diffuse bounce.
+int render_effects(const std::string& name, const bool bounce, RmScene scene, const RmParams* params, const int samples,
+                   const RmView* view, const RmLens* lens, const RmAreaLights* lights, const RmRoughGlass* rough, const RmMotion* motion,
+                   float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
+    if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, name + ": samples must be in [1, 8]");
+    Effects e;
+    e.lights = lights;
+    e.rough = rough;
+    e.motion = motion;
+    e.bounce = bounce;
+    int rc;
+    if (lights) {
+        if ((rc = check_area_lights(lights, &e.any_area)) != RM_OK) return rc;
+        if (lights->samples != samples) return fail(RM_ERR_INVALID_ARGUMENT, "lights: samples must equal the call's samples");
+    }
+    if (rough) {
+        if ((rc = check_rough(rough)) != RM_OK) return rc;
+        if (rough->samples != samples) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must equal the call's samples");
+    }
+    if (motion) {
+        if ((rc = check_motion(motion, &e.any_motion)) != RM_OK) return rc;
+        if (motion->samples != samples) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal the call's samples");
+    }
+    SampledCall c;
+    if ((rc = check_sampled_call(name, params, view, lens, samples, "lens: samples must equal the call's samples", out_rgb, out_rgb8, c)) != RM_OK)
+        return rc;
+    return render_sampled(scene, params, view, c, e, out_rgb, out_rgb8, stats);
+}
+
+}  // namespace
+
+// Extension mode (include/rm_b200.h): the sampled-frame calls.  Each makes the device-free checks of its own arguments and
+// renders through render_sampled, whose route_of picks the kernel; the routed kernel traces and resolves the output rows,
+// then, for the 8-bit frame, the tone-map kernel.
+int rm_render_lens(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, float* out_rgb, uint8_t* out_rgb8,
+                   RmStats* stats) {
+    int rc = check_lens(lens);
+    if (rc != RM_OK) return rc;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_lens", params, view, lens, lens->samples, "", out_rgb, out_rgb8, c)) != RM_OK) return rc;
+    // the pinhole frame needs no scene here: rm_render_supersampled looks it up itself
+    if (lens->aperture == 0. && c.identity) return rm_render_supersampled(scene, params, lens->samples, out_rgb, out_rgb8, stats);
+    return render_sampled(scene, params, view, c, Effects{}, out_rgb, out_rgb8, stats);
+}
+
+int rm_render_rough_glass(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, const RmRoughGlass* rough,
+                          float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
+    int rc = check_rough(rough);
+    if (rc != RM_OK) return rc;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_rough_glass", params, view, lens, rough->samples, "rough: samples must equal lens->samples", out_rgb,
+                                 out_rgb8, c)) != RM_OK)
+        return rc;
+    Effects e;
+    e.rough = rough;
+    return render_sampled(scene, params, view, c, e, out_rgb, out_rgb8, stats);
+}
+
+int rm_render_motion(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, const RmMotion* motion,
+                     float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
+    Effects e;
+    e.motion = motion;
+    int rc = check_motion(motion, &e.any_motion);
+    if (rc != RM_OK) return rc;
+    SampledCall c;
+    if ((rc = check_sampled_call("rm_render_motion", params, view, lens, motion->samples, "motion: samples must equal lens->samples", out_rgb,
+                                 out_rgb8, c)) != RM_OK)
+        return rc;
+    return render_sampled(scene, params, view, c, e, out_rgb, out_rgb8, stats);
+}
+
+int rm_render_indirect(RmScene scene, const RmParams* params, const RmView* view, const RmLens* lens, int samples, float* out_rgb,
+                       uint8_t* out_rgb8, RmStats* stats) {
+    if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_indirect: samples must be in [1, 8]");
+    SampledCall c;
+    int rc;
+    if ((rc = check_sampled_call("rm_render_indirect", params, view, lens, samples, "lens: samples must equal the call's samples", out_rgb,
+                                 out_rgb8, c)) != RM_OK)
+        return rc;
+    Effects e;
+    e.bounce = true;
+    return render_sampled(scene, params, view, c, e, out_rgb, out_rgb8, stats);
+}
+
 int rm_render_distributed(RmScene scene, const RmParams* params, int samples, const RmView* view, const RmLens* lens,
                           const RmAreaLights* lights, const RmRoughGlass* rough, const RmMotion* motion, float* out_rgb,
                           uint8_t* out_rgb8, RmStats* stats) {
-    if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_distributed: samples must be in [1, 8]");
-    const int S = samples;
-    bool any_area = false, any_motion = false;
-    int rc;
-    if (lights) {
-        if ((rc = check_area_lights(lights, &any_area)) != RM_OK) return rc;
-        if (lights->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lights: samples must equal the call's samples");
-    }
-    if (rough) {
-        if ((rc = check_rough(rough)) != RM_OK) return rc;
-        if (rough->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must equal the call's samples");
-    }
-    if (motion) {
-        if ((rc = check_motion(motion, &any_motion)) != RM_OK) return rc;
-        if (motion->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal the call's samples");
-    }
-    SampledCall c;
-    if ((rc = check_sampled_call("rm_render_distributed", params, view, lens, S, "lens: samples must equal the call's samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
-    bool any_rough = false;
-    {
-        std::lock_guard<std::mutex> lock(g.mu);
-        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
-        auto it = g.scenes.find(scene);
-        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-        if (lights && (size_t)lights->n_lights != it->second.flat.lights.size())
-            return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must equal the scene's light count");
-        if (rough && rough->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must equal the scene's primitive count");
-        if (motion && motion->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must equal the scene's primitive count");
-        if (rough) {
-            const std::vector<unsigned char> glass = glass_like_by_id(it->second.flat);
-            for (int k = 0; k < rough->n_prims && !any_rough; k++) any_rough = glass[k] && rough->roughness[k] > 0.;
-        }
-    }
-    // one sample (every offset (0, 0), every time 0), or a single effect that has a call of its own: that call's frame
-    if (S == 1 || (!any_area && !any_rough && !any_motion)) return rm_render_lens(scene, params, view, &c.lens, out_rgb, out_rgb8, stats);
-    if (!any_area && !any_motion) return rm_render_rough_glass(scene, params, view, lens, rough, out_rgb, out_rgb8, stats);
-    if (!any_area && !any_rough) return rm_render_motion(scene, params, view, lens, motion, out_rgb, out_rgb8, stats);
-    std::lock_guard<std::mutex> lock(g.mu);
-    auto it = g.scenes.find(scene);
-    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-    SceneEntry& se = it->second;
-    DevicePack<float>& dp = se.f32;
-    cudaStream_t s = g.stream;
-    if ((rc = ensure_pack<float>(se, dp)) != RM_OK) return rc;
-    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
-    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const bool walk = fp.accel != 0 && dp.ds.bvh.n_nodes > 0 && dp.ds.lay.n_lgt <= rm::kBvhMaxLights;
-    rm::Motion mo = rm::make_motion(S);
-    rm::DeviceScene<float> ds = dp.ds;
-    double reach = 0.;
-    if (any_motion && (rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
-    if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
-    const bool cull = params->cull_backfacing != 0;
-    std::vector<float> radius, gf;
-    rm::AreaPoints ap = rm::make_area_points(S, lights ? lights->radius : nullptr, lights ? lights->n_lights : 0, radius);
-    radius.resize(std::max<size_t>(radius.size(), se.flat.lights.size()), 0.f);   // no lights given: every light a point
-    rm::RoughGlass rg = rm::make_rough_glass(S, any_rough ? rough->roughness : nullptr, any_rough ? rough->n_prims : 0, gf);
-    // the radius table behind the 64 bytes the delivery zeroes
-    if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
-    if (any_rough && (rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
-    float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
-    ap.radius = d_radius;
-    rg.g = any_rough ? static_cast<const float*>(g.rough.p) : nullptr;
-    CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
-    if (any_rough) CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
-    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
-                                 [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
-                                     return rm::launch_distributed(ds, fp, lc, ap, rg, mo, any_motion, reach, cull, n_px, next, rgb, dmax, s);
-                                 });
+    return render_effects("rm_render_distributed", false, scene, params, samples, view, lens, lights, rough, motion, out_rgb, out_rgb8, stats);
 }
 
-// Extension mode (include/rm_b200.h): path_kernel traces and resolves the output rows with the diffuse bounce and every given
-// effect at once, then, for the 8-bit frame, the tone-map kernel.  max_depth = 1, or a scene in which no primitive bounces, is
-// rm_render_distributed's frame; s = 1, or no active effect, is rm_render_indirect's: those go there and give their frames bit
-// for bit.  The argument checks need no device, except the light and primitive counts, which need the scene.
 int rm_render_path(RmScene scene, const RmParams* params, int samples, const RmView* view, const RmLens* lens, const RmAreaLights* lights,
                    const RmRoughGlass* rough, const RmMotion* motion, float* out_rgb, uint8_t* out_rgb8, RmStats* stats) {
-    if (samples < 1 || samples > rm::kAreaMaxSamples) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_path: samples must be in [1, 8]");
-    const int S = samples;
-    bool any_area = false, any_motion = false;
-    int rc;
-    if (lights) {
-        if ((rc = check_area_lights(lights, &any_area)) != RM_OK) return rc;
-        if (lights->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "lights: samples must equal the call's samples");
+    return render_effects("rm_render_path", true, scene, params, samples, view, lens, lights, rough, motion, out_rgb, out_rgb8, stats);
+}
+
+// Extension mode (include/rm_b200.h): K0 writes this camera's raster records, area_light_kernel traces and shades the output
+// rows, then, for the 8-bit frame, the tone-map kernel.  s = 1 and all radii 0 are rm_render's frame and go there.  The
+// argument checks need no device, except the light count, which needs the scene.
+int rm_render_area_lights(RmScene scene, const RmParams* params, const RmAreaLights* lights, float* out_rgb, int32_t* out_prim_id,
+                          uint8_t* out_rgb8, RmStats* stats) {
+    bool any_area = false;
+    int rc = check_area_lights(lights, &any_area);
+    if (rc != RM_OK) return rc;
+    if ((rc = check_params(params)) != RM_OK) return rc;
+    if (params->precision != RM_FP32) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights computes in RM_FP32");
+    if (params->patch_row_stride > 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights renders contiguous patch rows (patch_row_stride <= 1)");
+    if (params->max_depth < 1) return fail(RM_ERR_INVALID_ARGUMENT, "rm_render_area_lights needs max_depth >= 1");
+    if (!out_rgb && !out_rgb8) return fail(RM_ERR_INVALID_ARGUMENT, "out_rgb and out_rgb8 are both null");
+    std::unique_lock<std::mutex> lock(g.mu);
+    SceneFrame f;
+    if ((rc = acquire_scene(scene, params, f)) != RM_OK) return rc;
+    if ((size_t)lights->n_lights != f.se->flat.lights.size()) return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must equal the scene's light count");
+    // one sample at the centre, or only point lights: the reference's lighting, rm_render's frame bit for bit
+    if (lights->samples == 1 || !any_area) {
+        lock.unlock();
+        return rm_render(scene, params, out_rgb, out_prim_id, out_rgb8, stats);
     }
-    if (rough) {
-        if ((rc = check_rough(rough)) != RM_OK) return rc;
-        if (rough->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "rough: samples must equal the call's samples");
-    }
-    if (motion) {
-        if ((rc = check_motion(motion, &any_motion)) != RM_OK) return rc;
-        if (motion->samples != S) return fail(RM_ERR_INVALID_ARGUMENT, "motion: samples must equal the call's samples");
-    }
-    SampledCall c;
-    if ((rc = check_sampled_call("rm_render_path", params, view, lens, S, "lens: samples must equal the call's samples", out_rgb, out_rgb8, c)) != RM_OK) return rc;
-    bool any_rough = false, any_bounce = false;
-    {
-        std::lock_guard<std::mutex> lock(g.mu);
-        if (!g.ready) return fail(RM_ERR_NOT_INITIALISED, "rm_init() has not been called (or failed): no CUDA device bound");
-        auto it = g.scenes.find(scene);
-        if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-        if (lights && (size_t)lights->n_lights != it->second.flat.lights.size())
-            return fail(RM_ERR_INVALID_ARGUMENT, "lights: n_lights must equal the scene's light count");
-        if (rough && rough->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "rough: n_prims must equal the scene's primitive count");
-        if (motion && motion->n_prims != it->second.n_prims) return fail(RM_ERR_INVALID_ARGUMENT, "motion: n_prims must equal the scene's primitive count");
-        if (rough) {
-            const std::vector<unsigned char> glass = glass_like_by_id(it->second.flat);
-            for (int k = 0; k < rough->n_prims && !any_rough; k++) any_rough = glass[k] && rough->roughness[k] > 0.;
-        }
-        any_bounce = any_diffuse_bounce(it->second.flat);
-    }
-    // one level, or no primitive that bounces: no diffuse ray is spawned, rm_render_distributed's frame (routed further there)
-    if (params->max_depth == 1 || !any_bounce)
-        return rm_render_distributed(scene, params, samples, view, lens, lights, rough, motion, out_rgb, out_rgb8, stats);
-    // one sample (every area, rough and time offset the identity), or no active effect: rm_render_indirect's frame
-    if (S == 1 || (!any_area && !any_rough && !any_motion)) return rm_render_indirect(scene, params, view, lens, S, out_rgb, out_rgb8, stats);
-    std::lock_guard<std::mutex> lock(g.mu);
-    auto it = g.scenes.find(scene);
-    if (it == g.scenes.end()) return fail(RM_ERR_INVALID_ARGUMENT, "unknown scene handle");
-    SceneEntry& se = it->second;
-    DevicePack<float>& dp = se.f32;
+    DevicePack<float>& dp = f.se->f32;
     cudaStream_t s = g.stream;
-    if ((rc = ensure_pack<float>(se, dp)) != RM_OK) return rc;
-    rm::FrameParams<float> fp = rm::make_frame_params<float>(*params);
-    fp.buf_row0 = fp.row_begin;                                 // the scratch frames are indexed from the call's first row
-    const bool walk = fp.accel != 0 && dp.ds.bvh.n_nodes > 0 && dp.ds.lay.n_lgt <= rm::kBvhMaxLights;
-    rm::Motion mo = rm::make_motion(S);
-    rm::DeviceScene<float> ds = dp.ds;
-    double reach = 0.;
-    if (any_motion && (rc = stage_motion(se, dp, motion, walk, s, mo, ds, reach)) != RM_OK) return rc;
-    if ((rc = order_scene_renders(se, s)) != RM_OK) return rc;
-    const rm::LensCamera lc = rm::make_lens_camera(*params, view ? c.vb.m : nullptr, c.lens);
-    const bool cull = params->cull_backfacing != 0;
-    std::vector<float> radius, gf;
-    rm::AreaPoints ap = rm::make_area_points(S, lights ? lights->radius : nullptr, lights ? lights->n_lights : 0, radius);
-    radius.resize(std::max<size_t>(radius.size(), se.flat.lights.size()), 0.f);   // no lights given: every light a point
-    rm::RoughGlass rg = rm::make_rough_glass(S, any_rough ? rough->roughness : nullptr, any_rough ? rough->n_prims : 0, gf);
-    const rm::Diffuse df = rm::make_diffuse(S);
+    const rm::FrameParams<float>& fp = f.fp;
+    const bool cull = f.cull;
+    const int n_lgt = lights->n_lights, S = lights->samples;
+    rm::AreaLights al = {};
+    std::vector<float> radius(std::max(n_lgt, 1), 0.f);
+    for (int l = 0; l < n_lgt; l++) {
+        const double r = lights->radius[l];
+        radius[l] = r > 0. ? std::max((float)std::min(r, (double)FLT_MAX), 1e-30f) : 0.f;
+    }
+    for (int a = 0; a < S; a++)
+        for (int b = 0; b < S; b++) {
+            double lx, ly;
+            rm::lens_offset(S, a, b, &lx, &ly);
+            al.off[2 * (a * S + b)] = (float)lx;
+            al.off[2 * (a * S + b) + 1] = (float)ly;
+        }
+    al.samples = S;
+    al.inv_ss = 1.f / (float)(S * S);
     // the radius table behind the 64 bytes the delivery zeroes
     if ((rc = g.small.ensure(std::max<size_t>(1024, 64 + radius.size() * 4))) != RM_OK) return rc;
-    if (any_rough && (rc = g.rough.ensure(gf.size() * 4)) != RM_OK) return rc;
     float* d_radius = reinterpret_cast<float*>(static_cast<char*>(g.small.p) + 64);
-    ap.radius = d_radius;
-    rg.g = any_rough ? static_cast<const float*>(g.rough.p) : nullptr;
+    al.radius = d_radius;
     CK(cudaMemcpyAsync(d_radius, radius.data(), radius.size() * 4, cudaMemcpyHostToDevice, s));
-    if (any_rough) CK(cudaMemcpyAsync(g.rough.p, gf.data(), gf.size() * 4, cudaMemcpyHostToDevice, s));
-    return deliver_sampled_frame(dp, fp, cull, out_rgb, nullptr, out_rgb8, stats, 1,
+    return deliver_sampled_frame(dp, fp, cull, out_rgb, out_prim_id, out_rgb8, stats, 2,
                                  [&](long long n_px, unsigned long long* next, float* rgb, float* dmax) {
-                                     return rm::launch_path(ds, fp, lc, ap, rg, mo, df, any_motion, reach, cull, n_px, next, rgb, dmax, s);
+                                     const cudaError_t e = rm::launch_prepare(dp.ds, cull, params->camera, s);
+                                     if (e != cudaSuccess) return e;
+                                     return rm::launch_area_lights(dp.ds, fp, al, cull, n_px, next, rgb,
+                                                                   out_prim_id ? static_cast<int*>(g.prim.p) : nullptr, dmax,
+                                                                   params->camera, s);
                                  });
 }
 

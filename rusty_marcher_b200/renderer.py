@@ -4,6 +4,7 @@
 string of renderer.rs:116-121) but runs the hot path on the GPU through the C ABI (rm_render)."""
 import ctypes as C
 import time
+import types
 
 import numpy as np
 
@@ -261,37 +262,9 @@ class Renderer:
         render_view() does (forward=None: the reference's camera looking down -z).  aperture = 0 without a view is
         render_supersampled()'s frame.  Fills frame.buffer (float32) over the rendered rows and, if given, rgb8 (H, W, 3)
         uint8 with normalize + to_vec of that frame; returns the same kind of status message as render()."""
-        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
-            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        aperture, focus = _lens_values(aperture, focus)
-        if self.precision != _abi.RM_FP32:
-            raise ValueError("render_lens computes in RM_FP32")
-        if int(self.width) != frame.width or int(self.height) != frame.height:
-            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
-        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
-                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
-            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
-        view = None
-        if forward is not None:
-            view = _view(forward, up)
-            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
-        lens = _abi.RmLens()
-        lens.aperture, lens.focus, lens.samples = aperture, focus, int(samples)
-        L = _abi.load()
-        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
-        now = time.perf_counter()
-        p = self.params(frame, scene, patch_rows)
-        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
-            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
-        stats = _abi.RmStats()
-        _abi.check(L.rm_render_lens(scene.device_handle(), C.byref(p), C.byref(view) if view is not None else None, C.byref(lens),
-                                    frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
-        self.last_stats = stats
-        ms = int((time.perf_counter() - now) * 1000)
-        fps = 1000. / ms if ms > 0 else float("inf")
-        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
-        print(message)
-        return message
+        return self._render_sampled("render_lens", frame, scene, samples, patch_rows, rgb8, lens=(aperture, focus), view=(forward, up),
+                                    check_stride=False,
+                                    call=lambda L, a: L.rm_render_lens(a.scene, a.params, a.view, a.lens, a.rgb, a.rgb8, a.stats))
 
     def render_area_lights(self, frame, scene, radii, samples=4, prim_id=None, rgb8=None, patch_rows=(0, -1)):
         """EXTENSION MODE (no reference counterpart): soft shadows.  Each of the scene's lights gets a radius for this frame
@@ -301,39 +274,9 @@ class Renderer:
         render()'s frame.  Fills frame.buffer (float32) over the rendered rows and, if given, prim_id (H, W) int32 (render()'s
         primary ids) and rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the same kind of status message
         as render()."""
-        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
-            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        r = _light_radii(scene, radii)
-        n = r.shape[0]
-        if self.precision != _abi.RM_FP32:
-            raise ValueError("render_area_lights computes in RM_FP32")
-        if int(self.width) != frame.width or int(self.height) != frame.height:
-            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
-        if len(patch_rows) > 2 and patch_rows[2] > 1:
-            raise ValueError("render_area_lights renders contiguous patch rows (stride <= 1)")
-        for name, a, dtype, shape in (("prim_id", prim_id, np.int32, (frame.height, frame.width)),
-                                      ("rgb8", rgb8, np.uint8, (frame.height, frame.width, 3))):
-            if a is not None and (not isinstance(a, np.ndarray) or a.dtype != dtype or a.shape != shape or not a.flags.c_contiguous
-                                  or not a.flags.writeable):
-                raise ValueError("%s must be a writeable C-contiguous %s array of shape %s" % (name, np.dtype(dtype).name, shape))
-        lights = _abi.RmAreaLights()
-        lights.n_lights, lights.radius, lights.samples = n, r.ctypes.data_as(C.POINTER(C.c_double)), int(samples)
-        L = _abi.load()
-        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
-        now = time.perf_counter()
-        p = self.params(frame, scene, patch_rows)
-        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
-            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
-        stats = _abi.RmStats()
-        _abi.check(L.rm_render_area_lights(scene.device_handle(), C.byref(p), C.byref(lights), frame.buffer.ctypes.data,
-                                           prim_id.ctypes.data if prim_id is not None else None,
-                                           rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
-        self.last_stats = stats
-        ms = int((time.perf_counter() - now) * 1000)
-        fps = 1000. / ms if ms > 0 else float("inf")
-        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
-        print(message)
-        return message
+        return self._render_sampled("render_area_lights", frame, scene, samples, patch_rows, rgb8, prim_id=prim_id,
+                                    effects=dict(light_radii=radii),
+                                    call=lambda L, a: L.rm_render_area_lights(a.scene, a.params, a.lights, a.rgb, a.prim_id, a.rgb8, a.stats))
 
     def render_rough_glass(self, frame, scene, roughness, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., rgb8=None,
                            patch_rows=(0, -1)):
@@ -345,43 +288,9 @@ class Renderer:
         thin lens (aperture 0: the pinhole).  samples = 1, or no rough glass-like shape, is render_lens()'s frame.  Fills
         frame.buffer (float32) over the rendered rows and, if given, rgb8 (H, W, 3) uint8 with normalize + to_vec of that
         frame; returns the same kind of status message as render()."""
-        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
-            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        per_prim = _roughness_by_prim(scene, roughness)
-        aperture, focus = _lens_values(aperture, focus)
-        if self.precision != _abi.RM_FP32:
-            raise ValueError("render_rough_glass computes in RM_FP32")
-        if int(self.width) != frame.width or int(self.height) != frame.height:
-            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
-        if len(patch_rows) > 2 and patch_rows[2] > 1:
-            raise ValueError("render_rough_glass renders contiguous patch rows (stride <= 1)")
-        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
-                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
-            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
-        view = None
-        if forward is not None:
-            view = _view(forward, up)
-            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
-        lens = _abi.RmLens()
-        lens.aperture, lens.focus, lens.samples = aperture, focus, int(samples)
-        rough = _abi.RmRoughGlass()
-        rough.n_prims, rough.roughness, rough.samples = per_prim.shape[0], per_prim.ctypes.data_as(C.POINTER(C.c_double)), int(samples)
-        L = _abi.load()
-        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
-        now = time.perf_counter()
-        p = self.params(frame, scene, patch_rows)
-        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
-            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
-        stats = _abi.RmStats()
-        _abi.check(L.rm_render_rough_glass(scene.device_handle(), C.byref(p), C.byref(view) if view is not None else None, C.byref(lens),
-                                           C.byref(rough), frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None,
-                                           C.byref(stats)))
-        self.last_stats = stats
-        ms = int((time.perf_counter() - now) * 1000)
-        fps = 1000. / ms if ms > 0 else float("inf")
-        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
-        print(message)
-        return message
+        return self._render_sampled("render_rough_glass", frame, scene, samples, patch_rows, rgb8, effects=dict(roughness=roughness),
+                                    lens=(aperture, focus), view=(forward, up),
+                                    call=lambda L, a: L.rm_render_rough_glass(a.scene, a.params, a.view, a.lens, a.rough, a.rgb, a.rgb8, a.stats))
 
     def render_motion(self, frame, scene, displacement, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., rgb8=None,
                       patch_rows=(0, -1)):
@@ -392,43 +301,9 @@ class Renderer:
         render_view() does, aperture / focus add render_lens()'s thin lens (aperture 0: the pinhole).  samples = 1, or no
         displacement at all, is render_lens()'s frame.  Fills frame.buffer (float32) over the rendered rows and, if given,
         rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the same kind of status message as render()."""
-        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
-            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        per_prim = _displacement_by_prim(scene, displacement)
-        aperture, focus = _lens_values(aperture, focus)
-        if self.precision != _abi.RM_FP32:
-            raise ValueError("render_motion computes in RM_FP32")
-        if int(self.width) != frame.width or int(self.height) != frame.height:
-            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
-        if len(patch_rows) > 2 and patch_rows[2] > 1:
-            raise ValueError("render_motion renders contiguous patch rows (stride <= 1)")
-        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
-                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
-            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
-        view = None
-        if forward is not None:
-            view = _view(forward, up)
-            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
-        lens = _abi.RmLens()
-        lens.aperture, lens.focus, lens.samples = aperture, focus, int(samples)
-        motion = _abi.RmMotion()
-        motion.n_prims, motion.displacement, motion.samples = per_prim.shape[0], per_prim.ctypes.data_as(C.POINTER(C.c_double)), int(samples)
-        L = _abi.load()
-        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
-        now = time.perf_counter()
-        p = self.params(frame, scene, patch_rows)
-        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
-            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
-        stats = _abi.RmStats()
-        _abi.check(L.rm_render_motion(scene.device_handle(), C.byref(p), C.byref(view) if view is not None else None, C.byref(lens),
-                                      C.byref(motion), frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None,
-                                      C.byref(stats)))
-        self.last_stats = stats
-        ms = int((time.perf_counter() - now) * 1000)
-        fps = 1000. / ms if ms > 0 else float("inf")
-        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
-        print(message)
-        return message
+        return self._render_sampled("render_motion", frame, scene, samples, patch_rows, rgb8, effects=dict(displacement=displacement),
+                                    lens=(aperture, focus), view=(forward, up),
+                                    call=lambda L, a: L.rm_render_motion(a.scene, a.params, a.view, a.lens, a.motion, a.rgb, a.rgb8, a.stats))
 
     def render_distributed(self, frame, scene, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., light_radii=None,
                            roughness=None, displacement=None, rgb8=None, patch_rows=(0, -1)):
@@ -441,55 +316,11 @@ class Renderer:
         samples = 1, or no active effect, is render_lens()'s frame; rough glass alone is render_rough_glass()'s and motion
         alone render_motion()'s.  Fills frame.buffer (float32) over the rendered rows and, if given, rgb8 (H, W, 3) uint8 with
         normalize + to_vec of that frame; returns the same kind of status message as render()."""
-        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
-            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        radii = None if light_radii is None else _light_radii(scene, light_radii)
-        rough_by_prim = None if roughness is None else _roughness_by_prim(scene, roughness)
-        disp_by_prim = None if displacement is None else _displacement_by_prim(scene, displacement)
-        aperture, focus = _lens_values(aperture, focus)
-        if self.precision != _abi.RM_FP32:
-            raise ValueError("render_distributed computes in RM_FP32")
-        if int(self.width) != frame.width or int(self.height) != frame.height:
-            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
-        if len(patch_rows) > 2 and patch_rows[2] > 1:
-            raise ValueError("render_distributed renders contiguous patch rows (stride <= 1)")
-        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
-                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
-            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
-        view = None
-        if forward is not None:
-            view = _view(forward, up)
-            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
-        s = int(samples)
-        lens = _abi.RmLens()
-        lens.aperture, lens.focus, lens.samples = aperture, focus, s
-        lights = rough = motion = None
-        if radii is not None:
-            lights = _abi.RmAreaLights()
-            lights.n_lights, lights.radius, lights.samples = radii.shape[0], radii.ctypes.data_as(C.POINTER(C.c_double)), s
-        if rough_by_prim is not None:
-            rough = _abi.RmRoughGlass()
-            rough.n_prims, rough.roughness, rough.samples = rough_by_prim.shape[0], rough_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s
-        if disp_by_prim is not None:
-            motion = _abi.RmMotion()
-            motion.n_prims, motion.displacement, motion.samples = disp_by_prim.shape[0], disp_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s
-        L = _abi.load()
-        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
-        now = time.perf_counter()
-        p = self.params(frame, scene, patch_rows)
-        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
-            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
-        stats = _abi.RmStats()
-        ref = lambda x: C.byref(x) if x is not None else None     # noqa: E731
-        _abi.check(L.rm_render_distributed(scene.device_handle(), C.byref(p), s, ref(view), C.byref(lens), ref(lights), ref(rough),
-                                           ref(motion), frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None,
-                                           C.byref(stats)))
-        self.last_stats = stats
-        ms = int((time.perf_counter() - now) * 1000)
-        fps = 1000. / ms if ms > 0 else float("inf")
-        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
-        print(message)
-        return message
+        return self._render_sampled("render_distributed", frame, scene, samples, patch_rows, rgb8,
+                                    effects=_given(light_radii=light_radii, roughness=roughness, displacement=displacement),
+                                    lens=(aperture, focus), view=(forward, up),
+                                    call=lambda L, a: L.rm_render_distributed(a.scene, a.params, a.samples, a.view, a.lens, a.lights, a.rough,
+                                                                              a.motion, a.rgb, a.rgb8, a.stats))
 
     def render_indirect(self, frame, scene, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., rgb8=None,
                         patch_rows=(0, -1)):
@@ -501,40 +332,8 @@ class Renderer:
         max_depth = 1, or a scene in which nothing bounces, is render_lens()'s frame.  Fills frame.buffer (float32) over the
         rendered rows and, if given, rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the same kind of
         status message as render()."""
-        if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
-            raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        aperture, focus = _lens_values(aperture, focus)
-        if self.precision != _abi.RM_FP32:
-            raise ValueError("render_indirect computes in RM_FP32")
-        if int(self.width) != frame.width or int(self.height) != frame.height:
-            raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
-        if len(patch_rows) > 2 and patch_rows[2] > 1:
-            raise ValueError("render_indirect renders contiguous patch rows (stride <= 1)")
-        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
-                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
-            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
-        view = None
-        if forward is not None:
-            view = _view(forward, up)
-            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
-        s = int(samples)
-        lens = _abi.RmLens()
-        lens.aperture, lens.focus, lens.samples = aperture, focus, s
-        L = _abi.load()
-        _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
-        now = time.perf_counter()
-        p = self.params(frame, scene, patch_rows)
-        if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
-            frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
-        stats = _abi.RmStats()
-        _abi.check(L.rm_render_indirect(scene.device_handle(), C.byref(p), C.byref(view) if view is not None else None, C.byref(lens), s,
-                                        frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
-        self.last_stats = stats
-        ms = int((time.perf_counter() - now) * 1000)
-        fps = 1000. / ms if ms > 0 else float("inf")
-        message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
-        print(message)
-        return message
+        return self._render_sampled("render_indirect", frame, scene, samples, patch_rows, rgb8, lens=(aperture, focus), view=(forward, up),
+                                    call=lambda L, a: L.rm_render_indirect(a.scene, a.params, a.view, a.lens, a.samples, a.rgb, a.rgb8, a.stats))
 
     def render_path(self, frame, scene, samples=4, forward=None, up=(0., 1., 0.), aperture=0., focus=1., light_radii=None,
                     roughness=None, displacement=None, rgb8=None, patch_rows=(0, -1)):
@@ -547,38 +346,52 @@ class Renderer:
         render_distributed()'s frame; otherwise samples = 1, or no active effect, is render_indirect()'s.  Fills frame.buffer
         (float32) over the rendered rows and, if given, rgb8 (H, W, 3) uint8 with normalize + to_vec of that frame; returns the
         same kind of status message as render()."""
+        return self._render_sampled("render_path", frame, scene, samples, patch_rows, rgb8,
+                                    effects=_given(light_radii=light_radii, roughness=roughness, displacement=displacement),
+                                    lens=(aperture, focus), view=(forward, up),
+                                    call=lambda L, a: L.rm_render_path(a.scene, a.params, a.samples, a.view, a.lens, a.lights, a.rough, a.motion,
+                                                                       a.rgb, a.rgb8, a.stats))
+
+    def _render_sampled(self, name, frame, scene, samples, patch_rows, rgb8, call, prim_id=None, effects=None, lens=None, view=None,
+                        check_stride=True):
+        """The sampled-frame methods: validates their arguments in one order -- samples, the per-light and per-primitive
+        values, the lens, precision, frame size, patch-row stride, output arrays, view -- builds the C structs and makes the
+        C call, call(lib, args), with args.scene, params, samples, view, lens, lights, rough, motion, rgb, prim_id, rgb8 and
+        stats as the C function takes them (None: not given).  `effects` holds the effect arguments the call was given, by
+        keyword (light_radii, roughness, displacement), each checked whatever its value; `lens` is (aperture, focus), `view`
+        (forward, up) with forward None for the reference's camera; check_stride=False leaves the patch-row stride to the C call."""
         if not isinstance(samples, (int, np.integer)) or isinstance(samples, bool) or not 1 <= samples <= 8:
             raise ValueError("samples must be an integer in [1, 8], got %r" % (samples,))
-        radii = None if light_radii is None else _light_radii(scene, light_radii)
-        rough_by_prim = None if roughness is None else _roughness_by_prim(scene, roughness)
-        disp_by_prim = None if displacement is None else _displacement_by_prim(scene, displacement)
-        aperture, focus = _lens_values(aperture, focus)
+        s = int(samples)
+        effects = effects or {}
+        radii = _light_radii(scene, effects["light_radii"]) if "light_radii" in effects else None
+        rough_by_prim = _roughness_by_prim(scene, effects["roughness"]) if "roughness" in effects else None
+        disp_by_prim = _displacement_by_prim(scene, effects["displacement"]) if "displacement" in effects else None
+        if lens is not None:
+            lens = _lens_values(*lens)
         if self.precision != _abi.RM_FP32:
-            raise ValueError("render_path computes in RM_FP32")
+            raise ValueError("%s computes in RM_FP32" % name)
         if int(self.width) != frame.width or int(self.height) != frame.height:
             raise ValueError("renderer was created for %dx%d, the frame is %dx%d" % (int(self.width), int(self.height), frame.width, frame.height))
-        if len(patch_rows) > 2 and patch_rows[2] > 1:
-            raise ValueError("render_path renders contiguous patch rows (stride <= 1)")
-        if rgb8 is not None and (not isinstance(rgb8, np.ndarray) or rgb8.dtype != np.uint8 or rgb8.shape != (frame.height, frame.width, 3)
-                                 or not rgb8.flags.c_contiguous or not rgb8.flags.writeable):
-            raise ValueError("rgb8 must be a writeable C-contiguous uint8 array of shape %s" % ((frame.height, frame.width, 3),))
-        view = None
-        if forward is not None:
-            view = _view(forward, up)
-            view_basis(forward, up)                             # ValueError for an invalid view, before any GPU work
-        s = int(samples)
-        lens = _abi.RmLens()
-        lens.aperture, lens.focus, lens.samples = aperture, focus, s
-        lights = rough = motion = None
+        if check_stride and len(patch_rows) > 2 and patch_rows[2] > 1:
+            raise ValueError("%s renders contiguous patch rows (stride <= 1)" % name)
+        for what, a, dtype, shape in (("prim_id", prim_id, np.int32, (frame.height, frame.width)),
+                                      ("rgb8", rgb8, np.uint8, (frame.height, frame.width, 3))):
+            if a is not None and (not isinstance(a, np.ndarray) or a.dtype != dtype or a.shape != shape or not a.flags.c_contiguous
+                                  or not a.flags.writeable):
+                raise ValueError("%s must be a writeable C-contiguous %s array of shape %s" % (what, np.dtype(dtype).name, shape))
+        a = types.SimpleNamespace(samples=s, view=None, lens=None, lights=None, rough=None, motion=None)
+        if view is not None and view[0] is not None:
+            a.view = C.byref(_view(*view))
+            view_basis(*view)                                   # ValueError for an invalid view, before any GPU work
+        if lens is not None:
+            a.lens = C.byref(_abi.RmLens(lens[0], lens[1], s))
         if radii is not None:
-            lights = _abi.RmAreaLights()
-            lights.n_lights, lights.radius, lights.samples = radii.shape[0], radii.ctypes.data_as(C.POINTER(C.c_double)), s
+            a.lights = C.byref(_abi.RmAreaLights(radii.shape[0], radii.ctypes.data_as(C.POINTER(C.c_double)), s))
         if rough_by_prim is not None:
-            rough = _abi.RmRoughGlass()
-            rough.n_prims, rough.roughness, rough.samples = rough_by_prim.shape[0], rough_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s
+            a.rough = C.byref(_abi.RmRoughGlass(rough_by_prim.shape[0], rough_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s))
         if disp_by_prim is not None:
-            motion = _abi.RmMotion()
-            motion.n_prims, motion.displacement, motion.samples = disp_by_prim.shape[0], disp_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s
+            a.motion = C.byref(_abi.RmMotion(disp_by_prim.shape[0], disp_by_prim.ctypes.data_as(C.POINTER(C.c_double)), s))
         L = _abi.load()
         _abi.init(_abi._initialised_device if _abi._initialised_device is not None else 0)
         now = time.perf_counter()
@@ -586,15 +399,20 @@ class Renderer:
         if frame.buffer.dtype != np.float32 or not frame.buffer.flags.c_contiguous:
             frame.buffer = np.zeros((frame.height, frame.width, 3), dtype=np.float32)
         stats = _abi.RmStats()
-        ref = lambda x: C.byref(x) if x is not None else None     # noqa: E731
-        _abi.check(L.rm_render_path(scene.device_handle(), C.byref(p), s, ref(view), C.byref(lens), ref(lights), ref(rough), ref(motion),
-                                    frame.buffer.ctypes.data, rgb8.ctypes.data if rgb8 is not None else None, C.byref(stats)))
+        a.scene, a.params, a.stats = scene.device_handle(), C.byref(p), C.byref(stats)
+        a.rgb, a.prim_id = frame.buffer.ctypes.data, prim_id.ctypes.data if prim_id is not None else None
+        a.rgb8 = rgb8.ctypes.data if rgb8 is not None else None
+        _abi.check(call(L, a))
         self.last_stats = stats
         ms = int((time.perf_counter() - now) * 1000)
         fps = 1000. / ms if ms > 0 else float("inf")
         message = "Scene rendered in %d ms (%d fps, %.2f MP/s)" % (ms, int(min(fps, 2**32 - 1)), fps * frame.height * frame.width / 1e6)
         print(message)
         return message
+
+def _given(**effects):
+    """render_distributed / render_path: the effect arguments that are not None (None leaves an effect out)."""
+    return {k: v for k, v in effects.items() if v is not None}
 
 
 def _light_radii(scene, radii):
